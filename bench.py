@@ -3,6 +3,9 @@
 
   python bench.py --gpus N --steps K --warmup W            # the sm_100a kernels
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+  python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed
+
+The K timed steps are split into --regions regions (default 3); the reported step time is the median region's.
 
 Metric (BASELINE.json): sampled-points/s of MSDeformAttn forward+backward, point = one
 (b,q,h,l,p) sample.  Workload at any N: BASELINE configs[1] per GPU -- the DINO-R50 deformable
@@ -66,7 +69,12 @@ def parse_args():
     ap.add_argument("--mode", default="op", choices=["op", "train"],
                     help="op: the core operator (the metric); train: batch-sharded module-level training step "
                          "(projections + fused op, fwd+bwd, grad all-reduce overlapped with backward, optimizer)")
-    ap.add_argument("--regions", type=int, default=3, help="timed regions of --steps steps each (median reported)")
+    ap.add_argument("--regions", type=int, default=3,
+                    help="timed regions the --steps timed steps are split into (median per-step time reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="op mode: write what the last timed step computed (out and the three gradients of every layer, "
+                         "float32, a fixed seeded sample of each large tensor, under 64 MB in all) as DIR/<name>.npy.  That "
+                         "step keeps its outputs alive, so the allocator may have to allocate inside the last timed region")
     ap.add_argument("--no-graph", action="store_true", help="train mode: do not try CUDA-graph capture")
     ap.add_argument("--amp", action="store_true", help="train mode: bf16 autocast (AMP config)")
     ap.add_argument("--tf32", action="store_true",
@@ -92,6 +100,12 @@ def config_dict(wl, args, extra=None):
     if extra:
         cfg.update(extra)
     return cfg
+
+
+def split_steps(steps, regions):
+    """The `steps` timed steps split as evenly as possible into up to `regions` timed regions."""
+    n = max(1, min(regions, steps))
+    return [steps // n + (r < steps % n) for r in range(n)]
 
 
 # --------------------------------------------------------------------------------------------
@@ -283,6 +297,10 @@ def onchip_block(wl, fwd_ms, bwd_ms, valid_frac):
 def main():
     args = parse_args()
     wl = WORKLOADS[args.workload]
+    if args.steps < 1:
+        raise SystemExit("bench.py: --steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "op"):
+        raise SystemExit("bench.py: --dump-outputs covers the sm_100a core op (--impl b200 --mode op) only")
     if args.impl == "reference":
         run_reference_arm(args, wl)
         return
@@ -336,7 +354,9 @@ def main():
     # training config's gradient all-reduce is measured where real gradients exist: --mode train.
     ev = lambda: torch.cuda.Event(enable_timing=True)
 
-    def step(record=None):
+    def step(record=None, keep=False):
+        """One step over all layers; with `keep`, returns every layer's (out, grad_value, grad_loc, grad_w)."""
+        kept = []
         for i, (value, shapes, lsi, loc, w, go) in enumerate(layers):
             if record is not None:
                 e0, e1, e2 = ev(), ev(), ev()
@@ -344,11 +364,14 @@ def main():
             out = ir_ads_b200.ms_deform_attn_forward(value, shapes, lsi, loc, w, 64)
             if record is not None:
                 e1.record()
-            ir_ads_b200.ms_deform_attn_backward(value, shapes, lsi, loc, w, go, 64)
+            grads = ir_ads_b200.ms_deform_attn_backward(value, shapes, lsi, loc, w, go, 64)
             if record is not None:
                 e2.record()
                 record.append((e0, e1, e2))
-            del out
+            if keep:
+                kept.append((out, *grads))
+            del out, grads
+        return kept
 
     def barrier():
         if dist_on:
@@ -361,24 +384,31 @@ def main():
         barrier()
         sampler = ClockSampler(local_rank)
         sampler.start()
-        # `regions` timed regions of exactly `steps` steps each, every one bracketed by barrier + synchronize;
-        # the median region is the reported one (one un-repeated sample gave an unexplained 0.90 outlier in r01)
+        # the `steps` timed steps are split into up to `regions` timed regions, every one bracketed by barrier +
+        # synchronize; the median region's per-step time is the reported one (one un-repeated sample gave an
+        # unexplained 0.90 outlier in r01)
+        region_steps = split_steps(args.steps, args.regions)
+        n_regions = len(region_steps)
         region_ms = []
         launches = 0
-        for _ in range(max(1, args.regions)):
+        last = None
+        for r, n in enumerate(region_steps):
             if flush is not None:
                 flush.zero_()
             barrier()
             launches0 = _lib.launch_count()
             t_begin, t_end = ev(), ev()
             t_begin.record()
-            for _ in range(args.steps):
-                step()
+            for s in range(n):
+                last = step(keep=bool(args.dump_outputs) and r == n_regions - 1 and s == n - 1)
             t_end.record()
             barrier()
-            launches = _lib.launch_count() - launches0
-            region_ms.append(t_begin.elapsed_time(t_end) / args.steps)
+            launches += _lib.launch_count() - launches0
+            region_ms.append(t_begin.elapsed_time(t_end) / n)
         clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last)
+        del last
 
         # per-kernel durations (same stream, separate short pass so event records do not perturb `value`)
         recs = []
@@ -431,7 +461,7 @@ def main():
             "warmup": max(args.warmup, 3), "ms_per_step": ms_step, "higher_is_better": True, "scaling": args.scaling,
             "vs_baseline": None, "dtype": "f32" if wl.value_dtype == "f32" else "bf16(value) + f32 accumulate",
             "data": "synthetic", "config": config_dict(wl, args),
-            "timed_regions": {"count": len(region_ms), "ms_per_step": [round(x, 4) for x in region_ms],
+            "timed_regions": {"count": len(region_ms), "steps": region_steps, "ms_per_step": [round(x, 4) for x in region_ms],
                               "reported": "median", "spread_pct": round(100.0 * (max(region_ms) - min(region_ms)) / ms_step, 2)},
             "roofline": roof,
             "gpu_launches": int(launches), "clocks": clocks,
@@ -531,21 +561,22 @@ def run_train_mode(args, wl, dev, rank, world, dist_on):
     sampler = ClockSampler(dev.index or 0)
     sampler.start()
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
+    region_steps = split_steps(args.steps, args.regions)
     region_ms = []
     launches = 0
     ev = lambda: torch.cuda.Event(enable_timing=True)
-    for _ in range(max(1, args.regions)):
+    for n in region_steps:
         flush.zero_()
         barrier()
         l0 = _lib.launch_count()
         t0, t1 = ev(), ev()
         t0.record()
-        for _ in range(args.steps):
+        for _ in range(n):
             step()
         t1.record()
         barrier()
-        launches = _lib.launch_count() - l0
-        region_ms.append(t0.elapsed_time(t1) / args.steps)
+        launches += _lib.launch_count() - l0
+        region_ms.append(t0.elapsed_time(t1) / n)
     clocks = sampler.stop()
     if dist_on:
         region_ms = [sharding.max_over_ranks(v, dev) for v in region_ms]
@@ -568,7 +599,7 @@ def run_train_mode(args, wl, dev, rank, world, dist_on):
                        "l2_hygiene": "256 MB L2 flush between timed regions",
                        "parallelism": f"image-batch sharding x{world}, no collective inside the op; "
                                       f"{L} all-reduces of 0.92 MB per step overlapped with backward"},
-            "timed_regions": {"count": len(region_ms), "ms_per_step": [round(v, 4) for v in region_ms],
+            "timed_regions": {"count": len(region_ms), "steps": region_steps, "ms_per_step": [round(v, 4) for v in region_ms],
                               "reported": "median", "spread_pct": round(100.0 * (max(region_ms) - min(region_ms)) / ms, 2)},
             "gpu_launches": int(launches) if graph is None else kernels_per_step * args.steps,
             "gpu_launches_note": "graph replays launch the captured kernels without passing the library's counter"
@@ -576,6 +607,29 @@ def run_train_mode(args, wl, dev, rank, world, dist_on):
             "clocks": clocks,
         }
         print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 60 << 20      # the whole dump, float32 (under 64 MB with the .npy headers)
+
+
+def dump_outputs(path, results):
+    """Save each layer's forward output and its three gradients as float32 `layer<i>_<name>.npy` under `path`.  A tensor
+    of more than DUMP_BYTES / (4 tensors x layers x 4 bytes) elements is reduced to that many elements at flat indices
+    drawn from a fixed seed (sorted), the same for every run and build, so that two builds can be compared element for
+    element."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    sample = DUMP_BYTES // (4 * 4 * max(1, len(results)))
+    index = {}
+    for i, tensors in enumerate(results):
+        for name, t in zip(("out", "grad_value", "grad_sampling_loc", "grad_attn_weight"), tensors):
+            n = t.numel()
+            if n > sample:
+                if n not in index:
+                    g = torch.Generator().manual_seed(n)
+                    index[n] = torch.randint(n, (sample,), generator=g).sort()[0].to(t.device)
+                t = t.reshape(-1)[index[n]]
+            np.save(os.path.join(path, f"layer{i}_{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def run_e2e(wl, layers, dev, dist_on, world, args):
@@ -592,7 +646,7 @@ def run_e2e(wl, layers, dev, dist_on, world, args):
     h2d = sum(t.numel() * t.element_size() for t in host_in)
     d2h = sum(t.numel() * t.element_size() for t in host_out)
     L = len(layers)
-    steps = max(2, min(args.steps, 10))   # the pipeline fills and drains once per measurement: amortise it
+    steps = args.steps
     s_in, s_cmp, s_out = (torch.cuda.Stream(dev) for _ in range(3))
     dev_in = [[torch.empty_like(t, device=dev) for t in host_in] for _ in range(2)]
     ev = lambda: torch.cuda.Event()

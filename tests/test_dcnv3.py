@@ -153,12 +153,10 @@ def test_dcnv3_generic_shapes_against_port(C, k, stride, pad, dil, scale, dtype)
 
 
 @pytest.mark.gpu
-def test_against_reference_dcnv3_cuda_kernels():
-    """Whole-tensor comparison with the reference's own DCNv3 kernels (compiled unmodified for sm_100a)."""
+def test_against_reference_dcnv3_formulation():
+    """Whole-tensor comparison with the reference's own formulation (dcnv3_core_pytorch as restated in
+    oracle/dcnv3_torch.py, pinned to reference-made vectors above) in float64 on the same GPU."""
     from ir_ads_b200.dcnv3 import DCNv3Function
-    from oracle import ref_cuda
-    if not ref_cuda.dcn_available():
-        pytest.skip("oracle/_ref/libdcnv3_refcuda.so not built")
     dev = "cuda:0"
     g = torch.Generator(device=dev).manual_seed(0)
     N, H, W, G, C, k = 2, 48, 64, 8, 32, 3
@@ -170,15 +168,17 @@ def test_against_reference_dcnv3_cuda_kernels():
         mask = torch.softmax(torch.randn(N, Ho, Wo, G, 9, device=dev, generator=g), -1).reshape(N, Ho, Wo, G * 9)
         go = torch.randn(N, Ho, Wo, G * C, device=dev, generator=g)
         args = (k, k, stride, stride, pad, pad, dil, dil, G, C, scale)
-        want = ref_cuda.dcnv3_forward_backward(inp, off, mask, go, *args)
+        want = dcnv3_torch.forward_backward(inp.double(), off.double(), mask.double(), go.double(), *args)
         leaves = [t.clone().requires_grad_(True) for t in (inp, off, mask)]
         out = DCNv3Function.apply(*leaves, *args, 256)
         out.backward(go)
         got = [out.detach()] + [t.grad for t in leaves]
+        # grad_offset is discontinuous where a sampling coordinate crosses a bilinear cell boundary, and the float64
+        # yardstick may pick the other cell within float32 location accuracy: those points are left out
+        m = torch.from_numpy(pixel_smooth_mask({"offset": off.cpu().numpy(), "args": args}, 1e-4)).to(dev).double()
         for a, b, key in zip(got, want, ("out", "grad_input", "grad_offset", "grad_mask")):
-            # same float32 coordinate arithmetic as the reference kernel => same bilinear cells, so even
-            # grad_offset needs no boundary mask
-            err = (a - b).abs().max().item()
+            mk = m if key == "grad_offset" else 1.0
+            err = ((a.double() - b) * mk).abs().max().item()
             assert err <= 1e-5 * b.abs().max().item() + 1e-6, (key, stride, err)
 
 
