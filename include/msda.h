@@ -17,7 +17,7 @@
  * (batch, spatial_size, num_heads, channels, num_levels, num_query, num_point), then outputs.
  * Differences, all deliberate:
  *   - plain C: no ATen / torch types, `void*` for the stream (a cudaStream_t);
- *   - a dtype tag instead of a C++ template: float, double, or bfloat16 value with float
+ *   - a dtype tag instead of a C++ template: float, double, bfloat16 or float16 value with float
  *     locations / weights (the reference has float and double only);
  *   - errors are RETURNED (the reference only printf's launch failures, cuh:948-952);
  *   - no im2col_step: the whole batch is one launch (ms_deform_attn_cuda.cu:51-76 chunked it);
@@ -61,6 +61,12 @@ extern "C" {
 #define MSDA_F32 0  /* value/out/grads float,  loc/w float  */
 #define MSDA_F64 1  /* everything double (gradcheck path; generic kernels only) */
 #define MSDA_BF16 2 /* value/out/grad_out/grad_value bfloat16, loc/w and their grads float, fp32 accumulate */
+/* value/out/grad_out/grad_value float16, loc/w and their grads float, fp32 accumulate.  Every kernel widens the
+ * float16 operands exactly, so out / grad_value equal the MSDA_F32 results on the widened tensors rounded once to
+ * float16, and the float gradients equal them bit for bit (grad_value with float reds: up to the run-to-run
+ * difference of the red order).  Added in ABI 3 without a version bump: an older library answers
+ * MSDA_ERR_INVALID_ARGUMENT ("unknown dtype tag"). */
+#define MSDA_F16 3
 
 /* status codes */
 #define MSDA_OK 0
@@ -187,15 +193,15 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
  *       (/root/reference/detrex/layers/csrc/DCNv3/dcnv3_im2col_cuda.cuh:840-868), i.e. _C.dcnv3_forward
  *       (csrc/vision.cpp:57); msda_dcnv3_backward replaces dcnv3_col2im_cuda<T> (:870-), _C.dcnv3_backward.
  * Argument order follows those launchers.  Layouts (contiguous, channels last, as dcn_v3.py:464-489):
- *   input  [N, H_in, W_in, group*group_channels]   dtype (MSDA_F32 or MSDA_BF16)
+ *   input  [N, H_in, W_in, group*group_channels]   dtype (MSDA_F32, MSDA_BF16 or MSDA_F16)
  *   offset [N, H_out, W_out, group*K*2] float, K = kernel_h*kernel_w, point index = i*kernel_h + j
  *          with i over kernel_w (the reference kernel's loop order), (x, y) per point, in pixels
  *   mask   [N, H_out, W_out, group*K]   float
  *   output / grad_output [N, H_out, W_out, group*group_channels] dtype
  * The input is NOT padded by the caller: pad_h / pad_w only shift the sampling grid and samples outside
  * the map read zeros, exactly like the reference kernel.  Supported: group_channels in {16,32,64,128},
- * K <= 64, float32 / bfloat16 input (MSDA_ERR_UNSUPPORTED otherwise).  bfloat16 backward needs a
- * workspace of N*H_in*W_in*C floats.
+ * K <= 64, float32 / bfloat16 / float16 input (MSDA_ERR_UNSUPPORTED otherwise).  The bfloat16 and float16
+ * backward need a workspace of N*H_in*W_in*C floats.
  */
 int msda_dcnv3_forward(void* stream, const void* input, const float* offset, const float* mask,
                        int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,

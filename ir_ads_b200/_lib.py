@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("MSDA_B200_LIB") or os.path.join(_PKG, "libmsda_b200.s
 HEADER_PATH = os.path.join(os.path.dirname(_PKG), "include", "msda.h")
 
 # include/msda.h
-MSDA_F32, MSDA_F64, MSDA_BF16 = 0, 1, 2
+MSDA_F32, MSDA_F64, MSDA_BF16, MSDA_F16 = 0, 1, 2, 3
 MSDA_OK = 0
 FLAG_DETERMINISTIC = 1 << 0
 FLAG_FORCE_GENERIC = 1 << 1

@@ -15,8 +15,7 @@ int bwd_fast(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const vo
 #endif
 #define CALL_BWD(D_, VT_, PT_, ORD_) \
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw, nullptr)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_BWD);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_BWD);
+  MSDA_DISPATCH_VT(CALL_BWD);
 #undef CALL_BWD
 #undef MSDA_DISPATCH_ORDER
 }

@@ -11,8 +11,7 @@ int bwd_fast_det(cudaStream_t st, const Dims& d, int dtype, const void* go, cons
 #define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
 #define CALL_BWD(D_, VT_, PT_, ORD_) \
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, unsigned long long>(st, d, go, value, shapes, lsi, loc, w, acc, gl, gw, det)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_BWD);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_BWD);
+  MSDA_DISPATCH_VT(CALL_BWD);
 #undef CALL_BWD
 #undef MSDA_DISPATCH_ORDER
 }
@@ -24,8 +23,7 @@ int bwd_fast_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go
 #define CALL_BWD(D_, VT_, PT_, ORD_)                                                                          \
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, msda::NoScatter>(st, d, go, value, shapes, lsi, loc, w,   \
                                                                     (msda::NoScatter*)nullptr, gl, gw, nullptr)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_BWD);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_BWD);
+  MSDA_DISPATCH_VT(CALL_BWD);
 #undef CALL_BWD
 #undef MSDA_DISPATCH_ORDER
 }
@@ -44,8 +42,7 @@ int bwd_fast_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, con
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, msda::EmitEntries>(st, d, go, value, shapes, lsi, loc, w,   \
                                                                       (msda::EmitEntries*)nullptr, gl, gw, nullptr, \
                                                                       msda::FusedArgs{}, ea)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_BWD);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_BWD);
+  MSDA_DISPATCH_VT(CALL_BWD);
 #undef CALL_BWD
 #undef MSDA_DISPATCH_ORDER
 }
@@ -72,8 +69,7 @@ int bwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* go, const v
 #define CALL_FB(D_, VT_, PT_, ORD_)                                                                               \
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPreFused>(st, d, go, value, shapes, lsi, off, logits, gv, \
                                                                            goff, glog, nullptr, fa)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_FB);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_FB);
+  MSDA_DISPATCH_VT(CALL_FB);
 #undef CALL_FB
 #undef MSDA_DISPATCH_ORDER
 }
@@ -86,8 +82,7 @@ int bwd_fused_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* g
 #define CALL_FB(D_, VT_, PT_, ORD_)                                                                              \
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, msda::NoScatter, msda::kPreFused>(                            \
       st, d, go, value, shapes, lsi, off, logits, (msda::NoScatter*)nullptr, goff, glog, nullptr, fa)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_FB);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_FB);
+  MSDA_DISPATCH_VT(CALL_FB);
 #undef CALL_FB
 #undef MSDA_DISPATCH_ORDER
 }
@@ -107,7 +102,9 @@ int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const voi
     default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);           \
   }
   if (dtype == MSDA_F32) DCN_D(float)
-  DCN_D(__nv_bfloat16)
+  if (dtype == MSDA_BF16) DCN_D(__nv_bfloat16)
+  if (dtype == MSDA_F16) DCN_D(__half)
+  return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
 #undef DCN_D
 #undef CALL_DB
 }

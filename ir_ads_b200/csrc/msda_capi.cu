@@ -48,7 +48,7 @@ int check_alignment(std::initializer_list<NamedPtr> ptrs) {
 
 bool fast_ok(const Dims& d, int dtype, unsigned flags) {
   if (flags & MSDA_FLAG_FORCE_GENERIC) return false;
-  if (dtype != MSDA_F32 && dtype != MSDA_BF16) return false;
+  if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16) return false;
   if (!(d.D == 16 || d.D == 32 || d.D == 64 || d.D == 128)) return false;
   if (d.L < 1 || d.L > msda::kFastMaxLevels) return false;
   if (d.L * d.P < 1 || d.L * d.P > msda::kFastMaxPoints) return false;
@@ -89,7 +89,7 @@ int check_dims(const Dims& d, int dtype) {
   if (d.B < 0 || d.S < 0 || d.H < 0 || d.D < 0 || d.L < 0 || d.Q < 0 || d.P < 0)
     return fail(MSDA_ERR_INVALID_ARGUMENT, "negative dimension (B=%d S=%d H=%d D=%d L=%d Q=%d P=%d)", d.B, d.S, d.H,
                 d.D, d.L, d.Q, d.P);
-  if (dtype != MSDA_F32 && dtype != MSDA_F64 && dtype != MSDA_BF16)
+  if (dtype != MSDA_F32 && dtype != MSDA_F64 && dtype != MSDA_BF16 && dtype != MSDA_F16)
     return fail(MSDA_ERR_INVALID_ARGUMENT, "unknown dtype tag %d", dtype);
   return MSDA_OK;
 }
@@ -238,7 +238,20 @@ int bwd_generic(cudaStream_t st, const Dims& d, const void* go, const void* valu
   return MSDA_OK;
 }
 
-size_t elem_size(int dtype) { return dtype == MSDA_F64 ? 8 : (dtype == MSDA_BF16 ? 2 : 4); }
+// bf16 / f16 values: 2-byte elements, grad_value accumulated in a float workspace and converted at the end
+bool two_byte(int dtype) { return dtype == MSDA_BF16 || dtype == MSDA_F16; }
+
+size_t elem_size(int dtype) { return dtype == MSDA_F64 ? 8 : (two_byte(dtype) ? 2 : 4); }
+
+// float workspace -> bf16 / f16 grad_value
+int cast_from_f32(cudaStream_t st, const float* src, void* dst, int64_t n, int dtype) {
+  const int grid = grid_for(n, 256, 148 * 16);
+  if (dtype == MSDA_BF16) msda::msda_cast_f32_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(src, (__nv_bfloat16*)dst, n);
+  else msda::msda_cast_f32_kernel<__half><<<grid, 256, 0, st>>>(src, (__half*)dst, n);
+  count_launch();
+  MSDA_CUDA(cudaGetLastError());
+  return MSDA_OK;
+}
 
 }  // namespace
 
@@ -279,7 +292,7 @@ const char* msda_dispatch_name(int channels, int num_levels, int num_point, int 
                                int dtype, unsigned flags, int backward) {
   Dims d{1, spatial_size, num_heads, channels, num_levels, 1, num_point};
   static thread_local char name[64];
-  const char* dt = dtype == MSDA_F64 ? "f64" : (dtype == MSDA_BF16 ? "bf16" : "f32");
+  const char* dt = dtype == MSDA_F64 ? "f64" : (dtype == MSDA_BF16 ? "bf16" : (dtype == MSDA_F16 ? "f16" : "f32"));
   if (fast_ok(d, dtype, flags))
     snprintf(name, sizeof(name), "%s_fast_d%d_%s", backward ? "bwd" : "fwd", channels, dt);
   else
@@ -317,9 +330,12 @@ int msda_forward(void* stream, const void* value, const int64_t* spatial_shapes,
       return fwd_generic<float, float>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
     case MSDA_F64:
       return fwd_generic<double, double>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
-    default:
+    case MSDA_BF16:
       return fwd_generic<__nv_bfloat16, float>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
+    case MSDA_F16:
+      return fwd_generic<__half, float>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
   }
+  return fail(MSDA_ERR_INVALID_ARGUMENT, "unknown dtype tag %d", dtype);
 }
 
 size_t msda_backward_workspace_bytes(int batch, int spatial_size, int num_heads, int channels, int num_levels,
@@ -332,8 +348,8 @@ size_t msda_backward_workspace_bytes(int batch, int spatial_size, int num_heads,
     if (det_sorted_ok(d, dtype, flags)) return det_layout(d).total;   // bins, cursors, scan sums, entries
     return n_value * sizeof(long long) + 64;   // 64-bit fixed-point accumulators + {amax bits x2, DetScale}
   }
-  // bf16 grad_value is accumulated in float and converted at the end
-  if (dtype == MSDA_BF16) return n_value * sizeof(float);
+  // bf16 / f16 grad_value is accumulated in float and converted at the end
+  if (two_byte(dtype)) return n_value * sizeof(float);
   return 0;
 }
 
@@ -371,8 +387,8 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
   const bool det = (flags & MSDA_FLAG_DETERMINISTIC) != 0;
   const bool have_samples = d.n_points() != 0 && d.n_value() != 0;
   // zero-fill grad_value -- unless a later pass writes every element anyway: the deterministic finalize / gather,
-  // or the float -> bf16 conversion of the workspace accumulators
-  const bool overwritten = have_samples && d.D != 0 && (det || dtype == MSDA_BF16);
+  // or the float -> bf16 / f16 conversion of the workspace accumulators
+  const bool overwritten = have_samples && d.D != 0 && (det || two_byte(dtype));
   if (d.n_value() && !overwritten) {
     if (!grad_value) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_value is null");
     MSDA_CUDA(cudaMemsetAsync(grad_value, 0, (size_t)d.n_value() * es, st));
@@ -418,7 +434,8 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
     if (!amax_in_emit) {
       if (dtype == MSDA_F32) msda::msda_amax_kernel<float><<<g_out, 256, 0, st>>>((const float*)grad_output, n_out, amax);
       else if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_out, 256, 0, st>>>((const double*)grad_output, n_out, amax);
-      else msda::msda_amax_kernel<__nv_bfloat16><<<g_out, 256, 0, st>>>((const __nv_bfloat16*)grad_output, n_out, amax);
+      else if (dtype == MSDA_BF16) msda::msda_amax_kernel<__nv_bfloat16><<<g_out, 256, 0, st>>>((const __nv_bfloat16*)grad_output, n_out, amax);
+      else msda::msda_amax_kernel<__half><<<g_out, 256, 0, st>>>((const __half*)grad_output, n_out, amax);
       count();
       if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_pts, 256, 0, st>>>((const double*)attn_weight, n_pts, amax + 1);
       else msda::msda_amax_kernel<float><<<g_pts, 256, 0, st>>>((const float*)attn_weight, n_pts, amax + 1);
@@ -470,7 +487,7 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
         count();
         msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax + n_warps, n_warps, amax + 1);
         count();
-        msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, 38);   // sorted route: float / bf16 only
+        msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, 38);   // sorted route: float / bf16 / f16 only
         count();
         MSDA_CUDA(cudaGetLastError());
       } else if (int s2 = bwd_fast_emit(st, d, dtype, grad_output, value, spatial_shapes, level_start_index,
@@ -481,20 +498,26 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
       if (!det_dense(d)) {
         if (dtype == MSDA_F32)
           return det_gather<float>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
-        return det_gather<__nv_bfloat16>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale,
-                                         grad_value);
+        if (dtype == MSDA_BF16)
+          return det_gather<__nv_bfloat16>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale,
+                                           grad_value);
+        return det_gather<__half>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
       }
       int s3;
       if (dtype == MSDA_F32)
         s3 = det_cell_reduce<float>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale, acc);
-      else
+      else if (dtype == MSDA_BF16)
         s3 = det_cell_reduce<__nv_bfloat16>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index,
                                             scale, acc);
+      else
+        s3 = det_cell_reduce<__half>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale,
+                                     acc);
       if (s3 != MSDA_OK) return s3;
       const int g_fin = grid_for(nv, 256, 148 * 16);
       const long long* sacc = reinterpret_cast<const long long*>(acc);
       if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_fin, 256, 0, st>>>(sacc, (float*)grad_value, nv, scale);
-      else msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_fin, 256, 0, st>>>(sacc, (__nv_bfloat16*)grad_value, nv, scale);
+      else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_fin, 256, 0, st>>>(sacc, (__nv_bfloat16*)grad_value, nv, scale);
+      else msda::msda_det_finalize_kernel<__half><<<g_fin, 256, 0, st>>>(sacc, (__half*)grad_value, nv, scale);
       count();
       MSDA_CUDA(cudaGetLastError());
       return MSDA_OK;
@@ -511,23 +534,28 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
       s = bwd_generic<double, double, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
                                                           sampling_loc, attn_weight, acc, grad_sampling_loc,
                                                           grad_attn_weight, scale);
-    else
+    else if (dtype == MSDA_BF16)
       s = bwd_generic<__nv_bfloat16, float, unsigned long long>(st, d, grad_output, value, spatial_shapes,
                                                                 level_start_index, sampling_loc, attn_weight, acc,
                                                                 grad_sampling_loc, grad_attn_weight, scale);
+    else
+      s = bwd_generic<__half, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
+                                                         sampling_loc, attn_weight, acc, grad_sampling_loc,
+                                                         grad_attn_weight, scale);
     if (s != MSDA_OK) return s;
     const int g_val = grid_for(nv, 256, 148 * 16);
     const long long* cacc = reinterpret_cast<const long long*>(acc);
     if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_val, 256, 0, st>>>(cacc, (float*)grad_value, nv, scale);
     else if (dtype == MSDA_F64) msda::msda_det_finalize_kernel<double><<<g_val, 256, 0, st>>>(cacc, (double*)grad_value, nv, scale);
-    else msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_val, 256, 0, st>>>(cacc, (__nv_bfloat16*)grad_value, nv, scale);
+    else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_val, 256, 0, st>>>(cacc, (__nv_bfloat16*)grad_value, nv, scale);
+    else msda::msda_det_finalize_kernel<__half><<<g_val, 256, 0, st>>>(cacc, (__half*)grad_value, nv, scale);
     count();
     MSDA_CUDA(cudaGetLastError());
     return MSDA_OK;
   }
 
   float* gv32 = static_cast<float*>(grad_value);
-  if (dtype == MSDA_BF16) {
+  if (two_byte(dtype)) {
     gv32 = static_cast<float*>(workspace);
     MSDA_CUDA(cudaMemsetAsync(gv32, 0, need, st));
   }
@@ -547,18 +575,15 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
     s = bwd_generic<double, double, double>(st, d, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
                                             attn_weight, static_cast<double*>(grad_value), grad_sampling_loc,
                                             grad_attn_weight);
-  } else {
+  } else if (dtype == MSDA_BF16) {
     s = bwd_generic<__nv_bfloat16, float, float>(st, d, grad_output, value, spatial_shapes, level_start_index,
                                                  sampling_loc, attn_weight, gv32, grad_sampling_loc, grad_attn_weight);
+  } else {
+    s = bwd_generic<__half, float, float>(st, d, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
+                                          attn_weight, gv32, grad_sampling_loc, grad_attn_weight);
   }
   if (s != MSDA_OK) return s;
-  if (dtype == MSDA_BF16) {
-    const int64_t n = d.n_value();
-    msda::msda_cast_f32_to_bf16_kernel<<<grid_for(n, 256, 148 * 16), 256, 0, st>>>(
-        gv32, static_cast<__nv_bfloat16*>(grad_value), n);
-    count();
-    MSDA_CUDA(cudaGetLastError());
-  }
+  if (two_byte(dtype)) return cast_from_f32(st, gv32, grad_value, d.n_value(), dtype);
   return MSDA_OK;
 }
 
@@ -579,7 +604,7 @@ int msda_fused_forward(void* stream, const void* value, const int64_t* spatial_s
   if (ref_dim != 2 && ref_dim != 4) return fail(MSDA_ERR_INVALID_ARGUMENT, "ref_dim must be 2 or 4, got %d", ref_dim);
   if (d.rows() * d.D == 0) return MSDA_OK;
   if (!msda_fused_supported(channels, num_levels, num_point, spatial_size, num_heads, dtype, flags) || d.S == 0)
-    return fail(MSDA_ERR_UNSUPPORTED, "fused path needs D in {16,32,64,128}, float/bf16 value, L<=16, 1<=L*P<=64");
+    return fail(MSDA_ERR_UNSUPPORTED, "fused path needs D in {16,32,64,128}, float/bf16/f16 value, L<=16, 1<=L*P<=64");
   if (!value || !spatial_shapes || !level_start_index || !sampling_offsets || !attn_logits || !reference_points ||
       !output)
     return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
@@ -610,7 +635,7 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
   if (ref_dim != 2 && ref_dim != 4) return fail(MSDA_ERR_INVALID_ARGUMENT, "ref_dim must be 2 or 4, got %d", ref_dim);
   if (!msda_fused_supported(channels, num_levels, num_point, spatial_size, num_heads, dtype, flags) ||
       d.n_value() == 0 || d.n_points() == 0)
-    return fail(MSDA_ERR_UNSUPPORTED, "fused path needs a non-empty problem, D in {16,32,64,128}, float/bf16 value");
+    return fail(MSDA_ERR_UNSUPPORTED, "fused path needs a non-empty problem, D in {16,32,64,128}, float/bf16/f16 value");
   if (!grad_output || !value || !spatial_shapes || !level_start_index || !sampling_offsets || !attn_logits ||
       !reference_points || !grad_value || !grad_offsets || !grad_logits)
     return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
@@ -627,7 +652,7 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
   if (need && (!workspace || workspace_bytes < need))
     return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
   float* gv32 = static_cast<float*>(grad_value);
-  if (dtype == MSDA_BF16) gv32 = static_cast<float*>(workspace);
+  if (two_byte(dtype)) gv32 = static_cast<float*>(workspace);
   MSDA_CUDA(cudaMemsetAsync(gv32, 0, (size_t)d.n_value() * sizeof(float), st));
   msda::FusedArgs fa{};
   fa.ref = reference_points;
@@ -643,13 +668,7 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
     s = bwd_fused(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits,
                   gv32, grad_offsets, grad_logits, fa);
   if (s != MSDA_OK) return s;
-  if (dtype == MSDA_BF16) {
-    const int64_t n = d.n_value();
-    msda::msda_cast_f32_to_bf16_kernel<<<grid_for(n, 256, 148 * 16), 256, 0, st>>>(
-        gv32, static_cast<__nv_bfloat16*>(grad_value), n);
-    count_launch();
-    MSDA_CUDA(cudaGetLastError());
-  }
+  if (two_byte(dtype)) return cast_from_f32(st, gv32, grad_value, d.n_value(), dtype);
   return MSDA_OK;
 }
 
@@ -663,7 +682,8 @@ int dcn_setup(int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h,
       group_channels < 1)
     return fail(MSDA_ERR_INVALID_ARGUMENT, "dcnv3: bad geometry");
   *d = Dims{batch, height_in * width_in, group, group_channels, 1, height_out * width_out, kernel_h * kernel_w};
-  if (dtype != MSDA_F32 && dtype != MSDA_BF16) return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: float32 / bfloat16 only");
+  if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16)
+    return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: float32 / bfloat16 / float16 only");
   if (d->rows() * d->D != 0 && !fast_ok(*d, dtype, 0))
     return fail(MSDA_ERR_UNSUPPORTED,
                 "dcnv3: needs group_channels in {16,32,64,128} and kernel_h*kernel_w <= 64 (got %d, %d)",
@@ -726,14 +746,14 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
     return s;
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(anchor));
-  const size_t need = dtype == MSDA_BF16 ? (size_t)d.n_value() * sizeof(float) : 0;
+  const size_t need = two_byte(dtype) ? (size_t)d.n_value() * sizeof(float) : 0;
   if (need && (!workspace || workspace_bytes < need))
     return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
-  float* gi32 = dtype == MSDA_BF16 ? static_cast<float*>(workspace) : static_cast<float*>(grad_input);
+  float* gi32 = two_byte(dtype) ? static_cast<float*>(workspace) : static_cast<float*>(grad_input);
   if (d.n_value()) {
     if (!grad_input) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_input is null");
     MSDA_CUDA(cudaMemsetAsync(gi32, 0, (size_t)d.n_value() * sizeof(float), st));
-    if (dtype == MSDA_BF16 && d.n_points() == 0)
+    if (two_byte(dtype) && d.n_points() == 0)
       MSDA_CUDA(cudaMemsetAsync(grad_input, 0, (size_t)d.n_value() * 2, st));
   }
   if (d.n_points() == 0) return MSDA_OK;
@@ -745,13 +765,7 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
   }
   if (!grad_output || !input || !offset || !mask) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
   if (int s = bwd_dcn(st, d, dtype, grad_output, input, offset, mask, gi32, grad_offset, grad_mask, fa)) return s;
-  if (dtype == MSDA_BF16) {
-    const int64_t n = d.n_value();
-    msda::msda_cast_f32_to_bf16_kernel<<<grid_for(n, 256, 148 * 16), 256, 0, st>>>(
-        gi32, static_cast<__nv_bfloat16*>(grad_input), n);
-    count_launch();
-    MSDA_CUDA(cudaGetLastError());
-  }
+  if (two_byte(dtype)) return cast_from_f32(st, gi32, grad_input, d.n_value(), dtype);
   return MSDA_OK;
 }
 

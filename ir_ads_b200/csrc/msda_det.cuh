@@ -274,6 +274,9 @@ __device__ __forceinline__ float det_ld(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float det_ld(const __nv_bfloat16* p) {
   return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
 }
+__device__ __forceinline__ float det_ld(const __half* p) {
+  return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
+}
 
 // No minimum-blocks bound on purpose: ptxas settles at 80 registers (3 CTAs per SM) and 2.09 ms at cfg 5; asking for
 // 4 CTAs (64 registers, 40 bytes of spills) gave 2.49 ms, and even a bound of 1 -- same register count, another

@@ -32,8 +32,11 @@
 // instructions than the reference's scalar atomicAdd (cuh:125-152).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 #include "msda_coords.cuh"
 
@@ -71,6 +74,20 @@ __device__ __forceinline__ float4 ld4(const __nv_bfloat16* p) {
   r.w = __uint_as_float(u.y & 0xffff0000u);
   return r;
 }
+// float16 -> float32: __half22float2 is ONE HADD2.F32 (FMA pipe, not the F2F conversion unit) per two channels, and
+// it is exact: every half (subnormals, Inf, NaN included) widens to the float32 with the same value
+__device__ __forceinline__ float2 half2_bits_to_float2(unsigned u) {
+  return __half22float2(*reinterpret_cast<const __half2*>(&u));
+}
+__device__ __forceinline__ unsigned pack_f16x2(float lo, float hi) {
+  const __half2 t = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<const unsigned*>(&t);
+}
+__device__ __forceinline__ float4 ld4(const __half* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  const float2 a = half2_bits_to_float2(u.x), b = half2_bits_to_float2(u.y);
+  return make_float4(a.x, a.y, b.x, b.y);
+}
 __device__ __forceinline__ void st4(float* p, const float4 v) { *reinterpret_cast<float4*>(p) = v; }
 __device__ __forceinline__ void st4(__nv_bfloat16* p, const float4 v) {
   const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
@@ -78,6 +95,9 @@ __device__ __forceinline__ void st4(__nv_bfloat16* p, const float4 v) {
   u.x = *reinterpret_cast<const unsigned*>(&lo);
   u.y = *reinterpret_cast<const unsigned*>(&hi);
   *reinterpret_cast<uint2*>(p) = u;
+}
+__device__ __forceinline__ void st4(__half* p, const float4 v) {
+  *reinterpret_cast<uint2*>(p) = make_uint2(pack_f16x2(v.x, v.y), pack_f16x2(v.z, v.w));
 }
 __device__ __forceinline__ void fma4(float4& acc, const float s, const float4 v) {
   acc.x = fmaf(s, v.x, acc.x); acc.y = fmaf(s, v.y, acc.y); acc.z = fmaf(s, v.z, acc.z); acc.w = fmaf(s, v.w, acc.w);
@@ -124,6 +144,24 @@ __device__ __forceinline__ Vec<N> ldv(const __nv_bfloat16* p) {
   }
   return r;
 }
+// float16: the same vector loads, widened pairwise (half2_bits_to_float2)
+__device__ __forceinline__ void widen_f16x2(float* dst, unsigned u) {
+  const float2 f = half2_bits_to_float2(u);
+  dst[0] = f.x;
+  dst[1] = f.y;
+}
+template <int N>
+__device__ __forceinline__ Vec<N> ldv(const __half* p) {
+  Vec<N> r;
+  if constexpr (N == 4) {
+    const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+    widen_f16x2(r.v, u.x); widen_f16x2(r.v + 2, u.y);
+  } else {
+    const uint4 u = __ldg(reinterpret_cast<const uint4*>(p));
+    widen_f16x2(r.v, u.x); widen_f16x2(r.v + 2, u.y); widen_f16x2(r.v + 4, u.z); widen_f16x2(r.v + 6, u.w);
+  }
+  return r;
+}
 // The bits of one lane load, converted to floats only where they are consumed (the forward keeps several
 // predicated loads in flight; holding them as packed bf16 keeps the kernel inside its register budget).
 template <int N, typename VT>
@@ -140,6 +178,14 @@ template <>
 struct Raw<8, __nv_bfloat16> {
   uint4 r = {0u, 0u, 0u, 0u};
 };
+template <>
+struct Raw<4, __half> {
+  uint2 r = {0u, 0u};
+};
+template <>
+struct Raw<8, __half> {
+  uint4 r = {0u, 0u, 0u, 0u};
+};
 template <int N>
 __device__ __forceinline__ Raw<N, float> ldraw(const float* p) {
   static_assert(N == 4, "float rows use 4 channels per lane");
@@ -150,6 +196,13 @@ __device__ __forceinline__ Raw<N, float> ldraw(const float* p) {
 template <int N>
 __device__ __forceinline__ Raw<N, __nv_bfloat16> ldraw(const __nv_bfloat16* p) {
   Raw<N, __nv_bfloat16> x;
+  if constexpr (N == 4) x.r = __ldg(reinterpret_cast<const uint2*>(p));
+  else x.r = __ldg(reinterpret_cast<const uint4*>(p));
+  return x;
+}
+template <int N>
+__device__ __forceinline__ Raw<N, __half> ldraw(const __half* p) {
+  Raw<N, __half> x;
   if constexpr (N == 4) x.r = __ldg(reinterpret_cast<const uint2*>(p));
   else x.r = __ldg(reinterpret_cast<const uint4*>(p));
   return x;
@@ -173,6 +226,16 @@ __device__ __forceinline__ Vec<8> unpack(const Raw<8, __nv_bfloat16>& x) {
   r.v[6] = __uint_as_float(x.r.w << 16); r.v[7] = __uint_as_float(x.r.w & 0xffff0000u);
   return r;
 }
+__device__ __forceinline__ Vec<4> unpack(const Raw<4, __half>& x) {
+  Vec<4> r;
+  widen_f16x2(r.v, x.r.x); widen_f16x2(r.v + 2, x.r.y);
+  return r;
+}
+__device__ __forceinline__ Vec<8> unpack(const Raw<8, __half>& x) {
+  Vec<8> r;
+  widen_f16x2(r.v, x.r.x); widen_f16x2(r.v + 2, x.r.y); widen_f16x2(r.v + 4, x.r.z); widen_f16x2(r.v + 6, x.r.w);
+  return r;
+}
 template <int N>
 __device__ __forceinline__ void stv(float* p, const Vec<N>& a) {
   static_assert(N == 4, "float rows use 4 channels per lane");
@@ -189,6 +252,15 @@ __device__ __forceinline__ void stv(__nv_bfloat16* p, const Vec<N>& a) {
   } else {
     *reinterpret_cast<uint4*>(p) = make_uint4(pack_bf16x2(a.v[0], a.v[1]), pack_bf16x2(a.v[2], a.v[3]),
                                               pack_bf16x2(a.v[4], a.v[5]), pack_bf16x2(a.v[6], a.v[7]));
+  }
+}
+template <int N>
+__device__ __forceinline__ void stv(__half* p, const Vec<N>& a) {
+  if constexpr (N == 4) {
+    *reinterpret_cast<uint2*>(p) = make_uint2(pack_f16x2(a.v[0], a.v[1]), pack_f16x2(a.v[2], a.v[3]));
+  } else {
+    *reinterpret_cast<uint4*>(p) = make_uint4(pack_f16x2(a.v[0], a.v[1]), pack_f16x2(a.v[2], a.v[3]),
+                                              pack_f16x2(a.v[4], a.v[5]), pack_f16x2(a.v[6], a.v[7]));
   }
 }
 template <int N>
@@ -513,8 +585,12 @@ __device__ __forceinline__ float2 dcn_location(const float2 off, int pt, int q, 
 
 // softmax over the row's NP logits by the row's LANES lanes; e_i = exp(x_i - max) is left in
 // scratch[pt] (one float per point, any 4-byte stride) and the sum is returned: w_i = e_i / sum.
-template <int LANES, int STRIDE>
+// VLANES = 2 * LANES (rows of 8 channels per lane) forms the sum in the order of VLANES lanes: lane `sub` adds up the
+// points of virtual lanes sub and sub + LANES separately and then the two -- the first butterfly step of the wider
+// order -- so the weights are bit for bit those of the 4-channel-per-lane rows (f16 forward == f32 forward).
+template <int LANES, int STRIDE, int VLANES = LANES>
 __device__ __forceinline__ float row_softmax(const float* logits_row, float* scratch, int NP, int sub) {
+  static_assert(VLANES == LANES || VLANES == 2 * LANES, "one or two virtual lanes per lane");
   float m = -3.402823466e38f;
   for (int pt = sub; pt < NP; pt += LANES) {
     const float x = __ldg(logits_row + pt);
@@ -523,12 +599,17 @@ __device__ __forceinline__ float row_softmax(const float* logits_row, float* scr
   }
 #pragma unroll
   for (int k = LANES / 2; k > 0; k >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, k));
-  float sum = 0.0f;
-  for (int pt = sub; pt < NP; pt += LANES) {
-    const float e = expf(scratch[pt * STRIDE] - m);
-    scratch[pt * STRIDE] = e;
-    sum += e;
-  }
+  auto partial = [&](int first) {
+    float s = 0.0f;
+    for (int pt = first; pt < NP; pt += VLANES) {
+      const float e = expf(scratch[pt * STRIDE] - m);
+      scratch[pt * STRIDE] = e;
+      s += e;
+    }
+    return s;
+  };
+  float sum = partial(sub);
+  if constexpr (VLANES != LANES) sum += partial(sub + LANES);
 #pragma unroll
   for (int k = LANES / 2; k > 0; k >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, k);
   return sum;
@@ -553,6 +634,9 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
   constexpr int DL = D * 4 / CPL;               // lane geometry: LANES = D / CPL lanes per row
   using G = Geom<DL, THREADS>;
   constexpr int LANES = G::LANES;
+  // f16 rows sum the fused softmax in the f32 rows' lane order (row_softmax), so the f16 forward is the f32 forward
+  // on the widened value; bf16 keeps its own order
+  constexpr int SM_LANES = std::is_same_v<VT, __half> ? D / 4 : LANES;
   constexpr bool FUSED = (PRE == kPreFused);
   constexpr bool DCN = (PRE == kPreDcn);
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -601,7 +685,7 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
       early_w[i] = (on && !FUSED) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
     }
     // the softmax shuffles need the whole warp; dead rows read row 0 and simply produce nothing
-    if constexpr (FUSED) early_sum = row_softmax<LANES, 1>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_oc), NP, sub);
+    if constexpr (FUSED) early_sum = row_softmax<LANES, 1, SM_LANES>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_oc), NP, sub);
     load_levels_plain(tab, shapes, lsi, L);
   } else {
     if constexpr (DCN) set_single_level<G::TW, G::TH>(tab, fused.height_in, fused.width_in);
@@ -617,7 +701,7 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
       const float2* lp = reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2);
       const float* wp = w + cur.row * (int64_t)NP;
       float sm_sum = early_sum;
-      if constexpr (FUSED && !EARLY) sm_sum = row_softmax<LANES, 1>(wp, reinterpret_cast<float*>(s_oc), NP, sub);
+      if constexpr (FUSED && !EARLY) sm_sum = row_softmax<LANES, 1, SM_LANES>(wp, reinterpret_cast<float*>(s_oc), NP, sub);
       if (cur.live) {
         const float* rp = FUSED ? fused.ref + (cur.row / H) * (int64_t)L * fused.ref_dim : nullptr;
         // one record from a point's raw location / weight (FUSED: raw offset; the weight comes from the softmax)

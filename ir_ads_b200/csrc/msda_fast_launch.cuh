@@ -27,7 +27,7 @@ inline int64_t tile2d_bound(const Dims& d, int rpc) { return ((int64_t)d.S + rpc
 #endif
 constexpr int kFwdThreads = MSDA_FWD_THREADS, kBwdThreads = MSDA_BWD_THREADS;
 
-// channels per lane: 8 for bf16 rows of 32+ channels (16-byte lane loads), else 4
+// channels per lane: 8 for bf16 / f16 rows of 32+ channels (16-byte lane loads), else 4
 template <int D, typename VT>
 constexpr int cpl_of() { return (sizeof(VT) == 2 && D >= 32) ? 8 : 4; }
 
@@ -105,6 +105,15 @@ int launch_bwd_fast(cudaStream_t st, const Dims& d, const void* go, const void* 
     }                                                        \
   } while (0)
 #endif
+
+// CALL over the value types of the fast kernels (fast_ok admits no other dtype)
+#define MSDA_DISPATCH_VT(CALL)                                         \
+  do {                                                                 \
+    if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL);               \
+    if (dtype == MSDA_BF16) MSDA_DISPATCH_D(__nv_bfloat16, CALL);      \
+    if (dtype == MSDA_F16) MSDA_DISPATCH_D(__half, CALL);              \
+    return fail(MSDA_ERR_UNSUPPORTED, "fast path: dtype %d", dtype);   \
+  } while (0)
 
 // The product library instantiates ONE row order per pass -- LINEAR forward, STRIP backward, the pair that is fastest
 // on every measured config (profiles/r02t_sweep_row_orders.txt) -- and treats MSDA_FLAG_ORDER_* as hints it may

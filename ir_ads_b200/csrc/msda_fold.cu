@@ -79,6 +79,7 @@ bool fold_applies(const Dims& d, int dtype, unsigned flags) {
   if (flags & (MSDA_FLAG_FOLD_OFF | MSDA_FLAG_DETERMINISTIC | MSDA_FLAG_FORCE_GENERIC | MSDA_FLAG_ORDER_LINEAR |
                MSDA_FLAG_ORDER_STRIP | MSDA_FLAG_ORDER_TILE2D))
     return false;
+  if (dtype != MSDA_F32 && dtype != MSDA_BF16) return false;   // instantiated for float / bf16 values only
   if (!fast_ok(d, dtype, flags)) return false;
   if (d.Q != d.S) return false;                       // query i must be pixel i of the pyramid
   if (!(d.D == 32 || d.D == 64)) return false;

@@ -12,8 +12,7 @@ int fwd_fast(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const vo
   (void)flags;
 #endif
 #define CALL_FWD(D_, VT_, PT_, ORD_) launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_>(st, d, value, shapes, lsi, loc, w, out)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_FWD);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_FWD);
+  MSDA_DISPATCH_VT(CALL_FWD);
 #undef CALL_FWD
 #undef MSDA_DISPATCH_ORDER
 }
@@ -33,8 +32,7 @@ int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, cons
 #define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
 #define CALL_FF(D_, VT_, PT_, ORD_) \
   launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPreFused>(st, d, value, shapes, lsi, off, logits, out, fa)
-  if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL_FF);
-  MSDA_DISPATCH_D(__nv_bfloat16, CALL_FF);
+  MSDA_DISPATCH_VT(CALL_FF);
 #undef CALL_FF
 #undef MSDA_DISPATCH_ORDER
 }
@@ -53,7 +51,9 @@ int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const 
     default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);           \
   }
   if (dtype == MSDA_F32) DCN_D(float)
-  DCN_D(__nv_bfloat16)
+  if (dtype == MSDA_BF16) DCN_D(__nv_bfloat16)
+  if (dtype == MSDA_F16) DCN_D(__half)
+  return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
 #undef DCN_D
 #undef CALL_DF
 }

@@ -1,4 +1,4 @@
-// msda_generic.cuh -- shape-agnostic MSDeformAttn kernels (any D, L, P; float / double / bf16 value).
+// msda_generic.cuh -- shape-agnostic MSDeformAttn kernels (any D, L, P; float / double / bf16 / f16 value).
 //
 // These cover what the fast kernels (msda_fast.cuh) do not: head dims outside {16,32,64,128},
 // float64 (the reference's gradcheck path, tests/test_ms_deform_attn.py:131-133 walks
@@ -13,6 +13,7 @@
 //             warp shuffles + one shared-memory hop; grad_value goes out as scalar atomics.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -22,17 +23,20 @@ namespace msda {
 
 template <typename VT> struct Compute { using type = float; };
 template <> struct Compute<double> { using type = double; };
+template <> struct Compute<__half> { using type = float; };
 
 template <typename CT, typename VT> __device__ __forceinline__ CT load_as(const VT* p) { return (CT)(*p); }
 template <> __device__ __forceinline__ float load_as<float, __nv_bfloat16>(const __nv_bfloat16* p) {
   return __bfloat162float(*p);
 }
+template <> __device__ __forceinline__ float load_as<float, __half>(const __half* p) { return __half2float(*p); }
 template <typename VT, typename CT> __device__ __forceinline__ void store_as(VT* p, CT v) { *p = (VT)v; }
 template <> __device__ __forceinline__ void store_as<__nv_bfloat16, float>(__nv_bfloat16* p, float v) {
   *p = __float2bfloat16_rn(v);
 }
+template <> __device__ __forceinline__ void store_as<__half, float>(__half* p, float v) { *p = __float2half_rn(v); }
 
-// value/out: VT; loc/w: CT (= float for float and bf16 values, double for double).
+// value/out: VT; loc/w: CT (= float for float, bf16 and f16 values, double for double).
 template <typename VT, typename CT>
 __global__ void __launch_bounds__(256)
 msda_fwd_generic_kernel(const VT* __restrict__ value, const int64_t* __restrict__ shapes,
@@ -157,10 +161,11 @@ msda_bwd_generic_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ 
   }
 }
 
-// scratch (float) -> bf16 grad_value
-__global__ void msda_cast_f32_to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, int64_t n) {
+// scratch (float) -> bf16 / f16 grad_value
+template <typename VT>
+__global__ void msda_cast_f32_kernel(const float* __restrict__ src, VT* __restrict__ dst, int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    dst[i] = __float2bfloat16_rn(src[i]);
+    store_as<VT, float>(dst + i, src[i]);
 }
 
 // ---- deterministic mode helpers ------------------------------------------------------------

@@ -11,6 +11,7 @@
 #include "../../include/msda.h"
 
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -47,7 +48,7 @@ struct NamedPtr {
 };
 int check_alignment(std::initializer_list<NamedPtr> ptrs);
 
-// D in {16,32,64,128}, float / bf16 value, L <= 16, 1 <= L*P <= 64, 32-bit offsets inside one image
+// D in {16,32,64,128}, float / bf16 / f16 value, L <= 16, 1 <= L*P <= 64, 32-bit offsets inside one image
 bool fast_ok(const Dims& d, int dtype, unsigned flags);
 
 inline int grid_for(int64_t work_items, int threads, int cap_blocks) {

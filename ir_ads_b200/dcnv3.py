@@ -7,10 +7,10 @@ input / offset / mask.  DCNv3 is MSDeformAttn with one level, K = kernel_h*kerne
 positions come from a convolution-style grid, and groups in the role of heads -- so it runs on the
 same kernels with a different record-building phase (ir_ads_b200/csrc/msda_fast.cuh, PRE == 2).
 
-Fast path: group_channels in {16, 32, 64, 128}, K <= 64, float32 / bfloat16 input (float16 is widened to float32
-around the op).  Every other shape / dtype the reference dispatches (any channel count, float64:
-detrex/layers/csrc/DCNv3/dcnv3_cuda.cu:66-80 uses AT_DISPATCH_FLOATING_TYPES_AND_HALF) runs as a composition on the
-GENERIC MSDeformAttn kernels (csrc/msda_generic.cuh, any D, float32 / float64): the convolution-grid sampling positions
+Fast path: group_channels in {16, 32, 64, 128}, K <= 64, float32 / bfloat16 / float16 input (float16 and bfloat16
+are widened exactly inside the kernels, accumulation is float32).  Every other shape / dtype the reference dispatches
+(any channel count, float64: detrex/layers/csrc/DCNv3/dcnv3_cuda.cu:66-80 uses AT_DISPATCH_FLOATING_TYPES_AND_HALF)
+runs as a composition on the GENERIC MSDeformAttn kernels (csrc/msda_generic.cuh, any D, float32 / float64): the convolution-grid sampling positions
 are formed with the reference kernel's arithmetic in PyTorch, normalised, and handed to
 MultiScaleDeformableAttnFunction with one level -- still CUDA only, still no CPU path.
 """
@@ -24,7 +24,9 @@ from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 
 from . import _lib
-from .functional import _DTYPE_TAG, _aligned, _ptr, _require
+from .functional import _aligned, _ptr, _require
+
+_DCN_TAG = {torch.float32: _lib.MSDA_F32, torch.bfloat16: _lib.MSDA_BF16, torch.float16: _lib.MSDA_F16}
 
 
 def _declare(handle):
@@ -51,8 +53,10 @@ def _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels):
     _require(C == group * group_channels, f"input channels {C} != group*group_channels {group * group_channels}")
     _require(tuple(offset.shape) == (N, H_out, W_out, group * K * 2), "offset must be [N, H_out, W_out, group*K*2]")
     _require(tuple(mask.shape) == (N, H_out, W_out, group * K), "mask must be [N, H_out, W_out, group*K]")
-    _require(input.dtype in (torch.float32, torch.bfloat16), f"unsupported input dtype {input.dtype}")
-    _require(offset.dtype == torch.float32 and mask.dtype == torch.float32, "offset / mask must be float32")
+    _require(input.dtype in _DCN_TAG, f"unsupported input dtype {input.dtype}")
+    # float16 offset / mask as well: the reference's _C takes them in the input's dtype (dcnv3_cuda.cu:66-80)
+    _require(offset.dtype in (torch.float32, torch.float16) and mask.dtype in (torch.float32, torch.float16),
+             "offset / mask must be float32 or float16")
     return N, H_in, W_in, H_out, W_out
 
 
@@ -60,37 +64,39 @@ def dcnv3_forward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, p
                   group, group_channels, offset_scale, im2col_step=256) -> torch.Tensor:
     """``detrex._C.dcnv3_forward``: returns ``[N, H_out, W_out, group*group_channels]``."""
     N, H_in, W_in, H_out, W_out = _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels)
-    input, offset, mask = _aligned(input), _aligned(offset), _aligned(mask)
+    input, offset, mask = _aligned(input), _aligned(offset.float()), _aligned(mask.float())
     out = torch.empty((N, H_out, W_out, group * group_channels), dtype=input.dtype, device=input.device)
     stream = torch.cuda.current_stream(input.device).cuda_stream
     status = _declare(_lib.lib()).msda_dcnv3_forward(
         ctypes.c_void_p(stream), _ptr(input), _ptr(offset), _ptr(mask), kernel_h, kernel_w, stride_h, stride_w, pad_h,
         pad_w, dilation_h, dilation_w, group, group_channels, float(offset_scale), N, H_in, W_in, H_out, W_out,
-        _ptr(out), _DTYPE_TAG[input.dtype], 0)
+        _ptr(out), _DCN_TAG[input.dtype], 0)
     _lib.check(status, "dcnv3_forward")
     return out
 
 
 def dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
                    group, group_channels, offset_scale, grad_output, im2col_step=256) -> List[torch.Tensor]:
-    """``detrex._C.dcnv3_backward``: ``[grad_input, grad_offset, grad_mask]``."""
+    """``detrex._C.dcnv3_backward``: ``[grad_input, grad_offset, grad_mask]``, each in the dtype of its input (the
+    offset / mask gradients are computed in float32)."""
     N, H_in, W_in, H_out, W_out = _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels)
     _require(grad_output.is_cuda and grad_output.dtype == input.dtype, "grad_output must match input's device / dtype")
     grad_output = _aligned(grad_output.contiguous())
-    input, offset, mask = _aligned(input), _aligned(offset), _aligned(mask)
+    off_dtype, mask_dtype = offset.dtype, mask.dtype
+    input, offset, mask = _aligned(input), _aligned(offset.float()), _aligned(mask.float())
     grad_input = torch.empty_like(input)
     grad_offset = torch.empty_like(offset)
     grad_mask = torch.empty_like(mask)
-    ws_bytes = input.numel() * 4 if input.dtype == torch.bfloat16 else 0
+    ws_bytes = input.numel() * 4 if input.dtype != torch.float32 else 0   # bf16 / f16: float accumulation buffer
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=input.device) if ws_bytes else None
     stream = torch.cuda.current_stream(input.device).cuda_stream
     status = _declare(_lib.lib()).msda_dcnv3_backward(
         ctypes.c_void_p(stream), _ptr(grad_output), _ptr(input), _ptr(offset), _ptr(mask), kernel_h, kernel_w,
         stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels, float(offset_scale), N, H_in,
         W_in, H_out, W_out, _ptr(grad_input), _ptr(grad_offset), _ptr(grad_mask),
-        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, _DTYPE_TAG[input.dtype], 0)
+        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, _DCN_TAG[input.dtype], 0)
     _lib.check(status, "dcnv3_backward")
-    return [grad_input, grad_offset, grad_mask]
+    return [grad_input, grad_offset.to(off_dtype), grad_mask.to(mask_dtype)]
 
 
 def fast_supported(input: torch.Tensor, kernel_h: int, kernel_w: int, group_channels: int) -> bool:
@@ -141,7 +147,6 @@ class DCNv3Function(Function):
         ctx.args = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels,
                     offset_scale)
         ctx.im2col_step = im2col_step
-        ctx.in_dtype = input.dtype
         ctx.composed = None
         if not fast_supported(input, kernel_h, kernel_w, group_channels):
             # any other channel count / float64: the composition on the generic kernels, graph kept for backward
@@ -150,11 +155,9 @@ class DCNv3Function(Function):
                 out = dcnv3_composed(*leaves, *ctx.args)
             ctx.composed = (leaves, out)
             return out.detach()
-        if input.dtype == torch.float16:
-            input = input.float()
         output = dcnv3_forward(input, offset.float(), mask.float(), *ctx.args, im2col_step)
         ctx.save_for_backward(input, offset, mask)
-        return output.to(ctx.in_dtype)
+        return output
 
     @staticmethod
     @once_differentiable
@@ -166,7 +169,7 @@ class DCNv3Function(Function):
         input, offset, mask = ctx.saved_tensors
         gi, go, gm = dcnv3_backward(input, offset.float(), mask.float(), *ctx.args, grad_output.to(input.dtype),
                                     ctx.im2col_step)
-        return (gi.to(ctx.in_dtype), go.to(offset.dtype), gm.to(mask.dtype)) + (None,) * 12
+        return (gi, go.to(offset.dtype), gm.to(mask.dtype)) + (None,) * 12
 
 
 # ------------------------------------------------------------------------------------------------

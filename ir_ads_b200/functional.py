@@ -7,7 +7,8 @@ order and error behaviour -- bound to libmsda_b200.so through ctypes instead of 
 
 Differences from the reference, all documented in SURVEY.md appendix B and DESIGN.md:
   * bf16 ``value`` is supported (locations / weights stay float32, fp32 accumulate); the reference
-    dispatches float and double only (ms_deform_attn_cuda.cu:65);
+    dispatches float and double only (ms_deform_attn_cuda.cu:65).  float16 is refused here as there; the fused
+    module path (MSDeformAttnFusedFunction) takes it natively;
   * ``im2col_step`` is accepted and ignored: one launch covers the batch, so the reference's
     ``batch % im2col_step == 0`` assert (ms_deform_attn_cuda.cu:53) has nothing to protect;
   * a non-contiguous ``grad_output`` is made contiguous instead of asserting (cu:99);
@@ -25,7 +26,12 @@ from torch.autograd.function import once_differentiable
 
 from . import _lib
 
+# value dtypes of the public operator (the reference's _C dispatches float / double only; bf16 is an extension)
 _DTYPE_TAG = {torch.float32: _lib.MSDA_F32, torch.float64: _lib.MSDA_F64, torch.bfloat16: _lib.MSDA_BF16}
+# value dtypes of the fused module path and of the library-internal calls: float16 as well (MSDA_F16: every kernel
+# widens it exactly and accumulates in float32).  The public operator keeps refusing float16, as the reference's does.
+_VALUE_TAG = {**_DTYPE_TAG, torch.float16: _lib.MSDA_F16}
+_FUSED_DTYPES = (torch.float32, torch.bfloat16, torch.float16)
 
 _state = {"deterministic": False, "flags": 0}
 
@@ -71,7 +77,7 @@ def _aligned(t):
     return t.clone(memory_format=torch.contiguous_format)
 
 
-def _check_inputs(value, spatial_shapes, level_start_index, sampling_loc, attn_weight):
+def _check_inputs(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, tags=_DTYPE_TAG):
     # mirrors the AT_ASSERTM block of ms_deform_attn_cuda.cu:29-39
     _require(value.is_cuda, "Not implemented on the CPU")  # ms_deform_attn.h:39
     for name, t in (("value", value), ("spatial_shapes", spatial_shapes),
@@ -91,7 +97,8 @@ def _check_inputs(value, spatial_shapes, level_start_index, sampling_loc, attn_w
     _require(tuple(attn_weight.shape) == (B, Q, H, L, P), "attn_weight shape does not match sampling_loc")
     _require(spatial_shapes.shape == (L, 2) and level_start_index.shape == (L,),
              "spatial_shapes must be [L, 2] and level_start_index [L]")
-    _require(value.dtype in _DTYPE_TAG, f"unsupported value dtype {value.dtype} (float32, float64, bfloat16)")
+    names = ", ".join(str(t).replace("torch.", "") for t in tags)
+    _require(value.dtype in tags, f"unsupported value dtype {value.dtype} ({names})")
     aux = torch.float64 if value.dtype == torch.float64 else torch.float32
     _require(sampling_loc.dtype == aux and attn_weight.dtype == aux,
              f"sampling_loc / attn_weight must be {aux} when value is {value.dtype}")
@@ -120,11 +127,12 @@ def ms_deform_attn_backward(value: torch.Tensor, spatial_shapes: torch.Tensor, l
 
 
 def _backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, grad_output,
-              need_grad_value: bool) -> List[torch.Tensor]:
+              need_grad_value: bool, tags=_DTYPE_TAG) -> List[torch.Tensor]:
     """The backward behind ms_deform_attn_backward.  ``need_grad_value=False`` (the autograd Function passes it when
     ``value`` does not require grad, e.g. a frozen memory branch) returns ``None`` for ``grad_value`` and, on the
-    shapes the fast kernels cover, skips its scatter -- the dominant cost of the backward -- altogether."""
-    B, S, H, D, L, Q, P = _check_inputs(value, spatial_shapes, level_start_index, sampling_loc, attn_weight)
+    shapes the fast kernels cover, skips its scatter -- the dominant cost of the backward -- altogether.  ``tags``:
+    the accepted value dtypes (library-internal callers pass _VALUE_TAG to hand float16 over natively)."""
+    B, S, H, D, L, Q, P = _check_inputs(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, tags)
     _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
     _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
     _require(grad_output.numel() == B * Q * H * D, "grad_output must be [B, Q, H*D]")
@@ -133,7 +141,7 @@ def _backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weigh
     grad_loc = torch.empty_like(sampling_loc)
     grad_w = torch.empty_like(attn_weight)
     flags = _flags(True)
-    tag = _DTYPE_TAG[value.dtype]
+    tag = tags[value.dtype]
     handle = _lib.lib()
     skip_scatter = (not need_grad_value and B * S * D > 0 and Q * L * P > 0
                     and b"_fast_" in handle.msda_dispatch_name(D, L, P, S, H, tag, flags, 1))
@@ -198,12 +206,12 @@ def multi_scale_deformable_attn_pytorch(value: torch.Tensor, value_spatial_shape
 # fused module path (SURVEY.md section 8f-1): softmax + sampling-location arithmetic inside the kernels
 # ------------------------------------------------------------------------------------------------
 def fused_supported(value: torch.Tensor, num_levels: int, num_points: int) -> bool:
-    """True when the fused kernels cover this problem (fast-kernel shapes, float32 / bfloat16 value);
+    """True when the fused kernels cover this problem (fast-kernel shapes, float32 / bfloat16 / float16 value);
     otherwise the module composes the pre-op chain in PyTorch."""
-    if not value.is_cuda or value.dtype not in (torch.float32, torch.bfloat16) or value.dim() != 4:
+    if not value.is_cuda or value.dtype not in _FUSED_DTYPES or value.dim() != 4:
         return False
     _, S, H, D = value.shape
-    return bool(_lib.lib().msda_fused_supported(D, num_levels, num_points, S, H, _DTYPE_TAG[value.dtype], _flags(False)))
+    return bool(_lib.lib().msda_fused_supported(D, num_levels, num_points, S, H, _VALUE_TAG[value.dtype], _flags(False)))
 
 
 def _mask_ptr(mask) -> ctypes.c_void_p:
@@ -221,7 +229,7 @@ def _check_fused_inputs(value, spatial_shapes, level_start_index, sampling_offse
         _require(t.is_cuda and t.device == value.device, f"{name} must be a CUDA tensor on {value.device}")
         _require(t.is_contiguous(), f"{name} tensor has to be contiguous")
     _require(value.dim() == 4, "value must be [B, S, H, D]")
-    _require(value.dtype in (torch.float32, torch.bfloat16), f"unsupported value dtype {value.dtype} (float32, bfloat16)")
+    _require(value.dtype in _FUSED_DTYPES, f"unsupported value dtype {value.dtype} (float32, bfloat16, float16)")
     _require(sampling_offsets.dim() == 6 and sampling_offsets.shape[-1] == 2, "sampling_offsets must be [B, Q, H, L, P, 2]")
     B, S, H, D = value.shape
     Bq, Q, Hq, L, P, _ = sampling_offsets.shape
@@ -262,7 +270,8 @@ def _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_poin
 class MSDeformAttnFusedFunction(Function):
     """``apply(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points,
     key_padding_mask=None)`` -> ``[B, Q, H*D]``.  ``sampling_offsets [B,Q,H,L,P,2]`` and ``attn_logits
-    [B,Q,H,L*P]`` are the raw outputs of the module's two Linear layers (float32); ``reference_points
+    [B,Q,H,L*P]`` are the raw outputs of the module's two Linear layers (float32); ``value`` is float32, bfloat16
+    or float16 (the output and ``grad_value`` share its dtype, accumulation is float32); ``reference_points
     [B,Q,L,2|4]`` float32.  Equivalent to softmax + location affine (multi_scale_deform_attn.py:300-332)
     followed by MultiScaleDeformableAttnFunction, without materialising locations / weights or their
     gradients.  With ``key_padding_mask [B,S]`` (bool or uint8, True = padded) it is additionally equivalent
@@ -286,7 +295,7 @@ class MSDeformAttnFusedFunction(Function):
         status = _lib.lib().msda_fused_forward(
             ctypes.c_void_p(stream), _ptr(value), _ptr(spatial_shapes), _ptr(level_start_index), _ptr(sampling_offsets),
             _ptr(attn_logits), _ptr(reference_points), ref_dim, _mask_ptr(mask), B, S, H, D, L, Q, P, _ptr(out),
-            _DTYPE_TAG[value.dtype], _flags(False))
+            _VALUE_TAG[value.dtype], _flags(False))
         _lib.check(status, "msda_fused_forward")
         ctx.save_for_backward(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points)
         ctx.value_mask = mask
@@ -313,7 +322,7 @@ class MSDeformAttnFusedFunction(Function):
             loc, weights = _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_points)
             v = value if mask is None else value.masked_fill(mask.bool()[..., None, None], 0)
             grad_value, g_loc, g_w = _backward(v, spatial_shapes, level_start_index, loc, weights, grad_output,
-                                               need_grad_value=ctx.needs_input_grad[0])
+                                               need_grad_value=ctx.needs_input_grad[0], tags=_VALUE_TAG)
             if grad_value is not None and mask is not None:
                 grad_value = grad_value.masked_fill(mask.bool()[..., None, None], 0)
             g_w = g_w.view(B, Q, H, L * P)
@@ -333,7 +342,7 @@ class MSDeformAttnFusedFunction(Function):
         grad_value = torch.empty_like(value)
         grad_off = torch.empty_like(sampling_offsets)
         grad_logits = torch.empty_like(attn_logits)
-        tag = _DTYPE_TAG[value.dtype]
+        tag = _VALUE_TAG[value.dtype]
         handle = _lib.lib()
         ws_bytes = int(handle.msda_backward_workspace_bytes(B, S, H, D, L, Q, P, tag, flags))
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None

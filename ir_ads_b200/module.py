@@ -12,9 +12,12 @@ What differs from the reference module:
     forward (py:286), which blocks the host 12 times per step; here the check runs on a HOST copy of the shapes
     when the caller has one (``level_shapes=[(H_l, W_l), ...]``, what ``encoder.flatten_levels`` returns: free),
     otherwise once per live shapes tensor OBJECT (keyed by the object, dropped when it dies -- never by address);
-  * bfloat16 activations (autocast bf16) go to the bf16-value kernel with float32 sampling
-    locations / weights instead of failing in the float-only dispatch; float16 is widened to
-    float32 around the op exactly as the reference does (py:343, :355-356);
+  * bfloat16 and float16 activations (autocast) go to the bf16 / f16-value kernels with float32 sampling
+    locations / weights and float32 accumulation instead of failing in the float-only dispatch.  The reference
+    widens float16 to float32 around the op (py:343, :355-356); here the fused path takes the float16 value as it is,
+    with the same output (the kernels widen exactly, so only the final rounding to float16 remains) and half the
+    value bytes read and saved for backward.  Only the unfused fallback (``fuse_pre_ops = False`` or shapes the
+    fused kernels do not cover) still widens float16, since the plain op, like the reference's, has no float16 form;
   * there is no CPU branch (py:350-353): a CPU tensor raises;
   * ``add_identity=False`` (keyword, default True) returns ``dropout(output_proj(...))`` WITHOUT the residual
     (py:363), for callers that fuse ``+ identity`` into the LayerNorm that follows (ir_ads_b200/epilogue.py).
@@ -147,9 +150,9 @@ class MultiScaleDeformableAttention(nn.Module):
 
         io_dtype = value.dtype
         value = value.view(bs, num_value, H, -1)
-        if io_dtype == torch.float16:
-            value = value.float()
         fused = self.fuse_pre_ops and fused_supported(value, L, P)
+        if io_dtype == torch.float16 and not fused:
+            value = value.float()                         # the plain op has no float16 form (py:343)
         if key_padding_mask is not None and not fused:
             value = value.masked_fill(key_padding_mask[..., None, None], float(0))
         if fused:
