@@ -200,9 +200,24 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
  *   output / grad_output [N, H_out, W_out, group*group_channels] dtype
  * The input is NOT padded by the caller: pad_h / pad_w only shift the sampling grid and samples outside
  * the map read zeros, exactly like the reference kernel.  Supported: group_channels in {16,32,64,128},
- * K <= 64, float32 / bfloat16 / float16 input (MSDA_ERR_UNSUPPORTED otherwise).  The bfloat16 and float16
- * backward need a workspace of N*H_in*W_in*C floats.
+ * K <= 64, float32 / bfloat16 / float16 input (MSDA_ERR_UNSUPPORTED otherwise).
+ * The backward's workspace comes from msda_dcnv3_backward_workspace_bytes; less gives MSDA_ERR_WORKSPACE.  Without
+ * MSDA_FLAG_DETERMINISTIC that is 0 for float32 and N*H_in*W_in*C floats for bfloat16 / float16 (grad_input is
+ * accumulated in float with float reds, whose rounding depends on arrival order).
+ * msda_dcnv3_backward honours MSDA_FLAG_DETERMINISTIC, MSDA_FLAG_DET_ATOMIC and MSDA_FLAG_DET_SEPARATE_FILL and ignores
+ * every other bit.  With MSDA_FLAG_DETERMINISTIC grad_input is bit-reproducible: it is the deterministic backward of
+ * the equivalent one-level msda_backward problem (value = input [N, H_in*W_in, group, group_channels],
+ * Q = H_out*W_out, P = K), 64-bit fixed point summed by the sorted segment reduction or, with MSDA_FLAG_DET_ATOMIC or
+ * beyond its 32-bit index limits, by integer reds -- all routes give the same bits -- and converted once into the
+ * input's dtype.  grad_offset / grad_mask are the same bits as without the flag.  The workspace is then
+ *   256 + msda_backward_workspace_bytes(N, H_in*W_in, group, group_channels, 1, H_out*W_out, K, dtype,
+ *                                       flags & (DETERMINISTIC | DET_ATOMIC | DET_SEPARATE_FILL))
+ * bytes (the first 256 hold the one-level table the kernels read), except for empty problems (N, H_in*W_in or
+ * H_out*W_out zero), which need and do exactly what they do without the flag.
  */
+size_t msda_dcnv3_backward_workspace_bytes(int kernel_h, int kernel_w, int group, int group_channels, int batch,
+                                           int height_in, int width_in, int height_out, int width_out, int dtype,
+                                           unsigned flags);
 int msda_dcnv3_forward(void* stream, const void* input, const float* offset, const float* mask,
                        int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                        int dilation_h, int dilation_w, int group, int group_channels, float offset_scale,

@@ -60,6 +60,18 @@ int bwd_dcn(cudaStream_t, const Dims&, int, const void*, const void*, const void
             msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
 }
+int bwd_dcn_det(cudaStream_t, const Dims&, int, const void*, const void*, const void*, const void*,
+                unsigned long long*, void*, void*, const msda::DetScale*, msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
+}
+int bwd_dcn_noscatter(cudaStream_t, const Dims&, int, const void*, const void*, const void*, const void*, void*, void*,
+                      msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
+}
+int bwd_dcn_emit(cudaStream_t, const Dims&, int, const void*, const void*, const void*, const void*, void*, void*, int*,
+                 const int*, void*, float*, int64_t*, msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
+}
 #else
 // fused pre-op chain: STRIP order
 int bwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
@@ -108,6 +120,58 @@ int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const voi
 #undef DCN_D
 #undef CALL_DB
 }
+
+// the DCNv3 twins of the deterministic backward kernels above, dispatched over group_channels and dtype
+#define MSDA_DCN_DISPATCH(CALL)                                                              \
+  do {                                                                                       \
+    if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16)                        \
+      return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);                           \
+    switch (d.D) {                                                                           \
+      case 16: return dtype == MSDA_F32 ? CALL(16, float) : dtype == MSDA_BF16 ? CALL(16, __nv_bfloat16) : CALL(16, __half); \
+      case 32: return dtype == MSDA_F32 ? CALL(32, float) : dtype == MSDA_BF16 ? CALL(32, __nv_bfloat16) : CALL(32, __half); \
+      case 64: return dtype == MSDA_F32 ? CALL(64, float) : dtype == MSDA_BF16 ? CALL(64, __nv_bfloat16) : CALL(64, __half); \
+      case 128: return dtype == MSDA_F32 ? CALL(128, float) : dtype == MSDA_BF16 ? CALL(128, __nv_bfloat16) : CALL(128, __half); \
+      default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);         \
+    }                                                                                        \
+  } while (0)
+
+// DCNv3, 64-bit fixed-point reds (MSDA_FLAG_DET_ATOMIC, or problems beyond the sorted path's 32-bit indices): STRIP
+// order, as the float-red twin
+int bwd_dcn_det(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                const void* mask, unsigned long long* acc, void* goff, void* gmask, const msda::DetScale* det,
+                msda::FusedArgs fa) {
+#define CALL_DB(D_, VT_)                                                                                         \
+  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, unsigned long long, msda::kPreDcn>(st, d, go, input, nullptr, nullptr, \
+                                                                                 off, mask, acc, goff, gmask, det, fa)
+  MSDA_DCN_DISPATCH(CALL_DB);
+#undef CALL_DB
+}
+
+// DCNv3 without the scatter (grad_offset / grad_mask only): the sorted path with MSDA_FLAG_DET_SEPARATE_FILL
+int bwd_dcn_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                      const void* mask, void* goff, void* gmask, msda::FusedArgs fa) {
+#define CALL_DB(D_, VT_)                                                                                           \
+  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, msda::NoScatter, msda::kPreDcn>(                                     \
+      st, d, go, input, nullptr, nullptr, off, mask, (msda::NoScatter*)nullptr, goff, gmask, nullptr, fa)
+  MSDA_DCN_DISPATCH(CALL_DB);
+#undef CALL_DB
+}
+
+// DCNv3 backward that files every in-range point under its bilinear cell (sorted path).  LINEAR order, so that the
+// per-warp maxima have exactly the slots bwd_fast_emit counts for the equivalent one-level problem.
+int bwd_dcn_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                 const void* mask, void* goff, void* gmask, int* cursor, const int* bin_start, void* entries,
+                 float* warp_amax, int64_t* n_warps, msda::FusedArgs fa) {
+  const int64_t rpc = kBwdThreads / (d.D / 4);
+  if (n_warps) *n_warps = ((d.rows() + rpc - 1) / rpc) * (kBwdThreads / 32);
+  msda::EmitArgs ea{cursor, bin_start, static_cast<int4*>(entries), warp_amax};
+#define CALL_DB(D_, VT_)                                                                                           \
+  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 0, msda::EmitEntries, msda::kPreDcn>(                                   \
+      st, d, go, input, nullptr, nullptr, off, mask, (msda::EmitEntries*)nullptr, goff, gmask, nullptr, fa, ea)
+  MSDA_DCN_DISPATCH(CALL_DB);
+#undef CALL_DB
+}
+#undef MSDA_DCN_DISPATCH
 #endif
 
 }  // namespace msda_host

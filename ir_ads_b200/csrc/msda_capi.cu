@@ -253,6 +253,189 @@ int cast_from_f32(cudaStream_t st, const float* src, void* dst, int64_t n, int d
   return MSDA_OK;
 }
 
+// Where the points of the deterministic backward come from: the plain operator's sampling_loc / attn_weight, or the
+// DCNv3 sampling grid (offset / mask + geometry; `Dims` is then the equivalent one-level problem).  The count, gather
+// and cell-reduce kernels read the level table from device memory in both cases (DCNv3: the one-level slot
+// det_one_level_kernel writes into the workspace).
+struct DetSource {
+  const void* loc;               // plain: sampling_loc [B,Q,H,L,P,2]; DCNv3: offset [N,Ho,Wo,G*K*2]
+  const void* w;                 // plain: attn_weight;                 DCNv3: mask   [N,Ho,Wo,G*K]
+  const int64_t* shapes;
+  const int64_t* lsi;
+  const msda::FusedArgs* dcn;    // null: plain operator
+};
+
+// Bit-reproducible grad_value (MSDA_FLAG_DETERMINISTIC): 64-bit fixed-point accumulation (see include/msda.h), by the
+// sorted segment reduction where det_sorted_ok admits the problem, else by fixed-point reds.  `workspace` holds `need`
+// bytes laid out as msda_backward_workspace_bytes describes.  Writes every element of grad_value.
+int det_backward(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const void* grad_output, const void* value,
+                 const DetSource& src, void* grad_value, void* grad_sampling_loc, void* grad_attn_weight,
+                 void* workspace, size_t need) {
+  auto count = [] { count_launch(); };
+  const void* sampling_loc = src.loc;
+  const void* attn_weight = src.w;
+  const int64_t* spatial_shapes = src.shapes;
+  const int64_t* level_start_index = src.lsi;
+  const msda::FusedArgs dcn = src.dcn ? *src.dcn : msda::FusedArgs{};
+  const int64_t nv = d.n_value(), n_out = d.rows() * d.D, n_pts = d.n_points();
+  const bool sorted = det_sorted_ok(d, dtype, flags);
+  const DetLayout lay = sorted ? det_layout(d) : DetLayout{};
+  char* ws = static_cast<char*>(workspace);
+  auto* acc = reinterpret_cast<unsigned long long*>(ws + (sorted ? lay.off_acc : 0));
+  auto* amax = reinterpret_cast<unsigned*>(ws + (sorted ? lay.off_misc : (size_t)nv * 8));
+  auto* scale = reinterpret_cast<msda::DetScale*>(reinterpret_cast<char*>(amax) + 16);
+  if (sorted) {   // zero the bins, cursors, {amax, scale} and the accumulators; entries are fully overwritten
+    MSDA_CUDA(cudaMemsetAsync(ws, 0, lay.off_sums, st));
+    MSDA_CUDA(cudaMemsetAsync(ws + lay.off_misc, 0, lay.total - lay.off_misc, st));
+  } else {
+    MSDA_CUDA(cudaMemsetAsync(workspace, 0, need, st));
+  }
+  // The fixed-point scale comes from max |grad_out| x max |weight|.  On the sorted route the backward kernel that
+  // files the entries reads both tensors anyway and takes the two maxima itself (EmitArgs::amax); the scale is only
+  // needed by the reduction that follows it.  Every other route scatters with the scale and takes them up front.
+#ifndef MSDA_DET_AMAX_IN_EMIT
+#define MSDA_DET_AMAX_IN_EMIT 1
+#endif
+  const bool amax_in_emit = MSDA_DET_AMAX_IN_EMIT && sorted && !(flags & MSDA_FLAG_DET_SEPARATE_FILL);
+  const int g_out = grid_for(n_out, 256, 148 * 8), g_pts = grid_for(n_pts, 256, 148 * 8);
+  if (!amax_in_emit) {
+    if (dtype == MSDA_F32) msda::msda_amax_kernel<float><<<g_out, 256, 0, st>>>((const float*)grad_output, n_out, amax);
+    else if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_out, 256, 0, st>>>((const double*)grad_output, n_out, amax);
+    else if (dtype == MSDA_BF16) msda::msda_amax_kernel<__nv_bfloat16><<<g_out, 256, 0, st>>>((const __nv_bfloat16*)grad_output, n_out, amax);
+    else msda::msda_amax_kernel<__half><<<g_out, 256, 0, st>>>((const __half*)grad_output, n_out, amax);
+    count();
+    if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_pts, 256, 0, st>>>((const double*)attn_weight, n_pts, amax + 1);
+    else msda::msda_amax_kernel<float><<<g_pts, 256, 0, st>>>((const float*)attn_weight, n_pts, amax + 1);
+    count();
+    msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, dtype == MSDA_F64 ? 44 : 38);
+    count();
+    MSDA_CUDA(cudaGetLastError());
+  }
+  if (sorted) {
+    // sorted segment reduction (msda_det.cuh): count -> scan -> fill -> gather; no atomics on grad_value
+    int* bins = reinterpret_cast<int*>(ws);
+    int* cursor = reinterpret_cast<int*>(ws + lay.off_cursor);
+    int* sums = reinterpret_cast<int*>(ws + lay.off_sums);
+    int4* entries = reinterpret_cast<int4*>(ws + lay.off_entries);
+    const float* loc = static_cast<const float*>(sampling_loc);
+    const float* w = static_cast<const float*>(attn_weight);
+    const int g_bin = grid_for(n_pts, 256, 148 * 32);
+    if (src.dcn)
+      msda::det_bin_kernel<false, msda::kPreDcn><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H,
+                                                                       d.L, d.Q, d.P, n_pts, bins, nullptr, nullptr, dcn);
+    else
+      msda::det_bin_kernel<false><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H, d.L, d.Q, d.P,
+                                                         n_pts, bins, nullptr, nullptr, dcn);
+    count();
+    msda::det_scan_block_kernel<<<(unsigned)lay.scan_blocks, 256, 0, st>>>(bins, bins, sums, lay.n_scan);
+    count();
+    msda::det_scan_sums_kernel<<<1, 1024, 0, st>>>(sums, (int)lay.scan_blocks);
+    count();
+    msda::det_scan_add_kernel<<<(unsigned)lay.scan_blocks, 256, 0, st>>>(bins, sums, lay.n_scan);
+    count();
+    MSDA_CUDA(cudaGetLastError());
+    // entries are filed by the backward kernel itself (ACC = EmitEntries): the lane that has just built a point's
+    // record takes the cursor atomic and writes the 16-byte entry, so the separate fill pass (det_bin_kernel<true>:
+    // re-read of every location / weight + the coordinate arithmetic a second time) is gone
+    auto emit = [&](float* wamax, int64_t* n_warps) {
+      if (src.dcn)
+        return bwd_dcn_emit(st, d, dtype, grad_output, value, sampling_loc, attn_weight, grad_sampling_loc,
+                            grad_attn_weight, cursor, bins, entries, wamax, n_warps, dcn);
+      return bwd_fast_emit(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
+                           attn_weight, grad_sampling_loc, grad_attn_weight, cursor, bins, entries, wamax, n_warps);
+    };
+    if (flags & MSDA_FLAG_DET_SEPARATE_FILL) {
+      if (src.dcn)
+        msda::det_bin_kernel<true, msda::kPreDcn><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H,
+                                                                        d.L, d.Q, d.P, n_pts, cursor, bins, entries, dcn);
+      else
+        msda::det_bin_kernel<true><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H, d.L, d.Q, d.P,
+                                                          n_pts, cursor, bins, entries, dcn);
+      count();
+      MSDA_CUDA(cudaGetLastError());
+      if (int s2 = src.dcn ? bwd_dcn_noscatter(st, d, dtype, grad_output, value, sampling_loc, attn_weight,
+                                               grad_sampling_loc, grad_attn_weight, dcn)
+                           : bwd_fast_noscatter(st, d, dtype, grad_output, value, spatial_shapes, level_start_index,
+                                                sampling_loc, attn_weight, grad_sampling_loc, grad_attn_weight))
+        return s2;
+    } else if (amax_in_emit) {
+      // the kernel leaves two maxima per warp; reducing those short arrays replaces the sweeps over grad_out / weights
+      float* wamax = reinterpret_cast<float*>(ws + lay.off_wamax);
+      int64_t n_warps = 0;
+      if (int s2 = emit(wamax, &n_warps)) return s2;
+      const int g_w = grid_for(n_warps, 256, 148 * 8);
+      msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax, n_warps, amax);
+      count();
+      msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax + n_warps, n_warps, amax + 1);
+      count();
+      msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, 38);   // sorted route: float / bf16 / f16 only
+      count();
+      MSDA_CUDA(cudaGetLastError());
+    } else if (int s2 = emit(nullptr, nullptr)) {
+      return s2;
+    }
+    if (!det_dense(d)) {
+      if (dtype == MSDA_F32)
+        return det_gather<float>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
+      if (dtype == MSDA_BF16)
+        return det_gather<__nv_bfloat16>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale,
+                                         grad_value);
+      return det_gather<__half>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
+    }
+    int s3;
+    if (dtype == MSDA_F32)
+      s3 = det_cell_reduce<float>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale, acc);
+    else if (dtype == MSDA_BF16)
+      s3 = det_cell_reduce<__nv_bfloat16>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index,
+                                          scale, acc);
+    else
+      s3 = det_cell_reduce<__half>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale,
+                                   acc);
+    if (s3 != MSDA_OK) return s3;
+    const int g_fin = grid_for(nv, 256, 148 * 16);
+    const long long* sacc = reinterpret_cast<const long long*>(acc);
+    if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_fin, 256, 0, st>>>(sacc, (float*)grad_value, nv, scale);
+    else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_fin, 256, 0, st>>>(sacc, (__nv_bfloat16*)grad_value, nv, scale);
+    else msda::msda_det_finalize_kernel<__half><<<g_fin, 256, 0, st>>>(sacc, (__half*)grad_value, nv, scale);
+    count();
+    MSDA_CUDA(cudaGetLastError());
+    return MSDA_OK;
+  }
+  int s;
+  if (src.dcn)
+    s = bwd_dcn_det(st, d, dtype, grad_output, value, sampling_loc, attn_weight, acc, grad_sampling_loc,
+                    grad_attn_weight, scale, dcn);
+  else if (fast_ok(d, dtype, flags))
+    s = bwd_fast_det(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_loc, attn_weight,
+                     acc, grad_sampling_loc, grad_attn_weight, scale);
+  else if (dtype == MSDA_F32)
+    s = bwd_generic<float, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
+                                                      sampling_loc, attn_weight, acc, grad_sampling_loc,
+                                                      grad_attn_weight, scale);
+  else if (dtype == MSDA_F64)
+    s = bwd_generic<double, double, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
+                                                        sampling_loc, attn_weight, acc, grad_sampling_loc,
+                                                        grad_attn_weight, scale);
+  else if (dtype == MSDA_BF16)
+    s = bwd_generic<__nv_bfloat16, float, unsigned long long>(st, d, grad_output, value, spatial_shapes,
+                                                              level_start_index, sampling_loc, attn_weight, acc,
+                                                              grad_sampling_loc, grad_attn_weight, scale);
+  else
+    s = bwd_generic<__half, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
+                                                       sampling_loc, attn_weight, acc, grad_sampling_loc,
+                                                       grad_attn_weight, scale);
+  if (s != MSDA_OK) return s;
+  const int g_val = grid_for(nv, 256, 148 * 16);
+  const long long* cacc = reinterpret_cast<const long long*>(acc);
+  if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_val, 256, 0, st>>>(cacc, (float*)grad_value, nv, scale);
+  else if (dtype == MSDA_F64) msda::msda_det_finalize_kernel<double><<<g_val, 256, 0, st>>>(cacc, (double*)grad_value, nv, scale);
+  else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_val, 256, 0, st>>>(cacc, (__nv_bfloat16*)grad_value, nv, scale);
+  else msda::msda_det_finalize_kernel<__half><<<g_val, 256, 0, st>>>(cacc, (__half*)grad_value, nv, scale);
+  count();
+  MSDA_CUDA(cudaGetLastError());
+  return MSDA_OK;
+}
+
 }  // namespace
 
 // ============================================================================================
@@ -406,152 +589,10 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
                                                     num_point, dtype, flags);
   if (need && (!workspace || workspace_bytes < need))
     return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
-  auto count = [] { count_launch(); };
-
   if (det) {
-    // ---- bit-reproducible grad_value: 64-bit fixed-point accumulation (see include/msda.h) ----
-    const int64_t nv = d.n_value(), n_out = d.rows() * d.D, n_pts = d.n_points();
-    const bool sorted = det_sorted_ok(d, dtype, flags);
-    const DetLayout lay = sorted ? det_layout(d) : DetLayout{};
-    char* ws = static_cast<char*>(workspace);
-    auto* acc = reinterpret_cast<unsigned long long*>(ws + (sorted ? lay.off_acc : 0));
-    auto* amax = reinterpret_cast<unsigned*>(ws + (sorted ? lay.off_misc : (size_t)nv * 8));
-    auto* scale = reinterpret_cast<msda::DetScale*>(reinterpret_cast<char*>(amax) + 16);
-    if (sorted) {   // zero the bins, cursors, {amax, scale} and the accumulators; entries are fully overwritten
-      MSDA_CUDA(cudaMemsetAsync(ws, 0, lay.off_sums, st));
-      MSDA_CUDA(cudaMemsetAsync(ws + lay.off_misc, 0, lay.total - lay.off_misc, st));
-    } else {
-      MSDA_CUDA(cudaMemsetAsync(workspace, 0, need, st));
-    }
-    // The fixed-point scale comes from max |grad_out| x max |weight|.  On the sorted route the backward kernel that
-    // files the entries reads both tensors anyway and takes the two maxima itself (EmitArgs::amax); the scale is only
-    // needed by the reduction that follows it.  Every other route scatters with the scale and takes them up front.
-#ifndef MSDA_DET_AMAX_IN_EMIT
-#define MSDA_DET_AMAX_IN_EMIT 1
-#endif
-    const bool amax_in_emit = MSDA_DET_AMAX_IN_EMIT && sorted && !(flags & MSDA_FLAG_DET_SEPARATE_FILL);
-    const int g_out = grid_for(n_out, 256, 148 * 8), g_pts = grid_for(n_pts, 256, 148 * 8);
-    if (!amax_in_emit) {
-      if (dtype == MSDA_F32) msda::msda_amax_kernel<float><<<g_out, 256, 0, st>>>((const float*)grad_output, n_out, amax);
-      else if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_out, 256, 0, st>>>((const double*)grad_output, n_out, amax);
-      else if (dtype == MSDA_BF16) msda::msda_amax_kernel<__nv_bfloat16><<<g_out, 256, 0, st>>>((const __nv_bfloat16*)grad_output, n_out, amax);
-      else msda::msda_amax_kernel<__half><<<g_out, 256, 0, st>>>((const __half*)grad_output, n_out, amax);
-      count();
-      if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_pts, 256, 0, st>>>((const double*)attn_weight, n_pts, amax + 1);
-      else msda::msda_amax_kernel<float><<<g_pts, 256, 0, st>>>((const float*)attn_weight, n_pts, amax + 1);
-      count();
-      msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, dtype == MSDA_F64 ? 44 : 38);
-      count();
-      MSDA_CUDA(cudaGetLastError());
-    }
-    if (sorted) {
-      // sorted segment reduction (msda_det.cuh): count -> scan -> fill -> gather; no atomics on grad_value
-      int* bins = reinterpret_cast<int*>(ws);
-      int* cursor = reinterpret_cast<int*>(ws + lay.off_cursor);
-      int* sums = reinterpret_cast<int*>(ws + lay.off_sums);
-      int4* entries = reinterpret_cast<int4*>(ws + lay.off_entries);
-      const float* loc = static_cast<const float*>(sampling_loc);
-      const float* w = static_cast<const float*>(attn_weight);
-      const int g_bin = grid_for(n_pts, 256, 148 * 32);
-      msda::det_bin_kernel<false><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H, d.L, d.Q, d.P,
-                                                         n_pts, bins, nullptr, nullptr);
-      count();
-      msda::det_scan_block_kernel<<<(unsigned)lay.scan_blocks, 256, 0, st>>>(bins, bins, sums, lay.n_scan);
-      count();
-      msda::det_scan_sums_kernel<<<1, 1024, 0, st>>>(sums, (int)lay.scan_blocks);
-      count();
-      msda::det_scan_add_kernel<<<(unsigned)lay.scan_blocks, 256, 0, st>>>(bins, sums, lay.n_scan);
-      count();
-      MSDA_CUDA(cudaGetLastError());
-      // entries are filed by the backward kernel itself (ACC = EmitEntries): the lane that has just built a point's
-      // record takes the cursor atomic and writes the 16-byte entry, so the separate fill pass (det_bin_kernel<true>:
-      // re-read of every location / weight + the coordinate arithmetic a second time) is gone
-      if (flags & MSDA_FLAG_DET_SEPARATE_FILL) {
-        msda::det_bin_kernel<true><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H, d.L, d.Q, d.P,
-                                                          n_pts, cursor, bins, entries);
-        count();
-        MSDA_CUDA(cudaGetLastError());
-        if (int s2 = bwd_fast_noscatter(st, d, dtype, grad_output, value, spatial_shapes, level_start_index,
-                                        sampling_loc, attn_weight, grad_sampling_loc, grad_attn_weight))
-          return s2;
-      } else if (amax_in_emit) {
-        // the kernel leaves two maxima per warp; reducing those short arrays replaces the sweeps over grad_out / weights
-        float* wamax = reinterpret_cast<float*>(ws + lay.off_wamax);
-        int64_t n_warps = 0;
-        if (int s2 = bwd_fast_emit(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
-                                   attn_weight, grad_sampling_loc, grad_attn_weight, cursor, bins, entries, wamax,
-                                   &n_warps))
-          return s2;
-        const int g_w = grid_for(n_warps, 256, 148 * 8);
-        msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax, n_warps, amax);
-        count();
-        msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax + n_warps, n_warps, amax + 1);
-        count();
-        msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, 38);   // sorted route: float / bf16 / f16 only
-        count();
-        MSDA_CUDA(cudaGetLastError());
-      } else if (int s2 = bwd_fast_emit(st, d, dtype, grad_output, value, spatial_shapes, level_start_index,
-                                        sampling_loc, attn_weight, grad_sampling_loc, grad_attn_weight, cursor, bins,
-                                        entries, nullptr, nullptr)) {
-        return s2;
-      }
-      if (!det_dense(d)) {
-        if (dtype == MSDA_F32)
-          return det_gather<float>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
-        if (dtype == MSDA_BF16)
-          return det_gather<__nv_bfloat16>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale,
-                                           grad_value);
-        return det_gather<__half>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
-      }
-      int s3;
-      if (dtype == MSDA_F32)
-        s3 = det_cell_reduce<float>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale, acc);
-      else if (dtype == MSDA_BF16)
-        s3 = det_cell_reduce<__nv_bfloat16>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index,
-                                            scale, acc);
-      else
-        s3 = det_cell_reduce<__half>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale,
-                                     acc);
-      if (s3 != MSDA_OK) return s3;
-      const int g_fin = grid_for(nv, 256, 148 * 16);
-      const long long* sacc = reinterpret_cast<const long long*>(acc);
-      if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_fin, 256, 0, st>>>(sacc, (float*)grad_value, nv, scale);
-      else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_fin, 256, 0, st>>>(sacc, (__nv_bfloat16*)grad_value, nv, scale);
-      else msda::msda_det_finalize_kernel<__half><<<g_fin, 256, 0, st>>>(sacc, (__half*)grad_value, nv, scale);
-      count();
-      MSDA_CUDA(cudaGetLastError());
-      return MSDA_OK;
-    }
-    int s;
-    if (fast_ok(d, dtype, flags))
-      s = bwd_fast_det(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_loc, attn_weight,
-                       acc, grad_sampling_loc, grad_attn_weight, scale);
-    else if (dtype == MSDA_F32)
-      s = bwd_generic<float, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                        sampling_loc, attn_weight, acc, grad_sampling_loc,
-                                                        grad_attn_weight, scale);
-    else if (dtype == MSDA_F64)
-      s = bwd_generic<double, double, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                          sampling_loc, attn_weight, acc, grad_sampling_loc,
-                                                          grad_attn_weight, scale);
-    else if (dtype == MSDA_BF16)
-      s = bwd_generic<__nv_bfloat16, float, unsigned long long>(st, d, grad_output, value, spatial_shapes,
-                                                                level_start_index, sampling_loc, attn_weight, acc,
-                                                                grad_sampling_loc, grad_attn_weight, scale);
-    else
-      s = bwd_generic<__half, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                         sampling_loc, attn_weight, acc, grad_sampling_loc,
-                                                         grad_attn_weight, scale);
-    if (s != MSDA_OK) return s;
-    const int g_val = grid_for(nv, 256, 148 * 16);
-    const long long* cacc = reinterpret_cast<const long long*>(acc);
-    if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_val, 256, 0, st>>>(cacc, (float*)grad_value, nv, scale);
-    else if (dtype == MSDA_F64) msda::msda_det_finalize_kernel<double><<<g_val, 256, 0, st>>>(cacc, (double*)grad_value, nv, scale);
-    else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_val, 256, 0, st>>>(cacc, (__nv_bfloat16*)grad_value, nv, scale);
-    else msda::msda_det_finalize_kernel<__half><<<g_val, 256, 0, st>>>(cacc, (__half*)grad_value, nv, scale);
-    count();
-    MSDA_CUDA(cudaGetLastError());
-    return MSDA_OK;
+    const DetSource src{sampling_loc, attn_weight, spatial_shapes, level_start_index, nullptr};
+    return det_backward(st, d, dtype, flags, grad_output, value, src, grad_value, grad_sampling_loc, grad_attn_weight,
+                        workspace, need);
   }
 
   float* gv32 = static_cast<float*>(grad_value);
@@ -696,7 +737,27 @@ int dcn_setup(int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h,
   *fa = a;
   return MSDA_OK;
 }
+
+// the flags msda_dcnv3_backward honours; every other bit is ignored
+constexpr unsigned kDcnDetFlags = MSDA_FLAG_DETERMINISTIC | MSDA_FLAG_DET_ATOMIC | MSDA_FLAG_DET_SEPARATE_FILL;
+// deterministic workspace: the one-level table {H_in, W_in}, {0} (det_one_level_kernel) first, then the layout of the
+// equivalent one-level msda_backward problem
+constexpr size_t kDcnLevelSlot = 256;
 }  // namespace
+
+size_t msda_dcnv3_backward_workspace_bytes(int kernel_h, int kernel_w, int group, int group_channels, int batch,
+                                           int height_in, int width_in, int height_out, int width_out, int dtype,
+                                           unsigned flags) {
+  if (batch <= 0 || height_in <= 0 || width_in <= 0 || group <= 0 || group_channels <= 0) return 0;
+  const size_t n_value = (size_t)batch * height_in * width_in * group * group_channels;
+  // empty problems (no output pixel, no kernel point) need what they need without the flag
+  if ((flags & MSDA_FLAG_DETERMINISTIC) && height_out > 0 && width_out > 0 && kernel_h > 0 && kernel_w > 0)
+    return kDcnLevelSlot + msda_backward_workspace_bytes(batch, height_in * width_in, group, group_channels, 1,
+                                                         height_out * width_out, kernel_h * kernel_w, dtype,
+                                                         flags & kDcnDetFlags);
+  // bf16 / f16 grad_input is accumulated in float and converted at the end
+  return two_byte(dtype) ? n_value * sizeof(float) : 0;
+}
 
 int msda_dcnv3_forward(void* stream, const void* input, const float* offset, const float* mask, int kernel_h,
                        int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w,
@@ -729,13 +790,13 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
                         int height_in, int width_in, int height_out, int width_out, void* grad_input,
                         float* grad_offset, float* grad_mask, void* workspace, size_t workspace_bytes, int dtype,
                         unsigned flags) {
-  (void)flags;
   g_err[0] = 0;
   Dims d;
   msda::FusedArgs fa;
   if (int s = dcn_setup(kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
                         group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
     return s;
+  flags &= kDcnDetFlags;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (d.n_value() == 0 && d.n_points() == 0) return MSDA_OK;
   const void* anchor = d.n_value() ? grad_input : (const void*)grad_mask;
@@ -746,9 +807,26 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
     return s;
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(anchor));
-  const size_t need = two_byte(dtype) ? (size_t)d.n_value() * sizeof(float) : 0;
+  const size_t need = msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, batch, height_in,
+                                                          width_in, height_out, width_out, dtype, flags);
   if (need && (!workspace || workspace_bytes < need))
     return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if ((flags & MSDA_FLAG_DETERMINISTIC) && d.n_value() != 0 && d.n_points() != 0) {
+    // bit-reproducible grad_input: the deterministic backward of the equivalent one-level problem, which writes every
+    // element of grad_input in its own dtype (no float workspace, no zero-fill, no cast)
+    if (!grad_input || !grad_offset || !grad_mask || !grad_output || !input || !offset || !mask)
+      return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+    char* ws = static_cast<char*>(workspace);
+    int64_t* table = reinterpret_cast<int64_t*>(ws);
+    if (det_sorted_ok(d, dtype, flags)) {   // the count / gather / cell-reduce kernels read the level table
+      msda::det_one_level_kernel<<<1, 1, 0, st>>>(table, height_in, width_in);
+      count_launch();
+      MSDA_CUDA(cudaGetLastError());
+    }
+    const DetSource src{offset, mask, table, table + 2, &fa};
+    return det_backward(st, d, dtype, flags, grad_output, input, src, grad_input, grad_offset, grad_mask,
+                        ws + kDcnLevelSlot, need - kDcnLevelSlot);
+  }
   float* gi32 = two_byte(dtype) ? static_cast<float*>(workspace) : static_cast<float*>(grad_input);
   if (d.n_value()) {
     if (!grad_input) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_input is null");

@@ -96,11 +96,15 @@ __host__ __device__ __forceinline__ unsigned fastdiv(unsigned n, const FastDiv f
 }
 
 // FILL == false: count points per bin.  FILL == true: write entries (bins already scanned into `bin_start`).
-template <bool FILL>
+// PRE == kPreDcn: DCNv3 (L == 1, P == K, H == groups, Q == H_out * W_out): `loc` holds the offsets [N, Ho, Wo, G*K*2]
+// and `w` the mask; point pt = ((b*Q + q)*G + g)*K + k lands at dcn_location + locate_pixel -- the device functions
+// the DCN records of the backward kernel use, so this pass and the entry-filing backward agree on every cell.
+template <bool FILL, int PRE = kPrePlain>
 __global__ void __launch_bounds__(256)
 det_bin_kernel(const float* __restrict__ loc, const float* __restrict__ w, const int64_t* __restrict__ shapes,
                const int64_t* __restrict__ lsi, int H, int L, int Q, int P, int64_t n_points, int* __restrict__ counter,
-               const int* __restrict__ bin_start, int4* __restrict__ entries) {
+               const int* __restrict__ bin_start, int4* __restrict__ entries, const FusedArgs dcn) {
+  static_assert(PRE == kPrePlain || PRE == kPreDcn, "plain or DCNv3 points");
   __shared__ CellTab tab;
   __shared__ FastDiv div[4];   // by NP, P, H, Q
   const int NP = L * P;
@@ -118,7 +122,13 @@ det_bin_kernel(const float* __restrict__ loc, const float* __restrict__ w, const
     const int h = (int)(row - bq * (unsigned)H);
     const int64_t b = fastdiv(bq, dQ);
     const float2 xy = __ldg(reinterpret_cast<const float2*>(loc) + pt);
-    const Cell<float> c = locate<float>(xy.x, xy.y, tab.H[l], tab.W[l]);
+    Cell<float> c;
+    if constexpr (PRE == kPreDcn) {   // NP == P == K: l == 0, k = p32 - row * K
+      const float2 px = dcn_location(xy, (int)(p32 - row * (unsigned)NP), (int)(bq - (unsigned)b * (unsigned)Q), dcn);
+      c = locate_pixel(px.x, px.y, tab.H[0], tab.W[0]);
+    } else {
+      c = locate<float>(xy.x, xy.y, tab.H[l], tab.W[l]);
+    }
     if (c.valid == 0u) continue;
     const int64_t bin = (b * H + h) * (int64_t)tab.cells_per_bh + tab.cell_begin[l] + (c.y0 + 1) * (tab.W[l] + 1) + (c.x0 + 1);
     if (!FILL) {
@@ -128,6 +138,15 @@ det_bin_kernel(const float* __restrict__ loc, const float* __restrict__ w, const
       entries[pos] = make_int4((int)row, __float_as_int(c.lw), __float_as_int(c.lh), __float_as_int(__ldg(w + pt)));
     }
   }
+}
+
+// DCNv3 has no spatial_shapes / level_start_index tensors, only H_in and W_in: one thread writes the one-level table
+// {H_in, W_in}, {0} into a slot of the caller's workspace, and the count / gather / cell-reduce kernels read it like the
+// plain operator's.  No host copy and no sync, so the call stays capturable in a CUDA graph.
+__global__ void det_one_level_kernel(int64_t* __restrict__ table, int H, int W) {
+  table[0] = H;
+  table[1] = W;
+  table[2] = 0;
 }
 
 // ---- exclusive scan of n ints, 2048 per block --------------------------------------------------------

@@ -329,8 +329,9 @@ __device__ __forceinline__ void load_levels_plain(LevelTab* tab, const int64_t* 
   __syncthreads();
 }
 
-// DCNv3: a single level whose shape comes with the call, not from device tensors
-template <int TW, int TH>
+// DCNv3: a single level whose shape comes with the call, not from device tensors.  CELLS: also the bin table of the
+// deterministic sorted path (one extended (H+1) x (W+1) grid).
+template <int TW, int TH, bool CELLS = false>
 __device__ __forceinline__ void set_single_level(LevelTab* tab, int H, int W) {
   if (threadIdx.x == 0) {
     tab->H[0] = H;
@@ -339,6 +340,10 @@ __device__ __forceinline__ void set_single_level(LevelTab* tab, int H, int W) {
     tab->tiles_x[0] = (W + TW - 1) / TW;
     tab->tile_begin[0] = 0;
     tab->total_tiles = tab->tiles_x[0] * ((H + TH - 1) / TH);
+    if constexpr (CELLS) {
+      tab->cell_begin[0] = 0;
+      tab->cells_per_bh = (H + 1) * (W + 1);
+    }
   }
   __syncthreads();
 }
@@ -958,7 +963,9 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
   // FUSED: loc = raw offsets, w = logits in; grad_loc = grad of the offsets, grad_w = grad of the logits out
   static_assert(THREADS <= 256, "single-pass CTAs");
   constexpr bool EMIT = sizeof(ACC) == sizeof(EmitEntries);
-  static_assert(!EMIT || (ORDER == 0 && PRE == kPrePlain), "entries are emitted by the plain LINEAR backward");
+  // LINEAR only: EmitArgs::warp_amax has one slot pair per warp of the LINEAR grid (bwd_fast_emit / bwd_dcn_emit)
+  static_assert(!EMIT || (ORDER == 0 && (PRE == kPrePlain || PRE == kPreDcn)),
+                "entries are emitted by the plain and DCNv3 LINEAR backward");
   constexpr int DL = D * 4 / CPL;
   using G = Geom<DL, THREADS>;
   constexpr int LANES = G::LANES;
@@ -1007,13 +1014,24 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
       early_sum = row_softmax<LANES, 4>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
     load_levels_plain<EMIT>(tab, shapes, lsi, L);
   } else {
-    if constexpr (DCN) set_single_level<G::TW, G::TH>(tab, fused.height_in, fused.width_in);
+    if constexpr (DCN) set_single_level<G::TW, G::TH, EMIT>(tab, fused.height_in, fused.width_in);
     else if constexpr (ORDER == 0 || ORDER == 2) load_levels_plain(tab, shapes, lsi, L);
     else load_levels<G::TW, G::TH>(tab, shapes, lsi, L);
     walk = RowWalk<DL, THREADS, ORDER>(tab, B, H, rows);
     if (walk.done()) return;
     cur = walk.get(tab, L, H, Q);
   }
+  // file a point's entry under the bin of its cell (cells of the extended grid, det_bin_kernel's index exactly)
+  auto emit_entry = [&](const Cell<float> c, int l, float aw) {
+    const int bin = (cur.b * H + cur.h) * tab->cells_per_bh + tab->cell_begin[l] + (c.y0 + 1) * (tab->W[l] + 1) +
+                    (c.x0 + 1);
+    const int pos = __ldg(emit.bin_start + bin) + atomicAdd(emit.cursor + bin, 1);
+#ifdef MSDA_DEBUG_BOUNDS   // the count pass must have counted this point in this very bin
+    MSDA_CHECK_OFFSET(pos - __ldg(emit.bin_start + bin), __ldg(emit.bin_start + bin + 1) - __ldg(emit.bin_start + bin),
+                      "emit entry");
+#endif
+    emit.entries[pos] = make_int4((int)cur.row, __float_as_int(c.lw), __float_as_int(c.lh), __float_as_int(aw));
+  };
   while (true) {
     if constexpr (!EARLY) go = cur.live ? ldv<CPL>(grad_out + cur.row * D + sub * CPL) : vzero<CPL>();
     const float* rp = FUSED ? fused.ref + (cur.row / H) * (int64_t)L * fused.ref_dim : nullptr;
@@ -1036,16 +1054,15 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
           PointRec r;
           if constexpr (DCN) {
             const float2 px = dcn_location(xy, pt, (int)((cur.row / H) % Q), fused);
-            r = record_from_cell(locate_pixel(px.x, px.y, tab->H[0], tab->W[0]), aw, tab->W[0], 0, H, cur.h, D);
+            const Cell<float> c = locate_pixel(px.x, px.y, tab->H[0], tab->W[0]);
+            r = record_from_cell(c, aw, tab->W[0], 0, H, cur.h, D);
+            if constexpr (EMIT) {
+              if (c.valid != 0u) emit_entry(c, 0, aw);
+            }
           } else if constexpr (EMIT) {
             const Cell<float> c = locate<float>(xy.x, xy.y, tab->H[l], tab->W[l]);
             r = record_from_cell(c, aw, tab->W[l], tab->start[l], H, cur.h, D);
-            if (c.valid != 0u) {   // same bin index as det_bin_kernel (msda_det.cuh): cells of the extended grid
-              const int bin = (cur.b * H + cur.h) * tab->cells_per_bh + tab->cell_begin[l] +
-                              (c.y0 + 1) * (tab->W[l] + 1) + (c.x0 + 1);
-              const int pos = __ldg(emit.bin_start + bin) + atomicAdd(emit.cursor + bin, 1);
-              emit.entries[pos] = make_int4((int)cur.row, __float_as_int(c.lw), __float_as_int(c.lh), __float_as_int(aw));
-            }
+            if (c.valid != 0u) emit_entry(c, l, aw);
           } else {
             r = make_record(xy.x, xy.y, aw, tab->H[l], tab->W[l], tab->start[l], H, cur.h, D);
           }

@@ -93,6 +93,15 @@ int bwd_fused_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* g
                         void* glog, msda::FusedArgs fa);
 int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
             const void* mask, float* gi, void* goff, void* gmask, msda::FusedArgs fa);
+// DCNv3 twins of bwd_fast_det / bwd_fast_noscatter / bwd_fast_emit (deterministic grad_input)
+int bwd_dcn_det(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                const void* mask, unsigned long long* acc, void* goff, void* gmask, const msda::DetScale* det,
+                msda::FusedArgs fa);
+int bwd_dcn_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                      const void* mask, void* goff, void* gmask, msda::FusedArgs fa);
+int bwd_dcn_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                 const void* mask, void* goff, void* gmask, int* cursor, const int* bin_start, void* entries,
+                 float* warp_amax, int64_t* n_warps, msda::FusedArgs fa);
 
 // ---- msda_fold.cu ----
 // does the folding backward cover this problem (encoder form Q == S, shapes it is instantiated for, flags)?

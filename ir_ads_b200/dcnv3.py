@@ -24,6 +24,7 @@ from torch.autograd import Function
 from torch.autograd.function import once_differentiable
 
 from . import _lib
+from . import functional
 from .functional import _aligned, _ptr, _require
 
 _DCN_TAG = {torch.float32: _lib.MSDA_F32, torch.bfloat16: _lib.MSDA_BF16, torch.float16: _lib.MSDA_F16}
@@ -37,6 +38,8 @@ def _declare(handle):
     handle.msda_dcnv3_forward.argtypes = [vp, vp, vp, vp] + [i] * 10 + [f] + [i] * 5 + [vp, i, u]
     handle.msda_dcnv3_backward.restype = i
     handle.msda_dcnv3_backward.argtypes = [vp, vp, vp, vp, vp] + [i] * 10 + [f] + [i] * 5 + [vp, vp, vp, vp, sz, i, u]
+    handle.msda_dcnv3_backward_workspace_bytes.restype = sz
+    handle.msda_dcnv3_backward_workspace_bytes.argtypes = [i] * 10 + [u]
     handle._dcn_declared = True
     return handle
 
@@ -78,7 +81,9 @@ def dcnv3_forward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, p
 def dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
                    group, group_channels, offset_scale, grad_output, im2col_step=256) -> List[torch.Tensor]:
     """``detrex._C.dcnv3_backward``: ``[grad_input, grad_offset, grad_mask]``, each in the dtype of its input (the
-    offset / mask gradients are computed in float32)."""
+    offset / mask gradients are computed in float32).  Under ``set_deterministic(True)`` or
+    ``torch.use_deterministic_algorithms(True)`` grad_input is bit-reproducible (MSDA_FLAG_DETERMINISTIC); grad_offset
+    and grad_mask are the same bits either way."""
     N, H_in, W_in, H_out, W_out = _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels)
     _require(grad_output.is_cuda and grad_output.dtype == input.dtype, "grad_output must match input's device / dtype")
     grad_output = _aligned(grad_output.contiguous())
@@ -87,14 +92,18 @@ def dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, 
     grad_input = torch.empty_like(input)
     grad_offset = torch.empty_like(offset)
     grad_mask = torch.empty_like(mask)
-    ws_bytes = input.numel() * 4 if input.dtype != torch.float32 else 0   # bf16 / f16: float accumulation buffer
+    flags = functional._flags(True)
+    tag = _DCN_TAG[input.dtype]
+    handle = _declare(_lib.lib())
+    ws_bytes = handle.msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, N, H_in, W_in,
+                                                          H_out, W_out, tag, flags)
     ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=input.device) if ws_bytes else None
     stream = torch.cuda.current_stream(input.device).cuda_stream
-    status = _declare(_lib.lib()).msda_dcnv3_backward(
+    status = handle.msda_dcnv3_backward(
         ctypes.c_void_p(stream), _ptr(grad_output), _ptr(input), _ptr(offset), _ptr(mask), kernel_h, kernel_w,
         stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels, float(offset_scale), N, H_in,
         W_in, H_out, W_out, _ptr(grad_input), _ptr(grad_offset), _ptr(grad_mask),
-        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, _DCN_TAG[input.dtype], 0)
+        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, flags)
     _lib.check(status, "dcnv3_backward")
     return [grad_input, grad_offset.to(off_dtype), grad_mask.to(mask_dtype)]
 
