@@ -232,6 +232,38 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
                         unsigned flags);
 
 /*
+ * Fused DCNv3 module path (an extension; the reference has no counterpart): the DCNv3 module's mask softmax
+ * (dcn_v3.py:476, softmax over the K points of every (output pixel, group)) runs inside the kernels, so the mask and
+ * its gradient never exist in HBM.  Arguments, layouts, geometry, supported shapes and dtypes are those of
+ * msda_dcnv3_forward / msda_dcnv3_backward, with
+ *   mask_logits       [N, H_out, W_out, group*K] float  the raw output of the module's mask Linear (pre-softmax)
+ *   grad_mask_logits  [N, H_out, W_out, group*K] float  its gradient (fully written by the library)
+ * in place of mask / grad_mask.  The result equals msda_dcnv3_forward / _backward called with
+ * mask = softmax(mask_logits) over each row of K, followed by the softmax's chain rule
+ * grad_logit_i = w_i * (grad_mask_i - sum_j grad_mask_j * w_j), up to float rounding of the softmax.  Non-finite
+ * logits behave as in torch.softmax: a -inf logit gets weight 0 (and gradient 0) while the rest of its row is
+ * normalised as usual; a row whose logits are all -inf, or that holds +inf or NaN, has NaN weights: its logits'
+ * gradient is NaN, and so are its output pixel and its grad_offset / grad_input contributions wherever one of its
+ * points samples inside the map (exactly what msda_dcnv3_* make of torch.softmax's NaN row).
+ * Backward uses the workspace rule of msda_dcnv3_backward_workspace_bytes with flags 0 (float reds).  It has no
+ * deterministic form: with MSDA_FLAG_DETERMINISTIC it returns MSDA_ERR_UNSUPPORTED before any device work (compose
+ * the softmax around msda_dcnv3_backward instead, whose grad_input is bit-reproducible).  Every other flag bit is
+ * ignored by both entry points.  Added in ABI 3 without a version bump: an older library lacks the two symbols.
+ */
+int msda_dcnv3_fused_forward(void* stream, const void* input, const float* offset, const float* mask_logits,
+                             int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                             int dilation_h, int dilation_w, int group, int group_channels, float offset_scale,
+                             int batch, int height_in, int width_in, int height_out, int width_out,
+                             void* output, int dtype, unsigned flags);
+int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void* input, const float* offset,
+                              const float* mask_logits, int kernel_h, int kernel_w, int stride_h, int stride_w,
+                              int pad_h, int pad_w, int dilation_h, int dilation_w, int group,
+                              int group_channels, float offset_scale, int batch, int height_in, int width_in,
+                              int height_out, int width_out, void* grad_input, float* grad_offset,
+                              float* grad_mask_logits, void* workspace, size_t workspace_bytes, int dtype,
+                              unsigned flags);
+
+/*
  * Fused residual add + LayerNorm (SURVEY.md section 8f-2): the epilogue that follows every MSDeformAttn call and every
  * FFN in the reference's transformer layers -- x = x + identity; x = norm(x)
  * (/root/reference/detrex/layers/transformer.py:152-192; the residuals are added at multi_scale_deform_attn.py:363 and

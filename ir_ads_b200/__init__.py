@@ -13,7 +13,7 @@ from .functional import (  # noqa: F401
     multi_scale_deformable_attn_pytorch,
     set_deterministic,
 )
-from .dcnv3 import DCNv3Function, dcnv3_backward, dcnv3_forward  # noqa: F401
+from .dcnv3 import DCNv3FusedFunction, DCNv3Function, dcnv3_backward, dcnv3_forward  # noqa: F401
 from .module import MultiScaleDeformableAttention  # noqa: F401
 
 __all__ = [
@@ -25,6 +25,7 @@ __all__ = [
     "set_deterministic",
     "kernel_flags",
     "DCNv3Function",
+    "DCNv3FusedFunction",
     "dcnv3_forward",
     "dcnv3_backward",
 ]

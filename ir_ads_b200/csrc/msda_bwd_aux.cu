@@ -60,6 +60,10 @@ int bwd_dcn(cudaStream_t, const Dims&, int, const void*, const void*, const void
             msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
 }
+int bwd_dcn_softmax(cudaStream_t, const Dims&, int, const void*, const void*, const void*, const void*, float*, void*,
+                    void*, msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
+}
 int bwd_dcn_det(cudaStream_t, const Dims&, int, const void*, const void*, const void*, const void*,
                 unsigned long long*, void*, void*, const msda::DetScale*, msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
@@ -99,12 +103,14 @@ int bwd_fused_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* g
 #undef MSDA_DISPATCH_ORDER
 }
 
-// DCNv3: runtime point count, STRIP order
-int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
-            const void* mask, float* gi, void* goff, void* gmask, msda::FusedArgs fa) {
-#define CALL_DB(D_, VT_)                                                                                           \
-  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, float, msda::kPreDcn>(st, d, go, input, nullptr, nullptr, off, mask, gi, \
-                                                                    goff, gmask, nullptr, fa)
+// DCNv3: runtime point count, STRIP order.  PRE: kPreDcn (w = mask, gw = its gradient) or kPreDcnSoftmax (w = mask
+// logits, gw = the logits' gradient)
+template <int PRE>
+int bwd_dcn_pre(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                const void* w, float* gi, void* goff, void* gw, msda::FusedArgs fa) {
+#define CALL_DB(D_, VT_)                                                                                             \
+  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, float, PRE>(st, d, go, input, nullptr, nullptr, off, w, gi, goff, gw, \
+                                                          nullptr, fa)
 #define DCN_D(VT_)                                                                         \
   switch (d.D) {                                                                           \
     case 16: return CALL_DB(16, VT_);                                                      \
@@ -119,6 +125,17 @@ int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const voi
   return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
 #undef DCN_D
 #undef CALL_DB
+}
+
+int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+            const void* mask, float* gi, void* goff, void* gmask, msda::FusedArgs fa) {
+  return bwd_dcn_pre<msda::kPreDcn>(st, d, dtype, go, input, off, mask, gi, goff, gmask, fa);
+}
+
+// fused DCNv3 module path: the softmax's chain rule runs in the kernel, which writes the mask logits' gradient
+int bwd_dcn_softmax(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                    const void* mask_logits, float* gi, void* goff, void* glogits, msda::FusedArgs fa) {
+  return bwd_dcn_pre<msda::kPreDcnSoftmax>(st, d, dtype, go, input, off, mask_logits, gi, goff, glogits, fa);
 }
 
 // the DCNv3 twins of the deterministic backward kernels above, dispatched over group_channels and dtype

@@ -759,6 +759,87 @@ size_t msda_dcnv3_backward_workspace_bytes(int kernel_h, int kernel_w, int group
   return two_byte(dtype) ? n_value * sizeof(float) : 0;
 }
 
+namespace {
+// The body of msda_dcnv3_forward (softmax false: `w` = mask) and msda_dcnv3_fused_forward (softmax true: `w` = mask
+// logits), after dcn_setup.
+int dcn_forward(void* stream, const Dims& d, const msda::FusedArgs& fa, const void* input, const float* offset,
+                const float* w, void* output, int dtype, bool softmax) {
+  if (d.rows() * d.D == 0) return MSDA_OK;
+  if (!output) return fail(MSDA_ERR_INVALID_ARGUMENT, "output is null");
+  if (int s = check_alignment({{"input", input}, {"offset", offset}, {softmax ? "mask_logits" : "mask", w},
+                               {"output", output}}))
+    return s;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  DeviceGuard guard;
+  MSDA_CUDA(guard.enter(output));
+  if (d.S == 0) {
+    MSDA_CUDA(cudaMemsetAsync(output, 0, (size_t)(d.rows() * d.D) * elem_size(dtype), st));
+    return MSDA_OK;
+  }
+  if (!input || !offset || !w) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  return softmax ? fwd_dcn_softmax(st, d, dtype, input, offset, w, output, fa)
+                 : fwd_dcn(st, d, dtype, input, offset, w, output, fa);
+}
+
+// The body of msda_dcnv3_backward (softmax false: `w` = mask, grad_w = its gradient) and msda_dcnv3_fused_backward
+// (softmax true: `w` = mask logits, grad_w = their gradient; never with MSDA_FLAG_DETERMINISTIC), after dcn_setup.
+// `need` = msda_dcnv3_backward_workspace_bytes of the problem and flags.
+int dcn_backward(void* stream, const Dims& d, const msda::FusedArgs& fa, const void* grad_output, const void* input,
+                 const float* offset, const float* w, void* grad_input, float* grad_offset, float* grad_w,
+                 void* workspace, size_t workspace_bytes, size_t need, int dtype, unsigned flags, bool softmax) {
+  const char* w_name = softmax ? "mask_logits" : "mask";
+  const char* gw_name = softmax ? "grad_mask_logits" : "grad_mask";
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (d.n_value() == 0 && d.n_points() == 0) return MSDA_OK;
+  const void* anchor = d.n_value() ? grad_input : (const void*)grad_w;
+  if (!anchor) return fail(MSDA_ERR_INVALID_ARGUMENT, "gradient output pointer is null");
+  if (int s = check_alignment({{"grad_output", grad_output}, {"input", input}, {"offset", offset}, {w_name, w},
+                               {"grad_input", grad_input}, {"grad_offset", grad_offset}, {gw_name, grad_w},
+                               {"workspace", workspace}}))
+    return s;
+  DeviceGuard guard;
+  MSDA_CUDA(guard.enter(anchor));
+  if (need && (!workspace || workspace_bytes < need))
+    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if ((flags & MSDA_FLAG_DETERMINISTIC) && d.n_value() != 0 && d.n_points() != 0) {
+    // bit-reproducible grad_input: the deterministic backward of the equivalent one-level problem, which writes every
+    // element of grad_input in its own dtype (no float workspace, no zero-fill, no cast)
+    if (!grad_input || !grad_offset || !grad_w || !grad_output || !input || !offset || !w)
+      return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+    char* ws = static_cast<char*>(workspace);
+    int64_t* table = reinterpret_cast<int64_t*>(ws);
+    if (det_sorted_ok(d, dtype, flags)) {   // the count / gather / cell-reduce kernels read the level table
+      msda::det_one_level_kernel<<<1, 1, 0, st>>>(table, fa.height_in, fa.width_in);
+      count_launch();
+      MSDA_CUDA(cudaGetLastError());
+    }
+    const DetSource src{offset, w, table, table + 2, &fa};
+    return det_backward(st, d, dtype, flags, grad_output, input, src, grad_input, grad_offset, grad_w,
+                        ws + kDcnLevelSlot, need - kDcnLevelSlot);
+  }
+  float* gi32 = two_byte(dtype) ? static_cast<float*>(workspace) : static_cast<float*>(grad_input);
+  if (d.n_value()) {
+    if (!grad_input) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_input is null");
+    MSDA_CUDA(cudaMemsetAsync(gi32, 0, (size_t)d.n_value() * sizeof(float), st));
+    if (two_byte(dtype) && d.n_points() == 0)
+      MSDA_CUDA(cudaMemsetAsync(grad_input, 0, (size_t)d.n_value() * 2, st));
+  }
+  if (d.n_points() == 0) return MSDA_OK;
+  if (!grad_offset || !grad_w) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_offset / %s is null", gw_name);
+  if (d.n_value() == 0) {   // nothing to sample: the output does not depend on the offsets or the mask (or its logits)
+    MSDA_CUDA(cudaMemsetAsync(grad_offset, 0, (size_t)d.n_points() * 2 * sizeof(float), st));
+    MSDA_CUDA(cudaMemsetAsync(grad_w, 0, (size_t)d.n_points() * sizeof(float), st));
+    return MSDA_OK;
+  }
+  if (!grad_output || !input || !offset || !w) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  if (int s = softmax ? bwd_dcn_softmax(st, d, dtype, grad_output, input, offset, w, gi32, grad_offset, grad_w, fa)
+                      : bwd_dcn(st, d, dtype, grad_output, input, offset, w, gi32, grad_offset, grad_w, fa))
+    return s;
+  if (two_byte(dtype)) return cast_from_f32(st, gi32, grad_input, d.n_value(), dtype);
+  return MSDA_OK;
+}
+}  // namespace
+
 int msda_dcnv3_forward(void* stream, const void* input, const float* offset, const float* mask, int kernel_h,
                        int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w,
                        int group, int group_channels, float offset_scale, int batch, int height_in, int width_in,
@@ -770,18 +851,7 @@ int msda_dcnv3_forward(void* stream, const void* input, const float* offset, con
   if (int s = dcn_setup(kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
                         group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
     return s;
-  if (d.rows() * d.D == 0) return MSDA_OK;
-  if (!output) return fail(MSDA_ERR_INVALID_ARGUMENT, "output is null");
-  if (int s = check_alignment({{"input", input}, {"offset", offset}, {"mask", mask}, {"output", output}})) return s;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  DeviceGuard guard;
-  MSDA_CUDA(guard.enter(output));
-  if (d.S == 0) {
-    MSDA_CUDA(cudaMemsetAsync(output, 0, (size_t)(d.rows() * d.D) * elem_size(dtype), st));
-    return MSDA_OK;
-  }
-  if (!input || !offset || !mask) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
-  return fwd_dcn(st, d, dtype, input, offset, mask, output, fa);
+  return dcn_forward(stream, d, fa, input, offset, mask, output, dtype, false);
 }
 
 int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input, const float* offset,
@@ -797,54 +867,47 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
                         group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
     return s;
   flags &= kDcnDetFlags;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (d.n_value() == 0 && d.n_points() == 0) return MSDA_OK;
-  const void* anchor = d.n_value() ? grad_input : (const void*)grad_mask;
-  if (!anchor) return fail(MSDA_ERR_INVALID_ARGUMENT, "gradient output pointer is null");
-  if (int s = check_alignment({{"grad_output", grad_output}, {"input", input}, {"offset", offset}, {"mask", mask},
-                               {"grad_input", grad_input}, {"grad_offset", grad_offset}, {"grad_mask", grad_mask},
-                               {"workspace", workspace}}))
-    return s;
-  DeviceGuard guard;
-  MSDA_CUDA(guard.enter(anchor));
   const size_t need = msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, batch, height_in,
                                                           width_in, height_out, width_out, dtype, flags);
-  if (need && (!workspace || workspace_bytes < need))
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
-  if ((flags & MSDA_FLAG_DETERMINISTIC) && d.n_value() != 0 && d.n_points() != 0) {
-    // bit-reproducible grad_input: the deterministic backward of the equivalent one-level problem, which writes every
-    // element of grad_input in its own dtype (no float workspace, no zero-fill, no cast)
-    if (!grad_input || !grad_offset || !grad_mask || !grad_output || !input || !offset || !mask)
-      return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
-    char* ws = static_cast<char*>(workspace);
-    int64_t* table = reinterpret_cast<int64_t*>(ws);
-    if (det_sorted_ok(d, dtype, flags)) {   // the count / gather / cell-reduce kernels read the level table
-      msda::det_one_level_kernel<<<1, 1, 0, st>>>(table, height_in, width_in);
-      count_launch();
-      MSDA_CUDA(cudaGetLastError());
-    }
-    const DetSource src{offset, mask, table, table + 2, &fa};
-    return det_backward(st, d, dtype, flags, grad_output, input, src, grad_input, grad_offset, grad_mask,
-                        ws + kDcnLevelSlot, need - kDcnLevelSlot);
-  }
-  float* gi32 = two_byte(dtype) ? static_cast<float*>(workspace) : static_cast<float*>(grad_input);
-  if (d.n_value()) {
-    if (!grad_input) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_input is null");
-    MSDA_CUDA(cudaMemsetAsync(gi32, 0, (size_t)d.n_value() * sizeof(float), st));
-    if (two_byte(dtype) && d.n_points() == 0)
-      MSDA_CUDA(cudaMemsetAsync(grad_input, 0, (size_t)d.n_value() * 2, st));
-  }
-  if (d.n_points() == 0) return MSDA_OK;
-  if (!grad_offset || !grad_mask) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_offset / grad_mask is null");
-  if (d.n_value() == 0) {
-    MSDA_CUDA(cudaMemsetAsync(grad_offset, 0, (size_t)d.n_points() * 2 * sizeof(float), st));
-    MSDA_CUDA(cudaMemsetAsync(grad_mask, 0, (size_t)d.n_points() * sizeof(float), st));
-    return MSDA_OK;
-  }
-  if (!grad_output || !input || !offset || !mask) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
-  if (int s = bwd_dcn(st, d, dtype, grad_output, input, offset, mask, gi32, grad_offset, grad_mask, fa)) return s;
-  if (two_byte(dtype)) return cast_from_f32(st, gi32, grad_input, d.n_value(), dtype);
-  return MSDA_OK;
+  return dcn_backward(stream, d, fa, grad_output, input, offset, mask, grad_input, grad_offset, grad_mask, workspace,
+                      workspace_bytes, need, dtype, flags, false);
+}
+
+int msda_dcnv3_fused_forward(void* stream, const void* input, const float* offset, const float* mask_logits,
+                             int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
+                             int dilation_h, int dilation_w, int group, int group_channels, float offset_scale,
+                             int batch, int height_in, int width_in, int height_out, int width_out, void* output,
+                             int dtype, unsigned flags) {
+  (void)flags;
+  g_err[0] = 0;
+  Dims d;
+  msda::FusedArgs fa;
+  if (int s = dcn_setup(kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
+                        group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
+    return s;
+  return dcn_forward(stream, d, fa, input, offset, mask_logits, output, dtype, true);
+}
+
+int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void* input, const float* offset,
+                              const float* mask_logits, int kernel_h, int kernel_w, int stride_h, int stride_w,
+                              int pad_h, int pad_w, int dilation_h, int dilation_w, int group, int group_channels,
+                              float offset_scale, int batch, int height_in, int width_in, int height_out,
+                              int width_out, void* grad_input, float* grad_offset, float* grad_mask_logits,
+                              void* workspace, size_t workspace_bytes, int dtype, unsigned flags) {
+  g_err[0] = 0;
+  Dims d;
+  msda::FusedArgs fa;
+  if (int s = dcn_setup(kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
+                        group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
+    return s;
+  // the float-red kernel is the only fused form: a caller that needs bit-reproducible gradients composes the softmax
+  // around msda_dcnv3_backward (refused before any device work, empty problems included)
+  if (flags & MSDA_FLAG_DETERMINISTIC)
+    return fail(MSDA_ERR_UNSUPPORTED, "dcnv3 fused backward: no deterministic form (use msda_dcnv3_backward)");
+  const size_t need = msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, batch, height_in,
+                                                          width_in, height_out, width_out, dtype, 0u);
+  return dcn_backward(stream, d, fa, grad_output, input, offset, mask_logits, grad_input, grad_offset,
+                      grad_mask_logits, workspace, workspace_bytes, need, dtype, 0u, true);
 }
 
 int msda_debug_bookkeeping(void* stream, const float* sampling_loc, const int64_t* spatial_shapes,

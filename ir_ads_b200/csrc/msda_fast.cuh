@@ -529,13 +529,19 @@ struct FusedArgs {
   // group), the K = kernel_w*kernel_h points of a row sit at
   //   loc_w = p0_w - (dil_w*(kw-1)/2)*scale + (i*dil_w + offset_w)*scale   (pixel units, i outer, j inner)
   // `loc` holds the offsets [N, Ho, Wo, G*K*2], `w` the mask [N, Ho, Wo, G*K]; one level = the input map.
+  // PRE == 3 (fused DCNv3 module path): the same grid, `w` the mask LOGITS -- the DCNv3 module's softmax over the K
+  // points of a (pixel, group) row runs inside the kernels, as the fused MSDA chain's softmax over L*P does.
   int kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dil_h, dil_w;
   int height_in, width_in, width_out;
   float offset_scale;
 };
 // PRE: 0 = sampling_locations / attention_weights given (the reference operator), 1 = fused module chain,
-//      2 = DCNv3 sampling grid
-constexpr int kPrePlain = 0, kPreFused = 1, kPreDcn = 2;
+//      2 = DCNv3 sampling grid, 3 = DCNv3 sampling grid + softmax over the row's mask logits
+constexpr int kPrePlain = 0, kPreFused = 1, kPreDcn = 2, kPreDcnSoftmax = 3;
+// the record modes whose `w` holds logits: the row softmax in forward, its chain rule in backward
+__host__ __device__ constexpr bool pre_softmax(int pre) { return pre == kPreFused || pre == kPreDcnSoftmax; }
+// the record modes on the DCNv3 convolution grid
+__host__ __device__ constexpr bool pre_dcn(int pre) { return pre == kPreDcn || pre == kPreDcnSoftmax; }
 
 __device__ __forceinline__ float2 fused_location(const float2 off, const float* r, int ref_dim, int Hl, int Wl,
                                                  float num_P) {
@@ -642,8 +648,9 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
   // f16 rows sum the fused softmax in the f32 rows' lane order (row_softmax), so the f16 forward is the f32 forward
   // on the widened value; bf16 keeps its own order
   constexpr int SM_LANES = std::is_same_v<VT, __half> ? D / 4 : LANES;
-  constexpr bool FUSED = (PRE == kPreFused);
-  constexpr bool DCN = (PRE == kPreDcn);
+  constexpr bool SOFTMAX = pre_softmax(PRE);    // `w` holds logits: row softmax (fused MSDA chain, fused DCNv3)
+  constexpr bool FUSED = (PRE == kPreFused);    // MSDA chain only: location affine, reference points, padding mask
+  constexpr bool DCN = pre_dcn(PRE);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   LevelTab* tab = reinterpret_cast<LevelTab*>(smem_raw);
   float* recs = reinterpret_cast<float*>(smem_raw + sizeof(LevelTab));
@@ -671,11 +678,11 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
   // of the row are requested BEFORE the table's load + barrier: the two global-memory latencies of a CTA's
   // start-up overlap instead of adding up.
   // (FUSED: the raw offsets are requested and the row's softmax is done before the barrier.)
-  constexpr bool EARLY = (ORDER == 0 || ORDER == 2) && PRE != kPreDcn;
+  constexpr bool EARLY = (ORDER == 0 || ORDER == 2) && !DCN;
   constexpr int kEarly = 2;                              // row-loop iterations whose loads are issued early
   float2 early_xy[kEarly];
   float early_w[kEarly];
-  float early_sum = 1.0f;                                // FUSED: softmax denominator of the row
+  float early_sum = 1.0f;                                // SOFTMAX: softmax denominator of the row
   RowWalk<DL, THREADS, ORDER> walk;
   RowRef cur;
   if constexpr (EARLY) {
@@ -687,10 +694,10 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
       const int pt = sub + i * LANES;
       const bool on = cur.live && pt < NP;
       early_xy[i] = on ? __ldg(reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2) + pt) : make_float2(0.f, 0.f);
-      early_w[i] = (on && !FUSED) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
+      early_w[i] = (on && !SOFTMAX) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
     }
     // the softmax shuffles need the whole warp; dead rows read row 0 and simply produce nothing
-    if constexpr (FUSED) early_sum = row_softmax<LANES, 1, SM_LANES>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_oc), NP, sub);
+    if constexpr (SOFTMAX) early_sum = row_softmax<LANES, 1, SM_LANES>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_oc), NP, sub);
     load_levels_plain(tab, shapes, lsi, L);
   } else {
     if constexpr (DCN) set_single_level<G::TW, G::TH>(tab, fused.height_in, fused.width_in);
@@ -706,16 +713,16 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
       const float2* lp = reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2);
       const float* wp = w + cur.row * (int64_t)NP;
       float sm_sum = early_sum;
-      if constexpr (FUSED && !EARLY) sm_sum = row_softmax<LANES, 1, SM_LANES>(wp, reinterpret_cast<float*>(s_oc), NP, sub);
+      if constexpr (SOFTMAX && !EARLY) sm_sum = row_softmax<LANES, 1, SM_LANES>(wp, reinterpret_cast<float*>(s_oc), NP, sub);
       if (cur.live) {
         const float* rp = FUSED ? fused.ref + (cur.row / H) * (int64_t)L * fused.ref_dim : nullptr;
-        // one record from a point's raw location / weight (FUSED: raw offset; the weight comes from the softmax)
+        // one record from a point's raw location / weight (FUSED: raw offset; SOFTMAX: the weight comes from the
+        // softmax)
         auto build = [&](int pt, float2 xy, float aw) {
           const int l = level_of<PT>(pt, P);
-          if constexpr (FUSED) {
-            aw = __fdiv_rn(__int_as_float(s_oc[pt]), sm_sum);
+          if constexpr (SOFTMAX) aw = __fdiv_rn(__int_as_float(s_oc[pt]), sm_sum);
+          if constexpr (FUSED)
             xy = fused_location(xy, rp + l * fused.ref_dim, fused.ref_dim, tab->H[l], tab->W[l], fused.num_P);
-          }
           PointRec r;
           if constexpr (DCN) {
             const float2 px = dcn_location(xy, pt, (int)((cur.row / H) % Q), fused);
@@ -739,7 +746,7 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
           for (int i = 0; i < kEarly; ++i, pt += LANES)
             if (pt < NP) build(pt, early_xy[i], early_w[i]);
         }
-        for (; pt < NP; pt += LANES) build(pt, __ldg(lp + pt), FUSED ? 0.0f : __ldg(wp + pt));
+        for (; pt < NP; pt += LANES) build(pt, __ldg(lp + pt), SOFTMAX ? 0.0f : __ldg(wp + pt));
       }
     }
     __syncwarp();
@@ -966,11 +973,15 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
   // LINEAR only: EmitArgs::warp_amax has one slot pair per warp of the LINEAR grid (bwd_fast_emit / bwd_dcn_emit)
   static_assert(!EMIT || (ORDER == 0 && (PRE == kPrePlain || PRE == kPreDcn)),
                 "entries are emitted by the plain and DCNv3 LINEAR backward");
+  // the fused DCNv3 module path has no deterministic or no-scatter form (its deterministic backward is composed
+  // around the kPreDcn kernels, ir_ads_b200/dcnv3.py)
+  static_assert(PRE != kPreDcnSoftmax || std::is_same_v<ACC, float>, "the fused DCNv3 backward uses float reds");
   constexpr int DL = D * 4 / CPL;
   using G = Geom<DL, THREADS>;
   constexpr int LANES = G::LANES;
-  constexpr bool FUSED = (PRE == kPreFused);
-  constexpr bool DCN = (PRE == kPreDcn);
+  constexpr bool SOFTMAX = pre_softmax(PRE);    // `w` holds logits: softmax and its chain rule (grad_w = logits' grad)
+  constexpr bool FUSED = (PRE == kPreFused);    // MSDA chain only: location affine, reference points, padding mask
+  constexpr bool DCN = pre_dcn(PRE);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   LevelTab* tab = reinterpret_cast<LevelTab*>(smem_raw);
   float* recs = reinterpret_cast<float*>(smem_raw + sizeof(LevelTab));
@@ -988,11 +999,11 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
 
   // Single-pass orders know their row without the level table: the row's grad_out and its first locations /
   // weights are requested before the table's load + barrier (see the forward kernel).
-  constexpr bool EARLY = (ORDER == 0 || ORDER == 2) && PRE != kPreDcn;
+  constexpr bool EARLY = (ORDER == 0 || ORDER == 2) && !DCN;
   constexpr int kEarly = 2;
   float2 early_xy[kEarly];
   float early_w[kEarly];
-  float early_sum = 1.0f;                                // FUSED: softmax denominator of the row
+  float early_sum = 1.0f;                                // SOFTMAX: softmax denominator of the row
   // A warp stays converged for the full-mask shuffles below: rows that do not exist (edge tiles,
   // the tail of the last CTA) get all-zero weights, so they scatter nothing and never write.
   RowWalk<DL, THREADS, ORDER> walk;
@@ -1008,9 +1019,9 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
       const int pt = sub + i * LANES;
       const bool on = cur.live && pt < NP;
       early_xy[i] = on ? __ldg(reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2) + pt) : make_float2(0.f, 0.f);
-      early_w[i] = (on && !FUSED) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
+      early_w[i] = (on && !SOFTMAX) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
     }
-    if constexpr (FUSED)
+    if constexpr (SOFTMAX)
       early_sum = row_softmax<LANES, 4>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
     load_levels_plain<EMIT>(tab, shapes, lsi, L);
   } else {
@@ -1039,18 +1050,17 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
       const float2* lp = reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2);
       const float* wp = w + cur.row * (int64_t)NP;
       float sm_sum = early_sum;
-      if constexpr (FUSED && !EARLY) sm_sum = row_softmax<LANES, 4>(wp, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
-      // one record from a point's raw location / weight (FUSED: raw offset; the weight comes from the softmax);
-      // rows that do not exist get all-zero records
+      if constexpr (SOFTMAX && !EARLY) sm_sum = row_softmax<LANES, 4>(wp, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
+      // one record from a point's raw location / weight (FUSED: raw offset; SOFTMAX: the weight comes from the
+      // softmax); rows that do not exist get all-zero records
       auto build = [&](int pt, float2 xy, float aw) {
         float4 cw = zero;
         int4 fin = make_int4(0, 0, 0, 0);      // no validity bits: nothing is loaded, scattered or written
         if (cur.live) {
           const int l = level_of<PT>(pt, P);
-          if constexpr (FUSED) {
-            aw = __fdiv_rn(__int_as_float(s_fin[pt].w), sm_sum);
+          if constexpr (SOFTMAX) aw = __fdiv_rn(__int_as_float(s_fin[pt].w), sm_sum);
+          if constexpr (FUSED)
             xy = fused_location(xy, rp + l * fused.ref_dim, fused.ref_dim, tab->H[l], tab->W[l], fused.num_P);
-          }
           PointRec r;
           if constexpr (DCN) {
             const float2 px = dcn_location(xy, pt, (int)((cur.row / H) % Q), fused);
@@ -1086,7 +1096,7 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
         float aw = 0.0f;
         if (cur.live) {
           xy = __ldg(lp + pt);
-          if constexpr (!FUSED) aw = __ldg(wp + pt);
+          if constexpr (!SOFTMAX) aw = __ldg(wp + pt);
         }
         build(pt, xy, aw);
       }
@@ -1114,7 +1124,7 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     float* glp = grad_loc + cur.row * (int64_t)NP * 2;
     float* gwp = grad_w + cur.row * (int64_t)NP;
 
-    float sm_dot = 0.0f;   // FUSED: sum_j grad_aw_j * aw_j of the row (softmax backward)
+    float sm_dot = 0.0f;   // SOFTMAX: sum_j grad_aw_j * aw_j of the row (softmax backward)
     for (int c0 = 0; c0 < NP; c0 += 4) {
       float d[16];
 #pragma unroll
@@ -1206,10 +1216,11 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
           sm_dot = fmaf(g_aw, aw, sm_dot);
         } else {
           s_fin[mine] = make_int4(__float_as_int(g_x), __float_as_int(g_aw), __float_as_int(g_y), r.w);
+          if constexpr (SOFTMAX) sm_dot = fmaf(g_aw, aw, sm_dot);
         }
       }
     }
-    if constexpr (FUSED) {
+    if constexpr (SOFTMAX) {
       // softmax backward: grad_logit_i = aw_i * (grad_aw_i - sum_j grad_aw_j aw_j)
 #pragma unroll
       for (int k = LANES / 2; k > 0; k >>= 1) sm_dot += __shfl_xor_sync(0xffffffffu, sm_dot, k);
@@ -1222,7 +1233,7 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     if (cur.live) {
       auto gw_of = [&](const int4 r) {
         const float g_aw = __int_as_float(r.y);
-        return FUSED ? __int_as_float(r.w) * (g_aw - sm_dot) : g_aw;
+        return SOFTMAX ? __int_as_float(r.w) * (g_aw - sm_dot) : g_aw;
       };
       if ((NP & 1) == 0) {      // both row bases are then 16- / 8-byte aligned
         for (int pt = 2 * sub; pt < NP; pt += 2 * LANES) {

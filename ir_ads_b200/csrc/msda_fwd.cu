@@ -25,6 +25,9 @@ int fwd_fused(cudaStream_t, const Dims&, int, const void*, const int64_t*, const
 int fwd_dcn(cudaStream_t, const Dims&, int, const void*, const void*, const void*, void*, msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
 }
+int fwd_dcn_softmax(cudaStream_t, const Dims&, int, const void*, const void*, const void*, void*, msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
+}
 #else
 // fused pre-op chain: LINEAR order
 int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes, const int64_t* lsi,
@@ -37,11 +40,12 @@ int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, cons
 #undef MSDA_DISPATCH_ORDER
 }
 
-// DCNv3: runtime point count (K = kernel_h * kernel_w), LINEAR order
-int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off, const void* mask, void* out,
-            msda::FusedArgs fa) {
-#define CALL_DF(D_, VT_) \
-  launch_fwd_fast<D_, VT_, 0, kFwdThreads, 0, msda::kPreDcn>(st, d, input, nullptr, nullptr, off, mask, out, fa)
+// DCNv3: runtime point count (K = kernel_h * kernel_w), LINEAR order.  PRE: kPreDcn (w = mask) or kPreDcnSoftmax
+// (w = mask logits)
+template <int PRE>
+int fwd_dcn_pre(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off, const void* w,
+                void* out, msda::FusedArgs fa) {
+#define CALL_DF(D_, VT_) launch_fwd_fast<D_, VT_, 0, kFwdThreads, 0, PRE>(st, d, input, nullptr, nullptr, off, w, out, fa)
 #define DCN_D(VT_)                                                                         \
   switch (d.D) {                                                                           \
     case 16: return CALL_DF(16, VT_);                                                      \
@@ -56,6 +60,17 @@ int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const 
   return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
 #undef DCN_D
 #undef CALL_DF
+}
+
+int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off, const void* mask, void* out,
+            msda::FusedArgs fa) {
+  return fwd_dcn_pre<msda::kPreDcn>(st, d, dtype, input, off, mask, out, fa);
+}
+
+// fused DCNv3 module path: the softmax over each (pixel, group) row's K mask logits runs in the kernel
+int fwd_dcn_softmax(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off,
+                    const void* mask_logits, void* out, msda::FusedArgs fa) {
+  return fwd_dcn_pre<msda::kPreDcnSoftmax>(st, d, dtype, input, off, mask_logits, out, fa);
 }
 #endif
 

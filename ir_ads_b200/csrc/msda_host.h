@@ -71,6 +71,9 @@ int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, cons
               const void* off, const void* logits, void* out, msda::FusedArgs fa);
 int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off, const void* mask, void* out,
             msda::FusedArgs fa);
+// fused DCNv3 module path (kPreDcnSoftmax): mask logits in, the row softmax runs in the kernel
+int fwd_dcn_softmax(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off,
+                    const void* mask_logits, void* out, msda::FusedArgs fa);
 
 // ---- msda_bwd.cu ----
 int bwd_fast(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const void* go, const void* value,
@@ -93,6 +96,9 @@ int bwd_fused_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* g
                         void* glog, msda::FusedArgs fa);
 int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
             const void* mask, float* gi, void* goff, void* gmask, msda::FusedArgs fa);
+// fused DCNv3 module path: mask logits in, their gradient out (float reds only)
+int bwd_dcn_softmax(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
+                    const void* mask_logits, float* gi, void* goff, void* glogits, msda::FusedArgs fa);
 // DCNv3 twins of bwd_fast_det / bwd_fast_noscatter / bwd_fast_emit (deterministic grad_input)
 int bwd_dcn_det(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                 const void* mask, unsigned long long* acc, void* goff, void* gmask, const msda::DetScale* det,

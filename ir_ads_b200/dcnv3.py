@@ -13,6 +13,10 @@ are widened exactly inside the kernels, accumulation is float32).  Every other s
 runs as a composition on the GENERIC MSDeformAttn kernels (csrc/msda_generic.cuh, any D, float32 / float64): the convolution-grid sampling positions
 are formed with the reference kernel's arithmetic in PyTorch, normalised, and handed to
 MultiScaleDeformableAttnFunction with one level -- still CUDA only, still no CPU path.
+
+The ``DCNv3`` module runs its mask softmax inside the kernels on the fast shapes (``DCNv3FusedFunction``, PRE == 3):
+the kernels take the mask Linear's raw logits, so the mask and its gradient never reach HBM.  Elsewhere it composes
+``F.softmax`` and ``DCNv3Function`` as the reference does.
 """
 from __future__ import annotations
 
@@ -40,6 +44,11 @@ def _declare(handle):
     handle.msda_dcnv3_backward.argtypes = [vp, vp, vp, vp, vp] + [i] * 10 + [f] + [i] * 5 + [vp, vp, vp, vp, sz, i, u]
     handle.msda_dcnv3_backward_workspace_bytes.restype = sz
     handle.msda_dcnv3_backward_workspace_bytes.argtypes = [i] * 10 + [u]
+    # fused module path: the same signatures, mask logits in place of the mask
+    handle.msda_dcnv3_fused_forward.restype = i
+    handle.msda_dcnv3_fused_forward.argtypes = handle.msda_dcnv3_forward.argtypes
+    handle.msda_dcnv3_fused_backward.restype = i
+    handle.msda_dcnv3_fused_backward.argtypes = handle.msda_dcnv3_backward.argtypes
     handle._dcn_declared = True
     return handle
 
@@ -182,6 +191,102 @@ class DCNv3Function(Function):
 
 
 # ------------------------------------------------------------------------------------------------
+# fused module path: the DCNv3 module's mask softmax inside the kernels (csrc/msda_fast.cuh, PRE == 3)
+# ------------------------------------------------------------------------------------------------
+def _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels):
+    dims = _geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels)
+    _require(offset.dtype == torch.float32 and mask_logits.dtype == torch.float32,
+             "offset / mask_logits must be float32")
+    _require(fast_supported(input, kernel_h, kernel_w, group_channels),
+             f"fused DCNv3 needs group_channels in {{16, 32, 64, 128}}, kernel_h*kernel_w <= 64 and a float32 / "
+             f"bfloat16 / float16 input (got {group_channels}, {kernel_h * kernel_w}, {input.dtype})")
+    return dims
+
+
+def dcnv3_fused_forward(input, offset, mask_logits, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                        dilation_w, group, group_channels, offset_scale) -> torch.Tensor:
+    """``dcnv3_forward`` with ``mask = softmax(mask_logits)`` over each (pixel, group) row of K, the softmax done inside
+    the kernel (``msda_dcnv3_fused_forward``).  ``offset`` / ``mask_logits`` are float32."""
+    N, H_in, W_in, H_out, W_out = _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels)
+    input, offset, mask_logits = _aligned(input), _aligned(offset), _aligned(mask_logits)
+    out = torch.empty((N, H_out, W_out, group * group_channels), dtype=input.dtype, device=input.device)
+    stream = torch.cuda.current_stream(input.device).cuda_stream
+    status = _declare(_lib.lib()).msda_dcnv3_fused_forward(
+        ctypes.c_void_p(stream), _ptr(input), _ptr(offset), _ptr(mask_logits), kernel_h, kernel_w, stride_h, stride_w,
+        pad_h, pad_w, dilation_h, dilation_w, group, group_channels, float(offset_scale), N, H_in, W_in, H_out, W_out,
+        _ptr(out), _DCN_TAG[input.dtype], 0)
+    _lib.check(status, "dcnv3_fused_forward")
+    return out
+
+
+def dcnv3_fused_backward(input, offset, mask_logits, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                         dilation_w, group, group_channels, offset_scale, grad_output) -> List[torch.Tensor]:
+    """``[grad_input, grad_offset, grad_mask_logits]`` of ``dcnv3_fused_forward``: float reds, the softmax's chain rule
+    inside the kernel (``msda_dcnv3_fused_backward``).  There is no deterministic form; ``DCNv3FusedFunction``
+    composes one."""
+    N, H_in, W_in, H_out, W_out = _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels)
+    _require(grad_output.is_cuda and grad_output.dtype == input.dtype, "grad_output must match input's device / dtype")
+    grad_output = _aligned(grad_output.contiguous())
+    input, offset, mask_logits = _aligned(input), _aligned(offset), _aligned(mask_logits)
+    grad_input = torch.empty_like(input)
+    grad_offset = torch.empty_like(offset)
+    grad_logits = torch.empty_like(mask_logits)
+    tag = _DCN_TAG[input.dtype]
+    handle = _declare(_lib.lib())
+    ws_bytes = handle.msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, N, H_in, W_in,
+                                                          H_out, W_out, tag, 0)
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=input.device) if ws_bytes else None
+    stream = torch.cuda.current_stream(input.device).cuda_stream
+    status = handle.msda_dcnv3_fused_backward(
+        ctypes.c_void_p(stream), _ptr(grad_output), _ptr(input), _ptr(offset), _ptr(mask_logits), kernel_h, kernel_w,
+        stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels, float(offset_scale), N, H_in,
+        W_in, H_out, W_out, _ptr(grad_input), _ptr(grad_offset), _ptr(grad_logits),
+        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, 0)
+    _lib.check(status, "dcnv3_fused_backward")
+    return [grad_input, grad_offset, grad_logits]
+
+
+class DCNv3FusedFunction(Function):
+    """``apply(input, offset, mask_logits, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+    dilation_w, group, group_channels, offset_scale, im2col_step)``: ``DCNv3Function`` with the mask replaced by its
+    pre-softmax logits ``[N, H_out, W_out, group*K]`` -- the DCNv3 module's ``softmax(mask(x1).reshape(..., group,
+    K), -1)`` runs inside the kernels, so the mask and its gradient never reach HBM.  Gradients for ``input``,
+    ``offset`` and ``mask_logits``.  ``offset`` / ``mask_logits`` are float32; ``input`` is float32, bfloat16 or
+    float16 on the fast-kernel shapes (``fast_supported``) -- anything else raises, the module composes instead.
+
+    Deterministic mode (set_deterministic / torch.use_deterministic_algorithms), as MSDeformAttnFusedFunction: the
+    forward is the same fused kernel (it has no atomics); the backward forms the mask with torch.softmax, runs the
+    bit-reproducible ``dcnv3_backward`` and applies the softmax's chain rule with torch's own softmax backward -- the
+    same bits as ``torch.softmax`` followed by ``DCNv3Function`` in deterministic mode."""
+
+    @staticmethod
+    def forward(ctx, input, offset, mask_logits, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                dilation_w, group, group_channels, offset_scale, im2col_step):
+        ctx.args = (kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group, group_channels,
+                    offset_scale)
+        ctx.im2col_step = im2col_step
+        output = dcnv3_fused_forward(input, offset, mask_logits, *ctx.args)
+        ctx.save_for_backward(input, offset, mask_logits)
+        return output
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        input, offset, mask_logits = ctx.saved_tensors
+        grad_output = grad_output.to(input.dtype)
+        if not functional._flags(True) & _lib.FLAG_DETERMINISTIC:
+            return tuple(dcnv3_fused_backward(input, offset, mask_logits, *ctx.args, grad_output)) + (None,) * 12
+        N, H_out, W_out, _ = mask_logits.shape
+        with torch.enable_grad():
+            logits = mask_logits.detach().view(N, H_out, W_out, ctx.args[8], -1).requires_grad_(True)
+            mask = torch.softmax(logits, -1)
+        gi, go, gm = dcnv3_backward(input, offset, mask.detach().view(N, H_out, W_out, -1), *ctx.args, grad_output,
+                                    ctx.im2col_step)
+        (g_logits,) = torch.autograd.grad(mask, logits, gm.view_as(mask))
+        return (gi, go, g_logits.view_as(mask_logits)) + (None,) * 12
+
+
+# ------------------------------------------------------------------------------------------------
 # the DCNv3 operator module (InternImage), same constructor / parameter names as the reference
 # (/root/reference/detrex/layers/dcn_v3.py:373-500) so InternImage checkpoints load
 # ------------------------------------------------------------------------------------------------
@@ -277,10 +382,16 @@ class DCNv3(nn.Module):
         dtype = x.dtype
         x1 = self.dw_conv(input.permute(0, 3, 1, 2))
         offset = self.offset(x1)
-        mask = F.softmax(self.mask(x1).reshape(N, H, W, self.group, -1), -1).reshape(N, H, W, -1).type(dtype)
-        x = DCNv3Function.apply(x.contiguous(), offset.contiguous(), mask.contiguous(), self.kernel_size,
-                                self.kernel_size, self.stride, self.stride, self.pad, self.pad, self.dilation,
-                                self.dilation, self.group, self.group_channels, self.offset_scale, 256)
+        geometry = (self.kernel_size, self.kernel_size, self.stride, self.stride, self.pad, self.pad, self.dilation,
+                    self.dilation, self.group, self.group_channels, self.offset_scale, 256)
+        if fast_supported(x, self.kernel_size, self.kernel_size, self.group_channels):
+            # fused: the mask softmax runs inside the kernels on the float32 logits (under autocast the mask is
+            # therefore not rounded to the input dtype, as the composition below rounds it)
+            x = DCNv3FusedFunction.apply(x.contiguous(), offset.float().contiguous(),
+                                         self.mask(x1).float().reshape(N, H, W, -1).contiguous(), *geometry)
+        else:
+            mask = F.softmax(self.mask(x1).reshape(N, H, W, self.group, -1), -1).reshape(N, H, W, -1).type(dtype)
+            x = DCNv3Function.apply(x.contiguous(), offset.contiguous(), mask.contiguous(), *geometry)
         if self.center_feature_scale:
             scale = F.linear(x1, weight=self.center_feature_scale_proj_weight,
                              bias=self.center_feature_scale_proj_bias).sigmoid()
