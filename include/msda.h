@@ -67,6 +67,18 @@ extern "C" {
  * difference of the red order).  Added in ABI 3 without a version bump: an older library answers
  * MSDA_ERR_INVALID_ARGUMENT ("unknown dtype tag"). */
 #define MSDA_F16 3
+/* The autocast forms of the fused module paths (msda_fused_*, msda_dcnv3_fused_*): value / output / grad_output /
+ * grad_value (input / grad_input for DCNv3) AND the projection tensors -- sampling_offsets / attn_logits (DCNv3:
+ * offset / mask_logits) and their gradients -- in that 16-bit type, as the module's Linear layers produce them under
+ * autocast; reference_points stay float.  The kernels widen the 16-bit offsets / logits exactly, so output and
+ * grad_value are those of MSDA_BF16 / MSDA_F16 called with the widened tensors, and the offset / logit gradients are
+ * the float gradients of that call rounded once, to nearest even (what a cast of them gives), except that a NaN
+ * gradient's payload may differ from the cast's: only NaN-ness is promised.  Accepted by msda_fused_supported,
+ * msda_fused_forward / _backward, msda_dcnv3_fused_forward / _backward and the two backward workspace queries (which
+ * answer exactly what they answer for MSDA_BF16 / MSDA_F16); every other entry point refuses them as an unknown tag,
+ * before any device work.  Added in ABI 3 without a version bump: an older library refuses them the same way. */
+#define MSDA_BF16_AUX16 4
+#define MSDA_F16_AUX16 5
 
 /* status codes */
 #define MSDA_OK 0
@@ -166,25 +178,26 @@ int msda_backward(void* stream, const void* grad_output, const void* value,
  *                                               masked copy (one read + one write of value per layer, and the
  *                                               same again in backward) never exists
  * Backward returns grad_value plus the gradients w.r.t. the two RAW tensors (what the Linear layers'
- * backward consumes); it uses the same workspace rule as msda_backward.  Only the fast kernels have
- * a fused form: otherwise MSDA_ERR_UNSUPPORTED is returned (query with msda_fused_supported) and the
- * caller composes softmax / affine itself around msda_forward / msda_backward.
+ * backward consumes); it uses the same workspace rule as msda_backward.  With MSDA_BF16_AUX16 / MSDA_F16_AUX16
+ * sampling_offsets, attn_logits, grad_offsets and grad_logits are in the value's 16-bit type (hence `void*`).
+ * Only the fast kernels have a fused form: otherwise MSDA_ERR_UNSUPPORTED is returned (query with
+ * msda_fused_supported) and the caller composes softmax / affine itself around msda_forward / msda_backward.
  */
 int msda_fused_supported(int channels, int num_levels, int num_point, int spatial_size, int num_heads,
                          int dtype, unsigned flags);
 int msda_fused_forward(void* stream, const void* value, const int64_t* spatial_shapes,
-                       const int64_t* level_start_index, const float* sampling_offsets,
-                       const float* attn_logits, const float* reference_points, int ref_dim,
+                       const int64_t* level_start_index, const void* sampling_offsets,
+                       const void* attn_logits, const float* reference_points, int ref_dim,
                        const uint8_t* value_padding_mask, int batch, int spatial_size, int num_heads,
                        int channels, int num_levels, int num_query, int num_point, void* output, int dtype,
                        unsigned flags);
 int msda_fused_backward(void* stream, const void* grad_output, const void* value,
                         const int64_t* spatial_shapes, const int64_t* level_start_index,
-                        const float* sampling_offsets, const float* attn_logits,
+                        const void* sampling_offsets, const void* attn_logits,
                         const float* reference_points, int ref_dim, const uint8_t* value_padding_mask,
                         int batch, int spatial_size, int num_heads, int channels, int num_levels,
-                        int num_query, int num_point, void* grad_value, float* grad_offsets,
-                        float* grad_logits, void* workspace, size_t workspace_bytes, int dtype,
+                        int num_query, int num_point, void* grad_value, void* grad_offsets,
+                        void* grad_logits, void* workspace, size_t workspace_bytes, int dtype,
                         unsigned flags);
 
 /*
@@ -238,10 +251,13 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
  * msda_dcnv3_forward / msda_dcnv3_backward, with
  *   mask_logits       [N, H_out, W_out, group*K] float  the raw output of the module's mask Linear (pre-softmax)
  *   grad_mask_logits  [N, H_out, W_out, group*K] float  its gradient (fully written by the library)
- * in place of mask / grad_mask.  The result equals msda_dcnv3_forward / _backward called with
- * mask = softmax(mask_logits) over each row of K, followed by the softmax's chain rule
- * grad_logit_i = w_i * (grad_mask_i - sum_j grad_mask_j * w_j), up to float rounding of the softmax.  Non-finite
- * logits behave as in torch.softmax: a -inf logit gets weight 0 (and gradient 0) while the rest of its row is
+ * in place of mask / grad_mask (with MSDA_BF16_AUX16 / MSDA_F16_AUX16: offset, mask_logits and their gradients in
+ * the input's 16-bit type, hence `void*`; before those tags the prototypes read `const float* mask_logits` /
+ * `float* grad_mask_logits`, and since a float pointer converts to `void*` implicitly, such callers compile and link
+ * unchanged -- the same holds for the four pointers of msda_fused_forward / _backward).  The result equals
+ * msda_dcnv3_forward / _backward called with mask = softmax(mask_logits) over each row of K, followed by the softmax's
+ * chain rule grad_logit_i = w_i * (grad_mask_i - sum_j grad_mask_j * w_j), up to float rounding of the softmax.
+ * Non-finite logits behave as in torch.softmax: a -inf logit gets weight 0 (and gradient 0) while the rest of its row is
  * normalised as usual; a row whose logits are all -inf, or that holds +inf or NaN, has NaN weights: its logits'
  * gradient is NaN, and so are its output pixel and its grad_offset / grad_input contributions wherever one of its
  * points samples inside the map (exactly what msda_dcnv3_* make of torch.softmax's NaN row).
@@ -250,17 +266,17 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
  * the softmax around msda_dcnv3_backward instead, whose grad_input is bit-reproducible).  Every other flag bit is
  * ignored by both entry points.  Added in ABI 3 without a version bump: an older library lacks the two symbols.
  */
-int msda_dcnv3_fused_forward(void* stream, const void* input, const float* offset, const float* mask_logits,
+int msda_dcnv3_fused_forward(void* stream, const void* input, const void* offset, const void* mask_logits,
                              int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                              int dilation_h, int dilation_w, int group, int group_channels, float offset_scale,
                              int batch, int height_in, int width_in, int height_out, int width_out,
                              void* output, int dtype, unsigned flags);
-int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void* input, const float* offset,
-                              const float* mask_logits, int kernel_h, int kernel_w, int stride_h, int stride_w,
+int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void* input, const void* offset,
+                              const void* mask_logits, int kernel_h, int kernel_w, int stride_h, int stride_w,
                               int pad_h, int pad_w, int dilation_h, int dilation_w, int group,
                               int group_channels, float offset_scale, int batch, int height_in, int width_in,
-                              int height_out, int width_out, void* grad_input, float* grad_offset,
-                              float* grad_mask_logits, void* workspace, size_t workspace_bytes, int dtype,
+                              int height_out, int width_out, void* grad_input, void* grad_offset,
+                              void* grad_mask_logits, void* workspace, size_t workspace_bytes, int dtype,
                               unsigned flags);
 
 /*
@@ -268,13 +284,21 @@ int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void*
  * FFN in the reference's transformer layers -- x = x + identity; x = norm(x)
  * (/root/reference/detrex/layers/transformer.py:152-192; the residuals are added at multi_scale_deform_attn.py:363 and
  * detrex/layers/mlp.py:127-132) -- as one pass instead of an add kernel plus a LayerNorm kernel.
- *   a, b, y, grad_y, grad_x   [rows, channels]  dtype (MSDA_F32 or MSDA_BF16), contiguous
+ *   a, b, y, grad_y, grad_x   [rows, channels]  dtype (MSDA_F32, MSDA_BF16 or MSDA_F16), contiguous
  *   gamma, beta, grad_gamma, grad_beta  [channels] float;   mean, rstd  [rows] float (saved by forward for backward)
  * forward:  y = (a + b - mean) * rstd * gamma + beta, statistics over the channels, fp32 arithmetic.
  * backward: grad_x = d loss / d (a + b) -- the gradient of BOTH addends -- plus grad_gamma / grad_beta, reduced in a
  *           fixed order (bit-reproducible); a + b is recomputed, never stored.  Needs a workspace of
  *           msda_add_layernorm_workspace_bytes(rows, channels).
- * channels must be a multiple of 4 and at most 1024 (MSDA_ERR_UNSUPPORTED otherwise).
+ * channels must be a multiple of 4 and at most 1024 (MSDA_ERR_UNSUPPORTED otherwise, also for any other dtype tag).
+ *
+ * Mixed form, the one autocast produces (a 16-bit attention / FFN output added to a float32 residual): `a` is in
+ * a_dtype (MSDA_BF16 or MSDA_F16; anything else is MSDA_ERR_UNSUPPORTED), b / y / grad_y / grad_b are float32.
+ *   forward:  y = LayerNorm(float(a) + b) in float32 -- what norm(a + b) gives with torch's type promotion.
+ *   backward: grad_b = d loss / d (a + b) (float32) and grad_a = grad_b rounded once to a_dtype, to nearest even (the
+ *             cast autograd applies to a's gradient; a NaN's payload may differ, only NaN-ness is promised), written in
+ *             one pass; grad_gamma / grad_beta as above, in the same fixed order.  Same workspace query.
+ * Added in ABI 3 without a version bump: an older library lacks the two symbols.
  */
 size_t msda_add_layernorm_workspace_bytes(int64_t rows, int channels);
 int msda_add_layernorm_forward(void* stream, const void* a, const void* b, const float* gamma, const float* beta,
@@ -283,6 +307,13 @@ int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a,
                                 const float* mean, const float* rstd, int64_t rows, int channels, void* grad_x,
                                 float* grad_gamma, float* grad_beta, void* workspace, size_t workspace_bytes,
                                 int dtype);
+int msda_add_layernorm_mixed_forward(void* stream, const void* a, const float* b, const float* gamma,
+                                     const float* beta, int64_t rows, int channels, float eps, float* y, float* mean,
+                                     float* rstd, int a_dtype);
+int msda_add_layernorm_mixed_backward(void* stream, const float* grad_y, const void* a, const float* b,
+                                      const float* gamma, const float* mean, const float* rstd, int64_t rows,
+                                      int channels, void* grad_a, float* grad_b, float* grad_gamma, float* grad_beta,
+                                      void* workspace, size_t workspace_bytes, int a_dtype);
 
 /*
  * Test hook: the integer bookkeeping the float kernels derive from every sampling point.

@@ -17,6 +17,8 @@ HEADER_PATH = os.path.join(os.path.dirname(_PKG), "include", "msda.h")
 
 # include/msda.h
 MSDA_F32, MSDA_F64, MSDA_BF16, MSDA_F16 = 0, 1, 2, 3
+# fused module paths under autocast: offsets / logits and their gradients in the value's 16-bit type as well
+MSDA_BF16_AUX16, MSDA_F16_AUX16 = 4, 5
 MSDA_OK = 0
 FLAG_DETERMINISTIC = 1 << 0
 FLAG_FORCE_GENERIC = 1 << 1
@@ -76,6 +78,10 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.msda_add_layernorm_forward.argtypes = [vp, vp, vp, vp, vp, i64, i, f32, vp, vp, vp, i]
     lib.msda_add_layernorm_backward.restype = i
     lib.msda_add_layernorm_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, i, vp, vp, vp, vp, sz, i]
+    lib.msda_add_layernorm_mixed_forward.restype = i
+    lib.msda_add_layernorm_mixed_forward.argtypes = lib.msda_add_layernorm_forward.argtypes
+    lib.msda_add_layernorm_mixed_backward.restype = i
+    lib.msda_add_layernorm_mixed_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, i, vp, vp, vp, vp, vp, sz, i]
     lib.msda_debug_bookkeeping.restype = i
     lib.msda_debug_bookkeeping.argtypes = [vp, vp, vp, vp, i, i, i, i, i, i, i, vp, vp]
     lib.msda_debug_fastdiv.restype = u

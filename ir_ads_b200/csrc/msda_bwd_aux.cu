@@ -77,7 +77,8 @@ int bwd_dcn_emit(cudaStream_t, const Dims&, int, const void*, const void*, const
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
 }
 #else
-// fused pre-op chain: STRIP order
+// fused pre-op chain: STRIP order.  dtype MSDA_*_AUX16: offsets / logits and their gradients in the value's 16-bit
+// type
 int bwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
               const int64_t* lsi, const void* off, const void* logits, float* gv, void* goff, void* glog,
               msda::FusedArgs fa) {
@@ -85,7 +86,12 @@ int bwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* go, const v
 #define CALL_FB(D_, VT_, PT_, ORD_)                                                                               \
   launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPreFused>(st, d, go, value, shapes, lsi, off, logits, gv, \
                                                                            goff, glog, nullptr, fa)
+#define CALL_FB16(D_, VT_, PT_, ORD_)                                                                          \
+  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPreFused, VT_>(st, d, go, value, shapes, lsi, off, \
+                                                                                logits, gv, goff, glog, nullptr, fa)
+  MSDA_DISPATCH_VT_AUX16(CALL_FB16);
   MSDA_DISPATCH_VT(CALL_FB);
+#undef CALL_FB16
 #undef CALL_FB
 #undef MSDA_DISPATCH_ORDER
 }
@@ -104,24 +110,29 @@ int bwd_fused_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* g
 }
 
 // DCNv3: runtime point count, STRIP order.  PRE: kPreDcn (w = mask, gw = its gradient) or kPreDcnSoftmax (w = mask
-// logits, gw = the logits' gradient)
+// logits, gw = the logits' gradient; dtype MSDA_*_AUX16: offset / logits and their gradients in the input's 16-bit
+// type)
 template <int PRE>
 int bwd_dcn_pre(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                 const void* w, float* gi, void* goff, void* gw, msda::FusedArgs fa) {
-#define CALL_DB(D_, VT_)                                                                                             \
-  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, float, PRE>(st, d, go, input, nullptr, nullptr, off, w, gi, goff, gw, \
-                                                          nullptr, fa)
-#define DCN_D(VT_)                                                                         \
+#define CALL_DB(D_, VT_, AT_)                                                                                          \
+  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, float, PRE, AT_>(st, d, go, input, nullptr, nullptr, off, w, gi, goff, gw, \
+                                                               nullptr, fa)
+#define DCN_D(VT_, AT_)                                                                    \
   switch (d.D) {                                                                           \
-    case 16: return CALL_DB(16, VT_);                                                      \
-    case 32: return CALL_DB(32, VT_);                                                      \
-    case 64: return CALL_DB(64, VT_);                                                      \
-    case 128: return CALL_DB(128, VT_);                                                    \
+    case 16: return CALL_DB(16, VT_, AT_);                                                 \
+    case 32: return CALL_DB(32, VT_, AT_);                                                 \
+    case 64: return CALL_DB(64, VT_, AT_);                                                 \
+    case 128: return CALL_DB(128, VT_, AT_);                                               \
     default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);           \
   }
-  if (dtype == MSDA_F32) DCN_D(float)
-  if (dtype == MSDA_BF16) DCN_D(__nv_bfloat16)
-  if (dtype == MSDA_F16) DCN_D(__half)
+  if constexpr (PRE == msda::kPreDcnSoftmax) {
+    if (dtype == MSDA_BF16_AUX16) DCN_D(__nv_bfloat16, __nv_bfloat16)
+    if (dtype == MSDA_F16_AUX16) DCN_D(__half, __half)
+  }
+  if (dtype == MSDA_F32) DCN_D(float, float)
+  if (dtype == MSDA_BF16) DCN_D(__nv_bfloat16, float)
+  if (dtype == MSDA_F16) DCN_D(__half, float)
   return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
 #undef DCN_D
 #undef CALL_DB

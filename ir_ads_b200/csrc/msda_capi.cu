@@ -243,6 +243,13 @@ bool two_byte(int dtype) { return dtype == MSDA_BF16 || dtype == MSDA_F16; }
 
 size_t elem_size(int dtype) { return dtype == MSDA_F64 ? 8 : (two_byte(dtype) ? 2 : 4); }
 
+// The autocast tags of the fused entry points (include/msda.h): the value dtype they stand for, and whether the
+// offsets / logits and their gradients are 16-bit too.  Every other tag maps to itself.
+int fused_value_dtype(int dtype) {
+  return dtype == MSDA_BF16_AUX16 ? MSDA_BF16 : (dtype == MSDA_F16_AUX16 ? MSDA_F16 : dtype);
+}
+size_t aux_size(int dtype) { return (dtype == MSDA_BF16_AUX16 || dtype == MSDA_F16_AUX16) ? 2 : 4; }
+
 // float workspace -> bf16 / f16 grad_value
 int cast_from_f32(cudaStream_t st, const float* src, void* dst, int64_t n, int dtype) {
   const int grid = grid_for(n, 256, 148 * 16);
@@ -524,6 +531,7 @@ int msda_forward(void* stream, const void* value, const int64_t* spatial_shapes,
 size_t msda_backward_workspace_bytes(int batch, int spatial_size, int num_heads, int channels, int num_levels,
                                      int num_query, int num_point, int dtype, unsigned flags) {
   (void)num_levels; (void)num_query; (void)num_point;
+  dtype = fused_value_dtype(dtype);   // the autocast tags need what their value dtype needs
   if (batch <= 0 || spatial_size <= 0 || num_heads <= 0 || channels <= 0) return 0;
   const size_t n_value = (size_t)batch * spatial_size * num_heads * channels;
   if (flags & MSDA_FLAG_DETERMINISTIC) {
@@ -631,17 +639,17 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
 int msda_fused_supported(int channels, int num_levels, int num_point, int spatial_size, int num_heads, int dtype,
                          unsigned flags) {
   const Dims d{1, spatial_size, num_heads, channels, num_levels, 1, num_point};
-  return fast_ok(d, dtype, flags) && !(flags & MSDA_FLAG_DETERMINISTIC) ? 1 : 0;
+  return fast_ok(d, fused_value_dtype(dtype), flags) && !(flags & MSDA_FLAG_DETERMINISTIC) ? 1 : 0;
 }
 
 int msda_fused_forward(void* stream, const void* value, const int64_t* spatial_shapes,
-                       const int64_t* level_start_index, const float* sampling_offsets, const float* attn_logits,
+                       const int64_t* level_start_index, const void* sampling_offsets, const void* attn_logits,
                        const float* reference_points, int ref_dim, const uint8_t* value_padding_mask, int batch,
                        int spatial_size, int num_heads, int channels, int num_levels, int num_query, int num_point,
                        void* output, int dtype, unsigned flags) {
   g_err[0] = 0;
   const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-  if (int s = check_dims(d, dtype)) return s;
+  if (int s = check_dims(d, fused_value_dtype(dtype))) return s;
   if (ref_dim != 2 && ref_dim != 4) return fail(MSDA_ERR_INVALID_ARGUMENT, "ref_dim must be 2 or 4, got %d", ref_dim);
   if (d.rows() * d.D == 0) return MSDA_OK;
   if (!msda_fused_supported(channels, num_levels, num_point, spatial_size, num_heads, dtype, flags) || d.S == 0)
@@ -665,14 +673,15 @@ int msda_fused_forward(void* stream, const void* value, const int64_t* spatial_s
 }
 
 int msda_fused_backward(void* stream, const void* grad_output, const void* value, const int64_t* spatial_shapes,
-                        const int64_t* level_start_index, const float* sampling_offsets, const float* attn_logits,
+                        const int64_t* level_start_index, const void* sampling_offsets, const void* attn_logits,
                         const float* reference_points, int ref_dim, const uint8_t* value_padding_mask, int batch,
                         int spatial_size, int num_heads, int channels, int num_levels, int num_query, int num_point,
-                        void* grad_value, float* grad_offsets, float* grad_logits, void* workspace,
+                        void* grad_value, void* grad_offsets, void* grad_logits, void* workspace,
                         size_t workspace_bytes, int dtype, unsigned flags) {
   g_err[0] = 0;
   const Dims d{batch, spatial_size, num_heads, channels, num_levels, num_query, num_point};
-  if (int s = check_dims(d, dtype)) return s;
+  const int vdt = fused_value_dtype(dtype);   // dtype itself selects the kernels (16-bit offsets / logits or not)
+  if (int s = check_dims(d, vdt)) return s;
   if (ref_dim != 2 && ref_dim != 4) return fail(MSDA_ERR_INVALID_ARGUMENT, "ref_dim must be 2 or 4, got %d", ref_dim);
   if (!msda_fused_supported(channels, num_levels, num_point, spatial_size, num_heads, dtype, flags) ||
       d.n_value() == 0 || d.n_points() == 0)
@@ -693,7 +702,7 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
   if (need && (!workspace || workspace_bytes < need))
     return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
   float* gv32 = static_cast<float*>(grad_value);
-  if (two_byte(dtype)) gv32 = static_cast<float*>(workspace);
+  if (two_byte(vdt)) gv32 = static_cast<float*>(workspace);
   MSDA_CUDA(cudaMemsetAsync(gv32, 0, (size_t)d.n_value() * sizeof(float), st));
   msda::FusedArgs fa{};
   fa.ref = reference_points;
@@ -709,7 +718,7 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
     s = bwd_fused(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits,
                   gv32, grad_offsets, grad_logits, fa);
   if (s != MSDA_OK) return s;
-  if (two_byte(dtype)) return cast_from_f32(st, gv32, grad_value, d.n_value(), dtype);
+  if (two_byte(vdt)) return cast_from_f32(st, gv32, grad_value, d.n_value(), vdt);
   return MSDA_OK;
 }
 
@@ -748,6 +757,7 @@ constexpr size_t kDcnLevelSlot = 256;
 size_t msda_dcnv3_backward_workspace_bytes(int kernel_h, int kernel_w, int group, int group_channels, int batch,
                                            int height_in, int width_in, int height_out, int width_out, int dtype,
                                            unsigned flags) {
+  dtype = fused_value_dtype(dtype);   // the autocast tags need what their value dtype needs
   if (batch <= 0 || height_in <= 0 || width_in <= 0 || group <= 0 || group_channels <= 0) return 0;
   const size_t n_value = (size_t)batch * height_in * width_in * group * group_channels;
   // empty problems (no output pixel, no kernel point) need what they need without the flag
@@ -761,9 +771,9 @@ size_t msda_dcnv3_backward_workspace_bytes(int kernel_h, int kernel_w, int group
 
 namespace {
 // The body of msda_dcnv3_forward (softmax false: `w` = mask) and msda_dcnv3_fused_forward (softmax true: `w` = mask
-// logits), after dcn_setup.
-int dcn_forward(void* stream, const Dims& d, const msda::FusedArgs& fa, const void* input, const float* offset,
-                const float* w, void* output, int dtype, bool softmax) {
+// logits; dtype may be an autocast tag), after dcn_setup.
+int dcn_forward(void* stream, const Dims& d, const msda::FusedArgs& fa, const void* input, const void* offset,
+                const void* w, void* output, int dtype, bool softmax) {
   if (d.rows() * d.D == 0) return MSDA_OK;
   if (!output) return fail(MSDA_ERR_INVALID_ARGUMENT, "output is null");
   if (int s = check_alignment({{"input", input}, {"offset", offset}, {softmax ? "mask_logits" : "mask", w},
@@ -773,7 +783,7 @@ int dcn_forward(void* stream, const Dims& d, const msda::FusedArgs& fa, const vo
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(output));
   if (d.S == 0) {
-    MSDA_CUDA(cudaMemsetAsync(output, 0, (size_t)(d.rows() * d.D) * elem_size(dtype), st));
+    MSDA_CUDA(cudaMemsetAsync(output, 0, (size_t)(d.rows() * d.D) * elem_size(fused_value_dtype(dtype)), st));
     return MSDA_OK;
   }
   if (!input || !offset || !w) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
@@ -782,11 +792,12 @@ int dcn_forward(void* stream, const Dims& d, const msda::FusedArgs& fa, const vo
 }
 
 // The body of msda_dcnv3_backward (softmax false: `w` = mask, grad_w = its gradient) and msda_dcnv3_fused_backward
-// (softmax true: `w` = mask logits, grad_w = their gradient; never with MSDA_FLAG_DETERMINISTIC), after dcn_setup.
-// `need` = msda_dcnv3_backward_workspace_bytes of the problem and flags.
+// (softmax true: `w` = mask logits, grad_w = their gradient; never with MSDA_FLAG_DETERMINISTIC; dtype may be an
+// autocast tag), after dcn_setup.  `need` = msda_dcnv3_backward_workspace_bytes of the problem and flags.
 int dcn_backward(void* stream, const Dims& d, const msda::FusedArgs& fa, const void* grad_output, const void* input,
-                 const float* offset, const float* w, void* grad_input, float* grad_offset, float* grad_w,
-                 void* workspace, size_t workspace_bytes, size_t need, int dtype, unsigned flags, bool softmax) {
+                 const void* offset, const void* w, void* grad_input, void* grad_offset, void* grad_w,
+                 void* workspace, size_t workspace_bytes, size_t need, int tag, unsigned flags, bool softmax) {
+  const int dtype = fused_value_dtype(tag);   // the value dtype; `tag` selects the kernels
   const char* w_name = softmax ? "mask_logits" : "mask";
   const char* gw_name = softmax ? "grad_mask_logits" : "grad_mask";
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -827,12 +838,12 @@ int dcn_backward(void* stream, const Dims& d, const msda::FusedArgs& fa, const v
   if (d.n_points() == 0) return MSDA_OK;
   if (!grad_offset || !grad_w) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_offset / %s is null", gw_name);
   if (d.n_value() == 0) {   // nothing to sample: the output does not depend on the offsets or the mask (or its logits)
-    MSDA_CUDA(cudaMemsetAsync(grad_offset, 0, (size_t)d.n_points() * 2 * sizeof(float), st));
-    MSDA_CUDA(cudaMemsetAsync(grad_w, 0, (size_t)d.n_points() * sizeof(float), st));
+    MSDA_CUDA(cudaMemsetAsync(grad_offset, 0, (size_t)d.n_points() * 2 * aux_size(tag), st));
+    MSDA_CUDA(cudaMemsetAsync(grad_w, 0, (size_t)d.n_points() * aux_size(tag), st));
     return MSDA_OK;
   }
   if (!grad_output || !input || !offset || !w) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
-  if (int s = softmax ? bwd_dcn_softmax(st, d, dtype, grad_output, input, offset, w, gi32, grad_offset, grad_w, fa)
+  if (int s = softmax ? bwd_dcn_softmax(st, d, tag, grad_output, input, offset, w, gi32, grad_offset, grad_w, fa)
                       : bwd_dcn(st, d, dtype, grad_output, input, offset, w, gi32, grad_offset, grad_w, fa))
     return s;
   if (two_byte(dtype)) return cast_from_f32(st, gi32, grad_input, d.n_value(), dtype);
@@ -873,7 +884,7 @@ int msda_dcnv3_backward(void* stream, const void* grad_output, const void* input
                       workspace_bytes, need, dtype, flags, false);
 }
 
-int msda_dcnv3_fused_forward(void* stream, const void* input, const float* offset, const float* mask_logits,
+int msda_dcnv3_fused_forward(void* stream, const void* input, const void* offset, const void* mask_logits,
                              int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w,
                              int dilation_h, int dilation_w, int group, int group_channels, float offset_scale,
                              int batch, int height_in, int width_in, int height_out, int width_out, void* output,
@@ -883,22 +894,24 @@ int msda_dcnv3_fused_forward(void* stream, const void* input, const float* offse
   Dims d;
   msda::FusedArgs fa;
   if (int s = dcn_setup(kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
-                        group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
+                        group_channels, offset_scale, batch, height_in, width_in, height_out, width_out,
+                        fused_value_dtype(dtype), &d, &fa))
     return s;
   return dcn_forward(stream, d, fa, input, offset, mask_logits, output, dtype, true);
 }
 
-int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void* input, const float* offset,
-                              const float* mask_logits, int kernel_h, int kernel_w, int stride_h, int stride_w,
+int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void* input, const void* offset,
+                              const void* mask_logits, int kernel_h, int kernel_w, int stride_h, int stride_w,
                               int pad_h, int pad_w, int dilation_h, int dilation_w, int group, int group_channels,
                               float offset_scale, int batch, int height_in, int width_in, int height_out,
-                              int width_out, void* grad_input, float* grad_offset, float* grad_mask_logits,
+                              int width_out, void* grad_input, void* grad_offset, void* grad_mask_logits,
                               void* workspace, size_t workspace_bytes, int dtype, unsigned flags) {
   g_err[0] = 0;
   Dims d;
   msda::FusedArgs fa;
   if (int s = dcn_setup(kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, group,
-                        group_channels, offset_scale, batch, height_in, width_in, height_out, width_out, dtype, &d, &fa))
+                        group_channels, offset_scale, batch, height_in, width_in, height_out, width_out,
+                        fused_value_dtype(dtype), &d, &fa))
     return s;
   // the float-red kernel is the only fused form: a caller that needs bit-reproducible gradients composes the softmax
   // around msda_dcnv3_backward (refused before any device work, empty problems included)

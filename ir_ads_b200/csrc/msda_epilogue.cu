@@ -9,7 +9,9 @@
 //   backward  dx = dLN/d(a+b) (the gradient of BOTH inputs), dgamma, dbeta
 //             reads dy, a, b (the sum is recomputed, never stored)       writes dx, per-CTA partials of dgamma / dbeta
 // One warp per row, 16-byte lane accesses, two-pass mean / variance in registers (the row stays in registers), fp32
-// arithmetic for float and bfloat16 tensors.  dgamma / dbeta are reduced in a fixed order (per-CTA partial sums, then
+// arithmetic for float, bfloat16 and float16 tensors.  The mixed form (TA = 16-bit `a`, TB = float `b` / y / dy / dx)
+// is the one autocast produces -- a 16-bit attention / FFN output plus a float32 residual -- and the backward then
+// writes dx twice: as float for `b` and rounded for `a`.  dgamma / dbeta are reduced in a fixed order (per-CTA partial sums, then
 // one small kernel), so the whole backward is bit-reproducible.  HBM-bound: 3 tensor passes forward, 4 backward.
 #include "msda_host.h"
 
@@ -25,7 +27,20 @@ __device__ __forceinline__ float4 ld_f4(const __nv_bfloat16* p) {
   return make_float4(__uint_as_float(u.x << 16), __uint_as_float(u.x & 0xffff0000u), __uint_as_float(u.y << 16),
                      __uint_as_float(u.y & 0xffff0000u));
 }
+__device__ __forceinline__ float4 ld_f4(const __half* p) {
+  const uint2 u = *reinterpret_cast<const uint2*>(p);
+  const float2 lo = __half22float2(*reinterpret_cast<const __half2*>(&u.x));
+  const float2 hi = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+  return make_float4(lo.x, lo.y, hi.x, hi.y);
+}
 __device__ __forceinline__ void st_f4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ void st_f4(__half* p, float4 v) {
+  const __half2 lo = __floats2half2_rn(v.x, v.y), hi = __floats2half2_rn(v.z, v.w);
+  uint2 u;
+  u.x = *reinterpret_cast<const unsigned*>(&lo);
+  u.y = *reinterpret_cast<const unsigned*>(&hi);
+  *reinterpret_cast<uint2*>(p) = u;
+}
 __device__ __forceinline__ void st_f4(__nv_bfloat16* p, float4 v) {
   const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
   uint2 u;
@@ -39,10 +54,11 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
-// NV = float4 chunks per lane (C == 128 * NV exactly when EXACT, else C <= 128 * NV and chunks are predicated)
-template <typename T, int NV>
+// NV = float4 chunks per lane (C == 128 * NV exactly when EXACT, else C <= 128 * NV and chunks are predicated).
+// T = the type of b and y; TA = the type of a (T, or a 16-bit type when T is float: the mixed form)
+template <typename T, int NV, typename TA = T>
 __global__ void __launch_bounds__(kLnThreads)
-add_layernorm_fwd_kernel(const T* __restrict__ a, const T* __restrict__ b, const float* __restrict__ gamma,
+add_layernorm_fwd_kernel(const TA* __restrict__ a, const T* __restrict__ b, const float* __restrict__ gamma,
                          const float* __restrict__ beta, T* __restrict__ y, float* __restrict__ mean,
                          float* __restrict__ rstd, int64_t rows, int C, float eps) {
   const int lane = threadIdx.x & 31;
@@ -50,7 +66,7 @@ add_layernorm_fwd_kernel(const T* __restrict__ a, const T* __restrict__ b, const
   const int64_t stride = (int64_t)gridDim.x * (kLnThreads / 32);
   const float inv_c = 1.0f / (float)C;
   for (int64_t row = warp0; row < rows; row += stride) {
-    const T* pa = a + row * C;
+    const TA* pa = a + row * C;
     const T* pb = b + row * C;
     float4 s[NV];
     float sum = 0.0f;
@@ -93,12 +109,14 @@ add_layernorm_fwd_kernel(const T* __restrict__ a, const T* __restrict__ b, const
 
 // dx = rstd * (g - mean(g) - xhat * mean(g * xhat)),  g = dy * gamma,  xhat = (a + b - mean) * rstd
 // partial[blockIdx.x][0][c] = sum over the CTA's rows of dy * xhat (dgamma), [1][c] = sum of dy (dbeta)
-template <typename T, int NV>
+// Mixed form (TA != T): dx_a = dx rounded to TA, stored in the same pass
+template <typename T, int NV, typename TA = T>
 __global__ void __launch_bounds__(kLnThreads)
-add_layernorm_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ a, const T* __restrict__ b,
+add_layernorm_bwd_kernel(const T* __restrict__ dy, const TA* __restrict__ a, const T* __restrict__ b,
                          const float* __restrict__ gamma, const float* __restrict__ mean,
-                         const float* __restrict__ rstd, T* __restrict__ dx, float* __restrict__ partial,
-                         int64_t rows, int C) {
+                         const float* __restrict__ rstd, T* __restrict__ dx, TA* __restrict__ dx_a,
+                         float* __restrict__ partial, int64_t rows, int C) {
+  static_assert(std::is_same_v<TA, T> || (std::is_same_v<T, float> && sizeof(TA) == 2), "mixed form: 16-bit a, float b");
   extern __shared__ __align__(16) float red[];          // [warps][2][C]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t warp0 = (int64_t)blockIdx.x * (kLnThreads / 32) + warp;
@@ -133,9 +151,12 @@ add_layernorm_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ a, cons
 #pragma unroll
     for (int v = 0; v < NV; ++v) {
       const int c = (v * 32 + lane) * 4;
-      if (c < C)
-        st_f4(dx + row * C + c, make_float4(rs * (g[v].x - m1 - xh[v].x * m2), rs * (g[v].y - m1 - xh[v].y * m2),
-                                            rs * (g[v].z - m1 - xh[v].z * m2), rs * (g[v].w - m1 - xh[v].w * m2)));
+      if (c < C) {
+        const float4 r = make_float4(rs * (g[v].x - m1 - xh[v].x * m2), rs * (g[v].y - m1 - xh[v].y * m2),
+                                     rs * (g[v].z - m1 - xh[v].z * m2), rs * (g[v].w - m1 - xh[v].w * m2));
+        st_f4(dx + row * C + c, r);
+        if constexpr (!std::is_same_v<TA, T>) st_f4(dx_a + row * C + c, r);
+      }
     }
   }
   // CTA-level reduction of dgamma / dbeta in a fixed order (warp 0..7), then one partial row per CTA
@@ -177,7 +198,8 @@ int ln_grid(int64_t rows) {
 
 int check_ln(int64_t rows, int C, int dtype) {
   if (rows < 0 || C < 0) return fail(MSDA_ERR_INVALID_ARGUMENT, "negative size (rows=%lld C=%d)", (long long)rows, C);
-  if (dtype != MSDA_F32 && dtype != MSDA_BF16) return fail(MSDA_ERR_UNSUPPORTED, "add_layernorm: float32 / bfloat16 only");
+  if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16)
+    return fail(MSDA_ERR_UNSUPPORTED, "add_layernorm: float32 / bfloat16 / float16 only");
   if (C % 4 != 0 || C > 128 * kLnMaxVec)
     return fail(MSDA_ERR_UNSUPPORTED, "add_layernorm: channels must be a multiple of 4 and <= %d (got %d)", 128 * kLnMaxVec, C);
   return MSDA_OK;
@@ -185,33 +207,41 @@ int check_ln(int64_t rows, int C, int dtype) {
 
 }  // namespace
 
-extern "C" {
-
-size_t msda_add_layernorm_workspace_bytes(int64_t rows, int channels) {
+extern "C" size_t msda_add_layernorm_workspace_bytes(int64_t rows, int channels) {
   if (rows <= 0 || channels <= 0) return 0;
   return (size_t)ln_grid(rows) * 2 * (size_t)channels * sizeof(float);
 }
 
-int msda_add_layernorm_forward(void* stream, const void* a, const void* b, const float* gamma, const float* beta,
-                               int64_t rows, int channels, float eps, void* y, float* mean, float* rstd, int dtype) {
-  if (int s = check_ln(rows, channels, dtype)) return s;
+namespace {
+// The bodies of the same-dtype entry points (mixed false: a, b, y, grad_* all `dtype`) and of the mixed ones (mixed
+// true: `a` / grad_a in the 16-bit `dtype`, b, y, grad_y, grad_b float), after check_ln.
+int ln_forward(void* stream, const void* a, const void* b, const float* gamma, const float* beta, int64_t rows,
+               int channels, float eps, void* y, float* mean, float* rstd, int dtype, bool mixed) {
   if (rows == 0 || channels == 0) return MSDA_OK;
   if (!a || !b || !gamma || !beta || !y || !mean || !rstd) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
   if (int s = check_alignment({{"a", a}, {"b", b}, {"gamma", gamma}, {"beta", beta}, {"y", y}})) return s;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int grid = ln_grid(rows);
   const int nv = (channels + 127) / 128;
-#define LN_FWD(T_, NV_)                                                                                              \
-  add_layernorm_fwd_kernel<T_, NV_><<<grid, kLnThreads, 0, st>>>((const T_*)a, (const T_*)b, gamma, beta, (T_*)y, mean, \
-                                                                 rstd, rows, channels, eps)
-#define LN_FWD_NV(T_)                                   \
+#define LN_FWD(T_, NV_, TA_)                                                                                        \
+  add_layernorm_fwd_kernel<T_, NV_, TA_><<<grid, kLnThreads, 0, st>>>((const TA_*)a, (const T_*)b, gamma, beta, (T_*)y, \
+                                                                      mean, rstd, rows, channels, eps)
+#define LN_FWD_NV(T_, TA_)                              \
   switch (nv) {                                         \
-    case 1: LN_FWD(T_, 1); break;                       \
-    case 2: LN_FWD(T_, 2); break;                       \
-    case 3: case 4: LN_FWD(T_, 4); break;               \
-    default: LN_FWD(T_, 8); break;                      \
+    case 1: LN_FWD(T_, 1, TA_); break;                  \
+    case 2: LN_FWD(T_, 2, TA_); break;                  \
+    case 3: case 4: LN_FWD(T_, 4, TA_); break;          \
+    default: LN_FWD(T_, 8, TA_); break;                 \
   }
-  if (dtype == MSDA_F32) { LN_FWD_NV(float) } else { LN_FWD_NV(__nv_bfloat16) }
+  if (mixed) {
+    if (dtype == MSDA_BF16) { LN_FWD_NV(float, __nv_bfloat16) } else { LN_FWD_NV(float, __half) }
+  } else if (dtype == MSDA_F32) {
+    LN_FWD_NV(float, float)
+  } else if (dtype == MSDA_BF16) {
+    LN_FWD_NV(__nv_bfloat16, __nv_bfloat16)
+  } else {
+    LN_FWD_NV(__half, __half)
+  }
 #undef LN_FWD_NV
 #undef LN_FWD
   count_launch();
@@ -219,11 +249,9 @@ int msda_add_layernorm_forward(void* stream, const void* a, const void* b, const
   return MSDA_OK;
 }
 
-int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a, const void* b, const float* gamma,
-                                const float* mean, const float* rstd, int64_t rows, int channels, void* grad_x,
-                                float* grad_gamma, float* grad_beta, void* workspace, size_t workspace_bytes,
-                                int dtype) {
-  if (int s = check_ln(rows, channels, dtype)) return s;
+int ln_backward(void* stream, const void* grad_y, const void* a, const void* b, const float* gamma, const float* mean,
+                const float* rstd, int64_t rows, int channels, void* grad_x, void* grad_a, float* grad_gamma,
+                float* grad_beta, void* workspace, size_t workspace_bytes, int dtype, bool mixed) {
   if (channels == 0) return MSDA_OK;
   if (!grad_gamma || !grad_beta) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_gamma / grad_beta is null");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -232,8 +260,10 @@ int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a,
     MSDA_CUDA(cudaMemsetAsync(grad_beta, 0, (size_t)channels * sizeof(float), st));
     return MSDA_OK;
   }
-  if (!grad_y || !a || !b || !gamma || !mean || !rstd || !grad_x) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
-  if (int s = check_alignment({{"grad_y", grad_y}, {"a", a}, {"b", b}, {"gamma", gamma}, {"grad_x", grad_x},
+  if (!grad_y || !a || !b || !gamma || !mean || !rstd || !grad_x || (mixed && !grad_a))
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  if (int s = check_alignment({{"grad_y", grad_y}, {"a", a}, {"b", b}, {"gamma", gamma},
+                               {mixed ? "grad_b" : "grad_x", grad_x}, {"grad_a", mixed ? grad_a : nullptr},
                                {"workspace", workspace}}))
     return s;
   const size_t need = msda_add_layernorm_workspace_bytes(rows, channels);
@@ -243,21 +273,29 @@ int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a,
   const int nv = (channels + 127) / 128;
   const size_t smem = (size_t)(kLnThreads / 32) * 2 * channels * sizeof(float);
   float* partial = static_cast<float*>(workspace);
-#define LN_BWD(T_, NV_)                                                                                     \
+#define LN_BWD(T_, NV_, TA_)                                                                                \
   do {                                                                                                      \
-    auto k = add_layernorm_bwd_kernel<T_, NV_>;                                                             \
+    auto k = add_layernorm_bwd_kernel<T_, NV_, TA_>;                                                        \
     MSDA_CUDA(ensure_smem(k, smem));                                                                        \
-    k<<<grid, kLnThreads, smem, st>>>((const T_*)grad_y, (const T_*)a, (const T_*)b, gamma, mean, rstd,     \
-                                      (T_*)grad_x, partial, rows, channels);                                \
+    k<<<grid, kLnThreads, smem, st>>>((const T_*)grad_y, (const TA_*)a, (const T_*)b, gamma, mean, rstd,    \
+                                      (T_*)grad_x, (TA_*)grad_a, partial, rows, channels);                  \
   } while (0)
-#define LN_BWD_NV(T_)                                   \
+#define LN_BWD_NV(T_, TA_)                              \
   switch (nv) {                                         \
-    case 1: LN_BWD(T_, 1); break;                       \
-    case 2: LN_BWD(T_, 2); break;                       \
-    case 3: case 4: LN_BWD(T_, 4); break;               \
-    default: LN_BWD(T_, 8); break;                      \
+    case 1: LN_BWD(T_, 1, TA_); break;                  \
+    case 2: LN_BWD(T_, 2, TA_); break;                  \
+    case 3: case 4: LN_BWD(T_, 4, TA_); break;          \
+    default: LN_BWD(T_, 8, TA_); break;                 \
   }
-  if (dtype == MSDA_F32) { LN_BWD_NV(float) } else { LN_BWD_NV(__nv_bfloat16) }
+  if (mixed) {
+    if (dtype == MSDA_BF16) { LN_BWD_NV(float, __nv_bfloat16) } else { LN_BWD_NV(float, __half) }
+  } else if (dtype == MSDA_F32) {
+    LN_BWD_NV(float, float)
+  } else if (dtype == MSDA_BF16) {
+    LN_BWD_NV(__nv_bfloat16, __nv_bfloat16)
+  } else {
+    LN_BWD_NV(__half, __half)
+  }
 #undef LN_BWD_NV
 #undef LN_BWD
   count_launch();
@@ -266,6 +304,47 @@ int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a,
   count_launch();
   MSDA_CUDA(cudaGetLastError());
   return MSDA_OK;
+}
+
+// the mixed form: `a` bfloat16 or float16, everything else float
+int check_ln_mixed(int64_t rows, int C, int a_dtype) {
+  if (a_dtype != MSDA_BF16 && a_dtype != MSDA_F16)
+    return fail(MSDA_ERR_UNSUPPORTED, "add_layernorm mixed: `a` must be bfloat16 or float16 (b float32)");
+  return check_ln(rows, C, a_dtype);
+}
+}  // namespace
+
+extern "C" {
+
+int msda_add_layernorm_forward(void* stream, const void* a, const void* b, const float* gamma, const float* beta,
+                               int64_t rows, int channels, float eps, void* y, float* mean, float* rstd, int dtype) {
+  if (int s = check_ln(rows, channels, dtype)) return s;
+  return ln_forward(stream, a, b, gamma, beta, rows, channels, eps, y, mean, rstd, dtype, false);
+}
+
+int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a, const void* b, const float* gamma,
+                                const float* mean, const float* rstd, int64_t rows, int channels, void* grad_x,
+                                float* grad_gamma, float* grad_beta, void* workspace, size_t workspace_bytes,
+                                int dtype) {
+  if (int s = check_ln(rows, channels, dtype)) return s;
+  return ln_backward(stream, grad_y, a, b, gamma, mean, rstd, rows, channels, grad_x, nullptr, grad_gamma, grad_beta,
+                     workspace, workspace_bytes, dtype, false);
+}
+
+int msda_add_layernorm_mixed_forward(void* stream, const void* a, const float* b, const float* gamma,
+                                     const float* beta, int64_t rows, int channels, float eps, float* y, float* mean,
+                                     float* rstd, int a_dtype) {
+  if (int s = check_ln_mixed(rows, channels, a_dtype)) return s;
+  return ln_forward(stream, a, b, gamma, beta, rows, channels, eps, y, mean, rstd, a_dtype, true);
+}
+
+int msda_add_layernorm_mixed_backward(void* stream, const float* grad_y, const void* a, const float* b,
+                                      const float* gamma, const float* mean, const float* rstd, int64_t rows,
+                                      int channels, void* grad_a, float* grad_b, float* grad_gamma, float* grad_beta,
+                                      void* workspace, size_t workspace_bytes, int a_dtype) {
+  if (int s = check_ln_mixed(rows, channels, a_dtype)) return s;
+  return ln_backward(stream, grad_y, a, b, gamma, mean, rstd, rows, channels, grad_b, grad_a, grad_gamma, grad_beta,
+                     workspace, workspace_bytes, a_dtype, true);
 }
 
 }  // extern "C"

@@ -594,17 +594,57 @@ __device__ __forceinline__ float2 dcn_location(const float2 off, int pt, int q, 
   return loc;
 }
 
+// ---- element type of loc / w and their gradients (AT) ----------------------------------------------------------
+// float, or -- in the record modes whose `w` holds logits (fused MSDA chain, fused DCNv3) -- the value's own 16-bit
+// type, which is what the module's Linear layers produce under autocast.  Widening f16 / bf16 to float is exact, so the
+// kernels compute on the same floats either way; gradients are rounded once, to nearest even, as a cast would.
+__device__ __forceinline__ float2 ld_xy(const float* base, int pt) {   // the (x, y) pair of point pt
+  return __ldg(reinterpret_cast<const float2*>(base) + pt);
+}
+__device__ __forceinline__ float2 ld_xy(const __half* base, int pt) {
+  const unsigned u = __ldg(reinterpret_cast<const unsigned*>(base) + pt);
+  return __half22float2(*reinterpret_cast<const __half2*>(&u));
+}
+__device__ __forceinline__ float2 ld_xy(const __nv_bfloat16* base, int pt) {
+  const unsigned u = __ldg(reinterpret_cast<const unsigned*>(base) + pt);
+  return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u));
+}
+__device__ __forceinline__ float ld_aux(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_aux(const __half* p) { return __half2float(__ldg(p)); }
+__device__ __forceinline__ float ld_aux(const __nv_bfloat16* p) { return __bfloat162float(__ldg(p)); }
+// two gradients as one store: 8 bytes of float, 4 of f16 / bf16
+__device__ __forceinline__ void st_aux2(float* p, float a, float b) { *reinterpret_cast<float2*>(p) = make_float2(a, b); }
+__device__ __forceinline__ void st_aux2(__half* p, float a, float b) { *reinterpret_cast<unsigned*>(p) = pack_f16x2(a, b); }
+__device__ __forceinline__ void st_aux2(__nv_bfloat16* p, float a, float b) {
+  const __nv_bfloat162 t = __floats2bfloat162_rn(a, b);
+  *reinterpret_cast<unsigned*>(p) = *reinterpret_cast<const unsigned*>(&t);
+}
+// four gradients as one store: 16 bytes of float, 8 of f16 / bf16
+__device__ __forceinline__ void st_aux4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ void st_aux4(__half* p, float4 v) { st4(p, v); }
+__device__ __forceinline__ void st_aux4(__nv_bfloat16* p, float4 v) { st4(p, v); }
+__device__ __forceinline__ void st_aux1(float* p, float a) { *p = a; }
+__device__ __forceinline__ void st_aux1(__half* p, float a) { *p = __float2half_rn(a); }
+__device__ __forceinline__ void st_aux1(__nv_bfloat16* p, float a) { *p = __float2bfloat16_rn(a); }
+// the (value type, aux type) pairs the kernels are built for: AT == float, or AT == VT (16-bit) in a logits mode
+// (kPreFused, kPreDcnSoftmax) and the one row order per pass the product library carries for it (ORDER_16)
+template <typename VT, typename AT, int PRE, int ORDER, int ORDER_16>
+__host__ __device__ constexpr bool aux_ok() {
+  return std::is_same_v<AT, float> ||
+         (std::is_same_v<AT, VT> && sizeof(VT) == 2 && (PRE == 1 || PRE == 3) && ORDER == ORDER_16);
+}
+
 // softmax over the row's NP logits by the row's LANES lanes; e_i = exp(x_i - max) is left in
 // scratch[pt] (one float per point, any 4-byte stride) and the sum is returned: w_i = e_i / sum.
 // VLANES = 2 * LANES (rows of 8 channels per lane) forms the sum in the order of VLANES lanes: lane `sub` adds up the
 // points of virtual lanes sub and sub + LANES separately and then the two -- the first butterfly step of the wider
 // order -- so the weights are bit for bit those of the 4-channel-per-lane rows (f16 forward == f32 forward).
-template <int LANES, int STRIDE, int VLANES = LANES>
-__device__ __forceinline__ float row_softmax(const float* logits_row, float* scratch, int NP, int sub) {
+template <int LANES, int STRIDE, int VLANES = LANES, typename AT>
+__device__ __forceinline__ float row_softmax(const AT* logits_row, float* scratch, int NP, int sub) {
   static_assert(VLANES == LANES || VLANES == 2 * LANES, "one or two virtual lanes per lane");
   float m = -3.402823466e38f;
   for (int pt = sub; pt < NP; pt += LANES) {
-    const float x = __ldg(logits_row + pt);
+    const float x = ld_aux(logits_row + pt);
     scratch[pt * STRIDE] = x;
     m = fmaxf(m, x);
   }
@@ -631,17 +671,18 @@ __device__ __forceinline__ float row_softmax(const float* logits_row, float* scr
 // =============================================================================================
 // One pass per CTA (TILE2D: a grid-stride step for pathological pyramids); phase 1 reads loc/w straight from
 // global memory.
-template <int D, typename VT, int PT, int THREADS, int ORDER, int PRE, int CPL>
+template <int D, typename VT, int PT, int THREADS, int ORDER, int PRE, int CPL, typename AT = float>
 #ifndef MSDA_FWD_MINB
 #define MSDA_FWD_MINB 6
 #endif
 __global__ void __launch_bounds__(THREADS, MSDA_FWD_MINB * (256 / THREADS))
 msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ shapes,
-                     const int64_t* __restrict__ lsi, const float* __restrict__ loc,
-                     const float* __restrict__ w, VT* __restrict__ out, const FusedArgs fused, int B, int S, int H,
+                     const int64_t* __restrict__ lsi, const AT* __restrict__ loc,
+                     const AT* __restrict__ w, VT* __restrict__ out, const FusedArgs fused, int B, int S, int H,
                      int L, int Q, int P, int64_t rows) {
   // FUSED: `loc` holds raw sampling offsets and `w` attention logits (see FusedArgs)
   static_assert(THREADS <= 256, "single-pass CTAs");
+  static_assert(aux_ok<VT, AT, PRE, ORDER, 0>(), "16-bit offsets / logits: fused modes, value's dtype, LINEAR forward");
   constexpr int DL = D * 4 / CPL;               // lane geometry: LANES = D / CPL lanes per row
   using G = Geom<DL, THREADS>;
   constexpr int LANES = G::LANES;
@@ -693,8 +734,8 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
     for (int i = 0; i < kEarly; ++i) {
       const int pt = sub + i * LANES;
       const bool on = cur.live && pt < NP;
-      early_xy[i] = on ? __ldg(reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2) + pt) : make_float2(0.f, 0.f);
-      early_w[i] = (on && !SOFTMAX) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
+      early_xy[i] = on ? ld_xy(loc + cur.row * (int64_t)NP * 2, pt) : make_float2(0.f, 0.f);
+      early_w[i] = (on && !SOFTMAX) ? ld_aux(w + cur.row * (int64_t)NP + pt) : 0.0f;
     }
     // the softmax shuffles need the whole warp; dead rows read row 0 and simply produce nothing
     if constexpr (SOFTMAX) early_sum = row_softmax<LANES, 1, SM_LANES>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_oc), NP, sub);
@@ -710,8 +751,8 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
   while (true) {
     // ---- phase 1: records ----
     {
-      const float2* lp = reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2);
-      const float* wp = w + cur.row * (int64_t)NP;
+      const AT* lp = loc + cur.row * (int64_t)NP * 2;
+      const AT* wp = w + cur.row * (int64_t)NP;
       float sm_sum = early_sum;
       if constexpr (SOFTMAX && !EARLY) sm_sum = row_softmax<LANES, 1, SM_LANES>(wp, reinterpret_cast<float*>(s_oc), NP, sub);
       if (cur.live) {
@@ -746,7 +787,7 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
           for (int i = 0; i < kEarly; ++i, pt += LANES)
             if (pt < NP) build(pt, early_xy[i], early_w[i]);
         }
-        for (; pt < NP; pt += LANES) build(pt, __ldg(lp + pt), SOFTMAX ? 0.0f : __ldg(wp + pt));
+        for (; pt < NP; pt += LANES) build(pt, ld_xy(lp, pt), SOFTMAX ? 0.0f : ld_aux(wp + pt));
       }
     }
     __syncwarp();
@@ -959,13 +1000,13 @@ __device__ __forceinline__ void transpose_reduce_4x4(float (&d)[16], int sub) {
 #ifndef MSDA_BWD_MINB
 #define MSDA_BWD_MINB 4
 #endif
-template <int D, typename VT, int PT, int THREADS, int ORDER, typename ACC, int PRE, int CPL>
+template <int D, typename VT, int PT, int THREADS, int ORDER, typename ACC, int PRE, int CPL, typename AT = float>
 __global__ void __launch_bounds__(THREADS, MSDA_BWD_MINB * (256 / THREADS))
 msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ value,
                      const int64_t* __restrict__ shapes, const int64_t* __restrict__ lsi,
-                     const float* __restrict__ loc, const float* __restrict__ w,
-                     ACC* __restrict__ grad_value, float* __restrict__ grad_loc,
-                     float* __restrict__ grad_w, const DetScale* __restrict__ det, const FusedArgs fused,
+                     const AT* __restrict__ loc, const AT* __restrict__ w,
+                     ACC* __restrict__ grad_value, AT* __restrict__ grad_loc,
+                     AT* __restrict__ grad_w, const DetScale* __restrict__ det, const FusedArgs fused,
                      const EmitArgs emit, int B, int S, int H, int L, int Q, int P, int64_t rows) {
   // FUSED: loc = raw offsets, w = logits in; grad_loc = grad of the offsets, grad_w = grad of the logits out
   static_assert(THREADS <= 256, "single-pass CTAs");
@@ -976,6 +1017,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
   // the fused DCNv3 module path has no deterministic or no-scatter form (its deterministic backward is composed
   // around the kPreDcn kernels, ir_ads_b200/dcnv3.py)
   static_assert(PRE != kPreDcnSoftmax || std::is_same_v<ACC, float>, "the fused DCNv3 backward uses float reds");
+  static_assert(aux_ok<VT, AT, PRE, ORDER, 2>() && (std::is_same_v<AT, float> || std::is_same_v<ACC, float>),
+                "16-bit offsets / logits: fused modes, value's dtype, float reds, STRIP backward");
   constexpr int DL = D * 4 / CPL;
   using G = Geom<DL, THREADS>;
   constexpr int LANES = G::LANES;
@@ -1018,8 +1061,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     for (int i = 0; i < kEarly; ++i) {
       const int pt = sub + i * LANES;
       const bool on = cur.live && pt < NP;
-      early_xy[i] = on ? __ldg(reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2) + pt) : make_float2(0.f, 0.f);
-      early_w[i] = (on && !SOFTMAX) ? __ldg(w + cur.row * (int64_t)NP + pt) : 0.0f;
+      early_xy[i] = on ? ld_xy(loc + cur.row * (int64_t)NP * 2, pt) : make_float2(0.f, 0.f);
+      early_w[i] = (on && !SOFTMAX) ? ld_aux(w + cur.row * (int64_t)NP + pt) : 0.0f;
     }
     if constexpr (SOFTMAX)
       early_sum = row_softmax<LANES, 4>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
@@ -1047,8 +1090,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     if constexpr (!EARLY) go = cur.live ? ldv<CPL>(grad_out + cur.row * D + sub * CPL) : vzero<CPL>();
     const float* rp = FUSED ? fused.ref + (cur.row / H) * (int64_t)L * fused.ref_dim : nullptr;
     {
-      const float2* lp = reinterpret_cast<const float2*>(loc + cur.row * (int64_t)NP * 2);
-      const float* wp = w + cur.row * (int64_t)NP;
+      const AT* lp = loc + cur.row * (int64_t)NP * 2;
+      const AT* wp = w + cur.row * (int64_t)NP;
       float sm_sum = early_sum;
       if constexpr (SOFTMAX && !EARLY) sm_sum = row_softmax<LANES, 4>(wp, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
       // one record from a point's raw location / weight (FUSED: raw offset; SOFTMAX: the weight comes from the
@@ -1095,8 +1138,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
         float2 xy = make_float2(0.f, 0.f);
         float aw = 0.0f;
         if (cur.live) {
-          xy = __ldg(lp + pt);
-          if constexpr (!SOFTMAX) aw = __ldg(wp + pt);
+          xy = ld_xy(lp, pt);
+          if constexpr (!SOFTMAX) aw = ld_aux(wp + pt);
         }
         build(pt, xy, aw);
       }
@@ -1121,8 +1164,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
       gsc = reinterpret_cast<float*>(grad_value) + (int64_t)cur.b * S * HD + sub * 4;
       asm volatile("" : "+l"(gsc));
     }   // one 64-bit register each: address = base + off*size (IMAD.WIDE)
-    float* glp = grad_loc + cur.row * (int64_t)NP * 2;
-    float* gwp = grad_w + cur.row * (int64_t)NP;
+    AT* glp = grad_loc + cur.row * (int64_t)NP * 2;
+    AT* gwp = grad_w + cur.row * (int64_t)NP;
 
     float sm_dot = 0.0f;   // SOFTMAX: sum_j grad_aw_j * aw_j of the row (softmax backward)
     for (int c0 = 0; c0 < NP; c0 += 4) {
@@ -1229,7 +1272,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     // Write-out.  One lane per point storing 4 + 8 bytes as it finishes would send every 16-byte piece of grad_attn_weight
     // and every 32-byte piece of grad_sampling_loc through the SM's crossbar port as a request of its own (header + one
     // sector each: 16 port cycles per row at L*P = 16); the port is what binds this kernel.  Parked in the records and
-    // written by the row's lanes two points at a time, a row leaves as one 128-byte and one 64-byte request.
+    // written by the row's lanes two points at a time, a row leaves as one 128-byte and one 64-byte request (16-bit AT:
+    // the same full lines at half the bytes).
     if (cur.live) {
       auto gw_of = [&](const int4 r) {
         const float g_aw = __int_as_float(r.y);
@@ -1238,15 +1282,15 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
       if ((NP & 1) == 0) {      // both row bases are then 16- / 8-byte aligned
         for (int pt = 2 * sub; pt < NP; pt += 2 * LANES) {
           const int4 a = s_fin[pt], b = s_fin[pt + 1];
-          *reinterpret_cast<float4*>(glp + 2 * pt) =
-              make_float4(__int_as_float(a.x), __int_as_float(a.z), __int_as_float(b.x), __int_as_float(b.z));
-          *reinterpret_cast<float2*>(gwp + pt) = make_float2(gw_of(a), gw_of(b));
+          st_aux4(glp + 2 * pt,
+                  make_float4(__int_as_float(a.x), __int_as_float(a.z), __int_as_float(b.x), __int_as_float(b.z)));
+          st_aux2(gwp + pt, gw_of(a), gw_of(b));
         }
       } else {
         for (int pt = sub; pt < NP; pt += LANES) {
           const int4 a = s_fin[pt];
-          *reinterpret_cast<float2*>(glp + 2 * pt) = make_float2(__int_as_float(a.x), __int_as_float(a.z));
-          gwp[pt] = gw_of(a);
+          st_aux2(glp + 2 * pt, __int_as_float(a.x), __int_as_float(a.z));
+          st_aux1(gwp + pt, gw_of(a));
         }
       }
     }

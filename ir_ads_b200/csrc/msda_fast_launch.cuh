@@ -31,27 +31,28 @@ constexpr int kFwdThreads = MSDA_FWD_THREADS, kBwdThreads = MSDA_BWD_THREADS;
 template <int D, typename VT>
 constexpr int cpl_of() { return (sizeof(VT) == 2 && D >= 32) ? 8 : 4; }
 
-template <int D, typename VT, int PT, int THREADS, int ORDER, int PRE = 0>
+// AT: element type of loc / w (float, or the value's 16-bit type in the logits modes, msda::aux_ok)
+template <int D, typename VT, int PT, int THREADS, int ORDER, int PRE = 0, typename AT = float>
 int launch_fwd_fast(cudaStream_t st, const Dims& d, const void* value, const int64_t* shapes, const int64_t* lsi,
                     const void* loc, const void* w, void* out, msda::FusedArgs fa = msda::FusedArgs{}) {
   constexpr int CPL = cpl_of<D, VT>();
   using G = msda::Geom<D * 4 / CPL, THREADS>;
   const int NP = d.L * d.P;
   const size_t smem = sizeof(msda::LevelTab) + (size_t)G::RPC * msda::fwd_row_words(NP) * 4;
-  auto k = msda::msda_fwd_fast_kernel<D, VT, PT, THREADS, ORDER, PRE, CPL>;
+  auto k = msda::msda_fwd_fast_kernel<D, VT, PT, THREADS, ORDER, PRE, CPL, AT>;
   MSDA_CUDA(ensure_smem(k, smem));
   const int64_t rows = d.rows();
   unsigned grid = (unsigned)((rows + G::RPC - 1) / G::RPC);
   if (ORDER == 2) grid = (unsigned)((int64_t)d.B * d.H * ((d.Q + G::RPC - 1) / G::RPC));
   if (ORDER == 3) grid = (unsigned)((int64_t)d.B * d.H * tile2d_bound(d, G::RPC));
-  k<<<grid, THREADS, smem, st>>>((const VT*)value, shapes, lsi, (const float*)loc, (const float*)w, (VT*)out, fa,
+  k<<<grid, THREADS, smem, st>>>((const VT*)value, shapes, lsi, (const AT*)loc, (const AT*)w, (VT*)out, fa,
                                  d.B, d.S, d.H, d.L, d.Q, d.P, rows);
   count_launch();
   MSDA_CUDA(cudaGetLastError());
   return MSDA_OK;
 }
 
-template <int D, typename VT, int PT, int THREADS, int ORDER, typename ACC, int PRE = 0>
+template <int D, typename VT, int PT, int THREADS, int ORDER, typename ACC, int PRE = 0, typename AT = float>
 int launch_bwd_fast(cudaStream_t st, const Dims& d, const void* go, const void* value, const int64_t* shapes,
                     const int64_t* lsi, const void* loc, const void* w, ACC* gv, void* gl, void* gw,
                     const msda::DetScale* det, msda::FusedArgs fa = msda::FusedArgs{},
@@ -63,14 +64,14 @@ int launch_bwd_fast(cudaStream_t st, const Dims& d, const void* go, const void* 
   using G = msda::Geom<D * 4 / CPL, THREADS>;
   const int NP = d.L * d.P;
   const size_t smem = sizeof(msda::LevelTab) + (size_t)G::RPC * msda::bwd_row_words(NP) * 4;
-  auto k = msda::msda_bwd_fast_kernel<D, VT, PT, THREADS, ORDER, ACC, PRE, CPL>;
+  auto k = msda::msda_bwd_fast_kernel<D, VT, PT, THREADS, ORDER, ACC, PRE, CPL, AT>;
   MSDA_CUDA(ensure_smem(k, smem));
   const int64_t rows = d.rows();
   unsigned grid = (unsigned)((rows + G::RPC - 1) / G::RPC);
   if (ORDER == 2) grid = (unsigned)((int64_t)d.B * d.H * ((d.Q + G::RPC - 1) / G::RPC));
   if (ORDER == 3) grid = (unsigned)((int64_t)d.B * d.H * tile2d_bound(d, G::RPC));
-  k<<<grid, THREADS, smem, st>>>((const VT*)go, (const VT*)value, shapes, lsi, (const float*)loc, (const float*)w,
-                                 gv, (float*)gl, (float*)gw, det, fa, emit, d.B, d.S, d.H, d.L, d.Q, d.P, rows);
+  k<<<grid, THREADS, smem, st>>>((const VT*)go, (const VT*)value, shapes, lsi, (const AT*)loc, (const AT*)w,
+                                 gv, (AT*)gl, (AT*)gw, det, fa, emit, d.B, d.S, d.H, d.L, d.Q, d.P, rows);
   count_launch();
   MSDA_CUDA(cudaGetLastError());
   return MSDA_OK;
@@ -105,6 +106,14 @@ int launch_bwd_fast(cudaStream_t st, const Dims& d, const void* go, const void* 
     }                                                        \
   } while (0)
 #endif
+
+// CALL over the value types of the fused kernels with 16-bit offsets / logits (MSDA_BF16_AUX16, MSDA_F16_AUX16): the
+// value's own type is the aux type
+#define MSDA_DISPATCH_VT_AUX16(CALL)                                   \
+  do {                                                                 \
+    if (dtype == MSDA_BF16_AUX16) MSDA_DISPATCH_D(__nv_bfloat16, CALL);\
+    if (dtype == MSDA_F16_AUX16) MSDA_DISPATCH_D(__half, CALL);        \
+  } while (0)
 
 // CALL over the value types of the fast kernels (fast_ok admits no other dtype)
 #define MSDA_DISPATCH_VT(CALL)                                         \

@@ -53,7 +53,7 @@ def _declare(handle):
     return handle
 
 
-def _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels):
+def _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels, aux_checked=False):
     _require(input.is_cuda, "Not implemented on the CPU")
     for name, t in (("input", input), ("offset", offset), ("mask", mask)):
         _require(t.is_cuda and t.device == input.device, f"{name} must be a CUDA tensor on {input.device}")
@@ -67,7 +67,7 @@ def _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels):
     _require(tuple(mask.shape) == (N, H_out, W_out, group * K), "mask must be [N, H_out, W_out, group*K]")
     _require(input.dtype in _DCN_TAG, f"unsupported input dtype {input.dtype}")
     # float16 offset / mask as well: the reference's _C takes them in the input's dtype (dcnv3_cuda.cu:66-80)
-    _require(offset.dtype in (torch.float32, torch.float16) and mask.dtype in (torch.float32, torch.float16),
+    _require(aux_checked or (offset.dtype in (torch.float32, torch.float16) and mask.dtype in (torch.float32, torch.float16)),
              "offset / mask must be float32 or float16")
     return N, H_in, W_in, H_out, W_out
 
@@ -194,27 +194,32 @@ class DCNv3Function(Function):
 # fused module path: the DCNv3 module's mask softmax inside the kernels (csrc/msda_fast.cuh, PRE == 3)
 # ------------------------------------------------------------------------------------------------
 def _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels):
-    dims = _geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels)
-    _require(offset.dtype == torch.float32 and mask_logits.dtype == torch.float32,
-             "offset / mask_logits must be float32")
+    """The problem's dimensions and its dtype tag: offset / mask_logits float32, or both in the input's own 16-bit
+    type (the module's Linear outputs under autocast; MSDA_*_AUX16)."""
+    _require(input.dtype in _DCN_TAG, f"unsupported input dtype {input.dtype}")
+    _require(offset.dtype == mask_logits.dtype, "offset / mask_logits must share a dtype")
+    tag = functional._aux_tag(input.dtype, offset.dtype, "offset / mask_logits")
+    dims = _geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels, aux_checked=True)
     _require(fast_supported(input, kernel_h, kernel_w, group_channels),
              f"fused DCNv3 needs group_channels in {{16, 32, 64, 128}}, kernel_h*kernel_w <= 64 and a float32 / "
              f"bfloat16 / float16 input (got {group_channels}, {kernel_h * kernel_w}, {input.dtype})")
-    return dims
+    return dims, tag
 
 
 def dcnv3_fused_forward(input, offset, mask_logits, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
                         dilation_w, group, group_channels, offset_scale) -> torch.Tensor:
     """``dcnv3_forward`` with ``mask = softmax(mask_logits)`` over each (pixel, group) row of K, the softmax done inside
-    the kernel (``msda_dcnv3_fused_forward``).  ``offset`` / ``mask_logits`` are float32."""
-    N, H_in, W_in, H_out, W_out = _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels)
+    the kernel (``msda_dcnv3_fused_forward``).  ``offset`` / ``mask_logits`` are float32, or both in the input's
+    16-bit dtype."""
+    (N, H_in, W_in, H_out, W_out), tag = _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group,
+                                                         group_channels)
     input, offset, mask_logits = _aligned(input), _aligned(offset), _aligned(mask_logits)
     out = torch.empty((N, H_out, W_out, group * group_channels), dtype=input.dtype, device=input.device)
     stream = torch.cuda.current_stream(input.device).cuda_stream
     status = _declare(_lib.lib()).msda_dcnv3_fused_forward(
         ctypes.c_void_p(stream), _ptr(input), _ptr(offset), _ptr(mask_logits), kernel_h, kernel_w, stride_h, stride_w,
         pad_h, pad_w, dilation_h, dilation_w, group, group_channels, float(offset_scale), N, H_in, W_in, H_out, W_out,
-        _ptr(out), _DCN_TAG[input.dtype], 0)
+        _ptr(out), tag, 0)
     _lib.check(status, "dcnv3_fused_forward")
     return out
 
@@ -223,15 +228,15 @@ def dcnv3_fused_backward(input, offset, mask_logits, kernel_h, kernel_w, stride_
                          dilation_w, group, group_channels, offset_scale, grad_output) -> List[torch.Tensor]:
     """``[grad_input, grad_offset, grad_mask_logits]`` of ``dcnv3_fused_forward``: float reds, the softmax's chain rule
     inside the kernel (``msda_dcnv3_fused_backward``).  There is no deterministic form; ``DCNv3FusedFunction``
-    composes one."""
-    N, H_in, W_in, H_out, W_out = _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group, group_channels)
+    composes one.  The offset / logit gradients come back in the dtype of offset / mask_logits."""
+    (N, H_in, W_in, H_out, W_out), tag = _fused_geometry(input, offset, mask_logits, kernel_h, kernel_w, group,
+                                                         group_channels)
     _require(grad_output.is_cuda and grad_output.dtype == input.dtype, "grad_output must match input's device / dtype")
     grad_output = _aligned(grad_output.contiguous())
     input, offset, mask_logits = _aligned(input), _aligned(offset), _aligned(mask_logits)
     grad_input = torch.empty_like(input)
     grad_offset = torch.empty_like(offset)
     grad_logits = torch.empty_like(mask_logits)
-    tag = _DCN_TAG[input.dtype]
     handle = _declare(_lib.lib())
     ws_bytes = handle.msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, N, H_in, W_in,
                                                           H_out, W_out, tag, 0)
@@ -251,8 +256,10 @@ class DCNv3FusedFunction(Function):
     dilation_w, group, group_channels, offset_scale, im2col_step)``: ``DCNv3Function`` with the mask replaced by its
     pre-softmax logits ``[N, H_out, W_out, group*K]`` -- the DCNv3 module's ``softmax(mask(x1).reshape(..., group,
     K), -1)`` runs inside the kernels, so the mask and its gradient never reach HBM.  Gradients for ``input``,
-    ``offset`` and ``mask_logits``.  ``offset`` / ``mask_logits`` are float32; ``input`` is float32, bfloat16 or
-    float16 on the fast-kernel shapes (``fast_supported``) -- anything else raises, the module composes instead.
+    ``offset`` and ``mask_logits``.  ``offset`` / ``mask_logits`` are float32, or -- as autocast produces them -- both
+    in the input's dtype when that is bfloat16 / float16, and their gradients then come back in that dtype (the
+    float32 gradients rounded once inside the kernel); ``input`` is float32, bfloat16 or float16 on the fast-kernel
+    shapes (``fast_supported``) -- anything else raises, the module composes instead.
 
     Deterministic mode (set_deterministic / torch.use_deterministic_algorithms), as MSDeformAttnFusedFunction: the
     forward is the same fused kernel (it has no atomics); the backward forms the mask with torch.softmax, runs the
@@ -276,14 +283,16 @@ class DCNv3FusedFunction(Function):
         grad_output = grad_output.to(input.dtype)
         if not functional._flags(True) & _lib.FLAG_DETERMINISTIC:
             return tuple(dcnv3_fused_backward(input, offset, mask_logits, *ctx.args, grad_output)) + (None,) * 12
+        # 16-bit offset / logits are widened (exact) and the final gradients cast: the float32 route's bits
+        aux_dtype = offset.dtype
         N, H_out, W_out, _ = mask_logits.shape
         with torch.enable_grad():
-            logits = mask_logits.detach().view(N, H_out, W_out, ctx.args[8], -1).requires_grad_(True)
+            logits = mask_logits.detach().float().view(N, H_out, W_out, ctx.args[8], -1).requires_grad_(True)
             mask = torch.softmax(logits, -1)
-        gi, go, gm = dcnv3_backward(input, offset, mask.detach().view(N, H_out, W_out, -1), *ctx.args, grad_output,
-                                    ctx.im2col_step)
+        gi, go, gm = dcnv3_backward(input, offset.float(), mask.detach().view(N, H_out, W_out, -1), *ctx.args,
+                                    grad_output, ctx.im2col_step)
         (g_logits,) = torch.autograd.grad(mask, logits, gm.view_as(mask))
-        return (gi, go, g_logits.view_as(mask_logits)) + (None,) * 12
+        return (gi, go.to(aux_dtype), g_logits.view_as(mask_logits).to(aux_dtype)) + (None,) * 12
 
 
 # ------------------------------------------------------------------------------------------------
@@ -385,10 +394,14 @@ class DCNv3(nn.Module):
         geometry = (self.kernel_size, self.kernel_size, self.stride, self.stride, self.pad, self.pad, self.dilation,
                     self.dilation, self.group, self.group_channels, self.offset_scale, 256)
         if fast_supported(x, self.kernel_size, self.kernel_size, self.group_channels):
-            # fused: the mask softmax runs inside the kernels on the float32 logits (under autocast the mask is
-            # therefore not rounded to the input dtype, as the composition below rounds it)
-            x = DCNv3FusedFunction.apply(x.contiguous(), offset.float().contiguous(),
-                                         self.mask(x1).float().reshape(N, H, W, -1).contiguous(), *geometry)
+            # fused: the mask softmax runs inside the kernels on float32 logits (under autocast the mask is therefore
+            # not rounded to the input dtype, as the composition below rounds it).  16-bit Linear outputs in the
+            # input's dtype (autocast) go in as they are: the kernels widen them exactly and round their gradients.
+            mask_logits = self.mask(x1)
+            if not (offset.dtype == mask_logits.dtype == dtype and dtype in (torch.float16, torch.bfloat16)):
+                offset, mask_logits = offset.float(), mask_logits.float()
+            x = DCNv3FusedFunction.apply(x.contiguous(), offset.contiguous(),
+                                         mask_logits.reshape(N, H, W, -1).contiguous(), *geometry)
         else:
             mask = F.softmax(self.mask(x1).reshape(N, H, W, self.group, -1), -1).reshape(N, H, W, -1).type(dtype)
             x = DCNv3Function.apply(x.contiguous(), offset.contiguous(), mask.contiguous(), *geometry)

@@ -32,6 +32,19 @@ _DTYPE_TAG = {torch.float32: _lib.MSDA_F32, torch.float64: _lib.MSDA_F64, torch.
 # widens it exactly and accumulates in float32).  The public operator keeps refusing float16, as the reference's does.
 _VALUE_TAG = {**_DTYPE_TAG, torch.float16: _lib.MSDA_F16}
 _FUSED_DTYPES = (torch.float32, torch.bfloat16, torch.float16)
+# the fused paths' autocast tags: 16-bit value AND 16-bit offsets / logits (the Linear outputs as autocast produces them)
+_AUX16_TAG = {torch.bfloat16: _lib.MSDA_BF16_AUX16, torch.float16: _lib.MSDA_F16_AUX16}
+
+
+def _aux_tag(value_dtype, aux_dtype, what):
+    """The dtype tag of a fused call: the value's tag with float32 offsets / logits, its autocast tag when they are in
+    the value's own 16-bit type; any other mix is refused."""
+    if aux_dtype == torch.float32:
+        return _VALUE_TAG[value_dtype]
+    _require(aux_dtype == value_dtype and value_dtype in _AUX16_TAG,
+             f"{what} must be float32, or in the value's dtype when that is float16 / bfloat16 "
+             f"(got {aux_dtype} with a {value_dtype} value)")
+    return _AUX16_TAG[value_dtype]
 
 _state = {"deterministic": False, "flags": 0}
 
@@ -240,8 +253,9 @@ def _check_fused_inputs(value, spatial_shapes, level_start_index, sampling_offse
              "spatial_shapes / level_start_index must be int64")
     _require(tuple(spatial_shapes.shape) == (L, 2) and tuple(level_start_index.shape) == (L,),
              "spatial_shapes must be [L, 2] and level_start_index [L]")
-    _require(sampling_offsets.dtype == torch.float32 and attn_logits.dtype == torch.float32
-             and reference_points.dtype == torch.float32, "offsets / logits / reference_points must be float32")
+    _require(sampling_offsets.dtype == attn_logits.dtype, "sampling_offsets / attn_logits must share a dtype")
+    tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
+    _require(reference_points.dtype == torch.float32, "reference_points must be float32")
     _require(tuple(attn_logits.shape) == (B, Q, H, L * P), "attn_logits must be [B, Q, H, L*P]")
     ref_dim = reference_points.shape[-1]
     _require(tuple(reference_points.shape) == (B, Q, L, ref_dim) and ref_dim in (2, 4),
@@ -253,7 +267,7 @@ def _check_fused_inputs(value, spatial_shapes, level_start_index, sampling_offse
         _require(key_padding_mask.is_cuda and key_padding_mask.device == value.device,
                  f"key_padding_mask must be a CUDA tensor on {value.device}")
         mask = key_padding_mask.contiguous()   # one byte per pixel either way; non-zero = padded
-    return (B, S, H, D, L, Q, P, ref_dim), mask
+    return (B, S, H, D, L, Q, P, ref_dim), mask, tag
 
 
 def _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_points):
@@ -272,8 +286,10 @@ def _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_poin
 class MSDeformAttnFusedFunction(Function):
     """``apply(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points,
     key_padding_mask=None)`` -> ``[B, Q, H*D]``.  ``sampling_offsets [B,Q,H,L,P,2]`` and ``attn_logits
-    [B,Q,H,L*P]`` are the raw outputs of the module's two Linear layers (float32); ``value`` is float32, bfloat16
-    or float16 (the output and ``grad_value`` share its dtype, accumulation is float32); ``reference_points
+    [B,Q,H,L*P]`` are the raw outputs of the module's two Linear layers: float32, or -- as autocast produces them --
+    in value's dtype when that is bfloat16 / float16, and then their gradients come back in that dtype too (the float32
+    gradients rounded once inside the kernel: the bits of the float32 route followed by a cast).  ``value`` is
+    float32, bfloat16 or float16 (the output and ``grad_value`` share its dtype, accumulation is float32); ``reference_points
     [B,Q,L,2|4]`` float32.  Equivalent to softmax + location affine (multi_scale_deform_attn.py:300-332)
     followed by MultiScaleDeformableAttnFunction, without materialising locations / weights or their
     gradients.  With ``key_padding_mask [B,S]`` (bool or uint8, True = padded) it is additionally equivalent
@@ -288,7 +304,7 @@ class MSDeformAttnFusedFunction(Function):
     @staticmethod
     def forward(ctx, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points,
                 key_padding_mask=None):
-        (B, S, H, D, L, Q, P, ref_dim), mask = _check_fused_inputs(
+        (B, S, H, D, L, Q, P, ref_dim), mask, tag = _check_fused_inputs(
             value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points, key_padding_mask)
         value, sampling_offsets, attn_logits, reference_points = (
             _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
@@ -297,7 +313,7 @@ class MSDeformAttnFusedFunction(Function):
         status = _lib.lib().msda_fused_forward(
             ctypes.c_void_p(stream), _ptr(value), _ptr(spatial_shapes), _ptr(level_start_index), _ptr(sampling_offsets),
             _ptr(attn_logits), _ptr(reference_points), ref_dim, _mask_ptr(mask), B, S, H, D, L, Q, P, _ptr(out),
-            _VALUE_TAG[value.dtype], _flags(False))
+            tag, _flags(False))
         _lib.check(status, "msda_fused_forward")
         ctx.save_for_backward(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points)
         ctx.value_mask = mask
@@ -321,6 +337,9 @@ class MSDeformAttnFusedFunction(Function):
             # Composition around the unfused backward: the deterministic mode, and the rare case of reference points
             # that require grad (DINO detaches them) -- d loc / d ref is the identity on (x, y) and off / P * 0.5 on
             # (w, h), taken from grad_sampling_loc itself so that boxes with w == 0 or h == 0 keep their (x, y) grad.
+            # 16-bit offsets / logits are widened (exact) and the final gradients cast: the float32 route's bits.
+            aux_dtype = sampling_offsets.dtype
+            sampling_offsets, attn_logits = sampling_offsets.float(), attn_logits.float()
             loc, weights = _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_points)
             v = value if mask is None else value.masked_fill(mask.bool()[..., None, None], 0)
             grad_value, g_loc, g_w = _backward(v, spatial_shapes, level_start_index, loc, weights, grad_output,
@@ -340,11 +359,11 @@ class MSDeformAttnFusedFunction(Function):
                 g_xy = g_loc.sum(dim=(2, 4))
                 grad_ref = g_xy if ref_dim == 2 else torch.cat(
                     [g_xy, (g_loc * sampling_offsets * (0.5 / P)).sum(dim=(2, 4))], -1)
-            return grad_value, None, None, grad_off, grad_logits, grad_ref, None
+            return grad_value, None, None, grad_off.to(aux_dtype), grad_logits.to(aux_dtype), grad_ref, None
         grad_value = torch.empty_like(value)
         grad_off = torch.empty_like(sampling_offsets)
         grad_logits = torch.empty_like(attn_logits)
-        tag = _VALUE_TAG[value.dtype]
+        tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
         handle = _lib.lib()
         ws_bytes = int(handle.msda_backward_workspace_bytes(B, S, H, D, L, Q, P, tag, flags))
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None

@@ -16,7 +16,9 @@ What differs from the reference module:
     locations / weights and float32 accumulation instead of failing in the float-only dispatch.  The reference
     widens float16 to float32 around the op (py:343, :355-356); here the fused path takes the float16 value as it is,
     with the same output (the kernels widen exactly, so only the final rounding to float16 remains) and half the
-    value bytes read and saved for backward.  Only the unfused fallback (``fuse_pre_ops = False`` or shapes the
+    value bytes read and saved for backward.  The 16-bit sampling offsets / attention logits that autocast's Linears
+    produce go into the fused kernels as they are too (no float32 copy, no cast kernel either way; the same bits as
+    widening them).  Only the unfused fallback (``fuse_pre_ops = False`` or shapes the
     fused kernels do not cover) still widens float16, since the plain op, like the reference's, has no float16 form;
   * there is no CPU branch (py:350-353): a CPU tensor raises;
   * ``add_identity=False`` (keyword, default True) returns ``dropout(output_proj(...))`` WITHOUT the residual
@@ -157,10 +159,14 @@ class MultiScaleDeformableAttention(nn.Module):
             value = value.masked_fill(key_padding_mask[..., None, None], float(0))
         if fused:
             # the padding mask goes into the kernels (masked pixels read as zeros, zero grad_value): the masked
-            # copy of value (py:291-292) and its backward never exist
+            # copy of value (py:291-292) and its backward never exist.  16-bit offsets / logits in value's dtype (the
+            # Linear outputs under autocast) go in as they are: the kernels widen them exactly and round their
+            # gradients, so neither a float32 copy nor a cast kernel exists in either direction.
+            if not (offsets.dtype == logits.dtype == value.dtype and value.dtype in (torch.float16, torch.bfloat16)):
+                offsets, logits = offsets.float(), logits.float()
             output = MSDeformAttnFusedFunction.apply(
-                value.contiguous(), spatial_shapes, level_start_index, offsets.float().contiguous(),
-                logits.float().contiguous(), reference_points.float().contiguous(), key_padding_mask)
+                value.contiguous(), spatial_shapes, level_start_index, offsets.contiguous(),
+                logits.contiguous(), reference_points.float().contiguous(), key_padding_mask)
             if output.dtype != io_dtype:
                 output = output.to(io_dtype)
             output = self.output_proj(output)
