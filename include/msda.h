@@ -201,6 +201,50 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
                         unsigned flags);
 
 /*
+ * Packed (padding-free) form of the fused module path: a batch of differently sized images without padding, the
+ * equivalent of FlashAttention's "varlen" interface.  Image b's pixels of level l are its valid top-left rectangle
+ * h_v[b,l] x w_v[b,l] of the padded level (H_l, W_l), stored row-major with row pitch w_v; the levels of an image follow
+ * each other and the images are concatenated, so
+ *   value              [T_v, H, D]             dtype (T_v = total_value, the valid pixels of all images)
+ *   sampling_offsets   [T_q, H, L, P, 2]       float or (MSDA_*_AUX16) the value's 16-bit type
+ *   attn_logits        [T_q, H, L*P]           as sampling_offsets
+ *   reference_points   [T_q, L, ref_dim]       float
+ *   output / grad_output  [T_q, H*D]           dtype (T_q = total_query)
+ *   grad_value         [T_v, H, D]             dtype; grad_offsets / grad_logits shaped and typed like their inputs
+ *   spatial_shapes     [L, 2] int64            the PADDED level shapes (H_l, W_l)
+ *   image_meta         [batch, 4 + 3*L] int64  per image {value_start, value_count, query_start, query_count} and per
+ *                                              level {h_v, w_v, start of the level inside the image}; query rows
+ *                                              query_start .. +query_count belong to image b
+ * Queries of image b sample image b only.  Locations stay normalised over the padded level (the location affine and
+ * the gate use (H_l, W_l)); a bilinear corner counts iff it lies inside image b's valid rectangle.  So every query's
+ * output, grad_offsets and grad_logits are the same bits msda_fused_forward / _backward give for the padded batch with
+ * the rectangle as value_padding_mask, and grad_value equals theirs at the valid pixels up to the order of the float
+ * reds.  Encoder self-attention: the queries are the value tokens (query_start == value_start); decoder
+ * cross-attention: query_start = b*Q over packed memory.
+ * max_image_value / max_image_query: the largest value_count / query_count (host integers; the grid is sized for
+ * them and every image's value_count * H * D must stay below 2^31).  The metadata is read on the device only -- no
+ * host copy, sync or allocation, so both calls are CUDA-graph capturable -- and is TRUSTED: the product library does
+ * not check it against the totals; a -DMSDA_DEBUG_BOUNDS build traps on any corner outside its image.
+ * Empty problems (batch, total_query or H*D zero) are no-ops; total_value == 0 zero-fills the output (backward: the
+ * offset / logit gradients) without a kernel.  The backward uses float reds; with MSDA_FLAG_DETERMINISTIC it returns
+ * MSDA_ERR_UNSUPPORTED before any device work (unpack, use msda_fused_* / msda_backward, pack).  Its workspace is
+ * msda_packed_backward_workspace_bytes (T_v*H*D floats for 16-bit values, else 0).  Every other flag bit is ignored.
+ * Added in ABI 3 without a version bump: an older library lacks the three symbols.
+ */
+size_t msda_packed_backward_workspace_bytes(int total_value, int num_heads, int channels, int dtype, unsigned flags);
+int msda_packed_forward(void* stream, const void* value, const int64_t* spatial_shapes, const int64_t* image_meta,
+                        const void* sampling_offsets, const void* attn_logits, const float* reference_points,
+                        int ref_dim, int batch, int total_value, int num_heads, int channels, int num_levels,
+                        int total_query, int num_point, int max_image_value, int max_image_query, void* output,
+                        int dtype, unsigned flags);
+int msda_packed_backward(void* stream, const void* grad_output, const void* value, const int64_t* spatial_shapes,
+                         const int64_t* image_meta, const void* sampling_offsets, const void* attn_logits,
+                         const float* reference_points, int ref_dim, int batch, int total_value, int num_heads,
+                         int channels, int num_levels, int total_query, int num_point, int max_image_value,
+                         int max_image_query, void* grad_value, void* grad_offsets, void* grad_logits,
+                         void* workspace, size_t workspace_bytes, int dtype, unsigned flags);
+
+/*
  * DCNv3 core op (SURVEY.md section 8f-4): the other native op of detrex._C, same gather/scatter core.
  *   msda_dcnv3_forward   replaces dcnv3_im2col_cuda<T>
  *       (/root/reference/detrex/layers/csrc/DCNv3/dcnv3_im2col_cuda.cuh:840-868), i.e. _C.dcnv3_forward

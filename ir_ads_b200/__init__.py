@@ -6,6 +6,7 @@ Importing the package does not load the CUDA library; the first op call does, an
 if ir_ads_b200/libmsda_b200.so has not been built (no CPU / PyTorch fallback exists).
 """
 from .functional import (  # noqa: F401
+    MSDeformAttnPackedFunction,
     MultiScaleDeformableAttnFunction,
     kernel_flags,
     ms_deform_attn_backward,
@@ -15,6 +16,7 @@ from .functional import (  # noqa: F401
 )
 from .dcnv3 import DCNv3FusedFunction, DCNv3Function, dcnv3_backward, dcnv3_forward  # noqa: F401
 from .module import MultiScaleDeformableAttention  # noqa: F401
+from .packing import PackedLevels, pack_levels, packed_reference_points, unpack_tokens, valid_extents  # noqa: F401
 
 __all__ = [
     "MultiScaleDeformableAttention",
@@ -28,4 +30,10 @@ __all__ = [
     "DCNv3FusedFunction",
     "dcnv3_forward",
     "dcnv3_backward",
+    "MSDeformAttnPackedFunction",
+    "PackedLevels",
+    "valid_extents",
+    "pack_levels",
+    "packed_reference_points",
+    "unpack_tokens",
 ]

@@ -71,6 +71,13 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.msda_fused_backward.restype = i
     lib.msda_fused_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i, vp, i, i, i, i, i, i, i, vp, vp, vp, vp,
                                         sz, i, u]
+    lib.msda_packed_backward_workspace_bytes.restype = sz
+    lib.msda_packed_backward_workspace_bytes.argtypes = [i, i, i, i, u]
+    lib.msda_packed_forward.restype = i
+    lib.msda_packed_forward.argtypes = [vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, i, i, vp, i, u]
+    lib.msda_packed_backward.restype = i
+    lib.msda_packed_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i, i, i, i, vp, vp, vp,
+                                         vp, sz, i, u]
     i64, f32 = ctypes.c_int64, ctypes.c_float
     lib.msda_add_layernorm_workspace_bytes.restype = sz
     lib.msda_add_layernorm_workspace_bytes.argtypes = [i64, i]

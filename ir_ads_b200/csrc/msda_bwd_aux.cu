@@ -56,6 +56,10 @@ int bwd_fused_noscatter(cudaStream_t, const Dims&, int, const void*, const void*
                         const void*, const void*, void*, void*, msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no fused kernels");
 }
+int bwd_packed(cudaStream_t, const Dims&, int, const void*, const void*, const int64_t*, const int64_t*, const void*,
+               const void*, float*, void*, void*, msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no packed kernels");
+}
 int bwd_dcn(cudaStream_t, const Dims&, int, const void*, const void*, const void*, const void*, float*, void*, void*,
             msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
@@ -93,6 +97,24 @@ int bwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* go, const v
   MSDA_DISPATCH_VT(CALL_FB);
 #undef CALL_FB16
 #undef CALL_FB
+#undef MSDA_DISPATCH_ORDER
+}
+
+// fused chain over a packed batch: STRIP order, float reds, the same value / aux types as bwd_fused
+int bwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
+               const int64_t* meta, const void* off, const void* logits, float* gv, void* goff, void* glog,
+               msda::FusedArgs fa) {
+#define MSDA_DISPATCH_ORDER MSDA_ORDER_STRIP
+#define CALL_PB(D_, VT_, PT_, ORD_)                                                                                  \
+  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPrePacked>(st, d, go, value, shapes, meta, off,      \
+                                                                            logits, gv, goff, glog, nullptr, fa)
+#define CALL_PB16(D_, VT_, PT_, ORD_)                                                                             \
+  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPrePacked, VT_>(st, d, go, value, shapes, meta, off, \
+                                                                                 logits, gv, goff, glog, nullptr, fa)
+  MSDA_DISPATCH_VT_AUX16(CALL_PB16);
+  MSDA_DISPATCH_VT(CALL_PB);
+#undef CALL_PB16
+#undef CALL_PB
 #undef MSDA_DISPATCH_ORDER
 }
 

@@ -723,6 +723,127 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
 }
 
 namespace {
+// Checks shared by msda_packed_forward / _backward.  *d becomes the problem the kernels are launched for: B images,
+// S / Q = the largest image's value / query count (grid and 32-bit in-image offsets).  Returns MSDA_OK, an error, or
+// -1 for an empty problem (nothing to do).
+int packed_setup(int batch, int total_value, int num_heads, int channels, int num_levels, int total_query,
+                 int num_point, int max_image_value, int max_image_query, int ref_dim, int dtype, unsigned flags,
+                 Dims* d) {
+  *d = Dims{batch, max_image_value, num_heads, channels, num_levels, max_image_query, num_point};
+  if (int s = check_dims(*d, fused_value_dtype(dtype))) return s;
+  if (total_value < 0 || total_query < 0)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "negative token count (T_v=%d T_q=%d)", total_value, total_query);
+  if (ref_dim != 2 && ref_dim != 4) return fail(MSDA_ERR_INVALID_ARGUMENT, "ref_dim must be 2 or 4, got %d", ref_dim);
+  if (batch == 0 || total_query == 0 || (int64_t)num_heads * channels == 0) return -1;
+  if (max_image_query > total_query || max_image_value > total_value ||
+      (int64_t)max_image_query * batch < total_query || (int64_t)max_image_value * batch < total_value)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "largest image (%d queries, %d values) does not fit the totals (%d, %d)",
+                max_image_query, max_image_value, total_query, total_value);
+  if (!fast_ok(*d, fused_value_dtype(dtype), flags & ~MSDA_FLAG_DETERMINISTIC) ||
+      (int64_t)max_image_query * num_heads >= ((int64_t)1 << 31))
+    return fail(MSDA_ERR_UNSUPPORTED, "packed path needs D in {16,32,64,128}, float/bf16/f16 value, L<=16, 1<=L*P<=64");
+  return MSDA_OK;
+}
+}  // namespace
+
+size_t msda_packed_backward_workspace_bytes(int total_value, int num_heads, int channels, int dtype, unsigned flags) {
+  (void)flags;
+  if (total_value <= 0 || num_heads <= 0 || channels <= 0) return 0;
+  // bf16 / f16 grad_value is accumulated in float and converted at the end
+  return two_byte(fused_value_dtype(dtype)) ? (size_t)total_value * num_heads * channels * sizeof(float) : 0;
+}
+
+int msda_packed_forward(void* stream, const void* value, const int64_t* spatial_shapes, const int64_t* image_meta,
+                        const void* sampling_offsets, const void* attn_logits, const float* reference_points,
+                        int ref_dim, int batch, int total_value, int num_heads, int channels, int num_levels,
+                        int total_query, int num_point, int max_image_value, int max_image_query, void* output,
+                        int dtype, unsigned flags) {
+  g_err[0] = 0;
+  Dims d;
+  const int s0 = packed_setup(batch, total_value, num_heads, channels, num_levels, total_query, num_point,
+                              max_image_value, max_image_query, ref_dim, dtype, flags, &d);
+  if (s0 == -1) return MSDA_OK;
+  if (s0 != MSDA_OK) return s0;
+  if (!output) return fail(MSDA_ERR_INVALID_ARGUMENT, "output is null");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (total_value == 0) {   // no valid pixel anywhere: every sample reads zeros
+    DeviceGuard g;
+    MSDA_CUDA(g.enter(output));
+    MSDA_CUDA(cudaMemsetAsync(output, 0, (size_t)total_query * num_heads * channels * elem_size(fused_value_dtype(dtype)),
+                              st));
+    return MSDA_OK;
+  }
+  if (!value || !spatial_shapes || !image_meta || !sampling_offsets || !attn_logits || !reference_points)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  if (int s = check_alignment({{"value", value}, {"image_meta", image_meta}, {"sampling_offsets", sampling_offsets},
+                               {"attn_logits", attn_logits}, {"reference_points", reference_points},
+                               {"output", output}}))
+    return s;
+  DeviceGuard guard;
+  MSDA_CUDA(guard.enter(value));
+  msda::FusedArgs fa{};
+  fa.ref = reference_points;
+  fa.ref_dim = ref_dim;
+  fa.inv_P = 1.0f / (float)num_point;
+  fa.num_P = (float)num_point;
+  return fwd_packed(st, d, dtype, value, spatial_shapes, image_meta, sampling_offsets, attn_logits, output, fa);
+}
+
+int msda_packed_backward(void* stream, const void* grad_output, const void* value, const int64_t* spatial_shapes,
+                         const int64_t* image_meta, const void* sampling_offsets, const void* attn_logits,
+                         const float* reference_points, int ref_dim, int batch, int total_value, int num_heads,
+                         int channels, int num_levels, int total_query, int num_point, int max_image_value,
+                         int max_image_query, void* grad_value, void* grad_offsets, void* grad_logits,
+                         void* workspace, size_t workspace_bytes, int dtype, unsigned flags) {
+  g_err[0] = 0;
+  if (flags & MSDA_FLAG_DETERMINISTIC)
+    return fail(MSDA_ERR_UNSUPPORTED, "the packed backward has no deterministic form (float reds)");
+  Dims d;
+  const int s0 = packed_setup(batch, total_value, num_heads, channels, num_levels, total_query, num_point,
+                              max_image_value, max_image_query, ref_dim, dtype, flags, &d);
+  if (s0 == -1) return MSDA_OK;
+  if (s0 != MSDA_OK) return s0;
+  if (!grad_offsets || !grad_logits) return fail(MSDA_ERR_INVALID_ARGUMENT, "gradient output pointer is null");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int64_t n_points = (int64_t)total_query * num_heads * num_levels * num_point;
+  if (total_value == 0) {   // nothing was sampled: every gradient is zero
+    DeviceGuard g;
+    MSDA_CUDA(g.enter(grad_offsets));
+    MSDA_CUDA(cudaMemsetAsync(grad_offsets, 0, (size_t)n_points * 2 * aux_size(dtype), st));
+    MSDA_CUDA(cudaMemsetAsync(grad_logits, 0, (size_t)n_points * aux_size(dtype), st));
+    return MSDA_OK;
+  }
+  if (!grad_output || !value || !spatial_shapes || !image_meta || !sampling_offsets || !attn_logits ||
+      !reference_points || !grad_value)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  if (int s = check_alignment({{"grad_output", grad_output}, {"value", value}, {"image_meta", image_meta},
+                               {"sampling_offsets", sampling_offsets}, {"attn_logits", attn_logits},
+                               {"reference_points", reference_points}, {"grad_value", grad_value},
+                               {"grad_offsets", grad_offsets}, {"grad_logits", grad_logits},
+                               {"workspace", workspace}}))
+    return s;
+  const int vdt = fused_value_dtype(dtype);
+  const size_t need = msda_packed_backward_workspace_bytes(total_value, num_heads, channels, dtype, flags);
+  if (need && (!workspace || workspace_bytes < need))
+    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  DeviceGuard guard;
+  MSDA_CUDA(guard.enter(value));
+  const int64_t n_value = (int64_t)total_value * num_heads * channels;
+  float* gv32 = two_byte(vdt) ? static_cast<float*>(workspace) : static_cast<float*>(grad_value);
+  MSDA_CUDA(cudaMemsetAsync(gv32, 0, (size_t)n_value * sizeof(float), st));
+  msda::FusedArgs fa{};
+  fa.ref = reference_points;
+  fa.ref_dim = ref_dim;
+  fa.inv_P = 1.0f / (float)num_point;
+  fa.num_P = (float)num_point;
+  const int s = bwd_packed(st, d, dtype, grad_output, value, spatial_shapes, image_meta, sampling_offsets, attn_logits,
+                           gv32, grad_offsets, grad_logits, fa);
+  if (s != MSDA_OK) return s;
+  if (two_byte(vdt)) return cast_from_f32(st, gv32, grad_value, n_value, vdt);
+  return MSDA_OK;
+}
+
+namespace {
 // DCNv3 as an MSDeformAttn problem: value = input [N, H_in*W_in, G, C], one level, Q = H_out*W_out, P = K.
 int dcn_setup(int kernel_h, int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h,
               int dilation_w, int group, int group_channels, float offset_scale, int batch, int height_in,

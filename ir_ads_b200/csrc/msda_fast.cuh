@@ -277,12 +277,20 @@ __device__ __forceinline__ float dotv(const Vec<N>& a, const Vec<N>& b) {
 }
 
 // ---- level / tile table in shared memory -----------------------------------------------------
+// Packed batches (kPrePacked) keep H / W = the padded level (location scaling and gating), start = the level's first
+// token inside the image, and the image's valid rectangle h_v x w_v in the tile fields, which they do not use.
 struct LevelTab {
   int H[kFastMaxLevels];
   int W[kFastMaxLevels];
   int start[kFastMaxLevels];
-  int tiles_x[kFastMaxLevels];     // tile orders only
-  int tile_begin[kFastMaxLevels];  // tile orders only: first tile index of the level
+  union {
+    int tiles_x[kFastMaxLevels];   // tile orders only
+    int Wv[kFastMaxLevels];        // packed only: valid width = row pitch of the level inside the image
+  };
+  union {
+    int tile_begin[kFastMaxLevels];  // tile orders only: first tile index of the level
+    int Hv[kFastMaxLevels];          // packed only: valid height
+  };
   int total_tiles;                 // tile orders only
   int cells_per_bh;                // EMIT only (deterministic sorted path): bins per (image, head), see msda_det.cuh
   int cell_begin[kFastMaxLevels];  // EMIT only: first bin of the level inside one (image, head) block
@@ -325,6 +333,24 @@ __device__ __forceinline__ void load_levels_plain(LevelTab* tab, const int64_t* 
       if ((int)threadIdx.x == L - 1)
         tab->cells_per_bh = acc + ((int)shapes[2 * threadIdx.x] + 1) * ((int)shapes[2 * threadIdx.x + 1] + 1);
     }
+  }
+  __syncthreads();
+}
+
+// ---- packed batches (kPrePacked) -----------------------------------------------------------------
+// Image b's metadata row, kPackedMetaFixed + 3*L int64: {value_start, value_count, query_start, query_count} and, per
+// level, {h_v, w_v, start of the level inside the image}.  A CTA works on rows of ONE image, so the row is loaded once.
+constexpr int kPackedMetaFixed = 4;
+__host__ __device__ constexpr int packed_meta_stride(int L) { return kPackedMetaFixed + 3 * L; }
+
+__device__ __forceinline__ void load_levels_packed(LevelTab* tab, const int64_t* shapes, const int64_t* img, int L) {
+  if (threadIdx.x < L) {
+    const int64_t* lv = img + kPackedMetaFixed + 3 * threadIdx.x;
+    tab->H[threadIdx.x] = (int)shapes[2 * threadIdx.x];
+    tab->W[threadIdx.x] = (int)shapes[2 * threadIdx.x + 1];
+    tab->Hv[threadIdx.x] = (int)lv[0];
+    tab->Wv[threadIdx.x] = (int)lv[1];
+    tab->start[threadIdx.x] = (int)lv[2];
   }
   __syncthreads();
 }
@@ -451,6 +477,62 @@ struct RowWalk {
   }
 };
 
+// The CTA's image and this thread's row.  LINEAR (forward): blockIdx.x = image * chunks + chunk, a chunk = RPC
+// consecutive (query, head) rows of the image, chunks = ceil(max_q * H / RPC).  STRIP (backward): blockIdx.x =
+// (image * chunks + chunk) * H + head, a chunk = RPC consecutive queries, chunks = ceil(max_q / RPC).  Every image
+// gets the grid of the largest one; a CTA past its image's rows is surplus (uniform over the CTA) and exits.
+struct PackedRow {
+  RowRef r;
+  const int64_t* img;   // the image's metadata row
+  bool surplus;
+};
+template <int RPC, int ORDER>
+__device__ __forceinline__ PackedRow packed_row(const int64_t* meta, int L, int H, int max_q, int rin) {
+  static_assert(ORDER == 0 || ORDER == 2, "packed batches: LINEAR forward, STRIP backward");
+  PackedRow p;
+  const unsigned it = blockIdx.x;
+  unsigned b, chunk;
+  int h = 0;
+  if (ORDER == 2) {
+    const unsigned chunks = (unsigned)((max_q + RPC - 1) / RPC), bc = it / (unsigned)H;
+    h = (int)(it - bc * (unsigned)H);
+    b = bc / chunks;
+    chunk = bc - b * chunks;
+  } else {
+    const unsigned chunks = (unsigned)((max_q * H + RPC - 1) / RPC);
+    b = it / chunks;
+    chunk = it - b * chunks;
+  }
+  p.img = meta + (int64_t)b * packed_meta_stride(L);
+  const int64_t q0 = __ldg(p.img + 2);
+  const int nq = (int)__ldg(p.img + 3);
+  p.r.b = (int)b;
+  if (ORDER == 2) {
+    const int q = (int)chunk * RPC + rin;
+    p.surplus = (int)chunk * RPC >= nq;
+    p.r.live = q < nq;
+    p.r.h = h;
+    p.r.row = p.r.live ? (q0 + q) * H + h : 0;
+  } else {
+    const int local = (int)chunk * RPC + rin;
+    p.surplus = (int)chunk * RPC >= nq * H;
+    p.r.live = local < nq * H;
+    p.r.h = local % H;
+    p.r.row = p.r.live ? q0 * H + local : 0;
+  }
+  return p;
+}
+
+// The validity bits of a cell restricted to the image's valid rectangle [0, w_v) x [0, h_v) -- what a
+// key_padding_mask that is exactly that rectangle does to the bits (apply_value_mask) -- for a level stored with
+// row pitch w_v.
+__device__ __forceinline__ Cell<float> clip_to_rect(Cell<float> c, int hv, int wv) {
+  const bool x0 = c.x0 < wv, x1 = c.x0 + 1 < wv, y0 = c.y0 < hv, y1 = c.y0 + 1 < hv;
+  c.valid &= (unsigned)(y0 && x0) | ((unsigned)(y0 && x1) << 1) | ((unsigned)(y1 && x0) << 2) |
+             ((unsigned)(y1 && x1) << 3);
+  return c;
+}
+
 // ---- per-point record --------------------------------------------------------------------------
 // oc = element offset, inside the image, of the bilinear cell's (x0, y0) corner -- NOT clamped: it lies outside the
 // map when that corner is padded, and is then never dereferenced -- with four corner-validity bits in its low bits
@@ -536,10 +618,16 @@ struct FusedArgs {
   float offset_scale;
 };
 // PRE: 0 = sampling_locations / attention_weights given (the reference operator), 1 = fused module chain,
-//      2 = DCNv3 sampling grid, 3 = DCNv3 sampling grid + softmax over the row's mask logits
-constexpr int kPrePlain = 0, kPreFused = 1, kPreDcn = 2, kPreDcnSoftmax = 3;
+//      2 = DCNv3 sampling grid, 3 = DCNv3 sampling grid + softmax over the row's mask logits,
+//      4 = fused module chain over a packed batch (valid pixels only, see packed_row; `lsi` is then the per-image
+//          metadata and `S` unused)
+constexpr int kPrePlain = 0, kPreFused = 1, kPreDcn = 2, kPreDcnSoftmax = 3, kPrePacked = 4;
 // the record modes whose `w` holds logits: the row softmax in forward, its chain rule in backward
-__host__ __device__ constexpr bool pre_softmax(int pre) { return pre == kPreFused || pre == kPreDcnSoftmax; }
+__host__ __device__ constexpr bool pre_softmax(int pre) {
+  return pre == kPreFused || pre == kPreDcnSoftmax || pre == kPrePacked;
+}
+// the record modes of the MSDA module chain: location affine from raw offsets and reference points
+__host__ __device__ constexpr bool pre_fused(int pre) { return pre == kPreFused || pre == kPrePacked; }
 // the record modes on the DCNv3 convolution grid
 __host__ __device__ constexpr bool pre_dcn(int pre) { return pre == kPreDcn || pre == kPreDcnSoftmax; }
 
@@ -631,7 +719,7 @@ __device__ __forceinline__ void st_aux1(__nv_bfloat16* p, float a) { *p = __floa
 template <typename VT, typename AT, int PRE, int ORDER, int ORDER_16>
 __host__ __device__ constexpr bool aux_ok() {
   return std::is_same_v<AT, float> ||
-         (std::is_same_v<AT, VT> && sizeof(VT) == 2 && (PRE == 1 || PRE == 3) && ORDER == ORDER_16);
+         (std::is_same_v<AT, VT> && sizeof(VT) == 2 && (PRE == 1 || PRE == 3 || PRE == 4) && ORDER == ORDER_16);
 }
 
 // softmax over the row's NP logits by the row's LANES lanes; e_i = exp(x_i - max) is left in
@@ -690,7 +778,9 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
   // on the widened value; bf16 keeps its own order
   constexpr int SM_LANES = std::is_same_v<VT, __half> ? D / 4 : LANES;
   constexpr bool SOFTMAX = pre_softmax(PRE);    // `w` holds logits: row softmax (fused MSDA chain, fused DCNv3)
-  constexpr bool FUSED = (PRE == kPreFused);    // MSDA chain only: location affine, reference points, padding mask
+  constexpr bool FUSED = pre_fused(PRE);        // MSDA chain only: location affine, reference points, padding mask
+  constexpr bool PACKED = (PRE == kPrePacked);  // packed batch: `lsi` = per-image metadata, one image per CTA
+  static_assert(!PACKED || ORDER == 0, "the packed forward is LINEAR");
   constexpr bool DCN = pre_dcn(PRE);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   LevelTab* tab = reinterpret_cast<LevelTab*>(smem_raw);
@@ -726,10 +816,18 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
   float early_sum = 1.0f;                                // SOFTMAX: softmax denominator of the row
   RowWalk<DL, THREADS, ORDER> walk;
   RowRef cur;
+  const int64_t* pimg = nullptr;                         // PACKED: the CTA's image metadata row
   if constexpr (EARLY) {
-    walk = RowWalk<DL, THREADS, ORDER>(tab, B, H, rows);
-    if (walk.done()) return;                             // uniform over the CTA
-    cur = walk.get(tab, L, H, Q);
+    if constexpr (PACKED) {
+      const PackedRow p = packed_row<G::RPC, ORDER>(lsi, L, H, Q, rin);
+      if (p.surplus) return;                             // uniform over the CTA
+      cur = p.r;
+      pimg = p.img;
+    } else {
+      walk = RowWalk<DL, THREADS, ORDER>(tab, B, H, rows);
+      if (walk.done()) return;                             // uniform over the CTA
+      cur = walk.get(tab, L, H, Q);
+    }
 #pragma unroll
     for (int i = 0; i < kEarly; ++i) {
       const int pt = sub + i * LANES;
@@ -739,7 +837,8 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
     }
     // the softmax shuffles need the whole warp; dead rows read row 0 and simply produce nothing
     if constexpr (SOFTMAX) early_sum = row_softmax<LANES, 1, SM_LANES>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_oc), NP, sub);
-    load_levels_plain(tab, shapes, lsi, L);
+    if constexpr (PACKED) load_levels_packed(tab, shapes, pimg, L);
+    else load_levels_plain(tab, shapes, lsi, L);
   } else {
     if constexpr (DCN) set_single_level<G::TW, G::TH>(tab, fused.height_in, fused.width_in);
     else if constexpr (ORDER == 0 || ORDER == 2) load_levels_plain(tab, shapes, lsi, L);
@@ -768,10 +867,13 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
           if constexpr (DCN) {
             const float2 px = dcn_location(xy, pt, (int)((cur.row / H) % Q), fused);
             r = record_from_cell(locate_pixel(px.x, px.y, tab->H[0], tab->W[0]), aw, tab->W[0], 0, H, cur.h, D);
+          } else if constexpr (PACKED) {
+            r = record_from_cell(clip_to_rect(locate<float>(xy.x, xy.y, tab->H[l], tab->W[l]), tab->Hv[l], tab->Wv[l]),
+                                 aw, tab->Wv[l], tab->start[l], H, cur.h, D);
           } else {
             r = make_record(xy.x, xy.y, aw, tab->H[l], tab->W[l], tab->start[l], H, cur.h, D);
           }
-          if constexpr (FUSED) {
+          if constexpr (FUSED && !PACKED) {
             if (fused.value_mask) apply_value_mask(r, fused.value_mask + (int64_t)cur.b * S, tab->W[l], S);
           }
           if constexpr (REC16) {
@@ -794,12 +896,15 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
 
     // ---- phase 2: gather ----
     if (cur.live) {
-      const VT* vimg = value + (int64_t)cur.b * S * HD + sub * CPL;
+      const VT* vimg = value + (PACKED ? __ldg(pimg) * HD : (int64_t)cur.b * S * HD) + sub * CPL;
       asm volatile("" : "+l"(vimg));   // keep the row base as ONE 64-bit register: corner address = base + off*4 (IMAD.WIDE)
+#ifdef MSDA_DEBUG_BOUNDS
+      const int lim = PACKED ? (int)__ldg(pimg + 1) * HD : S * HD;   // the image's elements
+#endif
       Vec<CPL> acc = vzero<CPL>();
       int pt = 0;
       for (int l = 0; l < L; ++l) {
-        const int dyl = tab->W[l] * HD;
+        const int dyl = (PACKED ? tab->Wv[l] : tab->W[l]) * HD;   // row pitch of the level inside the image
         const int np = (PT > 0) ? PT : P;
 #pragma unroll
         for (int p = 0; p < np; ++p, ++pt) {
@@ -820,10 +925,10 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
           // branches, and the loads of the next point are scheduled under the FMAs of this one.
           const int o00 = oc & ~15;
 #ifdef MSDA_DEBUG_BOUNDS
-          if (oc & 1) MSDA_CHECK_OFFSET(o00, S * HD, "fwd k0");
-          if (oc & 2) MSDA_CHECK_OFFSET(o00 + HD, S * HD, "fwd k1");
-          if (oc & 4) MSDA_CHECK_OFFSET(o00 + dyl, S * HD, "fwd k2");
-          if (oc & 8) MSDA_CHECK_OFFSET(o00 + dyl + HD, S * HD, "fwd k3");
+          if (oc & 1) MSDA_CHECK_OFFSET(o00, lim, "fwd k0");
+          if (oc & 2) MSDA_CHECK_OFFSET(o00 + HD, lim, "fwd k1");
+          if (oc & 4) MSDA_CHECK_OFFSET(o00 + dyl, lim, "fwd k2");
+          if (oc & 8) MSDA_CHECK_OFFSET(o00 + dyl + HD, lim, "fwd k3");
 #endif
           if constexpr (sizeof(VT) == 4) {
             Raw<CPL, VT> v0, v1, v2, v3;
@@ -852,6 +957,7 @@ msda_fwd_fast_kernel(const VT* __restrict__ value, const int64_t* __restrict__ s
       }
       stv<CPL>(out + cur.row * D + sub * CPL, acc);
     }
+    if constexpr (PACKED) break;   // single pass
     walk.next();    // single-pass orders end here; TILE2D only continues for a pathological pyramid
     if (walk.done()) break;
     __syncwarp();
@@ -1023,7 +1129,9 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
   using G = Geom<DL, THREADS>;
   constexpr int LANES = G::LANES;
   constexpr bool SOFTMAX = pre_softmax(PRE);    // `w` holds logits: softmax and its chain rule (grad_w = logits' grad)
-  constexpr bool FUSED = (PRE == kPreFused);    // MSDA chain only: location affine, reference points, padding mask
+  constexpr bool FUSED = pre_fused(PRE);        // MSDA chain only: location affine, reference points, padding mask
+  constexpr bool PACKED = (PRE == kPrePacked);  // packed batch: `lsi` = per-image metadata, one image per CTA
+  static_assert(!PACKED || (ORDER == 2 && std::is_same_v<ACC, float>), "the packed backward is STRIP with float reds");
   constexpr bool DCN = pre_dcn(PRE);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   LevelTab* tab = reinterpret_cast<LevelTab*>(smem_raw);
@@ -1052,10 +1160,18 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
   RowWalk<DL, THREADS, ORDER> walk;
   RowRef cur;
   Vec<CPL> go = vzero<CPL>();
+  const int64_t* pimg = nullptr;                         // PACKED: the CTA's image metadata row
   if constexpr (EARLY) {
-    walk = RowWalk<DL, THREADS, ORDER>(tab, B, H, rows);
-    if (walk.done()) return;                             // uniform over the CTA
-    cur = walk.get(tab, L, H, Q);
+    if constexpr (PACKED) {
+      const PackedRow p = packed_row<G::RPC, ORDER>(lsi, L, H, Q, rin);
+      if (p.surplus) return;                             // uniform over the CTA
+      cur = p.r;
+      pimg = p.img;
+    } else {
+      walk = RowWalk<DL, THREADS, ORDER>(tab, B, H, rows);
+      if (walk.done()) return;                             // uniform over the CTA
+      cur = walk.get(tab, L, H, Q);
+    }
     if (cur.live) go = ldv<CPL>(grad_out + cur.row * D + sub * CPL);
 #pragma unroll
     for (int i = 0; i < kEarly; ++i) {
@@ -1066,7 +1182,8 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     }
     if constexpr (SOFTMAX)
       early_sum = row_softmax<LANES, 4>(w + cur.row * (int64_t)NP, reinterpret_cast<float*>(s_fin) + 3, NP, sub);
-    load_levels_plain<EMIT>(tab, shapes, lsi, L);
+    if constexpr (PACKED) load_levels_packed(tab, shapes, pimg, L);
+    else load_levels_plain<EMIT>(tab, shapes, lsi, L);
   } else {
     if constexpr (DCN) set_single_level<G::TW, G::TH, EMIT>(tab, fused.height_in, fused.width_in);
     else if constexpr (ORDER == 0 || ORDER == 2) load_levels_plain(tab, shapes, lsi, L);
@@ -1116,10 +1233,13 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
             const Cell<float> c = locate<float>(xy.x, xy.y, tab->H[l], tab->W[l]);
             r = record_from_cell(c, aw, tab->W[l], tab->start[l], H, cur.h, D);
             if (c.valid != 0u) emit_entry(c, l, aw);
+          } else if constexpr (PACKED) {
+            r = record_from_cell(clip_to_rect(locate<float>(xy.x, xy.y, tab->H[l], tab->W[l]), tab->Hv[l], tab->Wv[l]),
+                                 aw, tab->Wv[l], tab->start[l], H, cur.h, D);
           } else {
             r = make_record(xy.x, xy.y, aw, tab->H[l], tab->W[l], tab->start[l], H, cur.h, D);
           }
-          if constexpr (FUSED) {
+          if constexpr (FUSED && !PACKED) {
             if (fused.value_mask) apply_value_mask(r, fused.value_mask + (int64_t)cur.b * S, tab->W[l], S);
           }
           cw = r.cw;
@@ -1150,7 +1270,10 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     constexpr bool SCATTER = sizeof(ACC) != sizeof(NoScatter) && !EMIT;
     static_assert(!(sizeof(ACC) == 8 && CPL != 4), "the fixed-point red path transposes 4 channels per lane");
 
-    const int64_t img = (int64_t)cur.b * S * HD + sub * CPL;
+    const int64_t img = (PACKED ? __ldg(pimg) * HD : (int64_t)cur.b * S * HD) + sub * CPL;
+#ifdef MSDA_DEBUG_BOUNDS
+    const int lim = PACKED ? (int)__ldg(pimg + 1) * HD : S * HD;   // the image's elements
+#endif
     const VT* vimg = value + img;
     ACC* gimg = grad_value + (DET ? img - sub * 3 : img);   // DET: lane offset is `sub`, not 4*sub
     asm volatile("" : "+l"(vimg), "+l"(gimg));
@@ -1161,7 +1284,7 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
     float* gsc = nullptr;
     if constexpr (SCATTER && !DET) {
       go_sc = load_scatter_layout<CPL, D>(grad_out + cur.row * D, sub, go);
-      gsc = reinterpret_cast<float*>(grad_value) + (int64_t)cur.b * S * HD + sub * 4;
+      gsc = reinterpret_cast<float*>(grad_value) + (PACKED ? __ldg(pimg) * HD : (int64_t)cur.b * S * HD) + sub * 4;
       asm volatile("" : "+l"(gsc));
     }   // one 64-bit register each: address = base + off*size (IMAD.WIDE)
     AT* glp = grad_loc + cur.row * (int64_t)NP * 2;
@@ -1179,14 +1302,14 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
           const int l = level_of<PT>(pt, P);
           const int o00 = oc & ~15;
           const int o01 = o00 + HD;
-          const int o10 = o00 + tab->W[l] * HD, o11 = o10 + HD;
+          const int o10 = o00 + (PACKED ? tab->Wv[l] : tab->W[l]) * HD, o11 = o10 + HD;
           // a corner whose validity bit is clear is not loaded (its offset may lie outside the map); its dot stays 0
           float d0 = 0.0f, d1 = 0.0f, d2 = 0.0f, d3 = 0.0f;
 #ifdef MSDA_DEBUG_BOUNDS
-          if ((oc & 1) || cw.x != 0.0f) MSDA_CHECK_OFFSET(o00, S * HD, "bwd k0");
-          if ((oc & 2) || cw.y != 0.0f) MSDA_CHECK_OFFSET(o01, S * HD, "bwd k1");
-          if ((oc & 4) || cw.z != 0.0f) MSDA_CHECK_OFFSET(o10, S * HD, "bwd k2");
-          if ((oc & 8) || cw.w != 0.0f) MSDA_CHECK_OFFSET(o11, S * HD, "bwd k3");
+          if ((oc & 1) || cw.x != 0.0f) MSDA_CHECK_OFFSET(o00, lim, "bwd k0");
+          if ((oc & 2) || cw.y != 0.0f) MSDA_CHECK_OFFSET(o01, lim, "bwd k1");
+          if ((oc & 4) || cw.z != 0.0f) MSDA_CHECK_OFFSET(o10, lim, "bwd k2");
+          if ((oc & 8) || cw.w != 0.0f) MSDA_CHECK_OFFSET(o11, lim, "bwd k3");
 #endif
 #ifdef MSDA_EXP_NO_GATHER   // experiment builds only (tools/ablate.sh): what does the scatter cost alone?
           d0 = d1 = d2 = d3 = dotv(go, go);
@@ -1315,6 +1438,7 @@ msda_bwd_fast_kernel(const VT* __restrict__ grad_out, const VT* __restrict__ val
         }
       }
     }
+    if constexpr (PACKED) break;   // single pass
     walk.next();
     if (walk.done()) break;
     __syncwarp();

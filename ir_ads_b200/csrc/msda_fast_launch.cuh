@@ -45,6 +45,8 @@ int launch_fwd_fast(cudaStream_t st, const Dims& d, const void* value, const int
   unsigned grid = (unsigned)((rows + G::RPC - 1) / G::RPC);
   if (ORDER == 2) grid = (unsigned)((int64_t)d.B * d.H * ((d.Q + G::RPC - 1) / G::RPC));
   if (ORDER == 3) grid = (unsigned)((int64_t)d.B * d.H * tile2d_bound(d, G::RPC));
+  // packed batch (d.Q = the largest image's query count): every image gets the LINEAR grid of that image
+  if (PRE == msda::kPrePacked) grid = (unsigned)((int64_t)d.B * (((int64_t)d.Q * d.H + G::RPC - 1) / G::RPC));
   k<<<grid, THREADS, smem, st>>>((const VT*)value, shapes, lsi, (const AT*)loc, (const AT*)w, (VT*)out, fa,
                                  d.B, d.S, d.H, d.L, d.Q, d.P, rows);
   count_launch();
@@ -68,6 +70,7 @@ int launch_bwd_fast(cudaStream_t st, const Dims& d, const void* go, const void* 
   MSDA_CUDA(ensure_smem(k, smem));
   const int64_t rows = d.rows();
   unsigned grid = (unsigned)((rows + G::RPC - 1) / G::RPC);
+  // (packed batches: d.Q = the largest image's query count, the STRIP grid of that image for every image)
   if (ORDER == 2) grid = (unsigned)((int64_t)d.B * d.H * ((d.Q + G::RPC - 1) / G::RPC));
   if (ORDER == 3) grid = (unsigned)((int64_t)d.B * d.H * tile2d_bound(d, G::RPC));
   k<<<grid, THREADS, smem, st>>>((const VT*)go, (const VT*)value, shapes, lsi, (const AT*)loc, (const AT*)w,

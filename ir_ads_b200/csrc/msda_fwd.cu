@@ -28,6 +28,10 @@ int fwd_dcn(cudaStream_t, const Dims&, int, const void*, const void*, const void
 int fwd_dcn_softmax(cudaStream_t, const Dims&, int, const void*, const void*, const void*, void*, msda::FusedArgs) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
 }
+int fwd_packed(cudaStream_t, const Dims&, int, const void*, const int64_t*, const int64_t*, const void*, const void*,
+               void*, msda::FusedArgs) {
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: no packed kernels");
+}
 #else
 // fused pre-op chain: LINEAR order.  dtype MSDA_*_AUX16: offsets / logits in the value's 16-bit type
 int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes, const int64_t* lsi,
@@ -42,6 +46,22 @@ int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, cons
   MSDA_DISPATCH_VT(CALL_FF);
 #undef CALL_FF16
 #undef CALL_FF
+#undef MSDA_DISPATCH_ORDER
+}
+
+// fused chain over a packed batch: LINEAR order, the same value / aux types as fwd_fused
+int fwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes,
+               const int64_t* meta, const void* off, const void* logits, void* out, msda::FusedArgs fa) {
+#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
+#define CALL_FP(D_, VT_, PT_, ORD_) \
+  launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPrePacked>(st, d, value, shapes, meta, off, logits, out, fa)
+#define CALL_FP16(D_, VT_, PT_, ORD_)                                                                           \
+  launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPrePacked, VT_>(st, d, value, shapes, meta, off, logits, \
+                                                                          out, fa)
+  MSDA_DISPATCH_VT_AUX16(CALL_FP16);
+  MSDA_DISPATCH_VT(CALL_FP);
+#undef CALL_FP16
+#undef CALL_FP
 #undef MSDA_DISPATCH_ORDER
 }
 

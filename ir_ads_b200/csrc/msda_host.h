@@ -75,6 +75,11 @@ int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const 
 int fwd_dcn_softmax(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off,
                     const void* mask_logits, void* out, msda::FusedArgs fa);
 
+// packed batch (kPrePacked): d.B images, d.S / d.Q the largest image's value / query count, `meta` the per-image
+// metadata rows (msda::packed_meta_stride), fa.value_mask unused.  LINEAR forward, STRIP backward with float reds.
+int fwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes,
+               const int64_t* meta, const void* off, const void* logits, void* out, msda::FusedArgs fa);
+
 // ---- msda_bwd.cu ----
 int bwd_fast(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const void* go, const void* value,
              const int64_t* shapes, const int64_t* lsi, const void* loc, const void* w, float* gv, void* gl, void* gw);
@@ -108,6 +113,10 @@ int bwd_dcn_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go,
 int bwd_dcn_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                  const void* mask, void* goff, void* gmask, int* cursor, const int* bin_start, void* entries,
                  float* warp_amax, int64_t* n_warps, msda::FusedArgs fa);
+
+int bwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
+               const int64_t* meta, const void* off, const void* logits, float* gv, void* goff, void* glog,
+               msda::FusedArgs fa);
 
 // ---- msda_fold.cu ----
 // does the folding backward cover this problem (encoder form Q == S, shapes it is instantiated for, flags)?

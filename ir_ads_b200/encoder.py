@@ -95,7 +95,9 @@ class DeformableEncoderLayer(nn.Module):
     """self_attn (MSDeformAttn) -> norm -> ffn -> norm, post-norm, batch-first
     (BaseTransformerLayer with operation_order ("self_attn", "norm", "ffn", "norm"), detrex/layers/transformer.py:152-192).
     Both ``x + identity; norm(x)`` epilogues run as ONE fused kernel each (ir_ads_b200/epilogue.py) where it applies
-    (CUDA, float32 / bfloat16); ``fuse_epilogue = False`` restores the op-by-op composition."""
+    (CUDA, float32 / bfloat16); ``fuse_epilogue = False`` restores the op-by-op composition.
+    ``packing=PackedLevels`` (ir_ads_b200/packing.py): ``query`` / ``query_pos`` are packed ``[T, C]`` rows and
+    ``reference_points`` ``[T, L, 2]`` (packed_reference_points); every step after the op works row by row."""
 
     def __init__(self, embed_dim=256, num_heads=8, feedforward_dim=1024, attn_dropout=0.1, ffn_dropout=0.1,
                  num_feature_levels=4, num_points=4):
@@ -116,20 +118,22 @@ class DeformableEncoderLayer(nn.Module):
             attn = self.attentions[0](query, None, None, None, query_pos=query_pos,
                                       key_padding_mask=query_key_padding_mask, reference_points=reference_points,
                                       spatial_shapes=spatial_shapes, level_start_index=level_start_index,
-                                      level_shapes=kwargs.get("level_shapes"), add_identity=False)
+                                      level_shapes=kwargs.get("level_shapes"), packing=kwargs.get("packing"),
+                                      add_identity=False)
             query = add_layer_norm(attn, query, self.norms[0])                    # norm(attn + identity)
             return add_layer_norm(self.ffns[0].layers(query), query, self.norms[1])   # norm(ffn(x) + x)
         query = self.attentions[0](query, None, None, None, query_pos=query_pos,
                                    key_padding_mask=query_key_padding_mask, reference_points=reference_points,
                                    spatial_shapes=spatial_shapes, level_start_index=level_start_index,
-                                   level_shapes=kwargs.get("level_shapes"))
+                                   level_shapes=kwargs.get("level_shapes"), packing=kwargs.get("packing"))
         query = self.norms[0](query)
         query = self.ffns[0](query)
         return self.norms[1](query)
 
 
 class DeformableEncoder(nn.Module):
-    """num_layers x DeformableEncoderLayer (+ optional final LayerNorm), DINOTransformerEncoder's contract."""
+    """num_layers x DeformableEncoderLayer (+ optional final LayerNorm), DINOTransformerEncoder's contract.
+    ``packing=`` is handed to every layer (a packed batch, see DeformableEncoderLayer)."""
 
     def __init__(self, embed_dim=256, num_heads=8, feedforward_dim=1024, attn_dropout=0.1, ffn_dropout=0.1,
                  num_layers=6, post_norm=False, num_feature_levels=4, num_points=4):
@@ -166,7 +170,9 @@ def decoder_reference_points_input(reference_points: torch.Tensor, valid_ratios:
 class DeformableCrossAttentionBlock(nn.Module):
     """The MSDeformAttn cross-attention + norm step of a DINO decoder layer (``cross_attn`` then ``norm`` in
     the layer's operation order, dino_transformer.py:124-150): queries attend to the encoder memory through
-    per-level reference boxes.  The decoder's self-attention (nn.MultiheadAttention) and FFN stay PyTorch."""
+    per-level reference boxes.  The decoder's self-attention (nn.MultiheadAttention) and FFN stay PyTorch.
+    ``packing=PackedLevels``: ``memory`` is the packed ``[T_v, C]`` encoder output of that batch (no key_padding_mask);
+    queries stay ``[B, Q, C]`` and attend to their own image's rows (``packing.cross(Q)``)."""
 
     def __init__(self, embed_dim=256, num_heads=8, attn_dropout=0.1, num_feature_levels=4, num_points=4):
         super().__init__()
@@ -176,8 +182,20 @@ class DeformableCrossAttentionBlock(nn.Module):
         self.norm = nn.LayerNorm(embed_dim)
 
     def forward(self, query, memory, query_pos, reference_points, valid_ratios, spatial_shapes, level_start_index,
-                key_padding_mask=None):
+                key_padding_mask=None, packing=None):
         ref_in = decoder_reference_points_input(reference_points, valid_ratios)
+        if packing is not None:
+            B, Q, C = query.shape
+            cross = packing.cross(Q)
+            rows = (query.reshape(B * Q, C), None if query_pos is None else query_pos.reshape(B * Q, C))
+            ref_rows = ref_in.reshape(B * Q, ref_in.shape[2], ref_in.shape[3])
+            if add_layer_norm_supported(query):
+                out = self.attn(rows[0], None, memory, None, query_pos=rows[1], key_padding_mask=key_padding_mask,
+                                reference_points=ref_rows, packing=cross, add_identity=False)
+                return add_layer_norm(out, rows[0], self.norm).view(B, Q, -1)
+            out = self.attn(rows[0], None, memory, None, query_pos=rows[1], key_padding_mask=key_padding_mask,
+                            reference_points=ref_rows, packing=cross)
+            return self.norm(out).view(B, Q, -1)
         if add_layer_norm_supported(query):
             out = self.attn(query, None, memory, None, query_pos=query_pos, key_padding_mask=key_padding_mask,
                             reference_points=ref_in, spatial_shapes=spatial_shapes, level_start_index=level_start_index,

@@ -390,3 +390,119 @@ def debug_bookkeeping(sampling_loc: torch.Tensor, spatial_shapes: torch.Tensor, 
                                                channels, L, Q, P, _ptr(offs), _ptr(frac))
     _lib.check(status, "msda_debug_bookkeeping")
     return offs, frac
+
+
+# ------------------------------------------------------------------------------------------------
+# packed (padding-free) batches of the fused module path: ir_ads_b200/packing.py, include/msda.h msda_packed_*
+# ------------------------------------------------------------------------------------------------
+def _check_packed_inputs(value, sampling_offsets, attn_logits, reference_points, packing):
+    _require(value.is_cuda, "Not implemented on the CPU")
+    for name, t in (("value", value), ("sampling_offsets", sampling_offsets), ("attn_logits", attn_logits),
+                    ("reference_points", reference_points), ("packing.meta", packing.meta),
+                    ("packing.spatial_shapes", packing.spatial_shapes)):
+        _require(t.is_cuda and t.device == value.device, f"{name} must be a CUDA tensor on {value.device}")
+        _require(t.is_contiguous(), f"{name} tensor has to be contiguous")
+    _require(value.dim() == 3, "value must be [T_v, H, D]")
+    _require(value.dtype in _FUSED_DTYPES, f"unsupported value dtype {value.dtype} (float32, bfloat16, float16)")
+    T_v, H, D = value.shape
+    L = packing.num_levels
+    _require(T_v == packing.total_value, f"value has {T_v} rows, the packing {packing.total_value}")
+    _require(sampling_offsets.dim() == 5 and sampling_offsets.shape[-1] == 2, "sampling_offsets must be [T_q, H, L, P, 2]")
+    T_q, Hq, Lq, P, _ = sampling_offsets.shape
+    _require(Hq == H and Lq == L, "sampling_offsets heads / levels do not match value / packing")
+    _require(T_q == packing.total_query, f"{T_q} query rows, the packing has {packing.total_query}")
+    _require(sampling_offsets.dtype == attn_logits.dtype, "sampling_offsets / attn_logits must share a dtype")
+    tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
+    _require(tuple(attn_logits.shape) == (T_q, H, L * P), "attn_logits must be [T_q, H, L*P]")
+    _require(reference_points.dtype == torch.float32, "reference_points must be float32")
+    ref_dim = reference_points.shape[-1]
+    _require(tuple(reference_points.shape) == (T_q, L, ref_dim) and ref_dim in (2, 4),
+             "reference_points must be [T_q, L, 2 or 4]")
+    return (T_v, H, D, L, T_q, P, ref_dim), tag
+
+
+class MSDeformAttnPackedFunction(Function):
+    """``apply(value, sampling_offsets, attn_logits, reference_points, packing)`` -> ``[T_q, H*D]``: the fused module
+    path over a packed batch (``packing``: an ``ir_ads_b200.packing.PackedLevels``).  ``value [T_v, H, D]``,
+    ``sampling_offsets [T_q, H, L, P, 2]``, ``attn_logits [T_q, H, L*P]``, ``reference_points [T_q, L, 2|4]``, dtypes
+    as MSDeformAttnFusedFunction.  Every query row gets the bits MSDeformAttnFusedFunction gives for the padded batch
+    with ``packing.padding_mask`` as key_padding_mask (output, offset and logit gradients); ``grad_value`` equals its
+    valid rows up to the order of the float reds.
+
+    Two cases leave the packed kernels: deterministic mode and ``reference_points`` that require grad.  Their backward
+    unpacks into the padded layout, runs MSDeformAttnFusedFunction's backward there and packs the gradients -- the bits
+    of the padded route (padding query rows get a zero output gradient)."""
+
+    @staticmethod
+    def forward(ctx, value, sampling_offsets, attn_logits, reference_points, packing):
+        (T_v, H, D, L, T_q, P, ref_dim), tag = _check_packed_inputs(value, sampling_offsets, attn_logits,
+                                                                    reference_points, packing)
+        value, sampling_offsets, attn_logits, reference_points = (
+            _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
+        out = torch.empty((T_q, H * D), dtype=value.dtype, device=value.device)
+        stream = torch.cuda.current_stream(value.device).cuda_stream
+        status = _lib.lib().msda_packed_forward(
+            ctypes.c_void_p(stream), _ptr(value), _ptr(packing.spatial_shapes), _ptr(packing.meta),
+            _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, packing.batch, T_v, H, D, L,
+            T_q, P, packing.max_value, packing.max_query, _ptr(out), tag, _flags(False))
+        _lib.check(status, "msda_packed_forward")
+        ctx.save_for_backward(value, sampling_offsets, attn_logits, reference_points)
+        ctx.packing = packing
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_output):
+        value, sampling_offsets, attn_logits, reference_points = ctx.saved_tensors
+        packing = ctx.packing
+        T_v, H, D = value.shape
+        T_q, _, L, P, _ = sampling_offsets.shape
+        ref_dim = reference_points.shape[-1]
+        _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
+        _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
+        _require(grad_output.numel() == T_q * H * D, "grad_output must be [T_q, H*D]")
+        grad_output = _aligned(grad_output.contiguous())
+        flags = _flags(True)
+        need_ref = ctx.needs_input_grad[3]
+        if (flags & _lib.FLAG_DETERMINISTIC) or need_ref:
+            return _packed_backward_padded(value, sampling_offsets, attn_logits, reference_points, grad_output,
+                                           packing, ctx.needs_input_grad)
+        grad_value = torch.empty_like(value)
+        grad_off = torch.empty_like(sampling_offsets)
+        grad_logits = torch.empty_like(attn_logits)
+        tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
+        handle = _lib.lib()
+        ws_bytes = int(handle.msda_packed_backward_workspace_bytes(T_v, H, D, tag, flags))
+        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None
+        stream = torch.cuda.current_stream(value.device).cuda_stream
+        status = handle.msda_packed_backward(
+            ctypes.c_void_p(stream), _ptr(grad_output), _ptr(value), _ptr(packing.spatial_shapes), _ptr(packing.meta),
+            _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, packing.batch, T_v, H, D, L,
+            T_q, P, packing.max_value, packing.max_query, _ptr(grad_value), _ptr(grad_off), _ptr(grad_logits),
+            _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, flags)
+        _lib.check(status, "msda_packed_backward")
+        return grad_value, grad_off, grad_logits, None, None
+
+
+def _packed_backward_padded(value, sampling_offsets, attn_logits, reference_points, grad_output, packing, needs):
+    """Backward of MSDeformAttnPackedFunction through the padded layout: unpack, MSDeformAttnFusedFunction's own
+    backward (deterministic composition, reference-point gradient), pack the gradients."""
+    from .packing import unpack_tokens
+    v, mask = unpack_tokens(value, packing)
+    off = unpack_tokens(sampling_offsets, packing, queries=True)[0]
+    lg = unpack_tokens(attn_logits, packing, queries=True)[0]
+    ref = unpack_tokens(reference_points, packing, queries=True)[0]
+    go = unpack_tokens(grad_output, packing, queries=True)[0]
+    with torch.enable_grad():
+        inputs = [t.detach().requires_grad_(bool(n)) for t, n in zip((v, off, lg, ref), needs[:4])]
+        out = MSDeformAttnFusedFunction.apply(inputs[0], packing.spatial_shapes, packing.level_start_index,
+                                              inputs[1], inputs[2], inputs[3], mask)
+        wanted = [t for t in inputs if t.requires_grad]
+        grads = iter(torch.autograd.grad(out, wanted, go, allow_unused=True))
+    got = [next(grads) if t.requires_grad else None for t in inputs]
+
+    def pack(g, index):
+        return None if g is None else g.reshape((-1,) + tuple(g.shape[2:])).index_select(0, index)
+
+    return (pack(got[0], packing.value_index), pack(got[1], packing.query_index), pack(got[2], packing.query_index),
+            pack(got[3], packing.query_index), None)

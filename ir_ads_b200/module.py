@@ -22,7 +22,10 @@ What differs from the reference module:
     fused kernels do not cover) still widens float16, since the plain op, like the reference's, has no float16 form;
   * there is no CPU branch (py:350-353): a CPU tensor raises;
   * ``add_identity=False`` (keyword, default True) returns ``dropout(output_proj(...))`` WITHOUT the residual
-    (py:363), for callers that fuse ``+ identity`` into the LayerNorm that follows (ir_ads_b200/epilogue.py).
+    (py:363), for callers that fuse ``+ identity`` into the LayerNorm that follows (ir_ads_b200/epilogue.py);
+  * ``packing=PackedLevels`` (keyword, ir_ads_b200/packing.py): a padding-free batch -- 2-D ``[T_q, C]`` query and
+    ``[T_v, C]`` value, ``reference_points [T_q, L, 2|4]``, no ``key_padding_mask`` -- through the packed fused
+    kernels (MSDeformAttnPackedFunction); the result is ``[T_q, C]``.
 """
 from __future__ import annotations
 
@@ -34,7 +37,8 @@ from typing import Optional
 import torch
 import torch.nn as nn
 
-from .functional import MSDeformAttnFusedFunction, MultiScaleDeformableAttnFunction, fused_supported
+from .functional import (MSDeformAttnFusedFunction, MSDeformAttnPackedFunction, MultiScaleDeformableAttnFunction,
+                         fused_supported)
 
 
 # shapes tensors already validated: id(tensor) -> (version, num_value); entries die with their tensor
@@ -120,6 +124,38 @@ class MultiScaleDeformableAttention(nn.Module):
             weakref.finalize(spatial_shapes, _SHAPE_CHECKS.pop, key, None)   # the id may be re-used after death
         _SHAPE_CHECKS[key] = (spatial_shapes._version, num_value)
 
+    def _forward_packed(self, query, value, identity, reference_points, key_padding_mask, packing, add_identity):
+        if key_padding_mask is not None:
+            raise ValueError("a packed batch has no padding: key_padding_mask must be None")
+        if query.dim() != 2 or value.dim() != 2:
+            raise ValueError("with packing=, query and value are 2-D [T, C] token rows")
+        if value.shape[0] != packing.total_value or query.shape[0] != packing.total_query:
+            raise AssertionError(f"{value.shape[0]} value / {query.shape[0]} query rows, the packing has "
+                                 f"{packing.total_value} / {packing.total_query}")
+        H, L, P = self.num_heads, self.num_levels, self.num_points
+        if packing.num_levels != L:
+            raise AssertionError(f"the packing has {packing.num_levels} levels, the module {L}")
+        if reference_points.shape[-1] not in (2, 4):
+            raise ValueError(
+                f"Last dim of reference_points must be 2 or 4, but get {reference_points.shape[-1]} instead.")
+        T_q = query.shape[0]
+        value = self.value_proj(value)
+        io_dtype = value.dtype
+        value = value.view(value.shape[0], H, -1)
+        if not (self.fuse_pre_ops and fused_supported(value.unsqueeze(0), L, P)):
+            raise RuntimeError("packed batches run on the fused kernels only (fuse_pre_ops, CUDA, float32 / bfloat16 / "
+                               "float16, head dim 16/32/64/128, L <= 16, L*P <= 64)")
+        offsets = self.sampling_offsets(query).view(T_q, H, L, P, 2)
+        logits = self.attention_weights(query).view(T_q, H, L * P)
+        if not (offsets.dtype == logits.dtype == value.dtype and value.dtype in (torch.float16, torch.bfloat16)):
+            offsets, logits = offsets.float(), logits.float()
+        output = MSDeformAttnPackedFunction.apply(value.contiguous(), offsets.contiguous(), logits.contiguous(),
+                                                  reference_points.float().contiguous(), packing)
+        if output.dtype != io_dtype:
+            output = output.to(io_dtype)
+        output = self.dropout(self.output_proj(output))
+        return output + identity if add_identity else output
+
     def forward(self, query: torch.Tensor, key: Optional[torch.Tensor] = None, value: Optional[torch.Tensor] = None,
                 identity: Optional[torch.Tensor] = None, query_pos: Optional[torch.Tensor] = None,
                 key_padding_mask: Optional[torch.Tensor] = None, reference_points: Optional[torch.Tensor] = None,
@@ -131,6 +167,10 @@ class MultiScaleDeformableAttention(nn.Module):
             identity = query
         if query_pos is not None:
             query = query + query_pos
+        packing = kwargs.get("packing")
+        if packing is not None:
+            return self._forward_packed(query, value, identity, reference_points, key_padding_mask, packing,
+                                        kwargs.get("add_identity", True))
         if not self.batch_first:
             query = query.permute(1, 0, 2)
             value = value.permute(1, 0, 2)
