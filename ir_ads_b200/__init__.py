@@ -17,6 +17,7 @@ from .functional import (  # noqa: F401
 from .dcnv3 import DCNv3FusedFunction, DCNv3Function, dcnv3_backward, dcnv3_forward  # noqa: F401
 from .module import MultiScaleDeformableAttention  # noqa: F401
 from .packing import PackedLevels, pack_levels, packed_reference_points, unpack_tokens, valid_extents  # noqa: F401
+from . import ops  # noqa: F401,E402  (registers the torch.library custom ops; loads no library)
 
 __all__ = [
     "MultiScaleDeformableAttention",
@@ -36,4 +37,5 @@ __all__ = [
     "pack_levels",
     "packed_reference_points",
     "unpack_tokens",
+    "ops",
 ]

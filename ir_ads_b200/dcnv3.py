@@ -93,6 +93,13 @@ def dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, 
     offset / mask gradients are computed in float32).  Under ``set_deterministic(True)`` or
     ``torch.use_deterministic_algorithms(True)`` grad_input is bit-reproducible (MSDA_FLAG_DETERMINISTIC); grad_offset
     and grad_mask are the same bits either way."""
+    return _dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                           dilation_w, group, group_channels, offset_scale, grad_output, functional._flags(True))
+
+
+def _dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w,
+                    group, group_channels, offset_scale, grad_output, flags) -> List[torch.Tensor]:
+    """dcnv3_backward under the MSDA_FLAG_* bits ``flags``."""
     N, H_in, W_in, H_out, W_out = _geometry(input, offset, mask, kernel_h, kernel_w, group, group_channels)
     _require(grad_output.is_cuda and grad_output.dtype == input.dtype, "grad_output must match input's device / dtype")
     grad_output = _aligned(grad_output.contiguous())
@@ -101,7 +108,6 @@ def dcnv3_backward(input, offset, mask, kernel_h, kernel_w, stride_h, stride_w, 
     grad_input = torch.empty_like(input)
     grad_offset = torch.empty_like(offset)
     grad_mask = torch.empty_like(mask)
-    flags = functional._flags(True)
     tag = _DCN_TAG[input.dtype]
     handle = _declare(_lib.lib())
     ws_bytes = handle.msda_dcnv3_backward_workspace_bytes(kernel_h, kernel_w, group, group_channels, N, H_in, W_in,
@@ -280,19 +286,25 @@ class DCNv3FusedFunction(Function):
     @once_differentiable
     def backward(ctx, grad_output):
         input, offset, mask_logits = ctx.saved_tensors
-        grad_output = grad_output.to(input.dtype)
-        if not functional._flags(True) & _lib.FLAG_DETERMINISTIC:
-            return tuple(dcnv3_fused_backward(input, offset, mask_logits, *ctx.args, grad_output)) + (None,) * 12
-        # 16-bit offset / logits are widened (exact) and the final gradients cast: the float32 route's bits
-        aux_dtype = offset.dtype
-        N, H_out, W_out, _ = mask_logits.shape
-        with torch.enable_grad():
-            logits = mask_logits.detach().float().view(N, H_out, W_out, ctx.args[8], -1).requires_grad_(True)
-            mask = torch.softmax(logits, -1)
-        gi, go, gm = dcnv3_backward(input, offset.float(), mask.detach().view(N, H_out, W_out, -1), *ctx.args,
-                                    grad_output, ctx.im2col_step)
-        (g_logits,) = torch.autograd.grad(mask, logits, gm.view_as(mask))
-        return (gi, go.to(aux_dtype), g_logits.view_as(mask_logits).to(aux_dtype)) + (None,) * 12
+        return tuple(_dcnv3_fused_backward_route(input, offset, mask_logits, ctx.args, grad_output,
+                                                 functional._flags(True))) + (None,) * 12
+
+
+def _dcnv3_fused_backward_route(input, offset, mask_logits, args, grad_output, flags):
+    """DCNv3FusedFunction's backward (also the body of ``ir_ads_b200::dcnv3_fused_backward``) under the MSDA_FLAG_*
+    bits ``flags``; ``args``: the eleven geometry arguments.  ``[grad_input, grad_offset, grad_mask_logits]``."""
+    grad_output = grad_output.to(input.dtype)
+    if not flags & _lib.FLAG_DETERMINISTIC:
+        return dcnv3_fused_backward(input, offset, mask_logits, *args, grad_output)
+    # 16-bit offset / logits are widened (exact) and the final gradients cast: the float32 route's bits
+    # The softmax's chain rule is the kernel autograd's SoftmaxBackward runs, called directly: inside a custom op
+    # (ir_ads_b200/ops.py) autograd is switched off below the dispatcher, and torch.enable_grad does not restore it.
+    aux_dtype = offset.dtype
+    N, H_out, W_out, _ = mask_logits.shape
+    mask = torch.softmax(mask_logits.detach().float().view(N, H_out, W_out, args[8], -1), -1)
+    gi, go, gm = _dcnv3_backward(input, offset.float(), mask.view(N, H_out, W_out, -1), *args, grad_output, flags)
+    g_logits = torch._softmax_backward_data(gm.view_as(mask), mask, -1, torch.float32)
+    return [gi, go.to(aux_dtype), g_logits.view_as(mask_logits).to(aux_dtype)]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -400,8 +412,13 @@ class DCNv3(nn.Module):
             mask_logits = self.mask(x1)
             if not (offset.dtype == mask_logits.dtype == dtype and dtype in (torch.float16, torch.bfloat16)):
                 offset, mask_logits = offset.float(), mask_logits.float()
-            x = DCNv3FusedFunction.apply(x.contiguous(), offset.contiguous(),
-                                         mask_logits.reshape(N, H, W, -1).contiguous(), *geometry)
+            if torch.compiler.is_compiling():
+                x = torch.ops.ir_ads_b200.dcnv3_fused(x.contiguous(), offset.contiguous(),
+                                                      mask_logits.reshape(N, H, W, -1).contiguous(), *geometry[:11],
+                                                      functional._deterministic())
+            else:
+                x = DCNv3FusedFunction.apply(x.contiguous(), offset.contiguous(),
+                                             mask_logits.reshape(N, H, W, -1).contiguous(), *geometry)
         else:
             mask = F.softmax(self.mask(x1).reshape(N, H, W, self.group, -1), -1).reshape(N, H, W, -1).type(dtype)
             x = DCNv3Function.apply(x.contiguous(), offset.contiguous(), mask.contiguous(), *geometry)

@@ -172,7 +172,8 @@ class DeformableCrossAttentionBlock(nn.Module):
     the layer's operation order, dino_transformer.py:124-150): queries attend to the encoder memory through
     per-level reference boxes.  The decoder's self-attention (nn.MultiheadAttention) and FFN stay PyTorch.
     ``packing=PackedLevels``: ``memory`` is the packed ``[T_v, C]`` encoder output of that batch (no key_padding_mask);
-    queries stay ``[B, Q, C]`` and attend to their own image's rows (``packing.cross(Q)``)."""
+    queries stay ``[B, Q, C]`` and attend to their own image's rows (``packing.cross(Q)``).  ``level_shapes``: the host
+    ``(H_l, W_l)`` list, handed to the module's shape check (no device read; what torch.compile needs)."""
 
     def __init__(self, embed_dim=256, num_heads=8, attn_dropout=0.1, num_feature_levels=4, num_points=4):
         super().__init__()
@@ -182,7 +183,7 @@ class DeformableCrossAttentionBlock(nn.Module):
         self.norm = nn.LayerNorm(embed_dim)
 
     def forward(self, query, memory, query_pos, reference_points, valid_ratios, spatial_shapes, level_start_index,
-                key_padding_mask=None, packing=None):
+                key_padding_mask=None, packing=None, level_shapes=None):
         ref_in = decoder_reference_points_input(reference_points, valid_ratios)
         if packing is not None:
             B, Q, C = query.shape
@@ -199,8 +200,9 @@ class DeformableCrossAttentionBlock(nn.Module):
         if add_layer_norm_supported(query):
             out = self.attn(query, None, memory, None, query_pos=query_pos, key_padding_mask=key_padding_mask,
                             reference_points=ref_in, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
-                            add_identity=False)
+                            level_shapes=level_shapes, add_identity=False)
             return add_layer_norm(out, query, self.norm)
         out = self.attn(query, None, memory, None, query_pos=query_pos, key_padding_mask=key_padding_mask,
-                        reference_points=ref_in, spatial_shapes=spatial_shapes, level_start_index=level_start_index)
+                        reference_points=ref_in, spatial_shapes=spatial_shapes, level_start_index=level_start_index,
+                        level_shapes=level_shapes)
         return self.norm(out)

@@ -74,6 +74,12 @@ def _flags(backward: bool) -> int:
     return f
 
 
+def _deterministic() -> bool:
+    """Whether backward passes take the bit-reproducible route.  The custom ops (ir_ads_b200/ops.py) take it as an
+    argument, read here while the graph is built, so that the compiler guards on it."""
+    return bool(_flags(True) & _lib.FLAG_DETERMINISTIC)
+
+
 def _ptr(t: torch.Tensor) -> ctypes.c_void_p:
     return ctypes.c_void_p(t.data_ptr())
 
@@ -142,11 +148,12 @@ def ms_deform_attn_backward(value: torch.Tensor, spatial_shapes: torch.Tensor, l
 
 
 def _backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, grad_output,
-              need_grad_value: bool, tags=_DTYPE_TAG) -> List[torch.Tensor]:
+              need_grad_value: bool, tags=_DTYPE_TAG, flags=None) -> List[torch.Tensor]:
     """The backward behind ms_deform_attn_backward.  ``need_grad_value=False`` (the autograd Function passes it when
     ``value`` does not require grad, e.g. a frozen memory branch) returns ``None`` for ``grad_value`` and, on the
     shapes the fast kernels cover, skips its scatter -- the dominant cost of the backward -- altogether.  ``tags``:
-    the accepted value dtypes (library-internal callers pass _VALUE_TAG to hand float16 over natively)."""
+    the accepted value dtypes (library-internal callers pass _VALUE_TAG to hand float16 over natively).  ``flags``:
+    the MSDA_FLAG_* bits, ``_flags(True)`` when not given."""
     B, S, H, D, L, Q, P = _check_inputs(value, spatial_shapes, level_start_index, sampling_loc, attn_weight, tags)
     _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
     _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
@@ -155,7 +162,7 @@ def _backward(value, spatial_shapes, level_start_index, sampling_loc, attn_weigh
     value, sampling_loc, attn_weight = _aligned(value), _aligned(sampling_loc), _aligned(attn_weight)
     grad_loc = torch.empty_like(sampling_loc)
     grad_w = torch.empty_like(attn_weight)
-    flags = _flags(True)
+    flags = _flags(True) if flags is None else flags
     tag = tags[value.dtype]
     handle = _lib.lib()
     skip_scatter = (not need_grad_value and B * S * D > 0 and Q * L * P > 0
@@ -226,7 +233,17 @@ def fused_supported(value: torch.Tensor, num_levels: int, num_points: int) -> bo
     if not value.is_cuda or value.dtype not in _FUSED_DTYPES or value.dim() != 4:
         return False
     _, S, H, D = value.shape
-    return bool(_lib.lib().msda_fused_supported(D, num_levels, num_points, S, H, _VALUE_TAG[value.dtype], _flags(False)))
+    if not isinstance(S, int):
+        # a dynamic value length under torch.compile: asked as 0, which leaves the 32-bit offset bound on S to the
+        # kernels' entry points (they refuse a problem past it)
+        S = 0
+    return _fused_supported_dims(D, num_levels, num_points, S, H, _VALUE_TAG[value.dtype], _flags(False))
+
+
+@torch.compiler.assume_constant_result
+def _fused_supported_dims(D, L, P, S, H, tag, flags) -> bool:
+    """Under torch.compile the answer is taken while the graph is built, for the traced shapes."""
+    return bool(_lib.lib().msda_fused_supported(D, L, P, S, H, tag, flags))
 
 
 def _mask_ptr(mask) -> ctypes.c_void_p:
@@ -304,77 +321,95 @@ class MSDeformAttnFusedFunction(Function):
     @staticmethod
     def forward(ctx, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points,
                 key_padding_mask=None):
-        (B, S, H, D, L, Q, P, ref_dim), mask, tag = _check_fused_inputs(
-            value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points, key_padding_mask)
-        value, sampling_offsets, attn_logits, reference_points = (
-            _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
-        out = torch.empty((B, Q, H * D), dtype=value.dtype, device=value.device)
-        stream = torch.cuda.current_stream(value.device).cuda_stream
-        status = _lib.lib().msda_fused_forward(
-            ctypes.c_void_p(stream), _ptr(value), _ptr(spatial_shapes), _ptr(level_start_index), _ptr(sampling_offsets),
-            _ptr(attn_logits), _ptr(reference_points), ref_dim, _mask_ptr(mask), B, S, H, D, L, Q, P, _ptr(out),
-            tag, _flags(False))
-        _lib.check(status, "msda_fused_forward")
-        ctx.save_for_backward(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points)
+        out, saved, mask = _fused_forward(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits,
+                                          reference_points, key_padding_mask)
+        ctx.save_for_backward(*saved)
         ctx.value_mask = mask
         return out
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_output):
-        value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points = ctx.saved_tensors
-        B, S, H, D = value.shape
-        _, Q, _, L, P, _ = sampling_offsets.shape
-        ref_dim = reference_points.shape[-1]
-        _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
-        _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
-        _require(grad_output.numel() == B * Q * H * D, "grad_output must be [B, Q, H*D]")
-        grad_output = _aligned(grad_output.contiguous())
-        flags = _flags(True)
-        mask = ctx.value_mask
-        need_ref = ctx.needs_input_grad[5]
-        if (flags & _lib.FLAG_DETERMINISTIC) or need_ref:
-            # Composition around the unfused backward: the deterministic mode, and the rare case of reference points
-            # that require grad (DINO detaches them) -- d loc / d ref is the identity on (x, y) and off / P * 0.5 on
-            # (w, h), taken from grad_sampling_loc itself so that boxes with w == 0 or h == 0 keep their (x, y) grad.
-            # 16-bit offsets / logits are widened (exact) and the final gradients cast: the float32 route's bits.
-            aux_dtype = sampling_offsets.dtype
-            sampling_offsets, attn_logits = sampling_offsets.float(), attn_logits.float()
-            loc, weights = _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_points)
-            v = value if mask is None else value.masked_fill(mask.bool()[..., None, None], 0)
-            grad_value, g_loc, g_w = _backward(v, spatial_shapes, level_start_index, loc, weights, grad_output,
-                                               need_grad_value=ctx.needs_input_grad[0], tags=_VALUE_TAG)
-            if grad_value is not None and mask is not None:
-                grad_value = grad_value.masked_fill(mask.bool()[..., None, None], 0)
-            g_w = g_w.view(B, Q, H, L * P)
-            w_flat = weights.view(B, Q, H, L * P)
-            grad_logits = w_flat * (g_w - (g_w * w_flat).sum(-1, keepdim=True))
-            if ref_dim == 2:
-                normalizer = torch.stack([spatial_shapes[..., 1], spatial_shapes[..., 0]], -1).to(g_loc.dtype)
-                grad_off = g_loc / normalizer[None, None, None, :, None, :]
-            else:
-                grad_off = g_loc * (reference_points[:, :, None, :, None, 2:] * (0.5 / P))
-            grad_ref = None
-            if need_ref:
-                g_xy = g_loc.sum(dim=(2, 4))
-                grad_ref = g_xy if ref_dim == 2 else torch.cat(
-                    [g_xy, (g_loc * sampling_offsets * (0.5 / P)).sum(dim=(2, 4))], -1)
-            return grad_value, None, None, grad_off.to(aux_dtype), grad_logits.to(aux_dtype), grad_ref, None
-        grad_value = torch.empty_like(value)
-        grad_off = torch.empty_like(sampling_offsets)
-        grad_logits = torch.empty_like(attn_logits)
-        tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
-        handle = _lib.lib()
-        ws_bytes = int(handle.msda_backward_workspace_bytes(B, S, H, D, L, Q, P, tag, flags))
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None
-        stream = torch.cuda.current_stream(value.device).cuda_stream
-        status = handle.msda_fused_backward(
-            ctypes.c_void_p(stream), _ptr(grad_output), _ptr(value), _ptr(spatial_shapes), _ptr(level_start_index),
-            _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, _mask_ptr(mask),
-            B, S, H, D, L, Q, P, _ptr(grad_value), _ptr(grad_off), _ptr(grad_logits),
-            _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, flags)
-        _lib.check(status, "msda_fused_backward")
-        return grad_value, None, None, grad_off, grad_logits, None, None
+        grad_value, grad_off, grad_logits, grad_ref = _fused_backward(
+            grad_output, *ctx.saved_tensors, ctx.value_mask, _flags(True), ctx.needs_input_grad[0],
+            ctx.needs_input_grad[5])
+        return grad_value, None, None, grad_off, grad_logits, grad_ref, None
+
+
+def _fused_forward(value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points,
+                   key_padding_mask):
+    """MSDeformAttnFusedFunction's forward (also the body of the ``ir_ads_b200::msda_fused`` op): the output, the
+    aligned tensors its backward reads and the contiguous padding mask."""
+    (B, S, H, D, L, Q, P, ref_dim), mask, tag = _check_fused_inputs(
+        value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points, key_padding_mask)
+    value, sampling_offsets, attn_logits, reference_points = (
+        _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
+    out = torch.empty((B, Q, H * D), dtype=value.dtype, device=value.device)
+    stream = torch.cuda.current_stream(value.device).cuda_stream
+    status = _lib.lib().msda_fused_forward(
+        ctypes.c_void_p(stream), _ptr(value), _ptr(spatial_shapes), _ptr(level_start_index), _ptr(sampling_offsets),
+        _ptr(attn_logits), _ptr(reference_points), ref_dim, _mask_ptr(mask), B, S, H, D, L, Q, P, _ptr(out),
+        tag, _flags(False))
+    _lib.check(status, "msda_fused_forward")
+    return out, (value, spatial_shapes, level_start_index, sampling_offsets, attn_logits, reference_points), mask
+
+
+def _fused_backward(grad_output, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits,
+                    reference_points, mask, flags, need_value, need_ref):
+    """MSDeformAttnFusedFunction's backward (also the body of ``ir_ads_b200::msda_fused_backward``) under the
+    MSDA_FLAG_* bits ``flags``: ``[grad_value, grad_offsets, grad_logits, grad_reference_points]``.  ``grad_value`` may
+    be None when ``need_value`` is False; ``grad_reference_points`` is None unless ``need_ref``."""
+    B, S, H, D = value.shape
+    _, Q, _, L, P, _ = sampling_offsets.shape
+    ref_dim = reference_points.shape[-1]
+    _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
+    _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
+    _require(grad_output.numel() == B * Q * H * D, "grad_output must be [B, Q, H*D]")
+    grad_output = _aligned(grad_output.contiguous())
+    value, sampling_offsets, attn_logits, reference_points = (
+        _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
+    if (flags & _lib.FLAG_DETERMINISTIC) or need_ref:
+        # Composition around the unfused backward: the deterministic mode, and the rare case of reference points
+        # that require grad (DINO detaches them) -- d loc / d ref is the identity on (x, y) and off / P * 0.5 on
+        # (w, h), taken from grad_sampling_loc itself so that boxes with w == 0 or h == 0 keep their (x, y) grad.
+        # 16-bit offsets / logits are widened (exact) and the final gradients cast: the float32 route's bits.
+        aux_dtype = sampling_offsets.dtype
+        sampling_offsets, attn_logits = sampling_offsets.float(), attn_logits.float()
+        loc, weights = _fused_pre_ops(spatial_shapes, sampling_offsets, attn_logits, reference_points)
+        v = value if mask is None else value.masked_fill(mask.bool()[..., None, None], 0)
+        grad_value, g_loc, g_w = _backward(v, spatial_shapes, level_start_index, loc, weights, grad_output,
+                                           need_grad_value=need_value, tags=_VALUE_TAG, flags=flags)
+        if grad_value is not None and mask is not None:
+            grad_value = grad_value.masked_fill(mask.bool()[..., None, None], 0)
+        g_w = g_w.view(B, Q, H, L * P)
+        w_flat = weights.view(B, Q, H, L * P)
+        grad_logits = w_flat * (g_w - (g_w * w_flat).sum(-1, keepdim=True))
+        if ref_dim == 2:
+            normalizer = torch.stack([spatial_shapes[..., 1], spatial_shapes[..., 0]], -1).to(g_loc.dtype)
+            grad_off = g_loc / normalizer[None, None, None, :, None, :]
+        else:
+            grad_off = g_loc * (reference_points[:, :, None, :, None, 2:] * (0.5 / P))
+        grad_ref = None
+        if need_ref:
+            g_xy = g_loc.sum(dim=(2, 4))
+            grad_ref = g_xy if ref_dim == 2 else torch.cat(
+                [g_xy, (g_loc * sampling_offsets * (0.5 / P)).sum(dim=(2, 4))], -1)
+        return grad_value, grad_off.to(aux_dtype), grad_logits.to(aux_dtype), grad_ref
+    grad_value = torch.empty_like(value)
+    grad_off = torch.empty_like(sampling_offsets)
+    grad_logits = torch.empty_like(attn_logits)
+    tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
+    handle = _lib.lib()
+    ws_bytes = int(handle.msda_backward_workspace_bytes(B, S, H, D, L, Q, P, tag, flags))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None
+    stream = torch.cuda.current_stream(value.device).cuda_stream
+    status = handle.msda_fused_backward(
+        ctypes.c_void_p(stream), _ptr(grad_output), _ptr(value), _ptr(spatial_shapes), _ptr(level_start_index),
+        _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, _mask_ptr(mask),
+        B, S, H, D, L, Q, P, _ptr(grad_value), _ptr(grad_off), _ptr(grad_logits),
+        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, flags)
+    _lib.check(status, "msda_fused_backward")
+    return grad_value, grad_off, grad_logits, None
 
 
 def debug_bookkeeping(sampling_loc: torch.Tensor, spatial_shapes: torch.Tensor, level_start_index: torch.Tensor,
@@ -435,56 +470,69 @@ class MSDeformAttnPackedFunction(Function):
 
     @staticmethod
     def forward(ctx, value, sampling_offsets, attn_logits, reference_points, packing):
-        (T_v, H, D, L, T_q, P, ref_dim), tag = _check_packed_inputs(value, sampling_offsets, attn_logits,
-                                                                    reference_points, packing)
-        value, sampling_offsets, attn_logits, reference_points = (
-            _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
-        out = torch.empty((T_q, H * D), dtype=value.dtype, device=value.device)
-        stream = torch.cuda.current_stream(value.device).cuda_stream
-        status = _lib.lib().msda_packed_forward(
-            ctypes.c_void_p(stream), _ptr(value), _ptr(packing.spatial_shapes), _ptr(packing.meta),
-            _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, packing.batch, T_v, H, D, L,
-            T_q, P, packing.max_value, packing.max_query, _ptr(out), tag, _flags(False))
-        _lib.check(status, "msda_packed_forward")
-        ctx.save_for_backward(value, sampling_offsets, attn_logits, reference_points)
+        out, saved = _packed_forward(value, sampling_offsets, attn_logits, reference_points, packing)
+        ctx.save_for_backward(*saved)
         ctx.packing = packing
         return out
 
     @staticmethod
     @once_differentiable
     def backward(ctx, grad_output):
-        value, sampling_offsets, attn_logits, reference_points = ctx.saved_tensors
-        packing = ctx.packing
-        T_v, H, D = value.shape
-        T_q, _, L, P, _ = sampling_offsets.shape
-        ref_dim = reference_points.shape[-1]
-        _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
-        _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
-        _require(grad_output.numel() == T_q * H * D, "grad_output must be [T_q, H*D]")
-        grad_output = _aligned(grad_output.contiguous())
-        flags = _flags(True)
-        need_ref = ctx.needs_input_grad[3]
-        if (flags & _lib.FLAG_DETERMINISTIC) or need_ref:
-            return _packed_backward_padded(value, sampling_offsets, attn_logits, reference_points, grad_output,
-                                           packing, ctx.needs_input_grad)
-        grad_value = torch.empty_like(value)
-        grad_off = torch.empty_like(sampling_offsets)
-        grad_logits = torch.empty_like(attn_logits)
-        tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
-        handle = _lib.lib()
-        ws_bytes = int(handle.msda_packed_backward_workspace_bytes(T_v, H, D, tag, flags))
-        ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None
-        stream = torch.cuda.current_stream(value.device).cuda_stream
-        status = handle.msda_packed_backward(
-            ctypes.c_void_p(stream), _ptr(grad_output), _ptr(value), _ptr(packing.spatial_shapes), _ptr(packing.meta),
-            _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, packing.batch, T_v, H, D, L,
-            T_q, P, packing.max_value, packing.max_query, _ptr(grad_value), _ptr(grad_off), _ptr(grad_logits),
-            _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, flags)
-        _lib.check(status, "msda_packed_backward")
-        return grad_value, grad_off, grad_logits, None, None
+        return _packed_backward(grad_output, *ctx.saved_tensors, ctx.packing, _flags(True), ctx.needs_input_grad[:4])
 
 
-def _packed_backward_padded(value, sampling_offsets, attn_logits, reference_points, grad_output, packing, needs):
+def _packed_forward(value, sampling_offsets, attn_logits, reference_points, packing):
+    """MSDeformAttnPackedFunction's forward (also the body of ``ir_ads_b200::msda_packed``): the output and the
+    aligned tensors its backward reads."""
+    (T_v, H, D, L, T_q, P, ref_dim), tag = _check_packed_inputs(value, sampling_offsets, attn_logits,
+                                                                reference_points, packing)
+    value, sampling_offsets, attn_logits, reference_points = (
+        _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
+    out = torch.empty((T_q, H * D), dtype=value.dtype, device=value.device)
+    stream = torch.cuda.current_stream(value.device).cuda_stream
+    status = _lib.lib().msda_packed_forward(
+        ctypes.c_void_p(stream), _ptr(value), _ptr(packing.spatial_shapes), _ptr(packing.meta),
+        _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, packing.batch, T_v, H, D, L,
+        T_q, P, packing.max_value, packing.max_query, _ptr(out), tag, _flags(False))
+    _lib.check(status, "msda_packed_forward")
+    return out, (value, sampling_offsets, attn_logits, reference_points)
+
+
+def _packed_backward(grad_output, value, sampling_offsets, attn_logits, reference_points, packing, flags, needs):
+    """MSDeformAttnPackedFunction's backward (also the body of ``ir_ads_b200::msda_packed_backward``) under the
+    MSDA_FLAG_* bits ``flags``; ``needs``: which of value, offsets, logits and reference points want a gradient.
+    Returns ``(grad_value, grad_offsets, grad_logits, grad_reference_points, None)``."""
+    T_v, H, D = value.shape
+    T_q, _, L, P, _ = sampling_offsets.shape
+    ref_dim = reference_points.shape[-1]
+    _require(grad_output.is_cuda and grad_output.device == value.device, "grad_output must be a CUDA tensor")
+    _require(grad_output.dtype == value.dtype, "grad_output dtype must match value")
+    _require(grad_output.numel() == T_q * H * D, "grad_output must be [T_q, H*D]")
+    grad_output = _aligned(grad_output.contiguous())
+    value, sampling_offsets, attn_logits, reference_points = (
+        _aligned(value), _aligned(sampling_offsets), _aligned(attn_logits), _aligned(reference_points))
+    if (flags & _lib.FLAG_DETERMINISTIC) or needs[3]:
+        return _packed_backward_padded(value, sampling_offsets, attn_logits, reference_points, grad_output,
+                                       packing, flags, needs)
+    grad_value = torch.empty_like(value)
+    grad_off = torch.empty_like(sampling_offsets)
+    grad_logits = torch.empty_like(attn_logits)
+    tag = _aux_tag(value.dtype, sampling_offsets.dtype, "sampling_offsets / attn_logits")
+    handle = _lib.lib()
+    ws_bytes = int(handle.msda_packed_backward_workspace_bytes(T_v, H, D, tag, flags))
+    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=value.device) if ws_bytes else None
+    stream = torch.cuda.current_stream(value.device).cuda_stream
+    status = handle.msda_packed_backward(
+        ctypes.c_void_p(stream), _ptr(grad_output), _ptr(value), _ptr(packing.spatial_shapes), _ptr(packing.meta),
+        _ptr(sampling_offsets), _ptr(attn_logits), _ptr(reference_points), ref_dim, packing.batch, T_v, H, D, L,
+        T_q, P, packing.max_value, packing.max_query, _ptr(grad_value), _ptr(grad_off), _ptr(grad_logits),
+        _ptr(ws) if ws is not None else ctypes.c_void_p(0), ws_bytes, tag, flags)
+    _lib.check(status, "msda_packed_backward")
+    return grad_value, grad_off, grad_logits, None, None
+
+
+def _packed_backward_padded(value, sampling_offsets, attn_logits, reference_points, grad_output, packing, flags,
+                            needs):
     """Backward of MSDeformAttnPackedFunction through the padded layout: unpack, MSDeformAttnFusedFunction's own
     backward (deterministic composition, reference-point gradient), pack the gradients."""
     from .packing import unpack_tokens
@@ -493,16 +541,11 @@ def _packed_backward_padded(value, sampling_offsets, attn_logits, reference_poin
     lg = unpack_tokens(attn_logits, packing, queries=True)[0]
     ref = unpack_tokens(reference_points, packing, queries=True)[0]
     go = unpack_tokens(grad_output, packing, queries=True)[0]
-    with torch.enable_grad():
-        inputs = [t.detach().requires_grad_(bool(n)) for t, n in zip((v, off, lg, ref), needs[:4])]
-        out = MSDeformAttnFusedFunction.apply(inputs[0], packing.spatial_shapes, packing.level_start_index,
-                                              inputs[1], inputs[2], inputs[3], mask)
-        wanted = [t for t in inputs if t.requires_grad]
-        grads = iter(torch.autograd.grad(out, wanted, go, allow_unused=True))
-    got = [next(grads) if t.requires_grad else None for t in inputs]
+    got = _fused_backward(go, v, packing.spatial_shapes, packing.level_start_index, off, lg, ref, mask, flags,
+                          bool(needs[0]), bool(needs[3]))
 
-    def pack(g, index):
-        return None if g is None else g.reshape((-1,) + tuple(g.shape[2:])).index_select(0, index)
+    def pack(g, index, need):
+        return None if g is None or not need else g.reshape((-1,) + tuple(g.shape[2:])).index_select(0, index)
 
-    return (pack(got[0], packing.value_index), pack(got[1], packing.query_index), pack(got[2], packing.query_index),
-            pack(got[3], packing.query_index), None)
+    return (pack(got[0], packing.value_index, needs[0]), pack(got[1], packing.query_index, needs[1]),
+            pack(got[2], packing.query_index, needs[2]), pack(got[3], packing.query_index, needs[3]), None)

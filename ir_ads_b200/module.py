@@ -38,7 +38,7 @@ import torch
 import torch.nn as nn
 
 from .functional import (MSDeformAttnFusedFunction, MSDeformAttnPackedFunction, MultiScaleDeformableAttnFunction,
-                         fused_supported)
+                         _deterministic, fused_supported)
 
 
 # shapes tensors already validated: id(tensor) -> (version, num_value); entries die with their tensor
@@ -149,8 +149,15 @@ class MultiScaleDeformableAttention(nn.Module):
         logits = self.attention_weights(query).view(T_q, H, L * P)
         if not (offsets.dtype == logits.dtype == value.dtype and value.dtype in (torch.float16, torch.bfloat16)):
             offsets, logits = offsets.float(), logits.float()
-        output = MSDeformAttnPackedFunction.apply(value.contiguous(), offsets.contiguous(), logits.contiguous(),
-                                                  reference_points.float().contiguous(), packing)
+        if torch.compiler.is_compiling():
+            output = torch.ops.ir_ads_b200.msda_packed(
+                value.contiguous(), offsets.contiguous(), logits.contiguous(), reference_points.float().contiguous(),
+                packing.meta, packing.spatial_shapes, packing.level_start_index, packing.value_index,
+                packing.query_index, packing.padding_mask, packing.max_value, packing.max_query, packing.query_pad,
+                _deterministic())
+        else:
+            output = MSDeformAttnPackedFunction.apply(value.contiguous(), offsets.contiguous(), logits.contiguous(),
+                                                      reference_points.float().contiguous(), packing)
         if output.dtype != io_dtype:
             output = output.to(io_dtype)
         output = self.dropout(self.output_proj(output))
@@ -204,9 +211,14 @@ class MultiScaleDeformableAttention(nn.Module):
             # gradients, so neither a float32 copy nor a cast kernel exists in either direction.
             if not (offsets.dtype == logits.dtype == value.dtype and value.dtype in (torch.float16, torch.bfloat16)):
                 offsets, logits = offsets.float(), logits.float()
-            output = MSDeformAttnFusedFunction.apply(
-                value.contiguous(), spatial_shapes, level_start_index, offsets.contiguous(),
-                logits.contiguous(), reference_points.float().contiguous(), key_padding_mask)
+            if torch.compiler.is_compiling():
+                output = torch.ops.ir_ads_b200.msda_fused(
+                    value.contiguous(), spatial_shapes, level_start_index, offsets.contiguous(), logits.contiguous(),
+                    reference_points.float().contiguous(), key_padding_mask, _deterministic())
+            else:
+                output = MSDeformAttnFusedFunction.apply(
+                    value.contiguous(), spatial_shapes, level_start_index, offsets.contiguous(),
+                    logits.contiguous(), reference_points.float().contiguous(), key_padding_mask)
             if output.dtype != io_dtype:
                 output = output.to(io_dtype)
             output = self.output_proj(output)
