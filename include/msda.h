@@ -324,6 +324,54 @@ int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void*
                               unsigned flags);
 
 /*
+ * Deformable convolution v1 / v2 (detectron2's DeformConv / ModulatedDeformConv, SURVEY.md section 2.1 row 12) as
+ * im2col + GEMM: these two entry points build the column matrix and scatter its gradient back; the products with the
+ * weight are dense GEMMs the caller runs (cuBLAS).  They replace detectron2/layers/csrc/deformable/
+ * deform_conv_cuda_kernel.cu:
+ *   msda_dcnv2_im2col   deformable_im2col (mask = NULL, DCNv1) and modulated_deformable_im2col_cuda (DCNv2)
+ *   msda_dcnv2_col2im   modulated_deformable_col2im_cuda (grad_input) + modulated_deformable_col2im_coord_cuda
+ *                       (grad_offset, grad_mask) in one pass; with mask = NULL the DCNv1 deformable_col2im +
+ *                       deformable_col2im_coord
+ * Layouts (contiguous; K = kernel_h*kernel_w, tap k = i*kernel_w + j; P = H_out*W_out):
+ *   input / grad_input       [N, H_in, W_in, C]                   dtype (channels last)
+ *   offset / grad_offset     [N, H_out, W_out, dg, K, 2]          (dy, dx) per tap, in pixels (detectron2's channel
+ *                                                                 order dg*K*2, channels last)
+ *   mask / grad_mask         [N, H_out, W_out, dg, K]             NULL for DCNv1 (grad_mask then unused)
+ *   columns / grad_columns   [N*P, groups, K, C/groups]           dtype; the (k, c) order of a row is that of
+ *                                                                 weight.permute(0, 2, 3, 1) [C_out, kh, kw, C/groups]
+ * dg = deformable_groups; channel c samples with the offsets of group c / (C/dg).  Sampling position of tap (i, j) at
+ * output (ho, wo): y = (ho*stride_h - pad_h + i*dilation_h) + dy, x likewise -- the integer base plus the offset, one
+ * rounding, as torchvision.ops.deform_conv2d -- bilinear, zero outside the map, a tap contributes only where
+ * y > -1 && y < H_in && x > -1 && x < W_in.  columns = mask * sample.  H_out / W_out must be what the geometry gives
+ * ((H_in + 2*pad_h - (dilation_h*(kernel_h-1) + 1)) / stride_h + 1), else MSDA_ERR_INVALID_ARGUMENT; C must be
+ * divisible by groups and by deformable_groups.
+ * dtype: MSDA_F32, MSDA_F64, MSDA_BF16, MSDA_F16 (offset / mask and their gradients float32, float64 for MSDA_F64) or
+ * MSDA_BF16_AUX16 / MSDA_F16_AUX16 (offset / mask and their gradients in the input's 16-bit type).  Fast kernels cover
+ * C/dg and C/groups multiples of 16 with float32 / bfloat16 / float16 input; every other shape, and float64, runs the
+ * generic kernels.  MSDA_FLAG_FORCE_GENERIC selects the generic kernels; every other flag bit is ignored, except that
+ * msda_dcnv2_col2im returns MSDA_ERR_UNSUPPORTED for MSDA_FLAG_DETERMINISTIC (grad_input is accumulated with float
+ * reds, whose rounding depends on arrival order; grad_offset / grad_mask are bit-reproducible in every case).
+ * col2im writes every element of grad_input, grad_offset and grad_mask.  Its workspace is
+ * msda_dcnv2_col2im_workspace_bytes: N*H_in*W_in*C floats for bfloat16 / float16 input (the float accumulator of
+ * grad_input), 0 otherwise (and 0 for an invalid geometry); less gives MSDA_ERR_WORKSPACE.  N = 0 or C = 0 are empty
+ * problems (col2im zero-fills grad_offset / grad_mask when C = 0).  Added in ABI 3 without a version bump: an older
+ * library lacks the three symbols.
+ */
+size_t msda_dcnv2_col2im_workspace_bytes(int batch, int channels, int height_in, int width_in, int height_out,
+                                         int width_out, int kernel_h, int kernel_w, int stride_h, int stride_w,
+                                         int pad_h, int pad_w, int dilation_h, int dilation_w, int groups,
+                                         int deformable_groups, int dtype, unsigned flags);
+int msda_dcnv2_im2col(void* stream, const void* input, const void* offset, const void* mask, int batch, int channels,
+                      int height_in, int width_in, int height_out, int width_out, int kernel_h, int kernel_w,
+                      int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w, int groups,
+                      int deformable_groups, void* columns, int dtype, unsigned flags);
+int msda_dcnv2_col2im(void* stream, const void* grad_columns, const void* input, const void* offset, const void* mask,
+                      int batch, int channels, int height_in, int width_in, int height_out, int width_out, int kernel_h,
+                      int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w,
+                      int groups, int deformable_groups, void* grad_input, void* grad_offset, void* grad_mask,
+                      void* workspace, size_t workspace_bytes, int dtype, unsigned flags);
+
+/*
  * Fused residual add + LayerNorm (SURVEY.md section 8f-2): the epilogue that follows every MSDeformAttn call and every
  * FFN in the reference's transformer layers -- x = x + identity; x = norm(x)
  * (/root/reference/detrex/layers/transformer.py:152-192; the residuals are added at multi_scale_deform_attn.py:363 and

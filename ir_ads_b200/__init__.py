@@ -1,6 +1,7 @@
 """B200-native multi-scale deformable attention -- drop-in for the MSDeformAttn hot path of
 yunduo-vision/IR-ADS (detrex.layers.MultiScaleDeformableAttention and the
-ms_deform_attn_forward / backward CUDA pair).  See DESIGN.md and include/msda.h.
+ms_deform_attn_forward / backward CUDA pair) -- plus DCNv3 and detectron2's deformable convolution
+(DeformConv / ModulatedDeformConv).  See DESIGN.md and include/msda.h.
 
 Importing the package does not load the CUDA library; the first op call does, and fails loudly
 if ir_ads_b200/libmsda_b200.so has not been built (no CPU / PyTorch fallback exists).
@@ -14,6 +15,7 @@ from .functional import (  # noqa: F401
     multi_scale_deformable_attn_pytorch,
     set_deterministic,
 )
+from .dcnv2 import DCNv2Function, DeformConv, ModulatedDeformConv, deform_conv, modulated_deform_conv  # noqa: F401
 from .dcnv3 import DCNv3FusedFunction, DCNv3Function, dcnv3_backward, dcnv3_forward  # noqa: F401
 from .module import MultiScaleDeformableAttention  # noqa: F401
 from .packing import PackedLevels, pack_levels, packed_reference_points, unpack_tokens, valid_extents  # noqa: F401
@@ -27,6 +29,11 @@ __all__ = [
     "multi_scale_deformable_attn_pytorch",
     "set_deterministic",
     "kernel_flags",
+    "DeformConv",
+    "ModulatedDeformConv",
+    "deform_conv",
+    "modulated_deform_conv",
+    "DCNv2Function",
     "DCNv3Function",
     "DCNv3FusedFunction",
     "dcnv3_forward",

@@ -89,6 +89,13 @@ def _declare(lib: ctypes.CDLL) -> None:
     lib.msda_add_layernorm_mixed_forward.argtypes = lib.msda_add_layernorm_forward.argtypes
     lib.msda_add_layernorm_mixed_backward.restype = i
     lib.msda_add_layernorm_mixed_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, i, vp, vp, vp, vp, vp, sz, i]
+    dcn2 = [i] * 16   # batch, channels, H_in, W_in, H_out, W_out, kernel, stride, pad, dilation (h, w), groups, dg
+    lib.msda_dcnv2_col2im_workspace_bytes.restype = sz
+    lib.msda_dcnv2_col2im_workspace_bytes.argtypes = dcn2 + [i, u]
+    lib.msda_dcnv2_im2col.restype = i
+    lib.msda_dcnv2_im2col.argtypes = [vp, vp, vp, vp] + dcn2 + [vp, i, u]
+    lib.msda_dcnv2_col2im.restype = i
+    lib.msda_dcnv2_col2im.argtypes = [vp, vp, vp, vp, vp] + dcn2 + [vp, vp, vp, vp, sz, i, u]
     lib.msda_debug_bookkeeping.restype = i
     lib.msda_debug_bookkeeping.argtypes = [vp, vp, vp, vp, i, i, i, i, i, i, i, vp, vp]
     lib.msda_debug_fastdiv.restype = u

@@ -1044,6 +1044,109 @@ int msda_dcnv3_fused_backward(void* stream, const void* grad_output, const void*
                       grad_mask_logits, workspace, workspace_bytes, need, dtype, 0u, true);
 }
 
+namespace {
+// Checks the deformable-convolution geometry and dtype tag (no device work) and fills `g`.
+int dcnv2_setup(int batch, int channels, int height_in, int width_in, int height_out, int width_out, int kernel_h,
+                int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w,
+                int groups, int deformable_groups, int dtype, Dcn2Dims* g) {
+  if (batch < 0 || channels < 0 || height_in < 1 || width_in < 1 || kernel_h < 1 || kernel_w < 1 || stride_h < 1 ||
+      stride_w < 1 || pad_h < 0 || pad_w < 0 || dilation_h < 1 || dilation_w < 1 || groups < 1 ||
+      deformable_groups < 1)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "dcnv2: bad geometry");
+  if (channels % groups != 0 || channels % deformable_groups != 0)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "dcnv2: channels (%d) must be divisible by groups (%d) and deformable_groups (%d)",
+                channels, groups, deformable_groups);
+  const int64_t ho = ((int64_t)height_in + 2 * pad_h - ((int64_t)dilation_h * (kernel_h - 1) + 1)) / stride_h + 1;
+  const int64_t wo = ((int64_t)width_in + 2 * pad_w - ((int64_t)dilation_w * (kernel_w - 1) + 1)) / stride_w + 1;
+  if (ho < 1 || wo < 1 || height_out != ho || width_out != wo)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "dcnv2: output %dx%d, the geometry gives %lldx%lld", height_out, width_out,
+                (long long)ho, (long long)wo);
+  if (dtype != MSDA_F32 && dtype != MSDA_F64 && dtype != MSDA_BF16 && dtype != MSDA_F16 && dtype != MSDA_BF16_AUX16 &&
+      dtype != MSDA_F16_AUX16)
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "unknown dtype tag %d", dtype);
+  if (ho * wo * deformable_groups * kernel_h * kernel_w >= ((int64_t)1 << 31) ||
+      (int64_t)height_in * width_in * channels >= ((int64_t)1 << 40))
+    return fail(MSDA_ERR_UNSUPPORTED, "dcnv2: image too large");
+  *g = Dcn2Dims{batch, channels, height_in, width_in, height_out, width_out, kernel_h, kernel_w, stride_h, stride_w,
+                pad_h, pad_w, dilation_h, dilation_w, groups, deformable_groups};
+  return MSDA_OK;
+}
+bool aux16(int dtype) { return dtype == MSDA_BF16_AUX16 || dtype == MSDA_F16_AUX16; }
+}  // namespace
+
+size_t msda_dcnv2_col2im_workspace_bytes(int batch, int channels, int height_in, int width_in, int height_out,
+                                         int width_out, int kernel_h, int kernel_w, int stride_h, int stride_w,
+                                         int pad_h, int pad_w, int dilation_h, int dilation_w, int groups,
+                                         int deformable_groups, int dtype, unsigned flags) {
+  (void)flags;
+  Dcn2Dims g;
+  if (dcnv2_setup(batch, channels, height_in, width_in, height_out, width_out, kernel_h, kernel_w, stride_h, stride_w,
+                  pad_h, pad_w, dilation_h, dilation_w, groups, deformable_groups, dtype, &g) != MSDA_OK)
+    return 0;
+  // bf16 / f16 grad_input is accumulated in float and converted at the end
+  return two_byte(fused_value_dtype(dtype)) ? (size_t)g.n_input() * sizeof(float) : 0;
+}
+
+int msda_dcnv2_im2col(void* stream, const void* input, const void* offset, const void* mask, int batch, int channels,
+                      int height_in, int width_in, int height_out, int width_out, int kernel_h, int kernel_w,
+                      int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w, int groups,
+                      int deformable_groups, void* columns, int dtype, unsigned flags) {
+  g_err[0] = 0;
+  Dcn2Dims g;
+  if (int s = dcnv2_setup(batch, channels, height_in, width_in, height_out, width_out, kernel_h, kernel_w, stride_h,
+                          stride_w, pad_h, pad_w, dilation_h, dilation_w, groups, deformable_groups, dtype, &g))
+    return s;
+  if (g.n_columns() == 0) return MSDA_OK;
+  if (!input || !offset || !columns) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  if (int s = check_alignment({{"input", input}, {"offset", offset}, {"mask", mask}, {"columns", columns}})) return s;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  DeviceGuard guard;
+  MSDA_CUDA(guard.enter(columns));
+  return dcnv2_im2col(st, g, fused_value_dtype(dtype), aux16(dtype), flags, input, offset, mask, columns);
+}
+
+int msda_dcnv2_col2im(void* stream, const void* grad_columns, const void* input, const void* offset, const void* mask,
+                      int batch, int channels, int height_in, int width_in, int height_out, int width_out, int kernel_h,
+                      int kernel_w, int stride_h, int stride_w, int pad_h, int pad_w, int dilation_h, int dilation_w,
+                      int groups, int deformable_groups, void* grad_input, void* grad_offset, void* grad_mask,
+                      void* workspace, size_t workspace_bytes, int dtype, unsigned flags) {
+  g_err[0] = 0;
+  Dcn2Dims g;
+  if (int s = dcnv2_setup(batch, channels, height_in, width_in, height_out, width_out, kernel_h, kernel_w, stride_h,
+                          stride_w, pad_h, pad_w, dilation_h, dilation_w, groups, deformable_groups, dtype, &g))
+    return s;
+  if (flags & MSDA_FLAG_DETERMINISTIC)
+    return fail(MSDA_ERR_UNSUPPORTED, "dcnv2 col2im: no deterministic form (grad_input uses float reds)");
+  if (g.n_points() == 0) return MSDA_OK;   // batch 0
+  const int vdt = fused_value_dtype(dtype);
+  const size_t aux = dtype == MSDA_F64 ? 8 : aux_size(dtype);
+  if (!grad_offset || (mask && !grad_mask)) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_offset / grad_mask is null");
+  if (g.n_input() != 0 && (!grad_columns || !input || !offset || !grad_input))
+    return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
+  if (int s = check_alignment({{"grad_columns", grad_columns}, {"input", input}, {"offset", offset}, {"mask", mask},
+                               {"grad_input", grad_input}, {"grad_offset", grad_offset},
+                               {"grad_mask", mask ? grad_mask : nullptr}, {"workspace", workspace}}))
+    return s;
+  const size_t need = two_byte(vdt) ? (size_t)g.n_input() * sizeof(float) : 0;
+  if (need && (!workspace || workspace_bytes < need))
+    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  DeviceGuard guard;
+  MSDA_CUDA(guard.enter(grad_offset));
+  if (g.n_input() == 0) {   // no channels: the output does not depend on the offsets or the mask
+    MSDA_CUDA(cudaMemsetAsync(grad_offset, 0, (size_t)g.n_points() * 2 * aux, st));
+    if (mask) MSDA_CUDA(cudaMemsetAsync(grad_mask, 0, (size_t)g.n_points() * aux, st));
+    return MSDA_OK;
+  }
+  void* acc = two_byte(vdt) ? workspace : grad_input;
+  MSDA_CUDA(cudaMemsetAsync(acc, 0, (size_t)g.n_input() * (vdt == MSDA_F64 ? 8 : 4), st));
+  if (int s = dcnv2_col2im(st, g, vdt, aux16(dtype), flags, grad_columns, input, offset, mask, acc, grad_offset,
+                           grad_mask))
+    return s;
+  if (two_byte(vdt)) return cast_from_f32(st, static_cast<const float*>(acc), grad_input, g.n_input(), vdt);
+  return MSDA_OK;
+}
+
 int msda_debug_bookkeeping(void* stream, const float* sampling_loc, const int64_t* spatial_shapes,
                            const int64_t* level_start_index, int batch, int spatial_size, int num_heads, int channels,
                            int num_levels, int num_query, int num_point, int64_t* corner_offsets, float* frac) {

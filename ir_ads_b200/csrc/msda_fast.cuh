@@ -551,15 +551,17 @@ struct PointRec {
   float lw, lh;  // fractional parts
 };
 
-// DCNv3 gives pixel coordinates directly (cuh:262-263 gate, :48-58 cell), no exact-product trick needed.
-__device__ __forceinline__ Cell<float> locate_pixel(float px, float py, int H, int W) {
-  Cell<float> c;
-  const bool ok = (py > -1.0f) && (px > -1.0f) && (py < (float)H) && (px < (float)W);
-  const float fy = floorf(py), fx = floorf(px);
+// DCNv3 gives pixel coordinates directly (cuh:262-263 gate, :48-58 cell), no exact-product trick needed.  DCNv2
+// (msda_dcnv2.cu) has the same gate and cell, in float or -- its generic kernels -- double.
+template <typename T>
+__device__ __forceinline__ Cell<T> locate_pixel(T px, T py, int H, int W) {
+  Cell<T> c;
+  const bool ok = (py > (T)-1) && (px > (T)-1) && (py < (T)H) && (px < (T)W);
+  const T fy = floor(py), fx = floor(px);
   c.y0 = ok ? (int)fy : 0;
   c.x0 = ok ? (int)fx : 0;
-  c.lh = ok ? py - fy : 0.0f;
-  c.lw = ok ? px - fx : 0.0f;
+  c.lh = ok ? py - fy : (T)0;
+  c.lw = ok ? px - fx : (T)0;
   unsigned v = 0;
   if (ok) {
     const bool y0ok = c.y0 >= 0, y1ok = c.y0 + 1 <= H - 1, x0ok = c.x0 >= 0, x1ok = c.x0 + 1 <= W - 1;

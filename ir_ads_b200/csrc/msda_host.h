@@ -7,6 +7,7 @@
 //   msda_bwd.cu      fast backward kernels, float reds (plain operator, all row orders)
 //   msda_bwd_aux.cu  fast backward kernels: fixed-point reds, no-scatter, fused module chain, DCNv3
 //   msda_fold.cu     encoder-form backward with on-SM folding of grad_value (msda_fold.cuh)
+//   msda_dcnv2.cu    deformable convolution im2col / col2im (fast + generic)
 #pragma once
 #include "../../include/msda.h"
 
@@ -117,6 +118,27 @@ int bwd_dcn_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, cons
 int bwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
                const int64_t* meta, const void* off, const void* logits, float* gv, void* goff, void* glog,
                msda::FusedArgs fa);
+
+// ---- msda_dcnv2.cu ----
+// Deformable convolution geometry (msda_dcnv2_im2col / _col2im): input [B,H,W,C], output [B,Ho,Wo,*].  A point is
+// (image, output pixel, deformable group, kernel tap); p = ((pixel*dg + d)*K + k) inside one image.
+struct Dcn2Dims {
+  int B, C, H, W, Ho, Wo, kh, kw, sh, sw, ph, pw, dh, dw, groups, dg;
+  __host__ __device__ int K() const { return kh * kw; }
+  __host__ __device__ int Cg() const { return C / groups; }
+  __host__ __device__ int Cdg() const { return C / dg; }
+  __host__ __device__ int points_per_image() const { return Ho * Wo * dg * kh * kw; }
+  int64_t n_points() const { return (int64_t)B * points_per_image(); }
+  int64_t n_input() const { return (int64_t)B * H * W * C; }
+  int64_t n_columns() const { return (int64_t)B * Ho * Wo * K() * C; }
+};
+// value dtype MSDA_F32 / F64 / BF16 / F16, aux16: offset / mask and their gradients in the value's 16-bit type.
+// grad_input_acc: float [B,H,W,C] (double for MSDA_F64), zeroed by the caller; the kernels add into it.
+int dcnv2_im2col(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsigned flags, const void* input,
+                 const void* offset, const void* mask, void* columns);
+int dcnv2_col2im(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsigned flags, const void* grad_columns,
+                 const void* input, const void* offset, const void* mask, void* grad_input_acc, void* grad_offset,
+                 void* grad_mask);
 
 // ---- msda_fold.cu ----
 // does the folding backward cover this problem (encoder form Q == S, shapes it is instantiated for, flags)?

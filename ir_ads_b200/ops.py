@@ -9,8 +9,10 @@ formula:
   ir_ads_b200::msda_packed / msda_packed_backward    MSDeformAttnPackedFunction
   ir_ads_b200::add_layer_norm / _backward            AddLayerNormFunction and AddLayerNormMixedFunction
   ir_ads_b200::dcnv3_fused / dcnv3_fused_backward    DCNv3FusedFunction
+  ir_ads_b200::dcnv2 / dcnv2_backward                DCNv2Function (deform_conv, modulated_deform_conv)
 
-``MultiScaleDeformableAttention``, ``epilogue.add_layer_norm`` and the ``DCNv3`` module call them only while
+``MultiScaleDeformableAttention``, ``epilogue.add_layer_norm``, the ``DCNv3`` module and the deformable convolutions
+(dcnv2.py) call them only while
 ``torch.compiler.is_compiling()``; eager code keeps calling the Functions.
 
 Choices the backward makes are op arguments, fixed when the graph is built: ``deterministic`` (read from
@@ -26,6 +28,7 @@ from typing import Optional, Tuple
 import torch
 
 from . import _lib
+from . import dcnv2 as _dcnv2
 from . import dcnv3 as _dcnv3
 from . import epilogue as _epilogue
 from . import functional as _functional
@@ -287,3 +290,68 @@ def _dcnv3_fused_grad(ctx, grad_output):
 
 
 dcnv3_fused.register_autograd(_dcnv3_fused_grad, setup_context=_dcnv3_fused_setup)
+
+
+# ------------------------------------------------------------------------------------------------
+# dcnv2: DCNv2Function (deform_conv with mask None and bias None, modulated_deform_conv)
+# ------------------------------------------------------------------------------------------------
+def _empty_in_format_of(shape, like: torch.Tensor, dtype=None) -> torch.Tensor:
+    """What dcnv2.py returns for a tensor shaped like ``like``: channels_last when ``like`` is, else contiguous."""
+    fmt = torch.channels_last if _dcnv2._channels_last(like) else torch.contiguous_format
+    return torch.empty(shape, dtype=dtype or like.dtype, device=like.device, memory_format=fmt)
+
+
+@torch.library.custom_op("ir_ads_b200::dcnv2", mutates_args=())
+def dcnv2(input: torch.Tensor, offset: torch.Tensor, mask: Optional[torch.Tensor], weight: torch.Tensor,
+          bias: Optional[torch.Tensor], stride_h: int, stride_w: int, pad_h: int, pad_w: int, dilation_h: int,
+          dilation_w: int, groups: int, deformable_groups: int, im2col_step: int) -> torch.Tensor:
+    """DCNv2Function's forward: ``[B, C_out, H_out, W_out]`` in input's dtype and memory format."""
+    g = _dcnv2._Geom(input, weight, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, groups,
+                     deformable_groups, im2col_step)
+    return _dcnv2._forward(input, offset, mask, weight, bias, g)
+
+
+@dcnv2.register_fake
+def _(input, offset, mask, weight, bias, *ints):
+    g = _dcnv2._Geom(input, weight, *ints)
+    return _empty_in_format_of((g.B, g.C_out, g.Ho, g.Wo), input)
+
+
+@torch.library.custom_op(
+    "ir_ads_b200::dcnv2_backward", mutates_args=(),
+    schema="(Tensor grad_output, Tensor input, Tensor offset, Tensor? mask, Tensor weight, Tensor? bias, "
+           "SymInt stride_h, SymInt stride_w, SymInt pad_h, SymInt pad_w, SymInt dilation_h, SymInt dilation_w, "
+           "SymInt groups, SymInt deformable_groups, SymInt im2col_step, bool need_input, bool need_offset, "
+           "bool need_mask, bool need_weight, bool need_bias) -> (Tensor?, Tensor?, Tensor?, Tensor?, Tensor?)")
+def dcnv2_backward(grad_output, input, offset, mask, weight, bias, stride_h, stride_w, pad_h, pad_w, dilation_h,
+                   dilation_w, groups, deformable_groups, im2col_step, need_input, need_offset, need_mask,
+                   need_weight, need_bias):
+    """``(grad_input, grad_offset, grad_mask, grad_weight, grad_bias)``, None where not needed (or no mask / bias)."""
+    g = _dcnv2._Geom(input, weight, stride_h, stride_w, pad_h, pad_w, dilation_h, dilation_w, groups,
+                     deformable_groups, im2col_step)
+    return _dcnv2._backward(grad_output, input, offset, mask, weight, bias, g,
+                            (need_input, need_offset, need_mask, need_weight, need_bias))
+
+
+@dcnv2_backward.register_fake
+def _(grad_output, input, offset, mask, weight, bias, *rest):
+    need_input, need_offset, need_mask, need_weight, need_bias = rest[9:]
+    return (_empty_in_format_of(input.shape, input) if need_input else None,
+            _empty_in_format_of(offset.shape, offset) if need_offset else None,
+            _empty_in_format_of(mask.shape, mask) if (mask is not None and need_mask) else None,
+            torch.empty_like(weight, memory_format=torch.contiguous_format) if need_weight else None,
+            torch.empty_like(bias) if (bias is not None and need_bias) else None)
+
+
+def _dcnv2_setup(ctx, inputs, output):
+    ctx.save_for_backward(*inputs[:5])
+    ctx.ints = inputs[5:14]
+
+
+def _dcnv2_grad(ctx, grad_output):
+    need = ctx.needs_input_grad
+    grads = dcnv2_backward(grad_output, *ctx.saved_tensors, *ctx.ints, *need[:5])
+    return tuple(grads) + (None,) * 9
+
+
+dcnv2.register_autograd(_dcnv2_grad, setup_context=_dcnv2_setup)
