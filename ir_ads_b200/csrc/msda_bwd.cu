@@ -8,16 +8,11 @@ int bwd_fast(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const vo
   // default row order of the backward: STRIP (measured 3 % faster than LINEAR at cfg 2: fewer L1 misses
   // on the crossbar-bound kernel); the forward keeps LINEAR
   if (!(flags & (MSDA_FLAG_ORDER_LINEAR | MSDA_FLAG_ORDER_TILE2D))) flags |= MSDA_FLAG_ORDER_STRIP;
-#ifdef MSDA_ALL_ORDERS
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_ANY
-#else
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_STRIP
-#endif
-#define CALL_BWD(D_, VT_, PT_, ORD_) \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw, nullptr)
-  MSDA_DISPATCH_VT(CALL_BWD);
-#undef CALL_BWD
-#undef MSDA_DISPATCH_ORDER
+  return dispatch_fast<FastTags, PlainOrders<kStrip>>(d, dtype, flags, [&](auto t, auto D, auto PT, auto order) {
+    using VT = typename decltype(t)::VT;
+    return launch_bwd_fast<D, VT, PT, kBwdThreads, order, float>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw,
+                                                                  nullptr);
+  });
 }
 
 }  // namespace msda_host

@@ -4,47 +4,48 @@
 
 namespace msda_host {
 
-// deterministic accumulate: LINEAR order
+namespace {
+// The per-warp slots of EmitArgs::warp_amax of the entry-filing backward (LINEAR order: one CTA per kBwdThreads /
+// (D / 4) rows, kBwdThreads / 32 warps each) go to *n_warps.
+msda::EmitArgs emit_args(const Dims& d, int* cursor, const int* bin_start, void* entries, float* warp_amax,
+                         int64_t* n_warps) {
+  const int64_t rpc = kBwdThreads / (d.D / 4);
+  if (n_warps) *n_warps = ((d.rows() + rpc - 1) / rpc) * (kBwdThreads / 32);
+  return msda::EmitArgs{cursor, bin_start, static_cast<int4*>(entries), warp_amax};
+}
+
+// The plain operator's backward without float reds, LINEAR order.  ACC: unsigned long long (64-bit fixed-point reds
+// into acc), NoScatter (scatter compiled out: grad_loc / grad_w only) or EmitEntries (no scatter; files every in-range
+// point under its bilinear cell for the deterministic sorted path, replacing det_bin_kernel<true> + the no-scatter
+// backward).
+template <typename ACC>
+int bwd_fast_acc(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
+                 const int64_t* lsi, const void* loc, const void* w, ACC* acc, void* gl, void* gw,
+                 const msda::DetScale* det, msda::EmitArgs ea = msda::EmitArgs{}) {
+  return dispatch_fast<FastTags, OrderList<kLinear>>(d, dtype, 0, [&](auto t, auto D, auto PT, auto order) {
+    using VT = typename decltype(t)::VT;
+    return launch_bwd_fast<D, VT, PT, kBwdThreads, order, ACC>(st, d, go, value, shapes, lsi, loc, w, acc, gl, gw, det,
+                                                               msda::FusedArgs{}, ea);
+  });
+}
+}  // namespace
+
 int bwd_fast_det(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
                  const int64_t* lsi, const void* loc, const void* w, unsigned long long* acc, void* gl, void* gw,
                  const msda::DetScale* det) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
-#define CALL_BWD(D_, VT_, PT_, ORD_) \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, unsigned long long>(st, d, go, value, shapes, lsi, loc, w, acc, gl, gw, det)
-  MSDA_DISPATCH_VT(CALL_BWD);
-#undef CALL_BWD
-#undef MSDA_DISPATCH_ORDER
+  return bwd_fast_acc(st, d, dtype, go, value, shapes, lsi, loc, w, acc, gl, gw, det);
 }
 
-// backward without the scatter (grad_loc / grad_w only), LINEAR order
 int bwd_fast_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value,
                        const int64_t* shapes, const int64_t* lsi, const void* loc, const void* w, void* gl, void* gw) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
-#define CALL_BWD(D_, VT_, PT_, ORD_)                                                                          \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, msda::NoScatter>(st, d, go, value, shapes, lsi, loc, w,   \
-                                                                    (msda::NoScatter*)nullptr, gl, gw, nullptr)
-  MSDA_DISPATCH_VT(CALL_BWD);
-#undef CALL_BWD
-#undef MSDA_DISPATCH_ORDER
+  return bwd_fast_acc<msda::NoScatter>(st, d, dtype, go, value, shapes, lsi, loc, w, nullptr, gl, gw, nullptr);
 }
 
-// backward without the scatter that also files every in-range point under its bilinear cell (deterministic sorted
-// path: replaces det_bin_kernel<true> + the plain no-scatter backward), LINEAR order
 int bwd_fast_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
                   const int64_t* lsi, const void* loc, const void* w, void* gl, void* gw, int* cursor,
                   const int* bin_start, void* entries, float* warp_amax, int64_t* n_warps) {
-  // one CTA per kBwdThreads / (D / 4) rows (LINEAR order), kBwdThreads / 32 warps each: the slots of EmitArgs::warp_amax
-  const int64_t rpc = kBwdThreads / (d.D / 4);
-  if (n_warps) *n_warps = ((d.rows() + rpc - 1) / rpc) * (kBwdThreads / 32);
-  msda::EmitArgs ea{cursor, bin_start, static_cast<int4*>(entries), warp_amax};
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
-#define CALL_BWD(D_, VT_, PT_, ORD_)                                                                            \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, msda::EmitEntries>(st, d, go, value, shapes, lsi, loc, w,   \
-                                                                      (msda::EmitEntries*)nullptr, gl, gw, nullptr, \
-                                                                      msda::FusedArgs{}, ea)
-  MSDA_DISPATCH_VT(CALL_BWD);
-#undef CALL_BWD
-#undef MSDA_DISPATCH_ORDER
+  const msda::EmitArgs ea = emit_args(d, cursor, bin_start, entries, warp_amax, n_warps);
+  return bwd_fast_acc<msda::EmitEntries>(st, d, dtype, go, value, shapes, lsi, loc, w, nullptr, gl, gw, nullptr, ea);
 }
 
 #ifdef MSDA_EXP_SLIM
@@ -81,147 +82,95 @@ int bwd_dcn_emit(cudaStream_t, const Dims&, int, const void*, const void*, const
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv3 kernels");
 }
 #else
-// fused pre-op chain: STRIP order.  dtype MSDA_*_AUX16: offsets / logits and their gradients in the value's 16-bit
-// type
+// fused pre-op chain, STRIP order.  PRE kPreFused (lsi: level start index) or kPrePacked (lsi: the per-image metadata
+// rows).  ACC float (float reds into gv) or NoScatter (gradients of the raw offsets / logits only).  dtype
+// MSDA_*_AUX16 (Tags = FusedTags): offsets / logits and their gradients in the value's 16-bit type
+template <int PRE, typename Tags, typename ACC>
+int bwd_fused_pre(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
+                  const int64_t* lsi, const void* off, const void* logits, ACC* gv, void* goff, void* glog,
+                  msda::FusedArgs fa) {
+  return dispatch_fast<Tags, OrderList<kStrip>>(d, dtype, 0, [&](auto t, auto D, auto PT, auto order) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
+    return launch_bwd_fast<D, VT, PT, kBwdThreads, order, ACC, PRE, AT>(st, d, go, value, shapes, lsi, off, logits, gv,
+                                                                        goff, glog, nullptr, fa);
+  });
+}
+
 int bwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
               const int64_t* lsi, const void* off, const void* logits, float* gv, void* goff, void* glog,
               msda::FusedArgs fa) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_STRIP
-#define CALL_FB(D_, VT_, PT_, ORD_)                                                                               \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPreFused>(st, d, go, value, shapes, lsi, off, logits, gv, \
-                                                                           goff, glog, nullptr, fa)
-#define CALL_FB16(D_, VT_, PT_, ORD_)                                                                          \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPreFused, VT_>(st, d, go, value, shapes, lsi, off, \
-                                                                                logits, gv, goff, glog, nullptr, fa)
-  MSDA_DISPATCH_VT_AUX16(CALL_FB16);
-  MSDA_DISPATCH_VT(CALL_FB);
-#undef CALL_FB16
-#undef CALL_FB
-#undef MSDA_DISPATCH_ORDER
+  return bwd_fused_pre<msda::kPreFused, FusedTags>(st, d, dtype, go, value, shapes, lsi, off, logits, gv, goff, glog,
+                                                   fa);
 }
 
-// fused chain over a packed batch: STRIP order, float reds, the same value / aux types as bwd_fused
 int bwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value, const int64_t* shapes,
                const int64_t* meta, const void* off, const void* logits, float* gv, void* goff, void* glog,
                msda::FusedArgs fa) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_STRIP
-#define CALL_PB(D_, VT_, PT_, ORD_)                                                                                  \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPrePacked>(st, d, go, value, shapes, meta, off,      \
-                                                                            logits, gv, goff, glog, nullptr, fa)
-#define CALL_PB16(D_, VT_, PT_, ORD_)                                                                             \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, float, msda::kPrePacked, VT_>(st, d, go, value, shapes, meta, off, \
-                                                                                 logits, gv, goff, glog, nullptr, fa)
-  MSDA_DISPATCH_VT_AUX16(CALL_PB16);
-  MSDA_DISPATCH_VT(CALL_PB);
-#undef CALL_PB16
-#undef CALL_PB
-#undef MSDA_DISPATCH_ORDER
+  return bwd_fused_pre<msda::kPrePacked, FusedTags>(st, d, dtype, go, value, shapes, meta, off, logits, gv, goff, glog,
+                                                    fa);
 }
 
-// fused chain, scatter compiled out: gradients of the raw offsets / logits only (deterministic fused backward)
 int bwd_fused_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* value,
                         const int64_t* shapes, const int64_t* lsi, const void* off, const void* logits, void* goff,
                         void* glog, msda::FusedArgs fa) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_STRIP
-#define CALL_FB(D_, VT_, PT_, ORD_)                                                                              \
-  launch_bwd_fast<D_, VT_, PT_, kBwdThreads, ORD_, msda::NoScatter, msda::kPreFused>(                            \
-      st, d, go, value, shapes, lsi, off, logits, (msda::NoScatter*)nullptr, goff, glog, nullptr, fa)
-  MSDA_DISPATCH_VT(CALL_FB);
-#undef CALL_FB
-#undef MSDA_DISPATCH_ORDER
+  return bwd_fused_pre<msda::kPreFused, FastTags, msda::NoScatter>(st, d, dtype, go, value, shapes, lsi, off, logits,
+                                                                   nullptr, goff, glog, fa);
 }
 
-// DCNv3: runtime point count, STRIP order.  PRE: kPreDcn (w = mask, gw = its gradient) or kPreDcnSoftmax (w = mask
-// logits, gw = the logits' gradient; dtype MSDA_*_AUX16: offset / logits and their gradients in the input's 16-bit
-// type)
-template <int PRE>
+// DCNv3: runtime point count.  PRE kPreDcn (w = mask, gw = its gradient) or kPreDcnSoftmax (w = mask logits, gw = the
+// logits' gradient; dtype MSDA_*_AUX16: offset / logits and their gradients in the input's 16-bit type).  ACC: float
+// reds, or the deterministic kinds of bwd_fast_acc (kPreDcn only).  STRIP order, except EmitEntries: LINEAR, so that
+// the per-warp maxima have exactly the slots emit_args counts for the equivalent one-level problem.
+template <int PRE, typename ACC>
 int bwd_dcn_pre(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
-                const void* w, float* gi, void* goff, void* gw, msda::FusedArgs fa) {
-#define CALL_DB(D_, VT_, AT_)                                                                                          \
-  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, float, PRE, AT_>(st, d, go, input, nullptr, nullptr, off, w, gi, goff, gw, \
-                                                               nullptr, fa)
-#define DCN_D(VT_, AT_)                                                                    \
-  switch (d.D) {                                                                           \
-    case 16: return CALL_DB(16, VT_, AT_);                                                 \
-    case 32: return CALL_DB(32, VT_, AT_);                                                 \
-    case 64: return CALL_DB(64, VT_, AT_);                                                 \
-    case 128: return CALL_DB(128, VT_, AT_);                                               \
-    default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);           \
-  }
-  if constexpr (PRE == msda::kPreDcnSoftmax) {
-    if (dtype == MSDA_BF16_AUX16) DCN_D(__nv_bfloat16, __nv_bfloat16)
-    if (dtype == MSDA_F16_AUX16) DCN_D(__half, __half)
-  }
-  if (dtype == MSDA_F32) DCN_D(float, float)
-  if (dtype == MSDA_BF16) DCN_D(__nv_bfloat16, float)
-  if (dtype == MSDA_F16) DCN_D(__half, float)
-  return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
-#undef DCN_D
-#undef CALL_DB
+                const void* w, ACC* gi, void* goff, void* gw, const msda::DetScale* det, msda::FusedArgs fa,
+                msda::EmitArgs ea = msda::EmitArgs{}) {
+  using Tags = std::conditional_t<PRE == msda::kPreDcnSoftmax, FusedTags, FastTags>;
+  constexpr int ORDER = std::is_same_v<ACC, msda::EmitEntries> ? kLinear : kStrip;
+  return with_types<Tags>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
+    return with_chunk(d.D, [&](auto D) {
+      return launch_bwd_fast<D, VT, 0, kBwdThreads, ORDER, ACC, PRE, AT>(st, d, go, input, nullptr, nullptr, off, w, gi,
+                                                                         goff, gw, det, fa, ea);
+    });
+  });
 }
 
 int bwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
             const void* mask, float* gi, void* goff, void* gmask, msda::FusedArgs fa) {
-  return bwd_dcn_pre<msda::kPreDcn>(st, d, dtype, go, input, off, mask, gi, goff, gmask, fa);
+  return bwd_dcn_pre<msda::kPreDcn>(st, d, dtype, go, input, off, mask, gi, goff, gmask, nullptr, fa);
 }
 
 // fused DCNv3 module path: the softmax's chain rule runs in the kernel, which writes the mask logits' gradient
 int bwd_dcn_softmax(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                     const void* mask_logits, float* gi, void* goff, void* glogits, msda::FusedArgs fa) {
-  return bwd_dcn_pre<msda::kPreDcnSoftmax>(st, d, dtype, go, input, off, mask_logits, gi, goff, glogits, fa);
+  return bwd_dcn_pre<msda::kPreDcnSoftmax>(st, d, dtype, go, input, off, mask_logits, gi, goff, glogits, nullptr, fa);
 }
 
-// the DCNv3 twins of the deterministic backward kernels above, dispatched over group_channels and dtype
-#define MSDA_DCN_DISPATCH(CALL)                                                              \
-  do {                                                                                       \
-    if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16)                        \
-      return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);                           \
-    switch (d.D) {                                                                           \
-      case 16: return dtype == MSDA_F32 ? CALL(16, float) : dtype == MSDA_BF16 ? CALL(16, __nv_bfloat16) : CALL(16, __half); \
-      case 32: return dtype == MSDA_F32 ? CALL(32, float) : dtype == MSDA_BF16 ? CALL(32, __nv_bfloat16) : CALL(32, __half); \
-      case 64: return dtype == MSDA_F32 ? CALL(64, float) : dtype == MSDA_BF16 ? CALL(64, __nv_bfloat16) : CALL(64, __half); \
-      case 128: return dtype == MSDA_F32 ? CALL(128, float) : dtype == MSDA_BF16 ? CALL(128, __nv_bfloat16) : CALL(128, __half); \
-      default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);         \
-    }                                                                                        \
-  } while (0)
-
-// DCNv3, 64-bit fixed-point reds (MSDA_FLAG_DET_ATOMIC, or problems beyond the sorted path's 32-bit indices): STRIP
-// order, as the float-red twin
+// 64-bit fixed-point reds: MSDA_FLAG_DET_ATOMIC, or problems beyond the sorted path's 32-bit indices
 int bwd_dcn_det(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                 const void* mask, unsigned long long* acc, void* goff, void* gmask, const msda::DetScale* det,
                 msda::FusedArgs fa) {
-#define CALL_DB(D_, VT_)                                                                                         \
-  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, unsigned long long, msda::kPreDcn>(st, d, go, input, nullptr, nullptr, \
-                                                                                 off, mask, acc, goff, gmask, det, fa)
-  MSDA_DCN_DISPATCH(CALL_DB);
-#undef CALL_DB
+  return bwd_dcn_pre<msda::kPreDcn>(st, d, dtype, go, input, off, mask, acc, goff, gmask, det, fa);
 }
 
-// DCNv3 without the scatter (grad_offset / grad_mask only): the sorted path with MSDA_FLAG_DET_SEPARATE_FILL
+// without the scatter (grad_offset / grad_mask only): the sorted path with MSDA_FLAG_DET_SEPARATE_FILL
 int bwd_dcn_noscatter(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                       const void* mask, void* goff, void* gmask, msda::FusedArgs fa) {
-#define CALL_DB(D_, VT_)                                                                                           \
-  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 2, msda::NoScatter, msda::kPreDcn>(                                     \
-      st, d, go, input, nullptr, nullptr, off, mask, (msda::NoScatter*)nullptr, goff, gmask, nullptr, fa)
-  MSDA_DCN_DISPATCH(CALL_DB);
-#undef CALL_DB
+  return bwd_dcn_pre<msda::kPreDcn, msda::NoScatter>(st, d, dtype, go, input, off, mask, nullptr, goff, gmask, nullptr,
+                                                     fa);
 }
 
-// DCNv3 backward that files every in-range point under its bilinear cell (sorted path).  LINEAR order, so that the
-// per-warp maxima have exactly the slots bwd_fast_emit counts for the equivalent one-level problem.
+// files every in-range point under its bilinear cell (sorted path)
 int bwd_dcn_emit(cudaStream_t st, const Dims& d, int dtype, const void* go, const void* input, const void* off,
                  const void* mask, void* goff, void* gmask, int* cursor, const int* bin_start, void* entries,
                  float* warp_amax, int64_t* n_warps, msda::FusedArgs fa) {
-  const int64_t rpc = kBwdThreads / (d.D / 4);
-  if (n_warps) *n_warps = ((d.rows() + rpc - 1) / rpc) * (kBwdThreads / 32);
-  msda::EmitArgs ea{cursor, bin_start, static_cast<int4*>(entries), warp_amax};
-#define CALL_DB(D_, VT_)                                                                                           \
-  launch_bwd_fast<D_, VT_, 0, kBwdThreads, 0, msda::EmitEntries, msda::kPreDcn>(                                   \
-      st, d, go, input, nullptr, nullptr, off, mask, (msda::EmitEntries*)nullptr, goff, gmask, nullptr, fa, ea)
-  MSDA_DCN_DISPATCH(CALL_DB);
-#undef CALL_DB
+  const msda::EmitArgs ea = emit_args(d, cursor, bin_start, entries, warp_amax, n_warps);
+  return bwd_dcn_pre<msda::kPreDcn, msda::EmitEntries>(st, d, dtype, go, input, off, mask, nullptr, goff, gmask,
+                                                       nullptr, fa, ea);
 }
-#undef MSDA_DCN_DISPATCH
 #endif
 
 }  // namespace msda_host

@@ -46,6 +46,12 @@ int check_alignment(std::initializer_list<NamedPtr> ptrs) {
   return MSDA_OK;
 }
 
+int check_workspace(const void* workspace, size_t workspace_bytes, size_t need) {
+  if (need && (!workspace || workspace_bytes < need))
+    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  return MSDA_OK;
+}
+
 bool fast_ok(const Dims& d, int dtype, unsigned flags) {
   if (flags & MSDA_FLAG_FORCE_GENERIC) return false;
   if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16) return false;
@@ -127,23 +133,12 @@ template <typename VT>
 int det_gather(cudaStream_t st, const Dims& d, const void* go, const int4* entries, const int* bin_start,
                const int64_t* shapes, const int64_t* lsi, const msda::DetScale* scale, void* gv) {
   const int64_t items = (int64_t)d.B * d.S * d.H;
-#define CALL_G(D_)                                                                                            \
-  do {                                                                                                        \
-    constexpr int RPC = 256 / (D_ / 4);                                                                       \
-    msda::det_gather_kernel<D_, VT><<<(unsigned)((items + RPC - 1) / RPC), 256, 0, st>>>(                     \
-        (const VT*)go, entries, bin_start, shapes, lsi, scale, (VT*)gv, d.B, d.S, d.H, d.L);                  \
-  } while (0)
-  switch (d.D) {
-    case 16: CALL_G(16); break;
-    case 32: CALL_G(32); break;
-    case 64: CALL_G(64); break;
-    case 128: CALL_G(128); break;
-    default: return fail(MSDA_ERR_UNSUPPORTED, "det gather: D=%d", d.D);
-  }
-#undef CALL_G
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return with_chunk(d.D, [&](auto D) {
+    constexpr int RPC = 256 / (D / 4);
+    msda::det_gather_kernel<D, VT><<<(unsigned)((items + RPC - 1) / RPC), 256, 0, st>>>(
+        (const VT*)go, entries, bin_start, shapes, lsi, scale, (VT*)gv, d.B, d.S, d.H, d.L);
+    return launched();
+  });
 }
 
 // dense problems reduce per cell (one pass over the entries), sparse ones gather per pixel (msda_det.cuh)
@@ -154,23 +149,20 @@ int det_cell_reduce(cudaStream_t st, const Dims& d, const void* go, const int4* 
                     int64_t n_bins, const int64_t* shapes, const int64_t* lsi, const msda::DetScale* scale,
                     unsigned long long* acc) {
   const int64_t slices = (d.n_points() + msda::kDetSlice - 1) / msda::kDetSlice;   // upper bound: gated points have no entry
-#define CALL_G(D_)                                                                                            \
-  do {                                                                                                        \
-    constexpr int GPC = 256 / (D_ / 4);                                                                       \
-    msda::det_cell_reduce_kernel<D_, VT><<<(unsigned)((slices + GPC - 1) / GPC), 256, 0, st>>>(               \
-        (const VT*)go, entries, bin_start, (int)n_bins, shapes, lsi, scale, acc, d.S, d.H, d.L);              \
-  } while (0)
-  switch (d.D) {
-    case 16: CALL_G(16); break;
-    case 32: CALL_G(32); break;
-    case 64: CALL_G(64); break;
-    case 128: CALL_G(128); break;
-    default: return fail(MSDA_ERR_UNSUPPORTED, "det cell reduce: D=%d", d.D);
-  }
-#undef CALL_G
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return with_chunk(d.D, [&](auto D) {
+    constexpr int GPC = 256 / (D / 4);
+    msda::det_cell_reduce_kernel<D, VT><<<(unsigned)((slices + GPC - 1) / GPC), 256, 0, st>>>(
+        (const VT*)go, entries, bin_start, (int)n_bins, shapes, lsi, scale, acc, d.S, d.H, d.L);
+    return launched();
+  });
+}
+
+// 64-bit fixed-point accumulators -> grad_value
+template <typename VT>
+int det_finalize(cudaStream_t st, const unsigned long long* acc, void* gv, int64_t nv, const msda::DetScale* scale) {
+  msda::msda_det_finalize_kernel<VT><<<grid_for(nv, 256, 148 * 16), 256, 0, st>>>(
+      reinterpret_cast<const long long*>(acc), (VT*)gv, nv, scale);
+  return launched();
 }
 
 // Workspace of the sorted deterministic path (all 16-byte aligned):
@@ -217,9 +209,7 @@ int fwd_generic(cudaStream_t st, const Dims& d, const void* value, const int64_t
   msda::msda_fwd_generic_kernel<VT, CT><<<grid, 256, 0, st>>>((const VT*)value, shapes, lsi, (const CT*)loc,
                                                               (const CT*)w, (VT*)out, d.S, d.H, d.D, d.L, d.Q, d.P,
                                                               total);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
 template <typename VT, typename CT, typename ACC>
@@ -233,9 +223,7 @@ int bwd_generic(cudaStream_t st, const Dims& d, const void* go, const void* valu
   msda::msda_bwd_generic_kernel<VT, CT, ACC><<<grid, threads, 0, st>>>(
       (const VT*)go, (const VT*)value, shapes, lsi, (const CT*)loc, (const CT*)w, gv, (CT*)gl, (CT*)gw, det, d.S, d.H,
       d.D, d.L, d.Q, d.P, rows);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
 // bf16 / f16 values: 2-byte elements, grad_value accumulated in a float workspace and converted at the end
@@ -255,9 +243,18 @@ int cast_from_f32(cudaStream_t st, const float* src, void* dst, int64_t n, int d
   const int grid = grid_for(n, 256, 148 * 16);
   if (dtype == MSDA_BF16) msda::msda_cast_f32_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(src, (__nv_bfloat16*)dst, n);
   else msda::msda_cast_f32_kernel<__half><<<grid, 256, 0, st>>>(src, (__half*)dst, n);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
+}
+
+// The FusedArgs of the MSDeformAttn module path: reference points, the 1/P offset normalisation, the value padding mask
+msda::FusedArgs module_args(const float* reference_points, int ref_dim, int num_point, const uint8_t* value_mask) {
+  msda::FusedArgs fa{};
+  fa.ref = reference_points;
+  fa.ref_dim = ref_dim;
+  fa.inv_P = 1.0f / (float)num_point;
+  fa.num_P = (float)num_point;
+  fa.value_mask = value_mask;
+  return fa;
 }
 
 // Where the points of the deterministic backward come from: the plain operator's sampling_loc / attn_weight, or the
@@ -278,7 +275,6 @@ struct DetSource {
 int det_backward(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const void* grad_output, const void* value,
                  const DetSource& src, void* grad_value, void* grad_sampling_loc, void* grad_attn_weight,
                  void* workspace, size_t need) {
-  auto count = [] { count_launch(); };
   const void* sampling_loc = src.loc;
   const void* attn_weight = src.w;
   const int64_t* spatial_shapes = src.shapes;
@@ -306,17 +302,17 @@ int det_backward(cudaStream_t st, const Dims& d, int dtype, unsigned flags, cons
   const bool amax_in_emit = MSDA_DET_AMAX_IN_EMIT && sorted && !(flags & MSDA_FLAG_DET_SEPARATE_FILL);
   const int g_out = grid_for(n_out, 256, 148 * 8), g_pts = grid_for(n_pts, 256, 148 * 8);
   if (!amax_in_emit) {
-    if (dtype == MSDA_F32) msda::msda_amax_kernel<float><<<g_out, 256, 0, st>>>((const float*)grad_output, n_out, amax);
-    else if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_out, 256, 0, st>>>((const double*)grad_output, n_out, amax);
-    else if (dtype == MSDA_BF16) msda::msda_amax_kernel<__nv_bfloat16><<<g_out, 256, 0, st>>>((const __nv_bfloat16*)grad_output, n_out, amax);
-    else msda::msda_amax_kernel<__half><<<g_out, 256, 0, st>>>((const __half*)grad_output, n_out, amax);
-    count();
-    if (dtype == MSDA_F64) msda::msda_amax_kernel<double><<<g_pts, 256, 0, st>>>((const double*)attn_weight, n_pts, amax + 1);
-    else msda::msda_amax_kernel<float><<<g_pts, 256, 0, st>>>((const float*)attn_weight, n_pts, amax + 1);
-    count();
-    msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, dtype == MSDA_F64 ? 44 : 38);
-    count();
-    MSDA_CUDA(cudaGetLastError());
+    if (int s = with_types<ValueTags>(dtype, [&](auto t) {
+          using VT = typename decltype(t)::VT;
+          using AT = typename decltype(t)::AT;
+          msda::msda_amax_kernel<VT><<<g_out, 256, 0, st>>>((const VT*)grad_output, n_out, amax);
+          count_launch();
+          msda::msda_amax_kernel<AT><<<g_pts, 256, 0, st>>>((const AT*)attn_weight, n_pts, amax + 1);
+          count_launch();
+          msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, std::is_same_v<VT, double> ? 44 : 38);
+          return launched();
+        }))
+      return s;
   }
   if (sorted) {
     // sorted segment reduction (msda_det.cuh): count -> scan -> fill -> gather; no atomics on grad_value
@@ -333,14 +329,13 @@ int det_backward(cudaStream_t st, const Dims& d, int dtype, unsigned flags, cons
     else
       msda::det_bin_kernel<false><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H, d.L, d.Q, d.P,
                                                          n_pts, bins, nullptr, nullptr, dcn);
-    count();
+    count_launch();
     msda::det_scan_block_kernel<<<(unsigned)lay.scan_blocks, 256, 0, st>>>(bins, bins, sums, lay.n_scan);
-    count();
+    count_launch();
     msda::det_scan_sums_kernel<<<1, 1024, 0, st>>>(sums, (int)lay.scan_blocks);
-    count();
+    count_launch();
     msda::det_scan_add_kernel<<<(unsigned)lay.scan_blocks, 256, 0, st>>>(bins, sums, lay.n_scan);
-    count();
-    MSDA_CUDA(cudaGetLastError());
+    if (int s = launched()) return s;
     // entries are filed by the backward kernel itself (ACC = EmitEntries): the lane that has just built a point's
     // record takes the cursor atomic and writes the 16-byte entry, so the separate fill pass (det_bin_kernel<true>:
     // re-read of every location / weight + the coordinate arithmetic a second time) is gone
@@ -358,8 +353,7 @@ int det_backward(cudaStream_t st, const Dims& d, int dtype, unsigned flags, cons
       else
         msda::det_bin_kernel<true><<<g_bin, 256, 0, st>>>(loc, w, spatial_shapes, level_start_index, d.H, d.L, d.Q, d.P,
                                                           n_pts, cursor, bins, entries, dcn);
-      count();
-      MSDA_CUDA(cudaGetLastError());
+      if (int s = launched()) return s;
       if (int s2 = src.dcn ? bwd_dcn_noscatter(st, d, dtype, grad_output, value, sampling_loc, attn_weight,
                                                grad_sampling_loc, grad_attn_weight, dcn)
                            : bwd_fast_noscatter(st, d, dtype, grad_output, value, spatial_shapes, level_start_index,
@@ -372,75 +366,41 @@ int det_backward(cudaStream_t st, const Dims& d, int dtype, unsigned flags, cons
       if (int s2 = emit(wamax, &n_warps)) return s2;
       const int g_w = grid_for(n_warps, 256, 148 * 8);
       msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax, n_warps, amax);
-      count();
+      count_launch();
       msda::msda_amax_kernel<float><<<g_w, 256, 0, st>>>(wamax + n_warps, n_warps, amax + 1);
-      count();
+      count_launch();
       msda::msda_det_scale_kernel<<<1, 1, 0, st>>>(amax, scale, 38);   // sorted route: float / bf16 / f16 only
-      count();
-      MSDA_CUDA(cudaGetLastError());
+      if (int s = launched()) return s;
     } else if (int s2 = emit(nullptr, nullptr)) {
       return s2;
     }
-    if (!det_dense(d)) {
-      if (dtype == MSDA_F32)
-        return det_gather<float>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
-      if (dtype == MSDA_BF16)
-        return det_gather<__nv_bfloat16>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale,
-                                         grad_value);
-      return det_gather<__half>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
-    }
-    int s3;
-    if (dtype == MSDA_F32)
-      s3 = det_cell_reduce<float>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale, acc);
-    else if (dtype == MSDA_BF16)
-      s3 = det_cell_reduce<__nv_bfloat16>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index,
-                                          scale, acc);
-    else
-      s3 = det_cell_reduce<__half>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index, scale,
-                                   acc);
-    if (s3 != MSDA_OK) return s3;
-    const int g_fin = grid_for(nv, 256, 148 * 16);
-    const long long* sacc = reinterpret_cast<const long long*>(acc);
-    if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_fin, 256, 0, st>>>(sacc, (float*)grad_value, nv, scale);
-    else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_fin, 256, 0, st>>>(sacc, (__nv_bfloat16*)grad_value, nv, scale);
-    else msda::msda_det_finalize_kernel<__half><<<g_fin, 256, 0, st>>>(sacc, (__half*)grad_value, nv, scale);
-    count();
-    MSDA_CUDA(cudaGetLastError());
-    return MSDA_OK;
+    return with_types<FastTags>(dtype, [&](auto t) {
+      using VT = typename decltype(t)::VT;
+      if (!det_dense(d))
+        return det_gather<VT>(st, d, grad_output, entries, bins, spatial_shapes, level_start_index, scale, grad_value);
+      if (int s = det_cell_reduce<VT>(st, d, grad_output, entries, bins, lay.bins, spatial_shapes, level_start_index,
+                                      scale, acc))
+        return s;
+      return det_finalize<VT>(st, acc, grad_value, nv, scale);
+    });
   }
-  int s;
-  if (src.dcn)
-    s = bwd_dcn_det(st, d, dtype, grad_output, value, sampling_loc, attn_weight, acc, grad_sampling_loc,
-                    grad_attn_weight, scale, dcn);
-  else if (fast_ok(d, dtype, flags))
-    s = bwd_fast_det(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_loc, attn_weight,
-                     acc, grad_sampling_loc, grad_attn_weight, scale);
-  else if (dtype == MSDA_F32)
-    s = bwd_generic<float, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                      sampling_loc, attn_weight, acc, grad_sampling_loc,
-                                                      grad_attn_weight, scale);
-  else if (dtype == MSDA_F64)
-    s = bwd_generic<double, double, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                        sampling_loc, attn_weight, acc, grad_sampling_loc,
-                                                        grad_attn_weight, scale);
-  else if (dtype == MSDA_BF16)
-    s = bwd_generic<__nv_bfloat16, float, unsigned long long>(st, d, grad_output, value, spatial_shapes,
-                                                              level_start_index, sampling_loc, attn_weight, acc,
-                                                              grad_sampling_loc, grad_attn_weight, scale);
-  else
-    s = bwd_generic<__half, float, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                       sampling_loc, attn_weight, acc, grad_sampling_loc,
-                                                       grad_attn_weight, scale);
-  if (s != MSDA_OK) return s;
-  const int g_val = grid_for(nv, 256, 148 * 16);
-  const long long* cacc = reinterpret_cast<const long long*>(acc);
-  if (dtype == MSDA_F32) msda::msda_det_finalize_kernel<float><<<g_val, 256, 0, st>>>(cacc, (float*)grad_value, nv, scale);
-  else if (dtype == MSDA_F64) msda::msda_det_finalize_kernel<double><<<g_val, 256, 0, st>>>(cacc, (double*)grad_value, nv, scale);
-  else if (dtype == MSDA_BF16) msda::msda_det_finalize_kernel<__nv_bfloat16><<<g_val, 256, 0, st>>>(cacc, (__nv_bfloat16*)grad_value, nv, scale);
-  else msda::msda_det_finalize_kernel<__half><<<g_val, 256, 0, st>>>(cacc, (__half*)grad_value, nv, scale);
-  count();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return with_types<ValueTags>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
+    int s;
+    if (src.dcn)
+      s = bwd_dcn_det(st, d, dtype, grad_output, value, sampling_loc, attn_weight, acc, grad_sampling_loc,
+                      grad_attn_weight, scale, dcn);
+    else if (fast_ok(d, dtype, flags))
+      s = bwd_fast_det(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_loc, attn_weight,
+                       acc, grad_sampling_loc, grad_attn_weight, scale);
+    else
+      s = bwd_generic<VT, AT, unsigned long long>(st, d, grad_output, value, spatial_shapes, level_start_index,
+                                                  sampling_loc, attn_weight, acc, grad_sampling_loc, grad_attn_weight,
+                                                  scale);
+    if (s != MSDA_OK) return s;
+    return det_finalize<VT>(st, acc, grad_value, nv, scale);
+  });
 }
 
 }  // namespace
@@ -515,17 +475,11 @@ int msda_forward(void* stream, const void* value, const int64_t* spatial_shapes,
   MSDA_CUDA(guard.enter(value));
   if (fast_ok(d, dtype, flags))
     return fwd_fast(st, d, dtype, flags, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
-  switch (dtype) {
-    case MSDA_F32:
-      return fwd_generic<float, float>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
-    case MSDA_F64:
-      return fwd_generic<double, double>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
-    case MSDA_BF16:
-      return fwd_generic<__nv_bfloat16, float>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
-    case MSDA_F16:
-      return fwd_generic<__half, float>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
-  }
-  return fail(MSDA_ERR_INVALID_ARGUMENT, "unknown dtype tag %d", dtype);
+  return with_types<ValueTags>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
+    return fwd_generic<VT, AT>(st, d, value, spatial_shapes, level_start_index, sampling_loc, attn_weight, output);
+  });
 }
 
 size_t msda_backward_workspace_bytes(int batch, int spatial_size, int num_heads, int channels, int num_levels,
@@ -595,8 +549,7 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
     return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
   const size_t need = msda_backward_workspace_bytes(batch, spatial_size, num_heads, channels, num_levels, num_query,
                                                     num_point, dtype, flags);
-  if (need && (!workspace || workspace_bytes < need))
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if (int s = check_workspace(workspace, workspace_bytes, need)) return s;
   if (det) {
     const DetSource src{sampling_loc, attn_weight, spatial_shapes, level_start_index, nullptr};
     return det_backward(st, d, dtype, flags, grad_output, value, src, grad_value, grad_sampling_loc, grad_attn_weight,
@@ -617,19 +570,14 @@ int msda_backward(void* stream, const void* grad_output, const void* value, cons
     else
       s = bwd_fast(st, d, dtype, flags, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
                    attn_weight, gv32, grad_sampling_loc, grad_attn_weight);
-  } else if (dtype == MSDA_F32) {
-    s = bwd_generic<float, float, float>(st, d, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
-                                         attn_weight, gv32, grad_sampling_loc, grad_attn_weight);
-  } else if (dtype == MSDA_F64) {
-    s = bwd_generic<double, double, double>(st, d, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
-                                            attn_weight, static_cast<double*>(grad_value), grad_sampling_loc,
-                                            grad_attn_weight);
-  } else if (dtype == MSDA_BF16) {
-    s = bwd_generic<__nv_bfloat16, float, float>(st, d, grad_output, value, spatial_shapes, level_start_index,
-                                                 sampling_loc, attn_weight, gv32, grad_sampling_loc, grad_attn_weight);
   } else {
-    s = bwd_generic<__half, float, float>(st, d, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
-                                          attn_weight, gv32, grad_sampling_loc, grad_attn_weight);
+    // grad_value accumulates in AT: float (the workspace for bf16 / f16 values), double for float64
+    s = with_types<ValueTags>(dtype, [&](auto t) {
+      using VT = typename decltype(t)::VT;
+      using AT = typename decltype(t)::AT;
+      return bwd_generic<VT, AT, AT>(st, d, grad_output, value, spatial_shapes, level_start_index, sampling_loc,
+                                     attn_weight, reinterpret_cast<AT*>(gv32), grad_sampling_loc, grad_attn_weight);
+    });
   }
   if (s != MSDA_OK) return s;
   if (two_byte(dtype)) return cast_from_f32(st, gv32, grad_value, d.n_value(), dtype);
@@ -662,12 +610,7 @@ int msda_fused_forward(void* stream, const void* value, const int64_t* spatial_s
     return s;
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(value));
-  msda::FusedArgs fa{};
-  fa.ref = reference_points;
-  fa.ref_dim = ref_dim;
-  fa.inv_P = 1.0f / (float)num_point;
-  fa.num_P = (float)num_point;
-  fa.value_mask = value_padding_mask;
+  const msda::FusedArgs fa = module_args(reference_points, ref_dim, num_point, value_padding_mask);
   return fwd_fused(static_cast<cudaStream_t>(stream), d, dtype, value, spatial_shapes, level_start_index,
                    sampling_offsets, attn_logits, output, fa);
 }
@@ -699,17 +642,11 @@ int msda_fused_backward(void* stream, const void* grad_output, const void* value
   MSDA_CUDA(guard.enter(value));
   const size_t need = msda_backward_workspace_bytes(batch, spatial_size, num_heads, channels, num_levels, num_query,
                                                     num_point, dtype, flags);
-  if (need && (!workspace || workspace_bytes < need))
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if (int s = check_workspace(workspace, workspace_bytes, need)) return s;
   float* gv32 = static_cast<float*>(grad_value);
   if (two_byte(vdt)) gv32 = static_cast<float*>(workspace);
   MSDA_CUDA(cudaMemsetAsync(gv32, 0, (size_t)d.n_value() * sizeof(float), st));
-  msda::FusedArgs fa{};
-  fa.ref = reference_points;
-  fa.ref_dim = ref_dim;
-  fa.inv_P = 1.0f / (float)num_point;
-  fa.num_P = (float)num_point;
-  fa.value_mask = value_padding_mask;
+  const msda::FusedArgs fa = module_args(reference_points, ref_dim, num_point, value_padding_mask);
   int s;
   if (fold_applies(d, dtype, flags))
     s = bwd_fold(st, d, dtype, grad_output, value, spatial_shapes, level_start_index, sampling_offsets, attn_logits,
@@ -781,11 +718,7 @@ int msda_packed_forward(void* stream, const void* value, const int64_t* spatial_
     return s;
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(value));
-  msda::FusedArgs fa{};
-  fa.ref = reference_points;
-  fa.ref_dim = ref_dim;
-  fa.inv_P = 1.0f / (float)num_point;
-  fa.num_P = (float)num_point;
+  const msda::FusedArgs fa = module_args(reference_points, ref_dim, num_point, nullptr);
   return fwd_packed(st, d, dtype, value, spatial_shapes, image_meta, sampling_offsets, attn_logits, output, fa);
 }
 
@@ -824,18 +757,13 @@ int msda_packed_backward(void* stream, const void* grad_output, const void* valu
     return s;
   const int vdt = fused_value_dtype(dtype);
   const size_t need = msda_packed_backward_workspace_bytes(total_value, num_heads, channels, dtype, flags);
-  if (need && (!workspace || workspace_bytes < need))
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if (int s = check_workspace(workspace, workspace_bytes, need)) return s;
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(value));
   const int64_t n_value = (int64_t)total_value * num_heads * channels;
   float* gv32 = two_byte(vdt) ? static_cast<float*>(workspace) : static_cast<float*>(grad_value);
   MSDA_CUDA(cudaMemsetAsync(gv32, 0, (size_t)n_value * sizeof(float), st));
-  msda::FusedArgs fa{};
-  fa.ref = reference_points;
-  fa.ref_dim = ref_dim;
-  fa.inv_P = 1.0f / (float)num_point;
-  fa.num_P = (float)num_point;
+  const msda::FusedArgs fa = module_args(reference_points, ref_dim, num_point, nullptr);
   const int s = bwd_packed(st, d, dtype, grad_output, value, spatial_shapes, image_meta, sampling_offsets, attn_logits,
                            gv32, grad_offsets, grad_logits, fa);
   if (s != MSDA_OK) return s;
@@ -931,8 +859,7 @@ int dcn_backward(void* stream, const Dims& d, const msda::FusedArgs& fa, const v
     return s;
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(anchor));
-  if (need && (!workspace || workspace_bytes < need))
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if (int s = check_workspace(workspace, workspace_bytes, need)) return s;
   if ((flags & MSDA_FLAG_DETERMINISTIC) && d.n_value() != 0 && d.n_points() != 0) {
     // bit-reproducible grad_input: the deterministic backward of the equivalent one-level problem, which writes every
     // element of grad_input in its own dtype (no float workspace, no zero-fill, no cast)
@@ -942,8 +869,7 @@ int dcn_backward(void* stream, const Dims& d, const msda::FusedArgs& fa, const v
     int64_t* table = reinterpret_cast<int64_t*>(ws);
     if (det_sorted_ok(d, dtype, flags)) {   // the count / gather / cell-reduce kernels read the level table
       msda::det_one_level_kernel<<<1, 1, 0, st>>>(table, fa.height_in, fa.width_in);
-      count_launch();
-      MSDA_CUDA(cudaGetLastError());
+      if (int s = launched()) return s;
     }
     const DetSource src{offset, w, table, table + 2, &fa};
     return det_backward(st, d, dtype, flags, grad_output, input, src, grad_input, grad_offset, grad_w,
@@ -1071,7 +997,6 @@ int dcnv2_setup(int batch, int channels, int height_in, int width_in, int height
                 pad_h, pad_w, dilation_h, dilation_w, groups, deformable_groups};
   return MSDA_OK;
 }
-bool aux16(int dtype) { return dtype == MSDA_BF16_AUX16 || dtype == MSDA_F16_AUX16; }
 }  // namespace
 
 size_t msda_dcnv2_col2im_workspace_bytes(int batch, int channels, int height_in, int width_in, int height_out,
@@ -1102,7 +1027,7 @@ int msda_dcnv2_im2col(void* stream, const void* input, const void* offset, const
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(columns));
-  return dcnv2_im2col(st, g, fused_value_dtype(dtype), aux16(dtype), flags, input, offset, mask, columns);
+  return dcnv2_im2col(st, g, dtype, flags, input, offset, mask, columns);
 }
 
 int msda_dcnv2_col2im(void* stream, const void* grad_columns, const void* input, const void* offset, const void* mask,
@@ -1128,8 +1053,7 @@ int msda_dcnv2_col2im(void* stream, const void* grad_columns, const void* input,
                                {"grad_mask", mask ? grad_mask : nullptr}, {"workspace", workspace}}))
     return s;
   const size_t need = two_byte(vdt) ? (size_t)g.n_input() * sizeof(float) : 0;
-  if (need && (!workspace || workspace_bytes < need))
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if (int s = check_workspace(workspace, workspace_bytes, need)) return s;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   DeviceGuard guard;
   MSDA_CUDA(guard.enter(grad_offset));
@@ -1140,8 +1064,7 @@ int msda_dcnv2_col2im(void* stream, const void* grad_columns, const void* input,
   }
   void* acc = two_byte(vdt) ? workspace : grad_input;
   MSDA_CUDA(cudaMemsetAsync(acc, 0, (size_t)g.n_input() * (vdt == MSDA_F64 ? 8 : 4), st));
-  if (int s = dcnv2_col2im(st, g, vdt, aux16(dtype), flags, grad_columns, input, offset, mask, acc, grad_offset,
-                           grad_mask))
+  if (int s = dcnv2_col2im(st, g, dtype, flags, grad_columns, input, offset, mask, acc, grad_offset, grad_mask))
     return s;
   if (two_byte(vdt)) return cast_from_f32(st, static_cast<const float*>(acc), grad_input, g.n_input(), vdt);
   return MSDA_OK;
@@ -1167,9 +1090,7 @@ int msda_debug_bookkeeping(void* stream, const float* sampling_loc, const int64_
     msda::msda_bookkeeping_kernel<<<grid_for(d.n_points(), 256, 148 * 16), 256, 0, st>>>(
         sampling_loc, spatial_shapes, level_start_index, d.S, d.H, d.D, d.L, d.Q, d.P, d.n_points(), corner_offsets,
         frac);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
 }  // extern "C"

@@ -239,39 +239,20 @@ namespace msda_host {
 
 namespace {
 
-// Calls f(VT*, AT*) (null pointers carrying the value and offset / mask types) for a value dtype and aux16.
-template <typename F>
-int with_types(int dtype, bool aux16, F&& f) {
-  switch (dtype) {
-    case MSDA_F32: return f((float*)nullptr, (float*)nullptr);
-    case MSDA_F64: return f((double*)nullptr, (double*)nullptr);
-    case MSDA_BF16:
-      return aux16 ? f((__nv_bfloat16*)nullptr, (__nv_bfloat16*)nullptr) : f((__nv_bfloat16*)nullptr, (float*)nullptr);
-    default: return aux16 ? f((__half*)nullptr, (__half*)nullptr) : f((__half*)nullptr, (float*)nullptr);
-  }
-}
-
-// Calls f(std::integral_constant<int, D>) for the chunk D of the fast kernels.
-template <typename F>
-int with_chunk(int D, F&& f) {
-  switch (D) {
-    case 16: return f(std::integral_constant<int, 16>{});
-    case 32: return f(std::integral_constant<int, 32>{});
-    case 64: return f(std::integral_constant<int, 64>{});
-    default: return f(std::integral_constant<int, 128>{});
-  }
-}
+// channels per lane of the fast kernels: one 16-byte load per corner
+template <typename VT>
+constexpr int dcn2_cpl() { return std::is_same_v<VT, float> ? 4 : 8; }
 
 // D of the fast kernels for this problem, 0 = the generic kernels: the largest of 128 / 64 / 32 / 16 dividing both
 // C/dg and C/groups (a chunk never straddles a deformable or a conv group), float / bf16 / f16, 32-bit element
 // offsets inside one image (one spare row of slack) and inside one image's thread range, B within grid.y.
-int fast_chunk(const Dcn2Dims& g, int dtype, unsigned flags) {
+template <typename VT>   // float / bf16 / f16
+int fast_chunk(const Dcn2Dims& g, unsigned flags) {
   if (flags & MSDA_FLAG_FORCE_GENERIC) return 0;
-  if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16) return 0;
   if (((int64_t)g.H * g.W + g.W + 1) * g.C >= ((int64_t)1 << 31) || g.B > 65535) return 0;
   for (int D = 128; D >= 16; D /= 2) {
     if (g.Cdg() % D != 0 || g.Cg() % D != 0) continue;
-    const int64_t lanes = D / (dtype == MSDA_F32 ? 4 : 8);
+    const int64_t lanes = D / dcn2_cpl<VT>();
     return ((int64_t)g.points_per_image() * lanes + 256 < ((int64_t)1 << 31)) ? D : 0;
   }
   return 0;
@@ -280,30 +261,27 @@ int fast_chunk(const Dcn2Dims& g, int dtype, unsigned flags) {
 }  // namespace
 
 #ifdef MSDA_EXP_SLIM
-int dcnv2_im2col(cudaStream_t, const Dcn2Dims&, int, bool, unsigned, const void*, const void*, const void*, void*) {
+int dcnv2_im2col(cudaStream_t, const Dcn2Dims&, int, unsigned, const void*, const void*, const void*, void*) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv2 kernels");
 }
-int dcnv2_col2im(cudaStream_t, const Dcn2Dims&, int, bool, unsigned, const void*, const void*, const void*,
-                 const void*, void*, void*, void*) {
+int dcnv2_col2im(cudaStream_t, const Dcn2Dims&, int, unsigned, const void*, const void*, const void*, const void*,
+                 void*, void*, void*) {
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no DCNv2 kernels");
 }
 #else
-int dcnv2_im2col(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsigned flags, const void* input,
-                 const void* offset, const void* mask, void* columns) {
-  const int D = fast_chunk(g, dtype, flags);
-  return with_types(dtype, aux16, [&](auto* vt, auto* at) {
-    using VT = std::remove_pointer_t<decltype(vt)>;
-    using AT = std::remove_pointer_t<decltype(at)>;
+int dcnv2_im2col(cudaStream_t st, const Dcn2Dims& g, int dtype, unsigned flags, const void* input, const void* offset,
+                 const void* mask, void* columns) {
+  return with_types<AllTags>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
     if constexpr (!std::is_same_v<VT, double>) {
-      if (D) {
-        return with_chunk(D, [&](auto dc) {
-          constexpr int DC = decltype(dc)::value, CPL = std::is_same_v<VT, float> ? 4 : 8;
+      if (const int D = fast_chunk<VT>(g, flags)) {
+        return with_chunk(D, [&](auto DC) {
+          constexpr int CPL = dcn2_cpl<VT>();
           const dim3 grid((unsigned)(((int64_t)g.points_per_image() * (DC / CPL) + 255) / 256), (unsigned)g.B);
           msda::msda_dcnv2_im2col_kernel<DC, CPL, VT, AT><<<grid, 256, 0, st>>>(
               (const VT*)input, (const AT*)offset, (const AT*)mask, (VT*)columns, g);
-          count_launch();
-          MSDA_CUDA(cudaGetLastError());
-          return MSDA_OK;
+          return launched();
         });
       }
     }
@@ -311,30 +289,25 @@ int dcnv2_im2col(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsi
     const int64_t total = g.n_points() * g.Cdg();
     msda::msda_dcnv2_im2col_generic_kernel<VT, AT, CT><<<grid_for(total, 256, 148 * 32), 256, 0, st>>>(
         (const VT*)input, (const AT*)offset, (const AT*)mask, (VT*)columns, g, total);
-    count_launch();
-    MSDA_CUDA(cudaGetLastError());
-    return MSDA_OK;
+    return launched();
   });
 }
 
-int dcnv2_col2im(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsigned flags, const void* grad_columns,
+int dcnv2_col2im(cudaStream_t st, const Dcn2Dims& g, int dtype, unsigned flags, const void* grad_columns,
                  const void* input, const void* offset, const void* mask, void* grad_input_acc, void* grad_offset,
                  void* grad_mask) {
-  const int D = fast_chunk(g, dtype, flags);
-  return with_types(dtype, aux16, [&](auto* vt, auto* at) {
-    using VT = std::remove_pointer_t<decltype(vt)>;
-    using AT = std::remove_pointer_t<decltype(at)>;
+  return with_types<AllTags>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
     if constexpr (!std::is_same_v<VT, double>) {
-      if (D) {
-        return with_chunk(D, [&](auto dc) {
-          constexpr int DC = decltype(dc)::value, CPL = std::is_same_v<VT, float> ? 4 : 8;
+      if (const int D = fast_chunk<VT>(g, flags)) {
+        return with_chunk(D, [&](auto DC) {
+          constexpr int CPL = dcn2_cpl<VT>();
           const dim3 grid((unsigned)(((int64_t)g.points_per_image() * (DC / CPL) + 255) / 256), (unsigned)g.B);
           msda::msda_dcnv2_col2im_kernel<DC, CPL, VT, AT><<<grid, 256, 0, st>>>(
               (const VT*)grad_columns, (const VT*)input, (const AT*)offset, (const AT*)mask, (float*)grad_input_acc,
               (AT*)grad_offset, (AT*)grad_mask, g);
-          count_launch();
-          MSDA_CUDA(cudaGetLastError());
-          return MSDA_OK;
+          return launched();
         });
       }
     }
@@ -343,9 +316,7 @@ int dcnv2_col2im(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsi
     msda::msda_dcnv2_col2im_generic_kernel<VT, AT, CT><<<grid_for(total, 256, 148 * 32), 256, 0, st>>>(
         (const VT*)grad_columns, (const VT*)input, (const AT*)offset, (const AT*)mask, (CT*)grad_input_acc,
         (AT*)grad_offset, (AT*)grad_mask, g, total);
-    count_launch();
-    MSDA_CUDA(cudaGetLastError());
-    return MSDA_OK;
+    return launched();
   });
 }
 #endif

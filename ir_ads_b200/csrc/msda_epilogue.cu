@@ -196,6 +196,18 @@ int ln_grid(int64_t rows) {
   return (int)(need < cap ? (need < 1 ? 1 : need) : cap);
 }
 
+// Calls f(Int<NV>{}) with the float4 chunks per lane the kernels are instantiated for: the least of 1, 2, 4, 8
+// covering C channels
+template <typename F>
+int with_nv(int C, F&& f) {
+  switch ((C + 127) / 128) {
+    case 1: return f(Int<1>{});
+    case 2: return f(Int<2>{});
+    case 3: case 4: return f(Int<4>{});
+    default: return f(Int<8>{});
+  }
+}
+
 int check_ln(int64_t rows, int C, int dtype) {
   if (rows < 0 || C < 0) return fail(MSDA_ERR_INVALID_ARGUMENT, "negative size (rows=%lld C=%d)", (long long)rows, C);
   if (dtype != MSDA_F32 && dtype != MSDA_BF16 && dtype != MSDA_F16)
@@ -213,45 +225,31 @@ extern "C" size_t msda_add_layernorm_workspace_bytes(int64_t rows, int channels)
 }
 
 namespace {
-// The bodies of the same-dtype entry points (mixed false: a, b, y, grad_* all `dtype`) and of the mixed ones (mixed
+// The bodies of the same-dtype entry points (MIXED false: a, b, y, grad_* all `dtype`) and of the mixed ones (MIXED
 // true: `a` / grad_a in the 16-bit `dtype`, b, y, grad_y, grad_b float), after check_ln.
+template <bool MIXED>
 int ln_forward(void* stream, const void* a, const void* b, const float* gamma, const float* beta, int64_t rows,
-               int channels, float eps, void* y, float* mean, float* rstd, int dtype, bool mixed) {
+               int channels, float eps, void* y, float* mean, float* rstd, int dtype) {
   if (rows == 0 || channels == 0) return MSDA_OK;
   if (!a || !b || !gamma || !beta || !y || !mean || !rstd) return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
   if (int s = check_alignment({{"a", a}, {"b", b}, {"gamma", gamma}, {"beta", beta}, {"y", y}})) return s;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int grid = ln_grid(rows);
-  const int nv = (channels + 127) / 128;
-#define LN_FWD(T_, NV_, TA_)                                                                                        \
-  add_layernorm_fwd_kernel<T_, NV_, TA_><<<grid, kLnThreads, 0, st>>>((const TA_*)a, (const T_*)b, gamma, beta, (T_*)y, \
-                                                                      mean, rstd, rows, channels, eps)
-#define LN_FWD_NV(T_, TA_)                              \
-  switch (nv) {                                         \
-    case 1: LN_FWD(T_, 1, TA_); break;                  \
-    case 2: LN_FWD(T_, 2, TA_); break;                  \
-    case 3: case 4: LN_FWD(T_, 4, TA_); break;          \
-    default: LN_FWD(T_, 8, TA_); break;                 \
-  }
-  if (mixed) {
-    if (dtype == MSDA_BF16) { LN_FWD_NV(float, __nv_bfloat16) } else { LN_FWD_NV(float, __half) }
-  } else if (dtype == MSDA_F32) {
-    LN_FWD_NV(float, float)
-  } else if (dtype == MSDA_BF16) {
-    LN_FWD_NV(__nv_bfloat16, __nv_bfloat16)
-  } else {
-    LN_FWD_NV(__half, __half)
-  }
-#undef LN_FWD_NV
-#undef LN_FWD
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return with_types<FastTags>(dtype, [&](auto t) {
+    using TA = typename decltype(t)::VT;
+    using T = std::conditional_t<MIXED, float, TA>;
+    return with_nv(channels, [&](auto NV) {
+      add_layernorm_fwd_kernel<T, NV, TA><<<grid, kLnThreads, 0, st>>>((const TA*)a, (const T*)b, gamma, beta, (T*)y,
+                                                                       mean, rstd, rows, channels, eps);
+      return launched();
+    });
+  });
 }
 
+template <bool MIXED>
 int ln_backward(void* stream, const void* grad_y, const void* a, const void* b, const float* gamma, const float* mean,
                 const float* rstd, int64_t rows, int channels, void* grad_x, void* grad_a, float* grad_gamma,
-                float* grad_beta, void* workspace, size_t workspace_bytes, int dtype, bool mixed) {
+                float* grad_beta, void* workspace, size_t workspace_bytes, int dtype) {
   if (channels == 0) return MSDA_OK;
   if (!grad_gamma || !grad_beta) return fail(MSDA_ERR_INVALID_ARGUMENT, "grad_gamma / grad_beta is null");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -260,50 +258,30 @@ int ln_backward(void* stream, const void* grad_y, const void* a, const void* b, 
     MSDA_CUDA(cudaMemsetAsync(grad_beta, 0, (size_t)channels * sizeof(float), st));
     return MSDA_OK;
   }
-  if (!grad_y || !a || !b || !gamma || !mean || !rstd || !grad_x || (mixed && !grad_a))
+  if (!grad_y || !a || !b || !gamma || !mean || !rstd || !grad_x || (MIXED && !grad_a))
     return fail(MSDA_ERR_INVALID_ARGUMENT, "null tensor pointer");
   if (int s = check_alignment({{"grad_y", grad_y}, {"a", a}, {"b", b}, {"gamma", gamma},
-                               {mixed ? "grad_b" : "grad_x", grad_x}, {"grad_a", mixed ? grad_a : nullptr},
+                               {MIXED ? "grad_b" : "grad_x", grad_x}, {"grad_a", MIXED ? grad_a : nullptr},
                                {"workspace", workspace}}))
     return s;
-  const size_t need = msda_add_layernorm_workspace_bytes(rows, channels);
-  if (!workspace || workspace_bytes < need)
-    return fail(MSDA_ERR_WORKSPACE, "workspace of %zu bytes required, %zu given", need, workspace_bytes);
+  if (int s = check_workspace(workspace, workspace_bytes, msda_add_layernorm_workspace_bytes(rows, channels))) return s;
   const int grid = ln_grid(rows);
-  const int nv = (channels + 127) / 128;
   const size_t smem = (size_t)(kLnThreads / 32) * 2 * channels * sizeof(float);
   float* partial = static_cast<float*>(workspace);
-#define LN_BWD(T_, NV_, TA_)                                                                                \
-  do {                                                                                                      \
-    auto k = add_layernorm_bwd_kernel<T_, NV_, TA_>;                                                        \
-    MSDA_CUDA(ensure_smem(k, smem));                                                                        \
-    k<<<grid, kLnThreads, smem, st>>>((const T_*)grad_y, (const TA_*)a, (const T_*)b, gamma, mean, rstd,    \
-                                      (T_*)grad_x, (TA_*)grad_a, partial, rows, channels);                  \
-  } while (0)
-#define LN_BWD_NV(T_, TA_)                              \
-  switch (nv) {                                         \
-    case 1: LN_BWD(T_, 1, TA_); break;                  \
-    case 2: LN_BWD(T_, 2, TA_); break;                  \
-    case 3: case 4: LN_BWD(T_, 4, TA_); break;          \
-    default: LN_BWD(T_, 8, TA_); break;                 \
-  }
-  if (mixed) {
-    if (dtype == MSDA_BF16) { LN_BWD_NV(float, __nv_bfloat16) } else { LN_BWD_NV(float, __half) }
-  } else if (dtype == MSDA_F32) {
-    LN_BWD_NV(float, float)
-  } else if (dtype == MSDA_BF16) {
-    LN_BWD_NV(__nv_bfloat16, __nv_bfloat16)
-  } else {
-    LN_BWD_NV(__half, __half)
-  }
-#undef LN_BWD_NV
-#undef LN_BWD
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
+  if (int s = with_types<FastTags>(dtype, [&](auto t) {
+        using TA = typename decltype(t)::VT;
+        using T = std::conditional_t<MIXED, float, TA>;
+        return with_nv(channels, [&](auto NV) {
+          auto k = add_layernorm_bwd_kernel<T, NV, TA>;
+          MSDA_CUDA(ensure_smem(k, smem));
+          k<<<grid, kLnThreads, smem, st>>>((const T*)grad_y, (const TA*)a, (const T*)b, gamma, mean, rstd, (T*)grad_x,
+                                            (TA*)grad_a, partial, rows, channels);
+          return launched();
+        });
+      }))
+    return s;
   add_layernorm_param_grad_kernel<<<(2 * channels + 255) / 256, 256, 0, st>>>(partial, grid, channels, grad_gamma, grad_beta);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
 // the mixed form: `a` bfloat16 or float16, everything else float
@@ -319,7 +297,7 @@ extern "C" {
 int msda_add_layernorm_forward(void* stream, const void* a, const void* b, const float* gamma, const float* beta,
                                int64_t rows, int channels, float eps, void* y, float* mean, float* rstd, int dtype) {
   if (int s = check_ln(rows, channels, dtype)) return s;
-  return ln_forward(stream, a, b, gamma, beta, rows, channels, eps, y, mean, rstd, dtype, false);
+  return ln_forward<false>(stream, a, b, gamma, beta, rows, channels, eps, y, mean, rstd, dtype);
 }
 
 int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a, const void* b, const float* gamma,
@@ -327,15 +305,15 @@ int msda_add_layernorm_backward(void* stream, const void* grad_y, const void* a,
                                 float* grad_gamma, float* grad_beta, void* workspace, size_t workspace_bytes,
                                 int dtype) {
   if (int s = check_ln(rows, channels, dtype)) return s;
-  return ln_backward(stream, grad_y, a, b, gamma, mean, rstd, rows, channels, grad_x, nullptr, grad_gamma, grad_beta,
-                     workspace, workspace_bytes, dtype, false);
+  return ln_backward<false>(stream, grad_y, a, b, gamma, mean, rstd, rows, channels, grad_x, nullptr, grad_gamma,
+                            grad_beta, workspace, workspace_bytes, dtype);
 }
 
 int msda_add_layernorm_mixed_forward(void* stream, const void* a, const float* b, const float* gamma,
                                      const float* beta, int64_t rows, int channels, float eps, float* y, float* mean,
                                      float* rstd, int a_dtype) {
   if (int s = check_ln_mixed(rows, channels, a_dtype)) return s;
-  return ln_forward(stream, a, b, gamma, beta, rows, channels, eps, y, mean, rstd, a_dtype, true);
+  return ln_forward<true>(stream, a, b, gamma, beta, rows, channels, eps, y, mean, rstd, a_dtype);
 }
 
 int msda_add_layernorm_mixed_backward(void* stream, const float* grad_y, const void* a, const float* b,
@@ -343,8 +321,8 @@ int msda_add_layernorm_mixed_backward(void* stream, const float* grad_y, const v
                                       int channels, void* grad_a, float* grad_b, float* grad_gamma, float* grad_beta,
                                       void* workspace, size_t workspace_bytes, int a_dtype) {
   if (int s = check_ln_mixed(rows, channels, a_dtype)) return s;
-  return ln_backward(stream, grad_y, a, b, gamma, mean, rstd, rows, channels, grad_b, grad_a, grad_gamma, grad_beta,
-                     workspace, workspace_bytes, a_dtype, true);
+  return ln_backward<true>(stream, grad_y, a, b, gamma, mean, rstd, rows, channels, grad_b, grad_a, grad_gamma,
+                           grad_beta, workspace, workspace_bytes, a_dtype);
 }
 
 }  // extern "C"

@@ -1,4 +1,5 @@
-// msda_fast_launch.cuh -- launch templates and dispatch macros shared by the fast-kernel translation units.
+// msda_fast_launch.cuh -- launch templates and the shape / row-order dispatch shared by the fast-kernel translation
+// units: dispatch_fast(d, dtype, flags, f) calls f(types, D, PT, ORDER) for the one fast kernel a problem runs on.
 #pragma once
 #include "msda_host.h"
 
@@ -49,9 +50,7 @@ int launch_fwd_fast(cudaStream_t st, const Dims& d, const void* value, const int
   if (PRE == msda::kPrePacked) grid = (unsigned)((int64_t)d.B * (((int64_t)d.Q * d.H + G::RPC - 1) / G::RPC));
   k<<<grid, THREADS, smem, st>>>((const VT*)value, shapes, lsi, (const AT*)loc, (const AT*)w, (VT*)out, fa,
                                  d.B, d.S, d.H, d.L, d.Q, d.P, rows);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
 template <int D, typename VT, int PT, int THREADS, int ORDER, typename ACC, int PRE = 0, typename AT = float>
@@ -75,75 +74,71 @@ int launch_bwd_fast(cudaStream_t st, const Dims& d, const void* go, const void* 
   if (ORDER == 3) grid = (unsigned)((int64_t)d.B * d.H * tile2d_bound(d, G::RPC));
   k<<<grid, THREADS, smem, st>>>((const VT*)go, (const VT*)value, shapes, lsi, (const AT*)loc, (const AT*)w,
                                  gv, (AT*)gl, (AT*)gw, det, fa, emit, d.B, d.S, d.H, d.L, d.Q, d.P, rows);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
-// CALL(D, VT, PT, ORDER) must be an expression returning int
+// Calls f(Int<PT>{}) for the point count of the fast kernels: 4 or 8 compiled in, 0 = any (runtime d.P).
+template <typename F>
+int with_points(int P, F&& f) {
+  if (P == 4) return f(Int<4>{});
+  if (P == 8) return f(Int<8>{});
+  return f(Int<0>{});
+}
+
+// Calls f(Int<D>{}, Int<PT>{}) for the channel and point count of the fast kernels.
+template <typename F>
+int with_shape(const Dims& d, F&& f) {
 #ifdef MSDA_EXP_SLIM
-// Kernel-variant experiment builds (tools/build_variant.sh): only D = 32, P in {4, 8} are instantiated, so a variant
-// compiles in well under a minute.  Never defined for the product library.
-#define MSDA_DISPATCH_D(VT_, CALL)                                          \
-  do {                                                                      \
-    if (d.D != 32) return fail(MSDA_ERR_UNSUPPORTED, "slim build: D=%d", d.D); \
-    if (d.P == 4) MSDA_DISPATCH_ORDER(32, VT_, 4, CALL);                    \
-    if (d.P == 8) MSDA_DISPATCH_ORDER(32, VT_, 8, CALL);                    \
-    return fail(MSDA_ERR_UNSUPPORTED, "slim build: P=%d", d.P);             \
-  } while (0)
+  // Kernel-variant experiment builds (tools/build_variant.sh): only D = 32, P in {4, 8} are instantiated, so a variant
+  // compiles in well under a minute.  Never defined for the product library.
+  if (d.D != 32) return fail(MSDA_ERR_UNSUPPORTED, "slim build: D=%d", d.D);
+  if (d.P == 4) return f(Int<32>{}, Int<4>{});
+  if (d.P == 8) return f(Int<32>{}, Int<8>{});
+  return fail(MSDA_ERR_UNSUPPORTED, "slim build: P=%d", d.P);
 #else
-#define MSDA_DISPATCH_PT(D_, VT_, CALL)                      \
-  do {                                                       \
-    if (d.P == 4) MSDA_DISPATCH_ORDER(D_, VT_, 4, CALL);     \
-    if (d.P == 8) MSDA_DISPATCH_ORDER(D_, VT_, 8, CALL);     \
-    MSDA_DISPATCH_ORDER(D_, VT_, 0, CALL);                   \
-  } while (0)
-#define MSDA_DISPATCH_D(VT_, CALL)                           \
-  do {                                                       \
-    switch (d.D) {                                           \
-      case 16: MSDA_DISPATCH_PT(16, VT_, CALL);              \
-      case 32: MSDA_DISPATCH_PT(32, VT_, CALL);              \
-      case 64: MSDA_DISPATCH_PT(64, VT_, CALL);              \
-      case 128: MSDA_DISPATCH_PT(128, VT_, CALL);            \
-      default: return fail(MSDA_ERR_UNSUPPORTED, "fast path: D=%d", d.D); \
-    }                                                        \
-  } while (0)
+  return with_chunk(d.D, [&](auto D) { return with_points(d.P, [&](auto PT) { return f(D, PT); }); });
 #endif
+}
 
-// CALL over the value types of the fused kernels with 16-bit offsets / logits (MSDA_BF16_AUX16, MSDA_F16_AUX16): the
-// value's own type is the aux type
-#define MSDA_DISPATCH_VT_AUX16(CALL)                                   \
-  do {                                                                 \
-    if (dtype == MSDA_BF16_AUX16) MSDA_DISPATCH_D(__nv_bfloat16, CALL);\
-    if (dtype == MSDA_F16_AUX16) MSDA_DISPATCH_D(__half, CALL);        \
-  } while (0)
+// Row orders (the kernels' ORDER argument) and the sets a family is instantiated for
+constexpr int kLinear = 0, kStrip = 2, kTile2d = 3;
+template <int... Orders>
+struct OrderList {};
+using AllOrders = OrderList<kLinear, kStrip, kTile2d>;
 
-// CALL over the value types of the fast kernels (fast_ok admits no other dtype)
-#define MSDA_DISPATCH_VT(CALL)                                         \
-  do {                                                                 \
-    if (dtype == MSDA_F32) MSDA_DISPATCH_D(float, CALL);               \
-    if (dtype == MSDA_BF16) MSDA_DISPATCH_D(__nv_bfloat16, CALL);      \
-    if (dtype == MSDA_F16) MSDA_DISPATCH_D(__half, CALL);              \
-    return fail(MSDA_ERR_UNSUPPORTED, "fast path: dtype %d", dtype);   \
-  } while (0)
-
-// The product library instantiates ONE row order per pass -- LINEAR forward, STRIP backward, the pair that is fastest
-// on every measured config (profiles/r02t_sweep_row_orders.txt) -- and treats MSDA_FLAG_ORDER_* as hints it may
-// ignore (results never depend on the order).  Experiment builds (-DMSDA_EXPERIMENTS) and the slim variant builds
-// of tools/build_variant.sh carry all three orders for both passes.
+// The product library instantiates ONE row order per pass of the plain operator -- LINEAR forward, STRIP backward, the
+// pair that is fastest on every measured config (profiles/r02t_sweep_row_orders.txt) -- and treats MSDA_FLAG_ORDER_*
+// as hints it may ignore (results never depend on the order).  Experiment builds (-DMSDA_EXPERIMENTS) and the slim
+// variant builds of tools/build_variant.sh carry all three orders for both passes.
 #if defined(MSDA_EXPERIMENTS) || defined(MSDA_EXP_SLIM)
-#define MSDA_ALL_ORDERS 1
+template <int Default>
+using PlainOrders = AllOrders;
+#else
+template <int Default>
+using PlainOrders = OrderList<Default>;
 #endif
 
-// all three row orders (the plain operator)
-#define MSDA_ORDER_ANY(D_, VT_, PT_, CALL)                       \
-  do {                                                           \
-    if (use_tile2d(d, flags)) return CALL(D_, VT_, PT_, 3);      \
-    if (use_strip(flags)) return CALL(D_, VT_, PT_, 2);          \
-    return CALL(D_, VT_, PT_, 0);                                \
-  } while (0)
-// one fixed order
-#define MSDA_ORDER_LINEAR(D_, VT_, PT_, CALL) return CALL(D_, VT_, PT_, 0)
-#define MSDA_ORDER_STRIP(D_, VT_, PT_, CALL) return CALL(D_, VT_, PT_, 2)
+// Calls f(Int<ORDER>{}): a family with one order always runs it, one with all three picks it from the flags.
+template <int Order, typename F>
+int with_order(OrderList<Order>, const Dims&, unsigned, F&& f) {
+  return f(Int<Order>{});
+}
+template <typename F>
+int with_order(AllOrders, const Dims& d, unsigned flags, F&& f) {
+  if (use_tile2d(d, flags)) return f(Int<kTile2d>{});
+  if (use_strip(flags)) return f(Int<kStrip>{});
+  return f(Int<kLinear>{});
+}
+
+// Calls f(TagTypes<dtype>{}, Int<D>{}, Int<PT>{}, Int<ORDER>{}) for a family instantiated for the dtype tags Tags
+// and the row orders Orders.
+template <typename Tags, typename Orders, typename F>
+int dispatch_fast(const Dims& d, int dtype, unsigned flags, F&& f) {
+  return with_types<Tags>(dtype, [&](auto t) {
+    return with_shape(d, [&](auto D, auto PT) {
+      return with_order(Orders{}, d, flags, [&](auto order) { return f(t, D, PT, order); });
+    });
+  });
+}
 
 }  // namespace msda_host

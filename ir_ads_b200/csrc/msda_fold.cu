@@ -40,39 +40,29 @@ int launch_fold(cudaStream_t st, const Dims& d, const void* go, const void* valu
   k<<<grid, msda::kFoldThreads, smem, st>>>((const VT*)go, (const VT*)value, shapes, lsi, (const float*)loc,
                                              (const float*)w, gv, (float*)gl, (float*)gw, fa, d.B, d.S, d.H, d.L, d.Q,
                                              d.P);
-  count_launch();
-  MSDA_CUDA(cudaGetLastError());
-  return MSDA_OK;
+  return launched();
 }
 
-#ifdef MSDA_EXP_SLIM
-// experiment builds: D = 32, P in {4, 8}, the plain operator only
 template <int D, typename VT, int PRE>
 int fold_pt(cudaStream_t st, const Dims& d, int nq, const void* go, const void* value, const int64_t* shapes,
             const int64_t* lsi, const void* loc, const void* w, float* gv, void* gl, void* gw, msda::FusedArgs fa) {
+  auto call = [&](auto PT, auto NQ) {
+    return launch_fold<D, VT, PT, NQ, PRE>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw, fa);
+  };
+#ifdef MSDA_EXP_SLIM
+  // experiment builds: D = 32, P in {4, 8}, the plain operator only
   if constexpr (D == 32 && PRE == msda::kPrePlain) {
-    if (d.P == 4 && nq == 64) return launch_fold<32, VT, 4, 64, PRE>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw, fa);
-    if (d.P == 8 && nq == 32) return launch_fold<32, VT, 8, 32, PRE>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw, fa);
+    if (d.P == 4 && nq == 64) return call(Int<4>{}, Int<64>{});
+    if (d.P == 8 && nq == 32) return call(Int<8>{}, Int<32>{});
   }
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: fold D=%d P=%d", d.D, d.P);
-}
 #else
-template <int D, typename VT, int PRE>
-int fold_pt(cudaStream_t st, const Dims& d, int nq, const void* go, const void* value, const int64_t* shapes,
-            const int64_t* lsi, const void* loc, const void* w, float* gv, void* gl, void* gw, msda::FusedArgs fa) {
-#define FOLD_CALL(PT_, NQ_) launch_fold<D, VT, PT_, NQ_, PRE>(st, d, go, value, shapes, lsi, loc, w, gv, gl, gw, fa)
   if constexpr (D == 32) {
-    if (nq == 32) {
-      if (d.P == 8) return FOLD_CALL(8, 32);
-      return FOLD_CALL(0, 32);
-    }
+    if (nq == 32) return d.P == 8 ? call(Int<8>{}, Int<32>{}) : call(Int<0>{}, Int<32>{});
   }
-  if (d.P == 4) return FOLD_CALL(4, 64);
-  if (d.P == 8) return FOLD_CALL(8, 64);
-  return FOLD_CALL(0, 64);
-#undef FOLD_CALL
-}
+  return with_points(d.P, [&](auto PT) { return call(PT, Int<64>{}); });
 #endif
+}
 }  // namespace
 
 bool fold_applies(const Dims& d, int dtype, unsigned flags) {
@@ -92,18 +82,15 @@ int bwd_fold(cudaStream_t st, const Dims& d, int dtype, const void* go, const vo
              const msda::FusedArgs* fa) {
   const int nq = fold_tile(d);
   const msda::FusedArgs a = fa ? *fa : msda::FusedArgs{};
-#define FOLD_D(VT_, PRE_)                                                                                 \
-  do {                                                                                                    \
-    if (d.D == 32) return fold_pt<32, VT_, PRE_>(st, d, nq, go, value, shapes, lsi, loc, w, gv, gl, gw, a); \
-    return fold_pt<64, VT_, PRE_>(st, d, nq, go, value, shapes, lsi, loc, w, gv, gl, gw, a);               \
-  } while (0)
-  if (fa) {
-    if (dtype == MSDA_F32) FOLD_D(float, msda::kPreFused);
-    FOLD_D(__nv_bfloat16, msda::kPreFused);
-  }
-  if (dtype == MSDA_F32) FOLD_D(float, msda::kPrePlain);
-  FOLD_D(__nv_bfloat16, msda::kPrePlain);
-#undef FOLD_D
+  // fold_applies admits float / bf16 values and D in {32, 64}
+  return with_types<TagList<MSDA_F32, MSDA_BF16>>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    auto run = [&](auto PRE) {
+      if (d.D == 32) return fold_pt<32, VT, PRE>(st, d, nq, go, value, shapes, lsi, loc, w, gv, gl, gw, a);
+      return fold_pt<64, VT, PRE>(st, d, nq, go, value, shapes, lsi, loc, w, gv, gl, gw, a);
+    };
+    return fa ? run(Int<msda::kPreFused>{}) : run(Int<msda::kPrePlain>{});
+  });
 }
 
 }  // namespace msda_host

@@ -5,16 +5,10 @@ namespace msda_host {
 
 int fwd_fast(cudaStream_t st, const Dims& d, int dtype, unsigned flags, const void* value, const int64_t* shapes,
              const int64_t* lsi, const void* loc, const void* w, void* out) {
-#ifdef MSDA_ALL_ORDERS
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_ANY
-#else
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
-  (void)flags;
-#endif
-#define CALL_FWD(D_, VT_, PT_, ORD_) launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_>(st, d, value, shapes, lsi, loc, w, out)
-  MSDA_DISPATCH_VT(CALL_FWD);
-#undef CALL_FWD
-#undef MSDA_DISPATCH_ORDER
+  return dispatch_fast<FastTags, PlainOrders<kLinear>>(d, dtype, flags, [&](auto t, auto D, auto PT, auto order) {
+    using VT = typename decltype(t)::VT;
+    return launch_fwd_fast<D, VT, PT, kFwdThreads, order>(st, d, value, shapes, lsi, loc, w, out);
+  });
 }
 
 #ifdef MSDA_EXP_SLIM
@@ -33,36 +27,26 @@ int fwd_packed(cudaStream_t, const Dims&, int, const void*, const int64_t*, cons
   return fail(MSDA_ERR_UNSUPPORTED, "slim build: no packed kernels");
 }
 #else
-// fused pre-op chain: LINEAR order.  dtype MSDA_*_AUX16: offsets / logits in the value's 16-bit type
-int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes, const int64_t* lsi,
-              const void* off, const void* logits, void* out, msda::FusedArgs fa) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
-#define CALL_FF(D_, VT_, PT_, ORD_) \
-  launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPreFused>(st, d, value, shapes, lsi, off, logits, out, fa)
-#define CALL_FF16(D_, VT_, PT_, ORD_)                                                                             \
-  launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPreFused, VT_>(st, d, value, shapes, lsi, off, logits, out, \
-                                                                         fa)
-  MSDA_DISPATCH_VT_AUX16(CALL_FF16);
-  MSDA_DISPATCH_VT(CALL_FF);
-#undef CALL_FF16
-#undef CALL_FF
-#undef MSDA_DISPATCH_ORDER
+// fused pre-op chain, PRE kPreFused (lsi: level start index) or kPrePacked (lsi: the per-image metadata rows): LINEAR
+// order.  dtype MSDA_*_AUX16: offsets / logits in the value's 16-bit type
+template <int PRE>
+int fwd_fused_pre(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes,
+                  const int64_t* lsi, const void* off, const void* logits, void* out, msda::FusedArgs fa) {
+  return dispatch_fast<FusedTags, OrderList<kLinear>>(d, dtype, 0, [&](auto t, auto D, auto PT, auto order) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
+    return launch_fwd_fast<D, VT, PT, kFwdThreads, order, PRE, AT>(st, d, value, shapes, lsi, off, logits, out, fa);
+  });
 }
 
-// fused chain over a packed batch: LINEAR order, the same value / aux types as fwd_fused
+int fwd_fused(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes, const int64_t* lsi,
+              const void* off, const void* logits, void* out, msda::FusedArgs fa) {
+  return fwd_fused_pre<msda::kPreFused>(st, d, dtype, value, shapes, lsi, off, logits, out, fa);
+}
+
 int fwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* value, const int64_t* shapes,
                const int64_t* meta, const void* off, const void* logits, void* out, msda::FusedArgs fa) {
-#define MSDA_DISPATCH_ORDER MSDA_ORDER_LINEAR
-#define CALL_FP(D_, VT_, PT_, ORD_) \
-  launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPrePacked>(st, d, value, shapes, meta, off, logits, out, fa)
-#define CALL_FP16(D_, VT_, PT_, ORD_)                                                                           \
-  launch_fwd_fast<D_, VT_, PT_, kFwdThreads, ORD_, msda::kPrePacked, VT_>(st, d, value, shapes, meta, off, logits, \
-                                                                          out, fa)
-  MSDA_DISPATCH_VT_AUX16(CALL_FP16);
-  MSDA_DISPATCH_VT(CALL_FP);
-#undef CALL_FP16
-#undef CALL_FP
-#undef MSDA_DISPATCH_ORDER
+  return fwd_fused_pre<msda::kPrePacked>(st, d, dtype, value, shapes, meta, off, logits, out, fa);
 }
 
 // DCNv3: runtime point count (K = kernel_h * kernel_w), LINEAR order.  PRE: kPreDcn (w = mask) or kPreDcnSoftmax
@@ -70,26 +54,14 @@ int fwd_packed(cudaStream_t st, const Dims& d, int dtype, const void* value, con
 template <int PRE>
 int fwd_dcn_pre(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off, const void* w,
                 void* out, msda::FusedArgs fa) {
-#define CALL_DF(D_, VT_, AT_) \
-  launch_fwd_fast<D_, VT_, 0, kFwdThreads, 0, PRE, AT_>(st, d, input, nullptr, nullptr, off, w, out, fa)
-#define DCN_D(VT_, AT_)                                                                    \
-  switch (d.D) {                                                                           \
-    case 16: return CALL_DF(16, VT_, AT_);                                                 \
-    case 32: return CALL_DF(32, VT_, AT_);                                                 \
-    case 64: return CALL_DF(64, VT_, AT_);                                                 \
-    case 128: return CALL_DF(128, VT_, AT_);                                               \
-    default: return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: group_channels=%d", d.D);           \
-  }
-  if constexpr (PRE == msda::kPreDcnSoftmax) {
-    if (dtype == MSDA_BF16_AUX16) DCN_D(__nv_bfloat16, __nv_bfloat16)
-    if (dtype == MSDA_F16_AUX16) DCN_D(__half, __half)
-  }
-  if (dtype == MSDA_F32) DCN_D(float, float)
-  if (dtype == MSDA_BF16) DCN_D(__nv_bfloat16, float)
-  if (dtype == MSDA_F16) DCN_D(__half, float)
-  return fail(MSDA_ERR_UNSUPPORTED, "dcnv3: dtype %d", dtype);
-#undef DCN_D
-#undef CALL_DF
+  using Tags = std::conditional_t<PRE == msda::kPreDcnSoftmax, FusedTags, FastTags>;
+  return with_types<Tags>(dtype, [&](auto t) {
+    using VT = typename decltype(t)::VT;
+    using AT = typename decltype(t)::AT;
+    return with_chunk(d.D, [&](auto D) {
+      return launch_fwd_fast<D, VT, 0, kFwdThreads, kLinear, PRE, AT>(st, d, input, nullptr, nullptr, off, w, out, fa);
+    });
+  });
 }
 
 int fwd_dcn(cudaStream_t st, const Dims& d, int dtype, const void* input, const void* off, const void* mask, void* out,

@@ -8,6 +8,9 @@
 //   msda_bwd_aux.cu  fast backward kernels: fixed-point reds, no-scatter, fused module chain, DCNv3
 //   msda_fold.cu     encoder-form backward with on-SM folding of grad_value (msda_fold.cuh)
 //   msda_dcnv2.cu    deformable convolution im2col / col2im (fast + generic)
+//   msda_epilogue.cu fused residual add + LayerNorm
+// Every launch site maps its runtime dtype tag and channel count onto template arguments with the dispatch templates
+// below (with_types, with_chunk); the fast units add the point-count and row-order dispatch of msda_fast_launch.cuh.
 #pragma once
 #include "../../include/msda.h"
 
@@ -17,6 +20,7 @@
 #include <stdint.h>
 
 #include <initializer_list>
+#include <type_traits>
 
 #include "msda_fast.cuh"
 
@@ -49,8 +53,67 @@ struct NamedPtr {
 };
 int check_alignment(std::initializer_list<NamedPtr> ptrs);
 
+// MSDA_OK, or MSDA_ERR_WORKSPACE when `need` bytes are required and fewer are given
+int check_workspace(const void* workspace, size_t workspace_bytes, size_t need);
+
+// The tail of every kernel launch: counts it (msda_kernel_launch_count) and returns MSDA_OK or the launch error.
+inline int launched() {
+  count_launch();
+  MSDA_CUDA(cudaGetLastError());
+  return MSDA_OK;
+}
+
 // D in {16,32,64,128}, float / bf16 / f16 value, L <= 16, 1 <= L*P <= 64, 32-bit offsets inside one image
 bool fast_ok(const Dims& d, int dtype, unsigned flags);
+
+// ---- dispatch templates ----
+// Each one calls a generic lambda with the template arguments a runtime value stands for, and instantiates it only
+// for the values it lists, so a launch site compiles exactly the kernels it can launch.
+template <int N>
+using Int = std::integral_constant<int, N>;
+
+// The types a dtype tag stands for: VT of the value (input, output, grad_output), AT of the offsets / weights and
+// their gradients (float; double for float64; the value's own type for the autocast tags *_AUX16).
+template <int Tag>
+struct TagTypes;
+template <> struct TagTypes<MSDA_F32> { using VT = float; using AT = float; };
+template <> struct TagTypes<MSDA_F64> { using VT = double; using AT = double; };
+template <> struct TagTypes<MSDA_BF16> { using VT = __nv_bfloat16; using AT = float; };
+template <> struct TagTypes<MSDA_F16> { using VT = __half; using AT = float; };
+template <> struct TagTypes<MSDA_BF16_AUX16> { using VT = __nv_bfloat16; using AT = __nv_bfloat16; };
+template <> struct TagTypes<MSDA_F16_AUX16> { using VT = __half; using AT = __half; };
+
+// The tag sets a kernel family is instantiated for
+template <int... Tags>
+struct TagList {};
+using FastTags = TagList<MSDA_F32, MSDA_BF16, MSDA_F16>;                                     // fast kernels (fast_ok)
+using FusedTags = TagList<MSDA_F32, MSDA_BF16, MSDA_F16, MSDA_BF16_AUX16, MSDA_F16_AUX16>;   // + 16-bit offsets / logits
+using ValueTags = TagList<MSDA_F32, MSDA_F64, MSDA_BF16, MSDA_F16>;                          // generic kernels
+using AllTags = TagList<MSDA_F32, MSDA_F64, MSDA_BF16, MSDA_F16, MSDA_BF16_AUX16, MSDA_F16_AUX16>;
+
+template <int... Tags, typename F>
+int with_types_in(TagList<Tags...>, int tag, F& f) {
+  int r = MSDA_OK;
+  if (((tag == Tags && (r = f(TagTypes<Tags>{}), true)) || ...)) return r;
+  return fail(MSDA_ERR_UNSUPPORTED, "no kernel for dtype tag %d", tag);
+}
+// Calls f(TagTypes<tag>{}) for a tag of the set List.
+template <typename List, typename F>
+int with_types(int tag, F&& f) {
+  return with_types_in(List{}, tag, f);
+}
+
+// Calls f(Int<D>{}) for the channel chunk D of the fast kernels, 16, 32, 64 or 128.
+template <typename F>
+int with_chunk(int D, F&& f) {
+  switch (D) {
+    case 16: return f(Int<16>{});
+    case 32: return f(Int<32>{});
+    case 64: return f(Int<64>{});
+    case 128: return f(Int<128>{});
+    default: return fail(MSDA_ERR_UNSUPPORTED, "no fast kernel for D=%d", D);
+  }
+}
 
 inline int grid_for(int64_t work_items, int threads, int cap_blocks) {
   int64_t g = (work_items + threads - 1) / threads;
@@ -132,11 +195,11 @@ struct Dcn2Dims {
   int64_t n_input() const { return (int64_t)B * H * W * C; }
   int64_t n_columns() const { return (int64_t)B * Ho * Wo * K() * C; }
 };
-// value dtype MSDA_F32 / F64 / BF16 / F16, aux16: offset / mask and their gradients in the value's 16-bit type.
+// dtype: any tag; MSDA_*_AUX16: offset / mask and their gradients in the value's 16-bit type.
 // grad_input_acc: float [B,H,W,C] (double for MSDA_F64), zeroed by the caller; the kernels add into it.
-int dcnv2_im2col(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsigned flags, const void* input,
-                 const void* offset, const void* mask, void* columns);
-int dcnv2_col2im(cudaStream_t st, const Dcn2Dims& g, int dtype, bool aux16, unsigned flags, const void* grad_columns,
+int dcnv2_im2col(cudaStream_t st, const Dcn2Dims& g, int dtype, unsigned flags, const void* input, const void* offset,
+                 const void* mask, void* columns);
+int dcnv2_col2im(cudaStream_t st, const Dcn2Dims& g, int dtype, unsigned flags, const void* grad_columns,
                  const void* input, const void* offset, const void* mask, void* grad_input_acc, void* grad_offset,
                  void* grad_mask);
 
