@@ -49,7 +49,7 @@ __device__ __forceinline__ void load_cell_tab(CellTab* t, const int64_t* shapes,
       t->W[l] = (int)shapes[2 * l + 1];
       t->start[l] = (int)lsi[l];
       t->cell_begin[l] = acc;
-      acc += (t->H[l] + 1) * (t->W[l] + 1);
+      acc += level_cells(t->H[l], t->W[l]);
     }
     t->cells_per_bh = acc;
   }
@@ -60,7 +60,8 @@ __device__ __forceinline__ void load_cell_tab(CellTab* t, const int64_t* shapes,
 // cfg 3 (1.4 points per pixel-head) 0.60 vs 0.81 ms, cfg 2 (16) 3.31 vs 3.02 ms, cfg 5 (39) 8.26 vs 5.65 ms
 constexpr int kDetDenseRatio = 4;
 
-// upper bound of bins per (image, head) that needs only S and L: (H+1)(W+1) <= 2HW + 2
+// upper bound of bins per (image, head) that needs only S and L: (H+1)(W+1) <= 2HW + 2 for H, W >= 1, and an empty
+// level owns no bins (level_cells)
 __host__ __device__ constexpr int64_t det_cells_bound(int64_t S, int64_t L) { return 2 * S + 2 * L; }
 
 // Division of a 31-bit unsigned by a run-time constant as multiply-high + shift (Granlund-Montgomery, the round-up

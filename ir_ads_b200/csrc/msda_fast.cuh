@@ -318,6 +318,12 @@ __device__ __forceinline__ void load_levels(LevelTab* tab, const int64_t* shapes
   __syncthreads();
 }
 
+// Bins one level owns on the deterministic sorted path: the cells of its extended (H+1) x (W+1) grid.  An empty level
+// (H or W <= 0) holds no valid point, so it owns none -- (H+1)(W+1) would add W+1 or H+1 bins without adding to S and
+// break det_cells_bound (msda_det.cuh).  Every table of that path (load_cell_tab, load_levels_plain<true>,
+// set_single_level<..., true>) sums this.
+__host__ __device__ __forceinline__ int level_cells(int H, int W) { return (H > 0 && W > 0) ? (H + 1) * (W + 1) : 0; }
+
 // LINEAR / STRIP orders need no tile table: one barrier, no serial section.  CELLS: also the bin table of the
 // deterministic sorted path (cells of the extended (H+1) x (W+1) grids, msda_det.cuh) -- thread l sums its own prefix.
 template <bool CELLS = false>
@@ -328,10 +334,10 @@ __device__ __forceinline__ void load_levels_plain(LevelTab* tab, const int64_t* 
     tab->start[threadIdx.x] = (int)lsi[threadIdx.x];
     if constexpr (CELLS) {
       int acc = 0;
-      for (int k = 0; k < (int)threadIdx.x; ++k) acc += ((int)shapes[2 * k] + 1) * ((int)shapes[2 * k + 1] + 1);
+      for (int k = 0; k < (int)threadIdx.x; ++k) acc += level_cells((int)shapes[2 * k], (int)shapes[2 * k + 1]);
       tab->cell_begin[threadIdx.x] = acc;
       if ((int)threadIdx.x == L - 1)
-        tab->cells_per_bh = acc + ((int)shapes[2 * threadIdx.x] + 1) * ((int)shapes[2 * threadIdx.x + 1] + 1);
+        tab->cells_per_bh = acc + level_cells((int)shapes[2 * threadIdx.x], (int)shapes[2 * threadIdx.x + 1]);
     }
   }
   __syncthreads();
@@ -368,7 +374,7 @@ __device__ __forceinline__ void set_single_level(LevelTab* tab, int H, int W) {
     tab->total_tiles = tab->tiles_x[0] * ((H + TH - 1) / TH);
     if constexpr (CELLS) {
       tab->cell_begin[0] = 0;
-      tab->cells_per_bh = (H + 1) * (W + 1);
+      tab->cells_per_bh = level_cells(H, W);
     }
   }
   __syncthreads();

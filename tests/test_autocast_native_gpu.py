@@ -395,7 +395,8 @@ def _close(got, exp, tol, what):
 
 @pytest.mark.parametrize("swap", [False, True])
 @pytest.mark.parametrize("dtype", HALVES)
-@pytest.mark.parametrize("rows,C", [((7, 33), 256), ((5000,), 64), ((3, 5), 100), ((2, 9), 1024), ((0,), 256)])
+@pytest.mark.parametrize("rows,C", [((7, 33), 256), ((5000,), 64), ((3, 5), 100), ((2, 9), 1024), ((0,), 256),
+                                    ((100000,), 256), ((3, 7), 200), ((5, 3), 516), ((9,), 772), ((4, 4), 1020)])
 def test_mixed_epilogue(rows, C, dtype, swap):
     from ir_ads_b200.epilogue import add_layer_norm
     torch.manual_seed(C)
@@ -426,7 +427,8 @@ def test_mixed_epilogue(rows, C, dtype, swap):
         _close(got, exp, 1e-5, what)
 
 
-@pytest.mark.parametrize("rows,C", [((7, 33), 256), ((5000,), 64), ((2, 9), 1024)])
+@pytest.mark.parametrize("rows,C", [((7, 33), 256), ((5000,), 64), ((2, 9), 1024), ((100000,), 256), ((3, 7), 200),
+                                    ((5, 3), 516), ((9,), 772), ((4, 4), 1020)])
 def test_f16_epilogue(rows, C):
     from ir_ads_b200.epilogue import AddLayerNormFunction
     torch.manual_seed(C)

@@ -71,16 +71,17 @@ def snap(off, kernel, stride, padding, dilation):
     return torch.stack((y, x), 3).view(off.shape)
 
 
-def oracle(case, go):
-    """torchvision in float64 on the CPU, at the kernels' float32 sampling positions: (out, {name: grad})."""
-    t = {n: (None if case[n] is None else case[n].detach().double().requires_grad_(True))
+def oracle(case, go, device="cpu"):
+    """torchvision in float64 (on the CPU unless `device` says otherwise), at the kernels' float32 sampling positions:
+    (out, {name: grad})."""
+    t = {n: (None if case[n] is None else case[n].detach().double().to(device).requires_grad_(True))
          for n in ("x", "off", "m", "w", "b")}
     kernel = tuple(case["w"].shape[2:])
     stride = case["stride"]
-    t["off"] = snap(case["off"], kernel, stride, case["padding"], case["dilation"]).requires_grad_(True)
+    t["off"] = snap(case["off"], kernel, stride, case["padding"], case["dilation"]).to(device).requires_grad_(True)
     out = tv_ops.deform_conv2d(t["x"], t["off"], t["w"], t["b"], stride=case["stride"], padding=case["padding"],
                                dilation=case["dilation"], mask=t["m"])
-    out.backward(go.double())
+    out.backward(go.double().to(device))
     return out.detach(), {n: t[n].grad for n in t if t[n] is not None}
 
 
@@ -232,6 +233,37 @@ def test_chunks_of_images_match_one_chunk():
         assert torch.equal(a[n], b[n])
     # grad_weight: one GEMM against per-chunk GEMMs summed; grad_input: float reds
     assert torch.allclose(a["w"], b["w"], rtol=1e-4, atol=1e-4) and torch.allclose(a["x"], b["x"], rtol=1e-5, atol=1e-5)
+
+
+@pytest.mark.parametrize("B", [65535, 65536])
+def test_batch_at_the_grid_y_limit(B):
+    """The fast im2col / col2im launches put the images of a chunk on grid.y, so they take at most 65535; a larger chunk
+    (im2col_step >= B hands the whole batch to one launch) goes to the generic kernels.  Both sides of that gate against
+    torchvision in float64 (on the GPU: 65536 tiny images).  At 65535 the offset gradients differ in their bits from the
+    generic kernels' (another summation order: the fast kernels ran); at 65536 both runs are the generic kernels."""
+    case = make(B, 16, 5, 5, 16, 3, 1, 1, 1, 1, 1, True, True, leave=True, seed=13)
+    go = torch.randn(case["out_shape"], generator=torch.Generator().manual_seed(7))
+    ref_out, ref_g = oracle(case, go, DEV)
+    # 3.3 million sampling positions: a few lie within float32 rounding of an integer, where the offset gradient jumps
+    # and either one-sided derivative is right -- those offsets are left out of the grad_offset comparison
+    s = snap(case["off"], (3, 3), 1, case["padding"], 1)
+    smooth = ((s - s.round()).abs() > 1e-4).view(B, 9, 2, 5, 5).all(2, keepdim=True).expand(B, 9, 2, 5, 5)
+    ref_g["off"] = ref_g["off"].cpu() * smooth.reshape(s.shape)
+    res = {}
+    for flags in (0, _lib.FLAG_FORCE_GENERIC):
+        n0 = _lib.launch_count()
+        with kernel_flags(flags):
+            out, g = ours(case, go, step=B)
+        assert _lib.launch_count() > n0
+        errs = {"out": nerr(out, ref_out)}
+        errs.update({n: nerr(g[n].cpu() * smooth.reshape(s.shape) if n == "off" else g[n], ref_g[n]) for n in ref_g})
+        assert all(e < 5e-5 for e in errs.values()), (flags, errs)
+        res[flags] = (out, g)
+    (out, g), (gout, gg) = res[0], res[_lib.FLAG_FORCE_GENERIC]
+    if B <= 65535:
+        assert not torch.equal(g["off"], gg["off"])
+    else:
+        assert torch.equal(out, gout) and torch.equal(g["off"], gg["off"]) and torch.equal(g["m"], gg["m"])
 
 
 def test_deterministic_mode_raises_and_warns():

@@ -10,8 +10,11 @@ DEV = "cuda:0"
 
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
+# 100 000 rows: more than the 148 * 8 CTAs of 8 warps (9472 rows), so every warp loops over rows and carries its
+# dgamma / dbeta partials; C = 200, 516, 772, 1020: the two- and eight-wide vector widths with predicated tail chunks
 @pytest.mark.parametrize("rows,C", [((7, 33), 256), ((1,), 4), ((5000,), 64), ((3, 5), 100), ((2, 9), 1024), ((11,), 384),
-                                    ((0,), 256)])
+                                    ((0,), 256), ((100000,), 256), ((3, 7), 200), ((5, 3), 516), ((9,), 772),
+                                    ((4, 4), 1020)])
 def test_add_layer_norm_matches_torch_fp64(rows, C, dtype):
     from ir_ads_b200.epilogue import AddLayerNormFunction
     torch.manual_seed(C + len(rows))
