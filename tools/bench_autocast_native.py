@@ -17,25 +17,24 @@ import argparse
 import contextlib
 import json
 import os
-import statistics
 import sys
+from functools import partial
 
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tools"))
 import ir_ads_b200.dcnv3 as dcnv3_mod  # noqa: E402
 import ir_ads_b200.encoder as encoder_mod  # noqa: E402
 import ir_ads_b200.module as module_mod  # noqa: E402
-from bench_dcnv3_fused import SHAPES as DCN_SHAPES, card  # noqa: E402
+from bench_dcnv3_fused import SHAPES as DCN_SHAPES  # noqa: E402
 from ir_ads_b200 import MultiScaleDeformableAttention  # noqa: E402
 from ir_ads_b200.encoder import DeformableEncoderLayer  # noqa: E402
 from ir_ads_b200.epilogue import AddLayerNormFunction  # noqa: E402
 from ir_ads_b200.workloads import LEVELS, _pixel_centres, level_tensors  # noqa: E402
+from timing import card, rotations, timed  # noqa: E402
 
 DEV = "cuda:0"
-L2_BYTES = 126 * 2 ** 20
 
 
 class _Widened:
@@ -79,21 +78,8 @@ def measure(fwd, xs, gos, params, dtype, iters, warmup):
                 out = fwd(xs[i])
             torch.autograd.grad(out, [xs[i]] + params, gos[i].to(out.dtype))
 
-    n = len(xs)
-    for i in range(warmup):
-        for r in routes:
-            step(r, i % n)
-    torch.cuda.synchronize()
-    times = {r: [] for r in routes}
-    for i in range(iters):
-        for r in routes:
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            step(r, i % n)
-            e1.record()
-            torch.cuda.synchronize()
-            times[r].append(e0.elapsed_time(e1))
-    ms = {r: round(statistics.median(v), 4) for r, v in times.items()}
+    t = timed({r: [(partial(step, r, i),) for i in range(len(xs))] for r in routes}, iters, warmup)
+    ms = {r: v for r, (v,) in t.items()}
     peak, kernels = {}, {}
     for r in routes:
         torch.cuda.synchronize()
@@ -124,7 +110,7 @@ def msda_module(dtype, iters, warmup):
         m.sampling_offsets.weight.normal_(0, 0.05)
         m.attention_weights.weight.normal_(0, 0.2)
     ref = _pixel_centres(levels, DEV)[None, :, None, :].expand(B, S, 4, 2).contiguous()
-    n = max(1, min(3, -(-3 * L2_BYTES // (B * S * 256 * 4 * 2))))
+    n = rotations(B * S * 256 * 4 * 2, 1, 3)
     xs = [torch.randn(B, S, 256, device=DEV).requires_grad_(True) for _ in range(n)]
     gos = [torch.randn(B, S, 256, device=DEV) for _ in range(n)]
     fwd = lambda x: m(x, reference_points=ref, spatial_shapes=shapes, level_start_index=lsi, level_shapes=levels)
@@ -142,7 +128,7 @@ def encoder_layer(dtype, iters, warmup):
         layer.attentions[0].attention_weights.weight.normal_(0, 0.2)
     ref = _pixel_centres(levels, DEV)[None, :, None, :].expand(B, S, 4, 2).contiguous()
     pos = torch.randn(B, S, 256, device=DEV) * 0.1
-    n = max(1, min(3, -(-3 * L2_BYTES // (B * S * 256 * 4 * 2))))
+    n = rotations(B * S * 256 * 4 * 2, 1, 3)
     xs = [torch.randn(B, S, 256, device=DEV).requires_grad_(True) for _ in range(n)]
     gos = [torch.randn(B, S, 256, device=DEV) for _ in range(n)]
     fwd = lambda x: layer(x, query_pos=pos, reference_points=ref, spatial_shapes=shapes, level_start_index=lsi,
@@ -158,7 +144,7 @@ def dcn_module(shape, dtype, iters, warmup):
         for lin in (m.offset, m.mask):
             lin.weight.normal_(0.0, 0.2)
             lin.bias.normal_(0.0, 1.0)
-    n = max(1, min(4, -(-3 * L2_BYTES // (N * H * W * G * C * 4 * 2))))
+    n = rotations(N * H * W * G * C * 4 * 2, 1, 4)
     xs = [torch.randn(N, H, W, G * C, device=DEV).requires_grad_(True) for _ in range(n)]
     gos = [torch.randn(N, H, W, G * C, device=DEV) for _ in range(n)]
     return measure(m, xs, gos, list(m.parameters()), dtype, iters, warmup)

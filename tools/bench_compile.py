@@ -3,8 +3,8 @@
 Workloads: cfg2 (DINO-R50 levels at 800x1333, B=8) and cfg4 (VOC-shape levels, B=2), unpadded, float32 and bf16
 autocast, fused add + LayerNorm epilogues on.  The three variants are compiled and warmed up first, then timed in
 alternating rounds in one process; every timed pass reads one of several input sets, together larger than the 126 MB
-L2.  Times are CUDA-event medians of whole steps (forward, backward, gradient accumulation).  One JSON line per
-(workload, dtype, variant), the card's name and power limit in each.
+L2.  Times are CUDA-event medians of whole steps (forward, backward, gradient accumulation).  The first JSON line names
+the card, its power limit and maximum SM clock, then one per (workload, dtype, variant).
 
   python tools/bench_compile.py [--iters 20] [--warmup 3] [--rounds 3] [--out FILE]
 """
@@ -14,7 +14,6 @@ import argparse
 import json
 import os
 import statistics
-import subprocess
 import sys
 
 import torch
@@ -22,16 +21,11 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ir_ads_b200.encoder import DeformableEncoder, get_reference_points  # noqa: E402
 from ir_ads_b200.workloads import LEVELS  # noqa: E402
+from timing import card  # noqa: E402
 
 C, HEADS = 256, 8
 DEV = torch.device("cuda")
 WORKLOADS = {"cfg2": ("dino_r50", 8), "cfg4": ("voc", 2)}
-
-
-def card():
-    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
-                         capture_output=True, text=True).stdout.strip().splitlines()
-    return out[0] if out else torch.cuda.get_device_name()
 
 
 def inputs(levels, batch, n_sets, gen):
@@ -51,8 +45,8 @@ def main():
     ap.add_argument("--workloads", default="cfg2,cfg4")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    gpu = card()
-    lines = []
+    lines = [card()]
+    print(json.dumps(lines[0]), flush=True)
     for name in args.workloads.split(","):
         level_key, batch = WORKLOADS[name]
         levels = [tuple(x) for x in LEVELS[level_key]]
@@ -109,7 +103,7 @@ def main():
                 med = statistics.median(t)
                 rec = {"workload": name, "batch": batch, "dtype": dtype, "variant": k, "median_ms": round(med, 3),
                        "p10_ms": round(sorted(t)[len(t) // 10], 3), "p90_ms": round(sorted(t)[len(t) * 9 // 10], 3),
-                       "speedup_vs_eager": round(base / med, 3), "samples": len(t), "gpu": gpu}
+                       "speedup_vs_eager": round(base / med, 3), "samples": len(t)}
                 print(json.dumps(rec), flush=True)
                 lines.append(rec)
             for p in enc.parameters():

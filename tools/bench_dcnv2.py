@@ -15,9 +15,8 @@ times each piece alone, on the same shapes.  Prints the card name and power limi
 import argparse
 import json
 import os
-import statistics
-import subprocess
 import sys
+from functools import partial
 
 import torch
 
@@ -25,38 +24,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from ir_ads_b200 import _lib, modulated_deform_conv  # noqa: E402
 from ir_ads_b200 import dcnv2 as _dcnv2  # noqa: E402
+from timing import card, rotations, timed  # noqa: E402
 
 # (name, C, H_in, W_in, stride)
 SHAPES = (("res3_s2", 128, 200, 334, 2), ("res3", 128, 100, 167, 1), ("res4", 256, 50, 84, 1), ("res5", 512, 25, 42, 1))
-L2_BYTES = 126 * 2 ** 20
-
-
-def card():
-    name = torch.cuda.get_device_name(0)
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
-                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
-    except (OSError, subprocess.SubprocessError, IndexError):
-        q = "unknown"
-    return {"device": name, "power_limit_and_max_sm_clock": q}
-
-
-def alternate(fns, iters, warmup, n_rot):
-    """median ms per call of every fn(i) (i = rotation index), the fns alternated call by call"""
-    for i in range(warmup):
-        for f in fns.values():
-            f(i % n_rot)
-    torch.cuda.synchronize()
-    times = {k: [] for k in fns}
-    for i in range(iters):
-        for k, f in fns.items():
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            f(i % n_rot)
-            e1.record()
-            torch.cuda.synchronize()
-            times[k].append(e0.elapsed_time(e1))
-    return {k: round(statistics.median(v), 4) for k, v in times.items()}
 
 
 def torchvision_status():
@@ -89,7 +60,7 @@ def make_sets(B, C, H, W, s, n_rot, dev):
 def bench_shape(name, C, H, W, s, B, amp, tv_ok, iters, warmup):
     dev = "cuda:0"
     set_bytes = B * C * H * W * 4 * 2
-    n_rot = max(2, min(8, -(-3 * L2_BYTES // set_bytes)))
+    n_rot = rotations(set_bytes, 2, 8)
     sets, Ho, Wo = make_sets(B, C, H, W, s, n_rot, dev)
     torch.manual_seed(0)
     w = (torch.randn(C, C, 3, 3, device=dev) / (9 * C) ** 0.5).requires_grad_(True)
@@ -126,9 +97,10 @@ def bench_shape(name, C, H, W, s, B, amp, tv_ok, iters, warmup):
     row = {"shape": name, "B": B, "C": C, "in": [H, W], "out": [Ho, Wo], "stride": s,
            "dtype": "bf16_autocast" if amp else "f32", "rotated_sets": n_rot,
            "gflop_fwd": round(2 * B * Ho * Wo * 9 * C * C / 1e9, 3)}
-    with torch.no_grad():
-        row["fwd_ms"] = alternate({k: (lambda i, f=f: f(i, False)) for k, f in arms.items()}, iters, warmup, n_rot)
-    row["fwd_bwd_ms"] = alternate({k: (lambda i, f=f: f(i, True)) for k, f in arms.items()}, iters, warmup, n_rot)
+    for key, bwd in (("fwd_ms", False), ("fwd_bwd_ms", True)):
+        with torch.set_grad_enabled(bwd):
+            t = timed({k: [(partial(f, i, bwd),) for i in range(n_rot)] for k, f in arms.items()}, iters, warmup)
+        row[key] = {k: ms for k, (ms,) in t.items()}
     for key in ("fwd_ms", "fwd_bwd_ms"):
         t = row[key]
         row[key.replace("_ms", "_ours_vs")] = {k: round(t[k] / t["ours"], 3) for k in t if k != "ours"}
@@ -177,7 +149,8 @@ def split(cl, w, B, C, H, W, s, dt, iters, warmup, n_rot):
     fns = {"im2col": im2col, "col2im": col2im,
            "gemm_fwd": lambda i: torch.mm(cols, wm.t()),
            "gemm_bwd": lambda i: (torch.mm(go, wm), torch.mm(go.t(), cols))}
-    return alternate(fns, iters, warmup, n_rot)
+    t = timed({k: [(partial(f, i),) for i in range(n_rot)] for k, f in fns.items()}, iters, warmup)
+    return {k: ms for k, (ms,) in t.items()}
 
 
 def main():
@@ -186,7 +159,6 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--batches", default="2,8")
     a = ap.parse_args()
-    assert torch.cuda.is_available(), "bench_dcnv2 measures on a CUDA device"
     info = card()
     reason = torchvision_status()
     info["torchvision_cuda_deform_conv2d"] = "runs" if reason is None else f"left out: {reason}"

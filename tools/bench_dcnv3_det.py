@@ -6,27 +6,17 @@ name and power limit first, then one JSON line per shape (and dtype)."""
 import argparse
 import json
 import os
-import statistics
-import subprocess
 import sys
+from functools import partial
 
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from ir_ads_b200 import _lib, dcnv3_backward, functional  # noqa: E402
+from timing import card, timed  # noqa: E402
 
 SHAPES = ((16, 200, 336, 4, 16), (16, 100, 168, 8, 16), (16, 50, 84, 16, 16), (16, 25, 42, 32, 16), (8, 100, 168, 8, 32))
-
-
-def card():
-    name = torch.cuda.get_device_name(0)
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
-                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
-    except (OSError, subprocess.SubprocessError, IndexError):
-        q = "unknown"
-    return {"device": name, "power_limit_and_max_sm_clock": q}
 
 
 def main():
@@ -52,24 +42,11 @@ def main():
                     return dcnv3_backward(inp, off, mask, *args, go)
 
             modes = {"default": 0, "deterministic": _lib.FLAG_DETERMINISTIC}
-            for _ in range(a.warmup):
-                for f in modes.values():
-                    call(f)
-            torch.cuda.synchronize()
-            times = {k: [] for k in modes}
-            for _ in range(a.iters):
-                for k, f in modes.items():
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record()
-                    call(f)
-                    e1.record()
-                    torch.cuda.synchronize()
-                    times[k].append(e0.elapsed_time(e1))
+            t = timed({k: [(partial(call, f),)] for k, f in modes.items()}, a.iters, a.warmup)
             # the two routes agree to float-summation accuracy (and the deterministic one with itself, bit for bit)
             d0, d1, d2 = call(0)[0].float(), call(modes["deterministic"])[0], call(modes["deterministic"])[0]
             row = {"shape": [N, H, W, G, C], "dtype": dname, "points": N * H * W * G * 9, "iters": a.iters,
-                   "default_bwd_ms": round(statistics.median(times["default"]), 4),
-                   "det_bwd_ms": round(statistics.median(times["deterministic"]), 4),
+                   "default_bwd_ms": t["default"][0], "det_bwd_ms": t["deterministic"][0],
                    "det_reproducible": bool(torch.equal(d1, d2)),
                    "det_vs_default_max_rel": float((d1.float() - d0).abs().max() / d0.abs().max().clamp_min(1e-30))}
             row["det_over_default"] = round(row["det_bwd_ms"] / row["default_bwd_ms"], 3)

@@ -11,9 +11,8 @@ shape:
 import argparse
 import json
 import os
-import statistics
-import subprocess
 import sys
+from functools import partial
 
 import torch
 
@@ -21,19 +20,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from ir_ads_b200 import DCNv3Function, DCNv3FusedFunction  # noqa: E402
 from ir_ads_b200.dcnv3 import DCNv3  # noqa: E402
+from timing import card, rotations, timed  # noqa: E402
 
 SHAPES = ((16, 200, 336, 4, 16), (16, 100, 168, 8, 16), (16, 50, 84, 16, 16), (16, 25, 42, 32, 16), (8, 100, 168, 8, 32))
-L2_BYTES = 126 * 2 ** 20
-
-
-def card():
-    name = torch.cuda.get_device_name(0)
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
-                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
-    except (OSError, subprocess.SubprocessError, IndexError):
-        q = "unknown"
-    return {"device": name, "power_limit_and_max_sm_clock": q}
 
 
 def softmax_rows(logits, G):
@@ -54,29 +43,11 @@ def composed_forward(m, input):
     return m.output_proj(x)
 
 
-def alternate(fns, iters, warmup, n_rot):
-    """median ms per call of every fn(i) (i = rotation index), the fns alternated call by call"""
-    for i in range(warmup):
-        for f in fns.values():
-            f(i % n_rot)
-    torch.cuda.synchronize()
-    times = {k: [] for k in fns}
-    for i in range(iters):
-        for k, f in fns.items():
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            f(i % n_rot)
-            e1.record()
-            torch.cuda.synchronize()
-            times[k].append(e0.elapsed_time(e1))
-    return {k: round(statistics.median(v), 4) for k, v in times.items()}
-
-
 def core(N, H, W, G, C, iters, warmup):
     dev = "cuda:0"
     K, args = 9, (3, 3, 1, 1, 1, 1, 1, 1, G, C, 1.0)
     set_bytes = N * H * W * (G * C * 4 * 2 + G * K * 3 * 4)
-    n_rot = max(1, min(8, -(-3 * L2_BYTES // set_bytes)))
+    n_rot = rotations(set_bytes, 1, 8)
     g = torch.Generator(device=dev).manual_seed(0)
     sets = []
     for _ in range(n_rot):
@@ -86,14 +57,15 @@ def core(N, H, W, G, C, iters, warmup):
         go = torch.randn(N, H, W, G * C, device=dev, generator=g)
         sets.append((inp, off, lg, go))
     with torch.no_grad():
-        fwd = alternate({
-            "fused": lambda i: DCNv3FusedFunction.apply(*sets[i][:3], *args, 256),
-            "unfused": lambda i: DCNv3Function.apply(sets[i][0], sets[i][1], softmax_rows(sets[i][2], G), *args, 256),
-        }, iters, warmup, n_rot)
+        fwd = {k: t for k, (t,) in timed({
+            "fused": [(partial(DCNv3FusedFunction.apply, *s[:3], *args, 256),) for s in sets],
+            "unfused": [(lambda s=s: DCNv3Function.apply(s[0], s[1], softmax_rows(s[2], G), *args, 256),)
+                        for s in sets],
+        }, iters, warmup).items()}
     outs = {"fused": [DCNv3FusedFunction.apply(*s[:3], *args, 256) for s in sets],
             "unfused": [DCNv3Function.apply(s[0], s[1], softmax_rows(s[2], G), *args, 256) for s in sets]}
-    bwd = alternate({k: (lambda i, k=k: torch.autograd.grad(outs[k][i], sets[i][:3], sets[i][3], retain_graph=True))
-                     for k in outs}, iters, warmup, n_rot)
+    bwd = {k: t for k, (t,) in timed({k: [(partial(torch.autograd.grad, o, s[:3], s[3], retain_graph=True),)
+                                             for o, s in zip(outs[k], sets)] for k in outs}, iters, warmup).items()}
     a = torch.autograd.grad(outs["fused"][0], sets[0][:3], sets[0][3], retain_graph=True)
     b = torch.autograd.grad(outs["unfused"][0], sets[0][:3], sets[0][3], retain_graph=True)
     rel = {k: float((x - y).abs().max() / y.abs().max().clamp_min(1e-30))
@@ -115,7 +87,7 @@ def module(N, H, W, G, C, iters, warmup, amp):
             lin.weight.normal_(0.0, 0.2)
             lin.bias.normal_(0.0, 1.0)
     set_bytes = N * H * W * G * C * 4 * 2
-    n_rot = max(1, min(4, -(-3 * L2_BYTES // set_bytes)))
+    n_rot = rotations(set_bytes, 1, 4)
     g = torch.Generator(device=dev).manual_seed(1)
     xs = [torch.randn(N, H, W, G * C, device=dev, generator=g).requires_grad_(True) for _ in range(n_rot)]
     gos = [torch.randn(N, H, W, G * C, device=dev, generator=g) for _ in range(n_rot)]
@@ -127,7 +99,8 @@ def module(N, H, W, G, C, iters, warmup, amp):
             out = fwds[k](xs[i])
         torch.autograd.grad(out, [xs[i]] + params, gos[i].to(out.dtype))
 
-    ms = alternate({k: (lambda i, k=k: step(k, i)) for k in fwds}, iters, warmup, n_rot)
+    ms = {k: t for k, (t,) in timed({k: [(partial(step, k, i),) for i in range(n_rot)] for k in fwds}, iters,
+                                    warmup).items()}
     peak = {}
     for k in fwds:
         torch.cuda.synchronize()

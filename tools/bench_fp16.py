@@ -14,8 +14,6 @@ import copy
 import ctypes
 import json
 import os
-import statistics
-import subprocess
 import sys
 
 import torch
@@ -25,15 +23,10 @@ sys.path.insert(0, ROOT)
 from ir_ads_b200 import MultiScaleDeformableAttention, _lib, dcnv3_backward, dcnv3_forward  # noqa: E402
 from ir_ads_b200.functional import _VALUE_TAG, MSDeformAttnFusedFunction  # noqa: E402
 from ir_ads_b200.workloads import LEVELS, WORKLOADS, level_tensors, make_workload_inputs  # noqa: E402
+from timing import card, timed  # noqa: E402
 
 DEV = "cuda:0"
 DTYPES = {"f32": torch.float32, "bf16": torch.bfloat16, "f16": torch.float16}
-
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    return {"device": torch.cuda.get_device_name(0), "nvidia_smi": q.stdout.strip().splitlines()[:1]}
 
 
 def _p(t):
@@ -69,24 +62,6 @@ class PlainOp:
                                             _p(self.ws), self.ws_bytes, self.tag, self.flags), "msda_backward")
 
 
-def timed(fns, iters, warmup=3):
-    """fns: {name: [callables of one iteration, one per rotating set]} -> {name: [median ms per stage]}; every
-    iteration runs each name once, in a fixed alternation."""
-    times = {k: [] for k in fns}
-    for it in range(iters + warmup):
-        for name, per_set in fns.items():
-            stages = per_set[it % len(per_set)]
-            ev = [torch.cuda.Event(enable_timing=True) for _ in range(len(stages) + 1)]
-            ev[0].record()
-            for i, stage in enumerate(stages):
-                stage()
-                ev[i + 1].record()
-            torch.cuda.synchronize()
-            if it >= warmup:
-                times[name].append([ev[i].elapsed_time(ev[i + 1]) for i in range(len(stages))])
-    return {k: [round(statistics.median(t[i] for t in v), 4) for i in range(len(v[0]))] for k, v in times.items()}
-
-
 def bench_op(iters):
     rows = []
     for cfg, det in (("cfg2", False), ("cfg3_f32", False), ("cfg5", True)):
@@ -98,7 +73,7 @@ def bench_op(iters):
             go = torch.randn(wl.batch, wl.queries, wl.num_heads * wl.head_dim, device=DEV)
             sets.append((value, shapes, lsi, loc, w, go))
         ops = {dt: [PlainOp(s, DTYPES[dt], flags) for s in sets] for dt in DTYPES}
-        res = timed({dt: [(o.fwd, o.bwd) for o in ops[dt]] for dt in DTYPES}, iters)
+        res = timed({dt: [(o.fwd, o.bwd) for o in ops[dt]] for dt in DTYPES}, iters, 3)
         for dt, (f, b) in res.items():
             rows.append({"section": "op", "workload": cfg.replace("_f32", ""), "det": det, "value": dt,
                          "fwd_ms": f, "bwd_ms": b})
@@ -143,7 +118,7 @@ def bench_module(iters, batch=8):
         return fwd, bwd
 
     res = timed({"fp16_native": [step(new, i) for i in range(3)], "fp16_widened": [step(old, i) for i in range(3)]},
-                iters)
+                iters, 3)
     return [{"section": "module", "shape": "encoder", "batch": batch, "route": k, "fwd_ms": f, "bwd_ms": b}
             for k, (f, b) in res.items()]
 
@@ -165,7 +140,7 @@ def bench_dcnv3(iters):
             inp, off, mask, go = s[0].to(dt), s[1], s[2], s[3].to(dt)
             return (lambda: dcnv3_forward(inp, off, mask, *args), lambda: dcnv3_backward(inp, off, mask, *args, go))
 
-        res = timed({dt: [stages(s, DTYPES[dt]) for s in sets] for dt in ("f32", "f16")}, iters)
+        res = timed({dt: [stages(s, DTYPES[dt]) for s in sets] for dt in ("f32", "f16")}, iters, 3)
         for dt, (f, b) in res.items():
             rows.append({"section": "dcnv3", "shape": [N, H, W, G, C], "input": dt, "fwd_ms": f, "bwd_ms": b})
     return rows

@@ -5,8 +5,8 @@ Usage: python tools/bench_layer.py [--batch 8] [--iters 10]"""
 import argparse
 import json
 import os
-import statistics
 import sys
+from functools import partial
 
 import torch
 
@@ -14,6 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from ir_ads_b200.encoder import DeformableEncoderLayer  # noqa: E402
 from ir_ads_b200.workloads import LEVELS, _pixel_centres, level_tensors  # noqa: E402
+from timing import card, timed  # noqa: E402
 
 
 def run(batch, iters, fused, amp, dev="cuda:0"):
@@ -27,20 +28,13 @@ def run(batch, iters, fused, amp, dev="cuda:0"):
     sets = [(torch.randn(batch, S, 256, device=dev, requires_grad=True), torch.randn(batch, S, 256, device=dev) * 0.1,
              torch.randn(batch, S, 256, device=dev)) for _ in range(3)]
     ctx = torch.autocast("cuda", dtype=torch.bfloat16) if amp else torch.autocast("cuda", enabled=False)
-    times = []
-    for it in range(iters + 3):
-        x, pos, go = sets[it % 3]
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
+
+    def step(x, pos, go):
         with ctx:
             out = layer(x, query_pos=pos, reference_points=ref, spatial_shapes=shapes, level_start_index=lsi,
                         level_shapes=levels)
         out.backward(go.to(out.dtype))
-        e1.record()
-        torch.cuda.synchronize()
-        if it >= 3:
-            times.append(e0.elapsed_time(e1))
-    return statistics.median(times)
+    return timed({"layer": [(partial(step, *s),) for s in sets]}, iters, 3)["layer"][0]
 
 
 def main():
@@ -48,6 +42,7 @@ def main():
     ap.add_argument("--batch", type=int, default=8)
     ap.add_argument("--iters", type=int, default=10)
     a = ap.parse_args()
+    print(json.dumps(card()), flush=True)
     res = {"what": "DeformableEncoderLayer fwd+bwd, DINO-R50 800x1333 encoder shape, ms (median)", "batch": a.batch}
     for amp in (False, True):
         for fused in (True, False):

@@ -8,6 +8,7 @@ import json
 import os
 import statistics
 import sys
+from functools import partial
 
 import torch
 
@@ -16,6 +17,7 @@ sys.path.insert(0, ROOT)
 from ir_ads_b200 import MultiScaleDeformableAttention  # noqa: E402
 from ir_ads_b200 import module as msda_module  # noqa: E402
 from ir_ads_b200.workloads import LEVELS, level_tensors  # noqa: E402
+from timing import card, timed  # noqa: E402
 
 
 class RefKernelFunction(torch.autograd.Function):
@@ -67,25 +69,21 @@ def run(kind, batch, iters, mode, dev="cuda:0", amp=None, masked=False):
                 mm[:, (9 * w) // 10:] = True
                 mask[1::2, start:start + h * w] = mm.reshape(-1)
                 start += h * w
-        times = []
-        for it in range(iters + 3):
-            q, val, ref, go = sets[it % 3]
-            q.grad = None
-            m.zero_grad(set_to_none=True)
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
+
+        def step(q, val, ref, go):
             with torch.autocast("cuda", dtype=amp, enabled=amp is not None):
                 out = m(q, value=val, key_padding_mask=mask, reference_points=ref, spatial_shapes=shapes,
                         level_start_index=lsi)
             out.backward(go.to(out.dtype))
-            e1.record()
-            torch.cuda.synchronize()
-            if it >= 3:
-                times.append(e0.elapsed_time(e1))
+            # so that the next call assigns its gradients instead of adding to these; after the launches, so the host
+            # work overlaps the backward kernels
+            q.grad = None
+            m.zero_grad(set_to_none=True)
+
+        t = timed({mode: [(partial(step, *s),) for s in sets]}, iters, 3)[mode][0]
     finally:
         msda_module.MultiScaleDeformableAttnFunction = saved
     pts = batch * Q * 8 * 4 * 4
-    t = statistics.median(times)
     return {"kind": kind, "batch": batch, "mode": mode, "amp": str(amp), "key_padding_mask": masked, "ms": round(t, 3),
             "gpts_s": round(pts / t / 1e6, 3)}
 
@@ -141,7 +139,8 @@ def main():
     ap.add_argument("--out", default="")
     ap.add_argument("--mask-only", action="store_true", help="only the key_padding_mask comparison (fused vs unfused)")
     a = ap.parse_args()
-    rows = []
+    rows = [card()]
+    print(json.dumps(rows[0]), flush=True)
     for kind in ("encoder", "decoder"):
         for mode in ("fused", "unfused"):
             for amp in (None, torch.bfloat16):

@@ -16,9 +16,8 @@ import argparse
 import json
 import os
 import random
-import statistics
-import subprocess
 import sys
+from functools import partial
 
 import torch
 
@@ -26,6 +25,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ir_ads_b200.encoder import DeformableEncoder, get_reference_points  # noqa: E402
 from ir_ads_b200.functional import MSDeformAttnFusedFunction, MSDeformAttnPackedFunction  # noqa: E402
 from ir_ads_b200.packing import PackedLevels, packed_reference_points, valid_extents  # noqa: E402
+from timing import card, timed  # noqa: E402
 
 C, HEADS, L, P = 256, 8, 4, 4
 DEV = torch.device("cuda")
@@ -53,31 +53,6 @@ def make_packing(sizes):
     padded = (-(-max(h for h, _ in sizes) // 32) * 32, -(-max(w for _, w in sizes) // 32) * 32)
     shapes = levels_of(padded)
     return PackedLevels(valid_extents(sizes, padded, shapes), shapes, DEV)
-
-
-def timed(fn, iters, warmup, sets):
-    for i in range(warmup):
-        fn(sets[i % len(sets)])
-    times = []
-    for i in range(iters):
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        fn(sets[i % len(sets)])
-        b.record()
-        b.synchronize()
-        times.append(a.elapsed_time(b))
-    return times
-
-
-def alternate(fns, iters, warmup, sets):
-    """fns: {name: fn(set)}; runs them interleaved, `iters` passes each; returns {name: [ms]}"""
-    out = {k: [] for k in fns}
-    for k, f in fns.items():
-        timed(f, 0, warmup, sets[k])
-    for i in range(iters):
-        for k, f in fns.items():
-            out[k] += timed(f, 1, 0, sets[k][i % len(sets[k]):] + sets[k][:i % len(sets[k])])
-    return out
 
 
 def op_sets(pk, vdt, n, gen):
@@ -119,14 +94,6 @@ def main():
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
-    if not torch.cuda.is_available():
-        raise SystemExit("bench_packed.py needs a CUDA device")
-    card = torch.cuda.get_device_name(0)
-    try:
-        power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
-                               capture_output=True, text=True).stdout.strip()
-    except OSError:
-        power = "unknown"
     rng = random.Random(a.seed)
     mixes = [("model%d" % i, draw_mix(rng)) for i in range(a.mixes)] + [("equal", [(800, 1066), (800, 1066)])]
     gen = torch.Generator().manual_seed(a.seed)
@@ -135,10 +102,10 @@ def main():
     lines = []
 
     def emit(rec):
-        rec.update(card=card, power_limit=power)
         print(json.dumps(rec), flush=True)
         lines.append(json.dumps(rec))
 
+    emit(card())
     for name, sizes in mixes:
         pk = make_packing(sizes)
         base = dict(mix=name, sizes=sizes, level_shapes=pk.level_shapes, tokens_padded=pk.batch * pk.padded_len,
@@ -155,10 +122,11 @@ def main():
             def run_pk(s):
                 MSDeformAttnPackedFunction.apply(s[0], s[1], s[2], s[3], pk).backward(s[4])
 
-            t = alternate({"padded": run_pad, "packed": run_pk}, a.iters, a.warmup, {"padded": pad, "packed": packed})
-            mp, mk = statistics.median(t["padded"]), statistics.median(t["packed"])
-            emit(dict(base, workload="op_fwd_bwd", dtype=str(vdt).replace("torch.", ""), padded_ms=round(mp, 4),
-                      packed_ms=round(mk, 4), speedup=round(mp / mk, 3)))
+            t = timed({"padded": [(partial(run_pad, s),) for s in pad],
+                       "packed": [(partial(run_pk, s),) for s in packed]}, a.iters, a.warmup)
+            (mp,), (mk,) = t["padded"], t["packed"]
+            emit(dict(base, workload="op_fwd_bwd", dtype=str(vdt).replace("torch.", ""), padded_ms=mp, packed_ms=mk,
+                      speedup=round(mp / mk, 3)))
             del pad, packed
         # ---- the 6-layer encoder ----
         pad, packed = enc_sets(pk, 2, gen)
@@ -174,9 +142,9 @@ def main():
                     out = enc(s[0], **kw)
                 out.float().sum().backward()
 
-            t = alternate({"padded": lambda s: run_enc(s, False), "packed": lambda s: run_enc(s, True)}, a.iters,
-                          a.warmup, {"padded": pad, "packed": packed})
-            mp, mk = statistics.median(t["padded"]), statistics.median(t["packed"])
+            t = timed({"padded": [(partial(run_enc, s, False),) for s in pad],
+                       "packed": [(partial(run_enc, s, True),) for s in packed]}, a.iters, a.warmup)
+            (mp,), (mk,) = t["padded"], t["packed"]
             emit(dict(base, workload="encoder6_fwd_bwd", dtype="bf16_autocast" if amp else "float32",
                       padded_ms=round(mp, 3), packed_ms=round(mk, 3), speedup=round(mp / mk, 3)))
         del pad, packed

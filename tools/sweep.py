@@ -5,8 +5,8 @@ Usage: python tools/sweep.py [--workloads cfg2,cfg3] [--flags 0,4,65536] [--iter
 import argparse
 import json
 import os
-import statistics
 import sys
+from functools import partial
 
 import torch
 
@@ -15,6 +15,7 @@ sys.path.insert(0, ROOT)
 import ir_ads_b200  # noqa: E402
 from ir_ads_b200 import functional  # noqa: E402
 from ir_ads_b200.workloads import WORKLOADS, make_workload_inputs  # noqa: E402
+from timing import card, timed  # noqa: E402
 
 
 def hbm_peak_gbs():
@@ -34,26 +35,15 @@ def time_variant(wl, dist, flags, iters, sets=3, dev="cuda:0", deterministic=Fal
         go = torch.randn(wl.batch, wl.queries, wl.num_heads * wl.head_dim, device=dev).to(odt)
         data.append((value, shapes, lsi, loc, w, go))
     functional.set_deterministic(deterministic)
-    tf, tb = [], []
     with functional.kernel_flags(flags):
-        for it in range(iters + 3):
-            value, shapes, lsi, loc, w, go = data[it % sets]
-            e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-            e[0].record()
-            ir_ads_b200.ms_deform_attn_forward(value, shapes, lsi, loc, w, 64)
-            e[1].record()
-            ir_ads_b200.ms_deform_attn_backward(value, shapes, lsi, loc, w, go, 64)
-            e[2].record()
-            torch.cuda.synchronize()
-            if it >= 3:
-                tf.append(e[0].elapsed_time(e[1]))
-                tb.append(e[1].elapsed_time(e[2]))
+        f, b = timed({"op": [(partial(ir_ads_b200.ms_deform_attn_forward, value, shapes, lsi, loc, w, 64),
+                              partial(ir_ads_b200.ms_deform_attn_backward, value, shapes, lsi, loc, w, go, 64))
+                             for value, shapes, lsi, loc, w, go in data]}, iters, 3)["op"]
     functional.set_deterministic(False)
-    f, b = statistics.median(tf), statistics.median(tb)
     fb, bb = wl.algorithmic_bytes()
     peak = hbm_peak_gbs()
-    return {"workload": wl.name, "dist": dist, "flags": flags, "det": deterministic, "fwd_ms": round(f, 4),
-            "bwd_ms": round(b, 4), "gpts_s": round(wl.points / (f + b) / 1e6, 3),
+    return {"workload": wl.name, "dist": dist, "flags": flags, "det": deterministic, "fwd_ms": f, "bwd_ms": b,
+            "gpts_s": round(wl.points / (f + b) / 1e6, 3),
             "fwd_frac_hbm": round(fb / f / 1e6 / peak, 4), "bwd_frac_hbm": round(bb / b / 1e6 / peak, 4),
             "fb_frac_hbm": round((fb + bb) / (f + b) / 1e6 / peak, 4)}
 
@@ -67,7 +57,8 @@ def main():
     ap.add_argument("--det", action="store_true")
     ap.add_argument("--out", default="")
     a = ap.parse_args()
-    rows = []
+    rows = [card()]
+    print(json.dumps(rows[0]), flush=True)
     for name in a.workloads.split(","):
         for dist in a.dists.split(","):
             for fl in a.flags.split(","):
